@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...        # the reference's CPU path (torch CPU distance + Cython rank)
+    python bench.py ... --dump-outputs DIR      # also write the last timed step's results as DIR/<name>.npy
 
 One "step" = one pass of the hot path over one synthetic evaluation set: features + labels in,
 (cmc, mAP) on the host out.  Workload (BASELINE.json configs[1]): Market1501-multimodal-shaped,
@@ -442,6 +443,18 @@ def extra_c4_shard(peaks, check_q):
 # ------------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------------
+def dump_outputs(path, cmc, mAP, info):
+    """What the last timed step returned to its caller, one DIR/<name>.npy each (float32 CMC, the rest float64;
+    counts and first-hit positions are exact in float64).  The workload is seeded, so two builds run with the same
+    arguments can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {"cmc": np.asarray(cmc, dtype=np.float32), "mAP": np.float64(mAP), "mINP": np.float64(info["mINP"]),
+              "ap": info["ap"].cpu().numpy().astype(np.float64), "first": info["first"].cpu().numpy().astype(np.float64),
+              "num_valid": np.float64(info["num_valid"]), "num_ties": np.float64(info["num_ties"])}
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a))
+
+
 def run_ours(args):
     import torch.distributed as dist
     from ieee_b200 import _lib
@@ -538,6 +551,8 @@ def run_ours(args):
     lab_d = [t.to(dev) for t in lab_host]
     ms_dev, launches, clocks, out = timed(lambda: step_device(qf_d, gf_d, *lab_d), args.steps, args.warmup)
     cmc, mAP, info = out
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, cmc, mAP, info)
     value = Q * args.steps / (ms_dev / 1e3)
     count_path = ("fused into the contraction's epilogue (no distance block): %d of %d 128-output spans spilled for the exact recount"
                   % (last_ev[0].fused_stats["spilled_spans"], last_ev[0].fused_stats["spans"])) if info.get("fused") else (
@@ -679,7 +694,11 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--c4-check", type=int, default=2048, help="query subsample of the C4-shaped shard held against the CPU oracle (0: off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline step's results of the last timed step to DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

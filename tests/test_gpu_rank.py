@@ -200,14 +200,24 @@ def test_max_rank_clamp_and_errors(capsys):
         evaluate_rank(d, qp, gp, qc, gc, use_metric_cuhk03=True)
     # kept lists shorter than max_rank (rank.py:150,167).  All but 2 gallery items are junk for camera-0 queries:
     gc2 = np.zeros(12, int); gp2 = np.zeros(12, int); gc2[:2] = 1
-    # (a) EVERY valid query keeps the same 2 items: the reference stacks rows of length 2 and returns 2 ranks
+    # (a) EVERY valid query keeps the same 2 items: the reference stacks rows of length 2 and returns 2 ranks.  Both
+    # kept items are relevant, so its result is CMC [1, 1] and mAP 1 whatever the order (the compiled reference's
+    # answer, kept here so that the check runs without it; still compared live where oracle/_ref is built)
     cmc_u, map_u = evaluate_rank(d, np.zeros(6, int), gp2, np.zeros(6, int), gc2, max_rank=5)
-    cmc_r, map_r = ref.evaluate_rank(d, np.zeros(6, int), gp2, np.zeros(6, int), gc2, max_rank=5, use_cython=False)
-    assert cmc_u.shape == (2,) and np.array_equal(cmc_u, cmc_r) and abs(map_u - map_r) < 1e-9
-    # (b) lists of different length (camera-1 queries keep 10): the reference dies building a ragged array (ValueError)
+    ref_cmc, ref_map = np.ones(2, np.float32), 1.0
+    assert cmc_u.shape == (2,) and np.array_equal(cmc_u, ref_cmc) and abs(map_u - ref_map) < 1e-9
+    cmc_r, map_r = R.evaluate_rank(d, np.zeros(6, int), gp2, np.zeros(6, int), gc2, max_rank=5, stable=False)
+    assert np.array_equal(cmc_r, ref_cmc) and abs(map_r - ref_map) < 1e-9
+    # (b) lists of different length (camera-1 queries keep 10): the reference dies building a ragged array (ValueError,
+    # rank.py:167, which the restatement repeats line for line)
     qc2 = np.array([0, 1, 0, 1, 0, 1])
     with pytest.raises(ValueError):
-        ref.evaluate_rank(d, np.zeros(6, int), gp2, qc2, gc2, max_rank=5, use_cython=False)
+        R.evaluate_rank(d, np.zeros(6, int), gp2, qc2, gc2, max_rank=5, stable=False)
+    if ref.available():
+        cmc_r, map_r = ref.evaluate_rank(d, np.zeros(6, int), gp2, np.zeros(6, int), gc2, max_rank=5, use_cython=False)
+        assert np.array_equal(cmc_r, ref_cmc) and abs(map_r - ref_map) < 1e-9
+        with pytest.raises(ValueError):
+            ref.evaluate_rank(d, np.zeros(6, int), gp2, qc2, gc2, max_rank=5, use_cython=False)
     with pytest.raises(ValueError, match="fewer than max_rank"):
         evaluate_rank(d, np.zeros(6, int), gp2, qc2, gc2, max_rank=5)
 
