@@ -692,21 +692,33 @@ distmat_umma_chunked_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const _
 // below fix_tau of its scale; one warp per entry re-reads that span of the block and recomputes every output below the
 // bound as sum_k (q_k - g_k)^2 from the packed planes -- exact operands (hi + lo is the packed value), fp32 FMA chain,
 // relative error ~1e-7 of d itself.
+// The list holds `cap` entries.  A block with more flagged spans (duplicates scattered through the gallery, or centring
+// switched off on a large block) counts past it: then the warps walk every (row, span) of the block instead and apply
+// the same re-test, so the same outputs are recomputed, bit for bit, at the cost of one more read of the block.
 // =====================================================================================================
 __global__ void __launch_bounds__(256) distmat_fixup_kernel(const __half* __restrict__ q_hi, const __half* __restrict__ q_lo,
                                                              const __half* __restrict__ g_hi, const __half* __restrict__ g_lo,
                                                              const float* __restrict__ sq, const float* __restrict__ sg,
                                                              const float* __restrict__ rq, const float* __restrict__ rg, int Dp,
-                                                             int G, float tau, const unsigned long long* __restrict__ list,
+                                                             int Q, int G, float tau, const unsigned long long* __restrict__ list,
                                                              uint32_t cap, float* __restrict__ out, int64_t ldo) {
   const unsigned long long n64 = list[0];
-  const uint32_t n = n64 < cap ? (uint32_t)n64 : cap;
+  const bool overflow = n64 > cap;
+  const unsigned long long spans = (unsigned long long)((G + 127) / 128);
+  const unsigned long long n = overflow ? (unsigned long long)Q * spans : n64;
   const int lane = threadIdx.x & 31;
   const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
-  for (uint32_t e = warp; e < n; e += nwarps) {
+  for (unsigned long long e = warp; e < n; e += nwarps) {
     // entry = (row, first column of a 128-column span) in which the contraction saw an output below the bound
-    const unsigned long long rc = list[1 + e];
-    const uint32_t row = (uint32_t)(rc >> 32), col0 = (uint32_t)rc;
+    uint32_t row, col0;
+    if (overflow) {
+      row = (uint32_t)(e / spans);
+      col0 = (uint32_t)(e - row * spans) * 128u;
+    } else {
+      const unsigned long long rc = list[1 + e];
+      row = (uint32_t)(rc >> 32);
+      col0 = (uint32_t)rc;
+    }
     const float a_s = sq[row], a_n = rq[row];
     const uint4* ah = reinterpret_cast<const uint4*>(q_hi + (size_t)row * Dp);
     const uint4* al = reinterpret_cast<const uint4*>(q_lo + (size_t)row * Dp);
@@ -925,8 +937,8 @@ static int launch_umma_chunked(const void* q_packed, int64_t Q, const void* g_pa
         reinterpret_cast<const __half*>(qb + lq.hi_off), reinterpret_cast<const __half*>(qb + lq.lo_off),
         reinterpret_cast<const __half*>(gb + lg.hi_off), reinterpret_cast<const __half*>(gb + lg.lo_off),
         reinterpret_cast<const float*>(qb + lq.scale_off), reinterpret_cast<const float*>(gb + lg.scale_off),
-        reinterpret_cast<const float*>(qb + lq.norm_off), reinterpret_cast<const float*>(gb + lg.norm_off), (int)lq.Dp, (int)G,
-        kFixTau, L.p.fix_list, L.p.fix_cap, out, ldo);
+        reinterpret_cast<const float*>(qb + lq.norm_off), reinterpret_cast<const float*>(gb + lg.norm_off), (int)lq.Dp, (int)Q,
+        (int)G, kFixTau, L.p.fix_list, L.p.fix_cap, out, ldo);
     count_launch(1, "distmat_fixup_kernel");
     IEEE_CUDA_CHECK(cudaGetLastError());
   }

@@ -132,7 +132,8 @@ int ieee_feature_center(const void* x, int dtype, int64_t ld, int64_t rows, int6
  * output below 2^-6 of its scale |q|^2 + |g|^2 -- near-duplicate pairs, where the expansion |q|^2 + |g|^2 - 2 q.g only
  * keeps the ABSOLUTE accuracy of its terms -- is listed by the contraction and recomputed as sum_k (q_k - g_k)^2 by
  * a second small kernel: all distances then sit within 1e-4 relative of the exact value.  Word 0 of the workspace
- * holds the number of pairs found (up to 2 Q + 4096 are recomputed). */
+ * holds the number of 128-output spans flagged; the list keeps 2 Q + 4096 of them, and when there are more the second
+ * kernel re-tests every span of the block instead, so none is missed. */
 size_t ieee_distmat_fixup_bytes(int64_t Q);
 int ieee_distmat_packed(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
                         int precision, float* out, int64_t ldo, void* fixup_workspace, ieee_stream_t stream);

@@ -25,13 +25,9 @@ TC_ACCUM_FLOOR_UNCHUNKED = 2e-5  # whole-K accumulation in TMEM (BF16 1-pass mod
 SPLIT_EPS = 2.0 ** -21   # fp16 hi+lo keeps 22 mantissa bits per operand: each product is off by <= ~2^-21 relative
 
 
-def assert_distance_parity(got, a, b, metric, rtol=RTOL, split=True, floor=None):
-    """|got - fp64 truth| <= rtol*|truth| + floor.
-
-    floor = the cancellation floor the reference's own fp32 GEMM sits on (a few ulps of |q|^2+|g|^2) plus, for
-    the f16x3 split, 4 sigma of its rounding model: independent per-product errors of 2^-21 relative, i.e.
-    2 * 4 * 2^-21 * sqrt(sum_k (a_k b_k)^2)  (~ 1e-8 relative at D=2304: below the fp32 floor).
-    """
+def parity_terms(a, b, metric):
+    """What assert_distance_parity measures against: (fp64 truth, the reference's fp32 result, |q|^2+|g|^2,
+    sqrt(sum_k (a_k b_k)^2)).  Worth computing once when several results of the same inputs are checked."""
     truth = R.distance_fp64(a, b, metric).numpy()
     ref = R.compute_distance_matrix(a, b, metric).numpy()
     a64, b64 = a.double(), b.double()
@@ -40,6 +36,18 @@ def assert_distance_parity(got, a, b, metric, rtol=RTOL, split=True, floor=None)
         b64 = b64 / b64.norm(dim=1, keepdim=True).clamp_min(1e-12)
     scale = ((a64 ** 2).sum(1, keepdim=True) + (b64 ** 2).sum(1, keepdim=True).t()).numpy()
     prod_rms = torch.sqrt((a64 ** 2) @ (b64 ** 2).t()).numpy()
+    return truth, ref, scale, prod_rms
+
+
+def assert_distance_parity(got, a, b, metric, rtol=RTOL, split=True, floor=None, terms=None):
+    """|got - fp64 truth| <= rtol*|truth| + floor.
+
+    floor = the cancellation floor the reference's own fp32 GEMM sits on (a few ulps of |q|^2+|g|^2) plus, for
+    the f16x3 split, 4 sigma of its rounding model: independent per-product errors of 2^-21 relative, i.e.
+    2 * 4 * 2^-21 * sqrt(sum_k (a_k b_k)^2)  (~ 1e-8 relative at D=2304: below the fp32 floor).
+    `terms`: parity_terms(a, b, metric), when the caller already has them.
+    """
+    truth, ref, scale, prod_rms = terms if terms is not None else parity_terms(a, b, metric)
     alpha = 2.0 if metric == "euclidean" else 1.0
     tol = rtol * np.abs(truth) + CANCEL_ULPS * scale
     if split:   # tensor-core path
