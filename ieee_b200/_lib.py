@@ -72,11 +72,6 @@ SIGNATURES = {
     "ieee_retrieve_prepared_workspace_bytes": (sz, [i64, i64, C.c_int, i32]),
     "ieee_retrieve_eval_prepared": (C.c_int, [vp, i64, C.c_int, i64, i64, C.c_int, C.c_int, C.c_int, vp, vp, vp, i64, vp, vp, vp, i32, i32,
                                               C.POINTER(i32), vp, i64, vp, vp, vp, vp, vp, vp, sz, vp]),
-    "ieee_retrieve_fused_workspace_bytes": (sz, [i64, i64, i64]),
-    "ieee_retrieve_fused_spill_capacity": (C.c_uint32, [i64, i64]),
-    "ieee_retrieve_eval_fused_prepared": (C.c_int, [vp, i64, C.c_int, i64, i64, C.c_int, C.c_int, vp, vp, vp, i64, vp, vp, vp, i32,
-                                                    vp, vp, vp, vp, vp, vp, sz, vp]),
-    "ieee_set_fused_chunk": (C.c_int, [C.c_int]),
     "ieee_topk": (C.c_int, [vp, i64, i64, i64, i64, vp, vp, vp, vp, i32, vp, vp, vp]),
     "ieee_topk_merge": (C.c_int, [vp, vp, i32, i64, i32, vp, vp, vp]),
     "ieee_gnn_rerank_workspace_bytes": (sz, [i64, i32]),

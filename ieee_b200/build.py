@@ -15,7 +15,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libieee_b200.so")
-SOURCES = ["capi.cu", "pack.cu", "distmat_sm100.cu", "distmat_simt.cu", "rank.cu", "rerank.cu", "fused.cu"]
+SOURCES = ["capi.cu", "pack.cu", "distmat_sm100.cu", "distmat_simt.cu", "rank.cu", "rerank.cu"]
 HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(os.path.dirname(HERE), "include", "ieee_b200.h")]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 

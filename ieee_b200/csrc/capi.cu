@@ -20,7 +20,6 @@ static std::atomic<long long> g_launches{0};
 int g_debug_flags = 0;
 int g_accum_chunk_kb = 6;
 int g_raster_panel = 0;
-int g_fused_chunk_kb = 0;
 static int g_centering = 1;
 
 // Step timeline (debug flag 128): every named launch on the traced stream is followed by an event record, so the gaps
@@ -110,13 +109,6 @@ size_t rerank_workspace_bytes(int64_t Q, int64_t G, int32_t k1, int32_t k2);
 int rerank(const float* q_g, int64_t ld_qg, const float* q_q, int64_t ld_qq, const float* g_g, int64_t ld_gg, int64_t Q,
            int64_t G, int32_t k1, int32_t k2, double lambda_value, float* out, int64_t ldo, void* workspace,
            size_t workspace_bytes, cudaStream_t stream);
-
-size_t fused_workspace_bytes(int64_t Q, int64_t G);
-uint32_t fused_spill_capacity(int64_t Q, int64_t G);
-int fused_eval(const void* q_packed, int64_t Q, const void* g_packed, const void* group, int64_t G, int64_t D, int metric,
-               const int64_t* q_pids, const int64_t* q_camids, const int64_t* g_camids, int32_t max_rank, float* cmc,
-               ieee_eval_summary* summary, double* per_query_ap, int32_t* per_query_first, unsigned long long* stats_out,
-               void* workspace, size_t workspace_bytes, cudaStream_t stream, int cta_group);
 
 size_t gnn_rerank_workspace_bytes(int64_t N, int32_t k1);
 int gnn_rerank(const float* neg_score, int64_t lds, int64_t N, int32_t k1, int32_t k2, float* A, int64_t ldA, void* workspace,
@@ -715,47 +707,6 @@ int ieee_gnn_rerank(const float* neg_score, int64_t lds, int64_t N, int32_t k1, 
   if (rc) return rc;
   return gnn_rerank(neg_score, lds, N, k1, k2, A, ldA, workspace, workspace_bytes, (cudaStream_t)stream);
 }
-
-// ---- retrieval + evaluation with the count fused into the contraction ----------------------------------------------
-size_t ieee_retrieve_fused_workspace_bytes(int64_t Q, int64_t G, int64_t D) {
-  if (Q <= 0 || G <= 0 || D <= 0) return 0;
-  return align256(ieee_packed_bytes(Q, D, IEEE_PREC_F16X3)) + fused_workspace_bytes(Q, G) + 256;
-}
-
-int ieee_set_fused_chunk(int k_slices) {
-  const int prev = g_fused_chunk_kb;
-  if (k_slices >= 0) g_fused_chunk_kb = k_slices;
-  return prev;
-}
-
-int ieee_retrieve_eval_fused_prepared(const void* qf, int64_t ldq, int dtype, int64_t Q, int64_t D, int metric, int normalize,
-                                      const void* g_packed, const void* group, const float* center, int64_t G,
-                                      const int64_t* q_pids, const int64_t* q_camids, const int64_t* g_camids,
-                                      int32_t max_rank, float* cmc, ieee_eval_summary* summary, double* per_query_ap,
-                                      int32_t* per_query_first, uint64_t* stats_out, void* workspace, size_t workspace_bytes,
-                                      ieee_stream_t stream_) {
-  int rc = check_device();
-  if (rc) return rc;
-  cudaStream_t stream = (cudaStream_t)stream_;
-  IEEE_REQUIRE(qf && g_packed && group && q_pids && q_camids && g_camids && cmc && summary && stats_out && workspace,
-               "retrieve (fused): null pointer");
-  IEEE_REQUIRE(Q > 0 && G > 0 && D > 0 && max_rank >= 1 && Q < (int64_t(1) << 31) && G < (int64_t(1) << 31),
-               "retrieve (fused): bad shape Q=%lld G=%lld D=%lld max_rank=%d", (long long)Q, (long long)G, (long long)D, max_rank);
-  IEEE_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "retrieve (fused): workspace must be 256-byte aligned");
-  if (workspace_bytes < ieee_retrieve_fused_workspace_bytes(Q, G, D)) {
-    set_error("retrieve (fused): workspace too small (%zu < %zu)", workspace_bytes, ieee_retrieve_fused_workspace_bytes(Q, G, D));
-    return IEEE_ERR_WORKSPACE;
-  }
-  uint8_t* w = static_cast<uint8_t*>(workspace);
-  void* q_packed = w;
-  const size_t qbytes = align256(ieee_packed_bytes(Q, D, IEEE_PREC_F16X3));
-  if ((rc = pack_features(qf, dtype, ldq, Q, D, metric, normalize, IEEE_PREC_F16X3, center, q_packed, stream))) return rc;
-  return fused_eval(q_packed, Q, g_packed, group, G, D, metric, q_pids, q_camids, g_camids, max_rank, cmc, summary, per_query_ap,
-                    per_query_first, reinterpret_cast<unsigned long long*>(stats_out), w + qbytes, workspace_bytes - qbytes, stream,
-                    cta_group_default());
-}
-
-uint32_t ieee_retrieve_fused_spill_capacity(int64_t Q, int64_t G) { return (Q > 0 && G > 0) ? fused_spill_capacity(Q, G) : 0; }
 
 // ---- peer exchange (gallery sharded over the GPUs of one box) ---------------------------------------------------
 // regions are sized for the largest query block (Qb_max); a block of Qb <= Qb_max rows uses a dense prefix of each

@@ -67,7 +67,6 @@ struct ZeroJob {
 
 void count_launch(int n = 1, const char* name = nullptr);   // a name puts the launch on the step timeline (debug flag 128)
 extern int g_debug_flags;       // ieee_set_debug_flags()
-extern int g_fused_chunk_kb;    // accumulation chunk of the fused-count contraction (0 = as the store kernel)
 extern int g_raster_panel;      // ieee_set_raster_panel(): m tiles per raster panel of the contraction (0 = sized for L2)
 extern int g_accum_chunk_kb;    // ieee_set_accum_chunk(): K-slices per tensor-core accumulation chunk (0 = whole K)   // bookkeeping behind ieee_launch_count()
 
@@ -124,22 +123,6 @@ inline PackedLayout packed_layout(int64_t rows, int64_t D, int precision) {
 
 // ---- gallery grouping (rank.cu): open-addressing hash pid -> slot; members of a slot = the gallery items of that identity
 static constexpr long long kEmptyPid = (long long)0x8080808080808080ull;   // memset(0x80) pattern; not a usable pid
-struct GroupTables { const long long* keys; const int32_t* cnt; const int32_t* off; const int32_t* members; int64_t T; };
-GroupTables group_tables(const void* blob, int64_t G);
-
-// ---- counting fused into the contraction's epilogue (fused.cu, distmat_sm100.cu) ------------------------------------
-constexpr int kFusedLC = 32;             // thresholds (same-identity gallery items) per query the epilogue tables hold
-struct FusedCount {
-  const float* thr;                      // [Q][LC] approximate distance of the query to its i-th same-identity item; pad -inf
-  const int32_t* tn;                     // [Q]     number of such items
-  const float* eps;                      // [Q]     half-width of the band in which an output is NOT decided by `thr`
-  int32_t* cnt;                          // [Q][LC] outputs definitely below thr[q][i] (atomicAdd)
-  unsigned int* spill_n;                 // [1]     spans handed to the resolve kernels
-  unsigned long long* spill_meta;        // [cap]   row << 32 | first column
-  float* spill_val;                      // [cap][128]
-  uint32_t spill_cap;
-  int LC;
-};
 
 // ---- exchange between the ranks of a sharded gallery over NVLink peer memory ----------------------------------
 // Every rank owns one exchange buffer (ieee_peer_alloc) that all ranks of the gallery group map (cudaIpc): the rank

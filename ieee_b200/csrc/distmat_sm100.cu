@@ -72,9 +72,6 @@ struct GemmParams {
   unsigned long long* fix_list;
   uint32_t fix_cap;
   float fix_tau;
-  // fused counting (distmat_umma_chunked_kernel<CG, true>): the epilogue bins its outputs against every row's
-  // approximate thresholds instead of writing them (see fused.cu)
-  FusedCount fc;
 };
 
 // Tile order.  Inside a panel of `panel_m` m tiles, m runs fastest (the CTAs of one wave share B tiles in L2);
@@ -320,19 +317,17 @@ constexpr int kEpiWarpsC = 8;
 constexpr int kThreadsC = 128 + 32 * kEpiWarpsC;
 constexpr int kPitchC = 17;                      // floats; padded 32 x 16 transpose tile (fallback store path)
 
-template <int CG, bool FUSED = false>
+template <int CG>
 struct GemmCfgC {
-  // fused counting trades one pipeline stage for the per-warp threshold tables
-  static constexpr int kStages = FUSED ? ((CG == 1) ? 3 : 5) : ((CG == 1) ? 4 : 6);
+  static constexpr int kStages = (CG == 1) ? 4 : 6;
   static constexpr int kBRows = BLOCK_N / CG;
   static constexpr uint32_t kABytes = BLOCK_M * BLOCK_K * 2;
   static constexpr uint32_t kBBytes = kBRows * BLOCK_K * 2;
   static constexpr uint32_t kStageBytes = kABytes + kBBytes;
-  // store epilogue: 32 x 16 fp32 (2 KB, SWIZZLE_64B) / 32 x 17 padded (2176 B); fused: kFusedLC x 33 thresholds
-  // (fused: (kFusedLC + 2) x 33 guarded thresholds + (kFusedLC + 2) x 32 byte counters)
-  static constexpr uint32_t kEpiTileBytes = FUSED ? ((kFusedLC + 2) * 33 * 4 + (kFusedLC + 2) / 2 * 32 * 4 + 127) / 128 * 128 : 2560;
+  // store epilogue: 32 x 16 fp32 (2 KB, SWIZZLE_64B) / 32 x 17 padded (2176 B)
+  static constexpr uint32_t kEpiTileBytes = 2560;
   static constexpr uint32_t kEpiColBytes = 2 * 128 * 4;
-  static constexpr uint32_t kEpiWarpBytes = FUSED ? 8192 : 4096;   // keeps every warp's tile 1024-byte aligned
+  static constexpr uint32_t kEpiWarpBytes = 4096;   // keeps every warp's tile 1024-byte aligned
   static constexpr uint32_t kEpiBytes = kEpiWarpsC * kEpiWarpBytes;
   static constexpr uint32_t kBarBytes = 256;
   static constexpr uint32_t kSmemBytes = kStages * kStageBytes + kEpiBytes + kBarBytes + 1024;
@@ -340,12 +335,15 @@ struct GemmCfgC {
   static_assert(kSmemBytes <= 232448, "shared memory budget");
 };
 
-template <int CG, bool FUSED>
+// p is __grid_constant__ so that every use reads its field from the parameter bank: taken by value, the compiler
+// hoists the fields into registers at kernel entry, and in this kernel, whose 168 registers are full, that adds spills.
+template <int CG>
 __global__ void __launch_bounds__(kThreadsC, 1)
 distmat_umma_chunked_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
                             const __grid_constant__ CUtensorMap tm_b_hi, const __grid_constant__ CUtensorMap tm_b_lo,
-                            const __grid_constant__ CUtensorMap tm_out, const GemmParams p, const int chunk_kb) {
-  using Cfg = GemmCfgC<CG, FUSED>;
+                            const __grid_constant__ CUtensorMap tm_out, const __grid_constant__ GemmParams p,
+                            const int chunk_kb) {
+  using Cfg = GemmCfgC<CG>;
   constexpr int kStages = Cfg::kStages;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -494,24 +492,6 @@ distmat_umma_chunked_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const _
         col_sg[j * 32 + lane] = (p.sg != nullptr && col < p.G) ? p.sg[col] : 1.0f;
       }
       __syncwarp();
-      // fused counting: this warp's 32 rows x their (approximate) thresholds, transposed into shared memory so that
-      // lane = row reads them conflict-free; loaded here, while the tensor cores are still busy with the tile
-      float eps_row = 0.f;
-      int n_row = 0;
-      if constexpr (FUSED) {
-        // Tg[1 + k][row] = k-th smallest threshold of the row (+inf beyond its list), Tg[0] = -inf, Tg[LC + 1] = +inf:
-        // pitch 33 keeps both the transposing writes and the lane = row reads free of bank conflicts
-        float* Tg = tile;
-        const int LC = p.fc.LC;
-        for (int j = lane; j < 32 * LC; j += 32) {
-          const int rr = j / LC, k = j - rr * LC;
-          Tg[(1 + k) * 33 + rr] = (row0 + rr < p.Q) ? p.fc.thr[(int64_t)(row0 + rr) * LC + k] : INFINITY;
-        }
-        Tg[lane] = -INFINITY;
-        Tg[(LC + 1) * 33 + lane] = INFINITY;
-        if (my_row < p.Q) { n_row = p.fc.tn[my_row]; eps_row = p.fc.eps[my_row]; }
-        __syncwarp();
-      }
       float r[128];
       for (int c = 0; c < num_chunks; ++c, ++ci) {
         const int acc = ci & 1;
@@ -538,86 +518,6 @@ distmat_umma_chunked_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const _
         }
       }
       if (row0 >= p.Q || (p.debug & 1)) continue;
-      if constexpr (FUSED) {
-        // ---- count instead of store ----------------------------------------------------------------------------
-        // d = fma(coef * sg, sum, rq + rg) in place; `viol` as in the store epilogue (near-duplicate pairs)
-        float viol = 0.f;
-#pragma unroll
-        for (int i = 0; i < 128; ++i) {
-          const float base = __fadd_rn(rq_row, col_rg[i]);
-          r[i] = __fmaf_rn(coef_row * col_sg[i], r[i], base);
-          viol = fminf(viol, __fmaf_rn(-p.fix_tau, base, r[i]));
-        }
-        if (col0 + 128 > p.G) {                  // ragged last tile: columns beyond G never count (warp-uniform)
-#pragma unroll
-          for (int i = 0; i < 128; ++i)
-            if (col0 + i >= p.G) r[i] = INFINITY;
-        }
-        // Every output is placed among the row's sorted thresholds with a branch-free binary search (6 conflict-free
-        // shared loads): pos = #{k : T_k <= d}.  It is within eps of a threshold iff it is within eps of one of its two
-        // neighbours there; if none of the 128 outputs is, the comparisons against the approximate thresholds are the
-        // comparisons against the exact ones, and the per-position byte counters give the counts.
-        const float* Tg = tile;
-        uint32_t* bins = reinterpret_cast<uint32_t*>(tile + (kFusedLC + 2) * 33);    // [(kFusedLC + 2) / 2][32]: two 16-bit counters per word
-#pragma unroll
-        for (int b = 0; b < (kFusedLC + 2) / 2; ++b) bins[b * 32 + lane] = 0;
-        // the first two levels of the search compare against registers
-        const float p15 = Tg[16 * 33 + lane], p7 = Tg[8 * 33 + lane], p23 = Tg[24 * 33 + lane];
-        bool band = false;
-        // eight outputs at a time: first their searches (loads only, so the eight dependent chains overlap), then eight
-        // fire-and-forget shared atomics on this lane's private counter column (the compiler may not move a shared
-        // load above a shared atomic it cannot prove disjoint, so the two are kept in separate phases)
-#pragma unroll
-        for (int i0 = 0; i0 < 128; i0 += 8) {
-          int pos8[8];
-#pragma unroll
-          for (int e = 0; e < 8; ++e) {
-            const float d = fminf(r[i0 + e], INFINITY);     // NaN -> +inf: ranks after everything (NumPy's order)
-            float below = -INFINITY, above = INFINITY;       // nearest thresholds probed on either side
-            bool le = p15 <= d;
-            int pos = le ? 16 : 0;
-            below = le ? p15 : below; above = le ? above : p15;
-            const float p2 = le ? p23 : p7;
-            le = p2 <= d;
-            pos += le ? 8 : 0; below = le ? p2 : below; above = le ? above : p2;
-#pragma unroll
-            for (int step = 4; step >= 1; step >>= 1) {
-              const float t = Tg[(pos + step) * 33 + lane];
-              le = t <= d;
-              pos += le ? step : 0; below = le ? t : below; above = le ? above : t;
-            }
-            const float t = Tg[(pos + 1) * 33 + lane];       // (the five levels cover T_0 .. T_30)
-            le = t <= d;
-            pos += le ? 1 : 0; below = le ? t : below; above = le ? above : t;
-            band |= (d - below < eps_row) | (above - d < eps_row);
-            pos8[e] = pos;
-          }
-#pragma unroll
-          for (int e = 0; e < 8; ++e) atomicAdd(bins + (pos8[e] >> 1) * 32 + lane, (pos8[e] & 1) ? 65536u : 1u);
-        }
-        __syncwarp();
-        const bool live = my_row < p.Q;
-        const bool spill = live && (band || (p.rq != nullptr && viol < 0.f));
-        if (spill) {
-          // hand the whole 128-output span to the resolve kernels: they compare it against the exact thresholds
-          const unsigned int slot = atomicAdd(p.fc.spill_n, 1u);
-          if (slot < p.fc.spill_cap) {
-            p.fc.spill_meta[slot] = ((unsigned long long)(uint32_t)my_row << 32) | (uint32_t)col0;
-            float4* dst = reinterpret_cast<float4*>(p.fc.spill_val + (size_t)slot * 128);
-#pragma unroll
-            for (int j = 0; j < 32; ++j) dst[j] = make_float4(r[4 * j], r[4 * j + 1], r[4 * j + 2], r[4 * j + 3]);
-          }
-        } else if (live) {
-          // outputs definitely below the k-th smallest threshold: those placed at positions 0 .. k
-          int run = 0;
-          for (int k = 0; k < n_row; ++k) {
-            const uint32_t w2 = bins[(k >> 1) * 32 + lane];
-            run += (k & 1) ? (w2 >> 16) : (w2 & 0xFFFFu);
-            if (run != 0) atomicAdd(p.fc.cnt + (int64_t)my_row * p.fc.LC + k, run);
-          }
-        }
-        continue;
-      }
       const bool fix_on = p.fix_list != nullptr && p.rq != nullptr;
       float viol = 0.f;                          // min over this thread's 128 outputs of d - fix_tau * (|q|^2 + |g|^2)
       // d = fma(coef * sg, sum, rq + rg), 16 columns at a time
@@ -899,19 +799,15 @@ constexpr float kFixTau = 0.015625f;
 
 size_t distmat_fixup_bytes(int64_t Q) { return align256((size_t(2 * Q + 4096) + 2) * 8); }
 
-template <int CG, bool FUSED>
+template <int CG>
 static int launch_umma_chunked(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
                                int precision, float* out, int64_t ldo, cudaStream_t stream, int chunk_kb, void* fix_ws,
-                               const FusedCount* fc = nullptr, bool fix_zeroed = false) {
-  using Cfg = GemmCfgC<CG, FUSED>;
+                               bool fix_zeroed) {
+  using Cfg = GemmCfgC<CG>;
   GemmLaunch L;
   int rc = gemm_setup<CG>(L, q_packed, Q, g_packed, G, D, metric, precision, out, ldo, 16, CU_TENSOR_MAP_SWIZZLE_64B);
   if (rc) return rc;
-  if constexpr (FUSED) {
-    L.p.fc = *fc;
-    L.p.fix_tau = (metric == IEEE_METRIC_EUCLIDEAN && !(g_debug_flags & 32)) ? kFixTau : 0.f;
-  }
-  const bool fix = !FUSED && fix_ws != nullptr && metric == IEEE_METRIC_EUCLIDEAN && precision == IEEE_PREC_F16X3 &&
+  const bool fix = fix_ws != nullptr && metric == IEEE_METRIC_EUCLIDEAN && precision == IEEE_PREC_F16X3 &&
                    !(g_debug_flags & 32);
   if (fix) {
     L.p.fix_list = static_cast<unsigned long long*>(fix_ws);
@@ -922,13 +818,13 @@ static int launch_umma_chunked(const void* q_packed, int64_t Q, const void* g_pa
       count_launch(0, "memset fix list");
     }
   }
-  IEEE_ENSURE_DYN_SMEM((distmat_umma_chunked_kernel<CG, FUSED>), Cfg::kSmemBytes);
+  IEEE_ENSURE_DYN_SMEM(distmat_umma_chunked_kernel<CG>, Cfg::kSmemBytes);
   cudaLaunchConfig_t cfg;
   cudaLaunchAttribute attr[1];
   cluster_launch_config(cfg, attr, L.groups * CG, kThreadsC, Cfg::kSmemBytes, CG, stream);
-  IEEE_CUDA_CHECK(cudaLaunchKernelEx(&cfg, distmat_umma_chunked_kernel<CG, FUSED>, L.ta_hi, L.ta_lo, L.tb_hi, L.tb_lo, L.t_out, L.p,
+  IEEE_CUDA_CHECK(cudaLaunchKernelEx(&cfg, distmat_umma_chunked_kernel<CG>, L.ta_hi, L.ta_lo, L.tb_hi, L.tb_lo, L.t_out, L.p,
                                      chunk_kb));
-  count_launch(1, FUSED ? "distmat_umma_chunked_kernel (counting epilogue)" : "distmat_umma_chunked_kernel");
+  count_launch(1, "distmat_umma_chunked_kernel");
   if (fix) {
     PackedLayout lq = packed_layout(Q, D, precision), lg = packed_layout(G, D, precision);
     const uint8_t* qb = static_cast<const uint8_t*>(q_packed);
@@ -950,27 +846,14 @@ int distmat_umma(const void* q_packed, int64_t Q, const void* g_packed, int64_t 
   // chunked accumulation serves the fp32-grade mode; the 1-pass BF16 mode keeps the whole K in TMEM (throughput mode)
   if (g_accum_chunk_kb > 0 && (precision == IEEE_PREC_F16X3 || (g_debug_flags & 8))) {
     if (cta_group == 2)
-      return launch_umma_chunked<2, false>(q_packed, Q, g_packed, G, D, metric, precision, out, ldo, stream, g_accum_chunk_kb, fix_ws,
-                                           nullptr, fix_zeroed);
-    return launch_umma_chunked<1, false>(q_packed, Q, g_packed, G, D, metric, precision, out, ldo, stream, g_accum_chunk_kb, fix_ws,
-                                         nullptr, fix_zeroed);
+      return launch_umma_chunked<2>(q_packed, Q, g_packed, G, D, metric, precision, out, ldo, stream, g_accum_chunk_kb, fix_ws,
+                                    fix_zeroed);
+    return launch_umma_chunked<1>(q_packed, Q, g_packed, G, D, metric, precision, out, ldo, stream, g_accum_chunk_kb, fix_ws,
+                                  fix_zeroed);
   }
   if (cta_group == 2)
     return launch_umma<2>(q_packed, Q, g_packed, G, D, metric, precision, out, ldo, stream);
   return launch_umma<1>(q_packed, Q, g_packed, G, D, metric, precision, out, ldo, stream);
-}
-
-// Contraction with the count fused into its epilogue (F16X3 only): nothing is written but counts and spilled spans.
-int distmat_umma_fused(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
-                       const FusedCount& fc, cudaStream_t stream, int cta_group) {
-  // same chunking as the store kernel by default: the two paths then produce bit-identical distances
-  const int chunk = g_fused_chunk_kb > 0 ? g_fused_chunk_kb : (g_accum_chunk_kb > 0 ? g_accum_chunk_kb : 1 << 20);
-  // the output pointer only decides the (unused) store path: any 16-byte aligned address with a padded pitch will do
-  float* dummy = reinterpret_cast<float*>(const_cast<float*>(fc.thr));
-  const int64_t ldo = round_up(G, 4);
-  if (cta_group == 2)
-    return launch_umma_chunked<2, true>(q_packed, Q, g_packed, G, D, metric, IEEE_PREC_F16X3, dummy, ldo, stream, chunk, nullptr, &fc);
-  return launch_umma_chunked<1, true>(q_packed, Q, g_packed, G, D, metric, IEEE_PREC_F16X3, dummy, ldo, stream, chunk, nullptr, &fc);
 }
 
 }  // namespace ieee

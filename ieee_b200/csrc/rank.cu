@@ -76,10 +76,6 @@ static inline GroupView group_view(const void* blob, int64_t G) {
   return v;
 }
 size_t gallery_group_bytes(int64_t G) { return group_view(nullptr, G).total; }
-GroupTables group_tables(const void* blob, int64_t G) {
-  const GroupView v = group_view(blob, G);
-  return GroupTables{v.keys, v.cnt, v.off, v.members, v.T};
-}
 
 __global__ void group_insert_kernel(const int64_t* __restrict__ g_pids, int64_t G, long long* keys, int32_t* cnt,
                                     int32_t* slot_of, int64_t T) {

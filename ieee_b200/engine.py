@@ -94,8 +94,7 @@ def _stages_for(Qb, cap, world, device, width=0):
     return st
 
 
-_FUSED_POOL = {}
-_FUSED_SKIP = {}          # label identities for which the fused path could not certify its result (values: references)
+_ONE_CALL_POOL = {}
 _RESULT_HOST = {}
 
 
@@ -108,19 +107,16 @@ def _result_buffer(device, nbytes):
     return buf
 
 
-def _fused_buffers(Q, D, precision, cap, k_eff, device):
-    """Workspace + result block of the one-call path, reused per shape (stream-ordered like the stage pool)."""
-    key = (Q, D, precision, cap, k_eff, str(device))
-    buf = _FUSED_POOL.get(key)
+def _one_call_buffers(key, ws_bytes, res_bytes, device):
+    """Workspace, result block and its pinned host copy of a one-call evaluation, reused per key (stream-ordered like
+    the stage pool)."""
+    buf = _ONE_CALL_POOL.get(key)
     if buf is None:
-        if len(_FUSED_POOL) > 8:
-            _FUSED_POOL.clear()
-        lib = _lib.load()
-        ws = torch.empty(lib.ieee_retrieve_prepared_workspace_bytes(Q, D, precision, cap), dtype=torch.uint8, device=device)
-        res_off = (4 * k_eff + 7) // 8 * 8                      # [cmc float32[k_eff] | pad | ieee_eval_summary]
-        res = torch.empty(res_off + C.sizeof(_lib.EvalSummary), dtype=torch.uint8, device=device)
-        res_host = torch.empty(res.shape, dtype=torch.uint8, pin_memory=True)
-        buf = _FUSED_POOL[key] = (ws, res, res_off, res_host)
+        if len(_ONE_CALL_POOL) > 8:
+            _ONE_CALL_POOL.clear()
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=device)
+        res = torch.empty(res_bytes, dtype=torch.uint8, device=device)
+        buf = _ONE_CALL_POOL[key] = (ws, res, torch.empty(res_bytes, dtype=torch.uint8, pin_memory=True))
     return buf
 
 
@@ -269,8 +265,6 @@ class RetrievalEvaluator:
         self._host_gallery = None
         self._label_keys = (_tensor_key(g_pids), _tensor_key(g_camids))
         self._label_refs = (g_pids, g_camids)
-        self._fused_failed = False
-        self.fused_stats = None
 
     def _prepare_gallery(self, qf_dev):
         """ieee_gallery_prepare: grouping + [centre from the query rows] + packing of a device-resident gallery -- and
@@ -476,55 +470,6 @@ class RetrievalEvaluator:
             self.chunks.append((c0, (ev, staged)))
         self._host_gallery = None
 
-    def _evaluate_fused(self, qf, q_pids, q_camids):
-        """The count fused into the contraction's epilogue (ieee_retrieve_eval_fused_prepared): no distance block, no
-        capacity query.  Returns None when the result was not certified (the caller then takes the staged path, and
-        this evaluator's labels are remembered as not eligible)."""
-        with torch.cuda.device(self.device):
-            lib = _lib.load()
-            Q, D = qf.shape
-            if qf.stride(1) != 1:
-                qf = qf.contiguous()
-            qp = _as_device(q_pids, torch.int64, self.device)
-            qc = _as_device(q_camids, torch.int64, self.device)
-            k_eff = min(self.max_rank, self.g_total)
-            key = ("fused", Q, self.G, D, k_eff, str(self.device))
-            buf = _FUSED_POOL.get(key)
-            if buf is None:
-                if len(_FUSED_POOL) > 8:
-                    _FUSED_POOL.clear()
-                ws = torch.empty(lib.ieee_retrieve_fused_workspace_bytes(Q, self.G, D), dtype=torch.uint8, device=self.device)
-                res_off = (32 + 4 * k_eff + 7) // 8 * 8                 # [stats uint64[3] + pad | cmc | summary]
-                res = torch.empty(res_off + C.sizeof(_lib.EvalSummary), dtype=torch.uint8, device=self.device)
-                buf = _FUSED_POOL[key] = (ws, res, res_off, torch.empty(res.shape, dtype=torch.uint8, pin_memory=True),
-                                          lib.ieee_retrieve_fused_spill_capacity(Q, self.G))
-            ws, res, res_off, res_host, spill_cap = buf
-            ap = torch.empty(Q, dtype=torch.float64, device=self.device)
-            first = torch.empty(Q, dtype=torch.int32, device=self.device)
-            cur = torch.cuda.current_stream()
-            self.labels.wait(cur)
-            gpk = self.chunks[0][1]
-            _lib.call("ieee_retrieve_eval_fused_prepared", qf.data_ptr(), qf.stride(0), _lib.DTYPES[qf.dtype], Q, D,
-                      _lib.METRICS[self.metric], int(self.normalize), gpk.buf.data_ptr(), self.labels.group.data_ptr(),
-                      _lib.ptr(self.center), self.G, qp.data_ptr(), qc.data_ptr(), self.labels.camids.data_ptr(), self.max_rank,
-                      res.data_ptr() + 32, res.data_ptr() + res_off, ap.data_ptr(), first.data_ptr(), res.data_ptr(),
-                      ws.data_ptr(), ws.numel(), cur.cuda_stream)
-            res_host.copy_(res, non_blocking=True)
-            cur.synchronize()
-            out = res_host.numpy()
-            stats = out[:24].view(np.uint64)
-            fallback, spilled = int(stats[0]), int(stats[2] & 0xFFFFFFFF)
-            self.fused_stats = {"fallback": fallback, "spilled_spans": spilled, "spill_capacity": spill_cap,
-                                "spans": Q * ((self.G + 127) // 128)}
-            if fallback or spilled > spill_cap:
-                return None
-            cmc_host = out[32: 32 + 4 * k_eff].view(np.float32).copy()
-            summary = _lib.EvalSummary.from_buffer_copy(out[res_off: res_off + 64].tobytes())
-        raise_for_status(summary, self.max_rank)
-        info = {"num_valid": summary.num_valid, "num_ties": summary.num_ties, "cap": 0, "ap": ap, "first": first,
-                "mINP": float(summary.mINP), "fused": True}
-        return cmc_host, float(summary.mAP), info
-
     def _evaluate_one_call(self, qf, q_pids, q_camids, return_distmat, use_cap_memo):
         """One GPU, gallery packed in HBM, queries in HBM, one distance block: the whole evaluation is ONE foreign
         call (ieee_retrieve_eval_prepared enqueues pack -> contraction -> gather -> count -> metrics -> reduce back to
@@ -548,7 +493,10 @@ class RetrievalEvaluator:
                     _memo_put(memo_key, (cap, 0), (self._label_refs, q_pids))
             k_eff = min(self.max_rank, self.g_total)
             prec = _lib.PRECISIONS[self.precision]
-            ws, res, res_off, res_host = _fused_buffers(Q, D, prec, cap, k_eff, self.device)
+            res_off = (4 * k_eff + 7) // 8 * 8                  # [cmc float32[k_eff] | pad | ieee_eval_summary]
+            ws, res, res_host = _one_call_buffers((Q, D, prec, cap, k_eff, str(self.device)),
+                                                  _lib.load().ieee_retrieve_prepared_workspace_bytes(Q, D, prec, cap),
+                                                  res_off + C.sizeof(_lib.EvalSummary), self.device)
             pitch = (self.G + 31) // 32 * 32
             if self._block is None or self._block.shape[0] < Q:
                 self._block = torch.empty((Q, pitch), dtype=torch.float32, device=self.device)[:, : self.G]
@@ -593,15 +541,10 @@ class RetrievalEvaluator:
             prec = _lib.PRECISIONS[self.precision]
             link = link_for(self.group, self.device, lib.ieee_peer_exchange_bytes(Q, Q, cap, W, self.world))
             ex = link.descriptor(Q, Q, Q, 0, cap, W, link.next_epoch())
-            key = ("peer", Q, D, prec, cap, k_eff, str(self.device))
-            buf = _FUSED_POOL.get(key)
-            if buf is None:
-                if len(_FUSED_POOL) > 8:
-                    _FUSED_POOL.clear()
-                ws = torch.empty(lib.ieee_retrieve_prepared_peer_workspace_bytes(Q, D, prec, cap), dtype=torch.uint8, device=self.device)
-                res = torch.empty(32 + 64 + 4 * k_eff, dtype=torch.uint8, device=self.device)
-                buf = _FUSED_POOL[key] = (ws, res, torch.empty(res.shape, dtype=torch.uint8, pin_memory=True))
-            ws, res, res_host = buf
+            # [stats int64[3] | pad | ieee_eval_summary | cmc float32[k_eff]]
+            ws, res, res_host = _one_call_buffers(("peer", Q, D, prec, cap, k_eff, str(self.device)),
+                                                  lib.ieee_retrieve_prepared_peer_workspace_bytes(Q, D, prec, cap),
+                                                  32 + 64 + 4 * k_eff, self.device)
             self._ensure_block(Q)
             # per-query results straight into fresh arrays (every rank derives all of them itself): nothing to copy out
             # of the exchange buffer after the result has arrived, when the GPU would be idle
@@ -634,7 +577,7 @@ class RetrievalEvaluator:
         return cmc_host, float(summary.mAP), info
 
     def evaluate(self, qf: torch.Tensor, q_pids, q_camids, return_distmat: bool = False, use_cap_memo: bool = True,
-                 one_call: bool | None = None, fused: bool | None = None):
+                 one_call: bool | None = None):
         """Returns (cmc float32 ndarray [K'], mAP float, info dict).  Queries are replicated on every rank.
         `qf` may live in (pinned) host memory: it is copied on the copy stream ahead of the gallery chunks."""
         if one_call is None:
@@ -649,22 +592,6 @@ class RetrievalEvaluator:
                     self._prepare_gallery(None)
         if (one_call and self.world == 1 and qf.is_cuda and self._host_gallery is None and len(self.chunks) == 1
                 and isinstance(self.chunks[0][1], PackedFeatures) and 0 < qf.shape[0] <= self._block_rows(qf.shape[0])):
-            # opt-in (fused=True / IEEE_B200_FUSED=1): certified and bit-identical to the staged path, but on the Market-shaped
-            # workload the pre-pass and the counting epilogue still cost more than the block round trip they replace
-            # (DESIGN.md section 3.6)
-            fused = os.environ.get("IEEE_B200_FUSED", "0") == "1" if fused is None else fused
-            skip_key = (self._label_keys, _tensor_key(q_pids)) if self._label_keys[0] is not None and _tensor_key(q_pids) is not None else None
-            if (fused and not return_distmat and self.precision == "f16x3" and not self._fused_failed
-                    and (skip_key is None or skip_key not in _FUSED_SKIP)):
-                out = self._evaluate_fused(qf, q_pids, q_camids)
-                if out is not None:
-                    return out
-                # e.g. an identity with more than 32 gallery items: these labels take the staged path from now on
-                self._fused_failed = True
-                if skip_key is not None:
-                    if len(_FUSED_SKIP) > 64:
-                        _FUSED_SKIP.clear()
-                    _FUSED_SKIP[skip_key] = (self._label_refs, q_pids)
             return self._evaluate_one_call(qf, q_pids, q_camids, return_distmat, use_cap_memo)
         if (one_call and use_cap_memo and self.world > 1 and self.exchange == "peer" and qf.is_cuda and self._host_gallery is None
                 and len(self.chunks) == 1 and isinstance(self.chunks[0][1], PackedFeatures)

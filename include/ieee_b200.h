@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define IEEE_B200_ABI_VERSION 3
+#define IEEE_B200_ABI_VERSION 4
 
 typedef void* ieee_stream_t; /* cudaStream_t */
 
@@ -312,27 +312,6 @@ int ieee_retrieve_eval_prepared(const void* qf, int64_t ldq, int dtype, int64_t 
                                 const void* q_packed /* NULL, or the query rows as packed by ieee_gallery_prepare (qf is
                                                         then not read and may be NULL) */,
                                 void* workspace, size_t workspace_bytes, ieee_stream_t stream);
-
-/* The same evaluation with the COUNT FUSED INTO THE CONTRACTION's epilogue (F16X3 arithmetic, one query block, one
- * GPU): the Q x G distance block is never written.  A pre-pass computes, in plain fp32, the distance of every query to
- * the gallery items of its identity (the only distances the positions depend on, rank.py:117-160) and a band that
- * bounds its deviation from the contraction's value; the epilogue counts every 128-output span none of whose outputs
- * falls into a band, and spills the others (a few per cent) for an exact recount against the contraction's own values.
- * Either the result is bit-identical to ieee_retrieve_eval_prepared's, or it is not certified:
- * stats_out (uint64[3], device): [0] != 0 (a band was violated, a query has more than 32 same-identity gallery items, a
- * non-finite threshold) or (uint32)stats_out[2] > ieee_retrieve_fused_spill_capacity(Q, G) (spill space exhausted) mean
- * the outputs must be discarded and the staged entry point called instead; [1] = tie pairs. */
-size_t ieee_retrieve_fused_workspace_bytes(int64_t Q, int64_t G, int64_t D);
-uint32_t ieee_retrieve_fused_spill_capacity(int64_t Q, int64_t G);
-int ieee_retrieve_eval_fused_prepared(const void* qf, int64_t ldq, int dtype, int64_t Q, int64_t D, int metric, int normalize,
-                                      const void* g_packed, const void* group, const float* center, int64_t G,
-                                      const int64_t* q_pids, const int64_t* q_camids, const int64_t* g_camids,
-                                      int32_t max_rank, float* cmc, ieee_eval_summary* summary, double* per_query_ap,
-                                      int32_t* per_query_first, uint64_t* stats_out, void* workspace, size_t workspace_bytes,
-                                      ieee_stream_t stream);
-/* Accumulation chunk of the fused contraction (0, default: the same as ieee_set_accum_chunk, which keeps the two paths
- * bit-identical).  Negative: query only.  Returns the previous value. */
-int ieee_set_fused_chunk(int k_slices);
 
 /* ------------------------------------------------------------------------------------------------
  * Junk-masked top-k ranked list: the first k entries of rank.py:117 + :136-140 per query (what

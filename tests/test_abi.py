@@ -31,9 +31,9 @@ def test_library_exports_every_declared_symbol():
     assert sorted(_lib.SIGNATURES) == header_functions()
 
 
-def test_abi_version_and_struct_layout():
+def test_abi_version_4_and_struct_layout():
     lib = _lib.load()
-    assert lib.ieee_abi_version() == 3
+    assert lib.ieee_abi_version() == 4
     assert ctypes.sizeof(_lib.EvalSummary) == 64
 
 

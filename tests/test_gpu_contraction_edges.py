@@ -113,23 +113,6 @@ def test_exact_duplicates_past_fixup_capacity_one_call_entry_points(exact_dups):
     assert np.array_equal(cmc, cmc_o) and abs(mAP - map_o) < 1e-9, (cmc[:3], mAP, cmc_o[:3], map_o)
 
 
-def test_exact_duplicates_fused_count_matches_staged(exact_dups):
-    """The counting epilogue spills every span holding a near-duplicate; past its spill capacity it hands the query
-    block to the staged path.  Either way the result is the staged path's, bit for bit."""
-    base, gal, mask, _ = exact_dups
-    qp, gp, qc, gc = dup_labels()
-    cmc_s, map_s, info_s = RetrievalEvaluator(gal.cuda(), gp, gc).evaluate(base.cuda(), qp, qc, one_call=True, fused=False)
-    ev = RetrievalEvaluator(gal.cuda(), gp, gc)
-    cmc_f, map_f, info_f = ev.evaluate(base.cuda(), qp, qc, one_call=True, fused=True)
-    st = ev.fused_stats
-    print("fused stats:", st)
-    assert st is not None and st["spilled_spans"] >= NB * NCOPY
-    certified = not st["fallback"] and st["spilled_spans"] <= st["spill_capacity"]
-    assert bool(info_f.get("fused")) == certified
-    assert np.array_equal(cmc_f, cmc_s) and map_f == map_s
-    assert info_f["num_valid"] == info_s["num_valid"] and info_f["num_ties"] == info_s["num_ties"]
-
-
 def test_near_duplicates_past_fixup_capacity(cta_group, near_dups):
     base, gal, mask, terms = near_dups
     truth, _, scale, _ = terms

@@ -73,7 +73,6 @@ def test_capacity_memo_is_checked_not_trusted(one_call):
     dev = torch.device("cuda")
     lab = [torch.from_numpy(x).to(dev) for x in (s.q_pids, s.q_camids, s.g_pids, s.g_camids)]
     ev = RetrievalEvaluator(s.gf.cuda(), lab[2], lab[3])
-    ev._fused_failed = True                                              # the capacity memo belongs to the staged path
     c1, m1, i1 = ev.evaluate(s.qf.cuda(), lab[0], lab[1], one_call=one_call)
     key = [k for k in engine._CAP_MEMO if k[0] == ev._label_keys][0]
     assert engine._CAP_MEMO[key][0] == i1["cap"]
@@ -118,7 +117,6 @@ def test_one_call_path_checks_the_capacity_hint():
     dev = torch.device("cuda")
     lab = [torch.from_numpy(x).to(dev) for x in (s.q_pids, s.q_camids, s.g_pids, s.g_camids)]
     ev = RetrievalEvaluator(s.gf.cuda(), lab[2], lab[3])
-    ev._fused_failed = True                                              # staged path
     c1, m1, i1 = ev.evaluate(s.qf.cuda(), lab[0], lab[1])
     key = [k for k in engine._CAP_MEMO if k[0] == ev._label_keys][0]
     engine._CAP_MEMO[key] = (3, 0)                                       # stale, too small
@@ -127,64 +125,44 @@ def test_one_call_path_checks_the_capacity_hint():
 
 
 @pytest.mark.parametrize("metric,normalize", [("euclidean", False), ("cosine", False), ("euclidean", True)])
-def test_fused_count_equals_staged_path(metric, normalize):
-    """The count fused into the contraction's epilogue (no distance block) against the staged path: bit-identical CMC,
-    mAP, per-query AP / first hit, mINP and tie count -- and certified (no fallback)."""
+def test_one_call_equals_staged_path_per_metric(metric, normalize):
+    """The one-call path against the staged path for every metric, with ~16 gallery items per identity and queries
+    whose identity the gallery does not have: bit-identical CMC, mAP, per-query AP / first hit, mINP and tie count."""
     s = make_retrieval_set(333, 2500, 160, 5, dim=320, sigma=2.5, seed=77)      # ~16 gallery items per identity
     s.q_pids[:3] = 10 ** 6                                               # identities the gallery does not have
     ev = RetrievalEvaluator(s.gf.cuda(), s.g_pids, s.g_camids, metric, normalize)
-    c1, m1, i1 = ev.evaluate(s.qf.cuda(), s.q_pids, s.q_camids, fused=True)
-    assert i1.get("fused") and ev.fused_stats["fallback"] == 0, ev.fused_stats
-    assert 0 < ev.fused_stats["spilled_spans"] < ev.fused_stats["spans"]
-    c2, m2, i2 = ev.evaluate(s.qf.cuda(), s.q_pids, s.q_camids, fused=False)
-    assert not i2.get("fused")
+    c1, m1, i1 = ev.evaluate(s.qf.cuda(), s.q_pids, s.q_camids, one_call=True)
+    c2, m2, i2 = ev.evaluate(s.qf.cuda(), s.q_pids, s.q_camids, one_call=False)
     assert np.array_equal(c1, c2) and m1 == m2 and i1["mINP"] == i2["mINP"] and i1["num_ties"] == i2["num_ties"]
     assert torch.equal(i1["first"], i2["first"]) and torch.equal(i1["ap"], i2["ap"]) and i1["num_valid"] == i2["num_valid"] == 330
 
 
-def test_fused_count_full_size_with_duplicates():
+def test_one_call_equals_staged_path_full_size_with_duplicates():
     """Market-shaped, feature width 2304, gallery rows duplicated (bit-equal distances: ties by gallery index) and the
-    query set containing gallery rows (exact zeros: the near-duplicate fix-up inside the spilled spans)."""
+    query set containing gallery rows (exact zeros: the near-duplicate fix-up): the one-call path against the staged
+    path, and both against the oracle on the GPU's own distances."""
     from ieee_b200.testing import market1501_shaped
     s = market1501_shaped(seed=3, num_q=700)
     gf, g_pids, g_camids = s.gf.clone(), s.g_pids.copy(), s.g_camids.copy()
-    small = np.isin(s.g_pids, np.nonzero(np.bincount(s.g_pids) <= 16)[0])  # identities that stay within 32 items when doubled
+    small = np.isin(s.g_pids, np.nonzero(np.bincount(s.g_pids) <= 16)[0])  # identities of at most 16 items
     src = np.nonzero(small[:8000])[0][:1000]
     dst = 15912 - np.arange(src.size)
     dst = dst[~np.isin(dst, src)]
     src = src[: dst.size]
     gf[dst] = gf[src]
     g_pids[dst], g_camids[dst] = g_pids[src], (g_camids[src] + 1) % 6
-    assert np.bincount(g_pids)[1:].max() <= 32
     qf = s.qf.clone()
     twins = np.nonzero(g_pids != 0)[0][100:150]                          # (pid 0 = distractors: 2 680 of them, no query)
     qf[:50] = gf[twins]                                                   # queries identical to gallery rows
     q_pids, q_camids = s.q_pids.copy(), s.q_camids.copy()
     q_pids[:50], q_camids[:50] = g_pids[twins], (g_camids[twins] + 2) % 6
     ev = RetrievalEvaluator(gf.cuda(), g_pids, g_camids)
-    c1, m1, i1 = ev.evaluate(qf.cuda(), q_pids, q_camids, fused=True)
-    assert i1.get("fused") and ev.fused_stats["fallback"] == 0, ev.fused_stats
-    c2, m2, i2 = ev.evaluate(qf.cuda(), q_pids, q_camids, fused=False, return_distmat=True)
+    c1, m1, i1 = ev.evaluate(qf.cuda(), q_pids, q_camids, return_distmat=True, one_call=True)
+    c2, m2, i2 = ev.evaluate(qf.cuda(), q_pids, q_camids, return_distmat=True, one_call=False)
+    assert torch.equal(i1["distmat"], i2["distmat"])
     assert i2["num_ties"] > 0 and i1["num_ties"] == i2["num_ties"]
     assert np.array_equal(c1, c2) and m1 == m2 and torch.equal(i1["first"], i2["first"]) and torch.equal(i1["ap"], i2["ap"])
-    d = i2["distmat"].cpu().numpy()
+    d = i1["distmat"].cpu().numpy()
     assert (d[np.arange(50), twins] == 0).all()                          # the duplicates really are at distance 0
     cmc_o, map_o = R.evaluate_rank(d, q_pids, g_pids, q_camids, g_camids, max_rank=20)
     assert np.array_equal(c1, cmc_o) and abs(m1 - map_o) < 1e-9
-
-
-def test_fused_count_falls_back_when_it_cannot_certify():
-    """An identity with more than 32 gallery items does not fit the epilogue's threshold table: the fused path says so
-    and evaluate() silently takes the staged path; labels are remembered, so the next evaluator does not try again."""
-    from ieee_b200 import engine
-    s = make_retrieval_set(120, 1500, 12, 3, dim=128, sigma=2.0, seed=10)      # ~125 gallery items per identity
-    dev = torch.device("cuda")
-    lab = [torch.from_numpy(x).to(dev) for x in (s.q_pids, s.q_camids, s.g_pids, s.g_camids)]
-    ev = RetrievalEvaluator(s.gf.cuda(), lab[2], lab[3])
-    c1, m1, i1 = ev.evaluate(s.qf.cuda(), lab[0], lab[1], fused=True)
-    assert not i1.get("fused") and ev.fused_stats["fallback"] & 1
-    c2, m2, i2 = ev.evaluate(s.qf.cuda(), lab[0], lab[1], fused=False)
-    assert np.array_equal(c1, c2) and m1 == m2
-    ev2 = RetrievalEvaluator(s.gf.cuda(), lab[2], lab[3])
-    ev2.evaluate(s.qf.cuda(), lab[0], lab[1], fused=True)
-    assert ev2.fused_stats is None                                           # not attempted: remembered per labels
