@@ -78,6 +78,10 @@ SIGNATURES = {
     "ieee_gnn_rerank": (C.c_int, [vp, i64, i64, i32, i32, vp, i64, vp, sz, vp]),
     "ieee_rerank_workspace_bytes": (sz, [i64, i64, i32, i32]),
     "ieee_rerank": (C.c_int, [vp, i64, vp, i64, vp, i64, i64, i64, i32, i32, C.c_double, vp, i64, vp, sz, vp]),
+    "ieee_rerank_stream_workspace_bytes": (sz, [i64, i64, i32, i32]),
+    "ieee_rerank_stream_scratch_bytes": (sz, [i64, i64, i32, sz]),
+    "ieee_rerank_stream_prepare": (C.c_int, [vp, i64, vp, i64, i64, C.c_int, C.c_int, i32, i32, sz, vp, vp, vp, sz, vp, sz, vp]),
+    "ieee_rerank_stream_block": (C.c_int, [vp, i64, i64, i32, i32, vp, i64, i64, C.c_double, vp, i64, vp, sz, vp]),
 }
 
 MAX_PEERS = 16

@@ -110,6 +110,16 @@ int rerank(const float* q_g, int64_t ld_qg, const float* q_q, int64_t ld_qq, con
            int64_t G, int32_t k1, int32_t k2, double lambda_value, float* out, int64_t ldo, void* workspace,
            size_t workspace_bytes, cudaStream_t stream);
 
+size_t rerank_stream_workspace_bytes(int64_t Q, int64_t G, int32_t k1, int32_t k2);
+size_t rerank_stream_scratch_bytes(int64_t Q, int64_t G, int32_t k1, size_t strip_bytes);
+int rerank_stream_prepare(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
+                          int precision, int32_t k1, int32_t k2, size_t strip_bytes, float* colmax, int32_t* rank,
+                          void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes, cudaStream_t stream,
+                          int cta_group);
+int rerank_stream_block(const void* workspace, int64_t Q, int64_t G, int32_t k1, int32_t k2, const float* colmax, int64_t row0,
+                        int64_t rows, double lambda_value, float* block, int64_t ld, void* scratch, size_t scratch_bytes,
+                        cudaStream_t stream);
+
 size_t gnn_rerank_workspace_bytes(int64_t N, int32_t k1);
 int gnn_rerank(const float* neg_score, int64_t lds, int64_t N, int32_t k1, int32_t k2, float* A, int64_t ldA, void* workspace,
                size_t workspace_bytes, cudaStream_t stream);
@@ -697,6 +707,33 @@ int ieee_rerank(const float* q_g, int64_t ld_qg, const float* q_q, int64_t ld_qq
   if (rc) return rc;
   return rerank(q_g, ld_qg, q_q, ld_qq, g_g, ld_gg, Q, G, k1, k2, lambda_value, out, ldo, workspace, workspace_bytes,
                 (cudaStream_t)stream);
+}
+
+size_t ieee_rerank_stream_workspace_bytes(int64_t Q, int64_t G, int32_t k1, int32_t k2) {
+  return rerank_stream_workspace_bytes(Q, G, k1, k2);
+}
+
+size_t ieee_rerank_stream_scratch_bytes(int64_t Q, int64_t G, int32_t k1, size_t strip_bytes) {
+  return rerank_stream_scratch_bytes(Q, G, k1, strip_bytes);
+}
+
+int ieee_rerank_stream_prepare(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
+                               int precision, int32_t k1, int32_t k2, size_t strip_bytes, float* colmax, int32_t* rank,
+                               void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
+                               ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return rerank_stream_prepare(q_packed, Q, g_packed, G, D, metric, precision, k1, k2, strip_bytes, colmax, rank, workspace,
+                               workspace_bytes, scratch, scratch_bytes, (cudaStream_t)stream, cta_group_default());
+}
+
+int ieee_rerank_stream_block(const void* workspace, int64_t Q, int64_t G, int32_t k1, int32_t k2, const float* colmax,
+                             int64_t row0, int64_t rows, double lambda_value, float* block, int64_t ld, void* scratch,
+                             size_t scratch_bytes, ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return rerank_stream_block(workspace, Q, G, k1, k2, colmax, row0, rows, lambda_value, block, ld, scratch, scratch_bytes,
+                             (cudaStream_t)stream);
 }
 
 size_t ieee_gnn_rerank_workspace_bytes(int64_t N, int32_t k1) { return gnn_rerank_workspace_bytes(N, k1); }

@@ -121,6 +121,27 @@ inline PackedLayout packed_layout(int64_t rows, int64_t D, int precision) {
   return L;
 }
 
+// Rows [r0, r0 + rows) of a packed operand that holds `total` rows, as pointers into its sections: a contraction over
+// them reads the same bytes a contraction over the whole operand reads for those rows.
+struct PackedRows {
+  const uint8_t *hi, *lo;       // lo == hi when the operand has no lo plane
+  const float *norm, *scale;
+  int64_t rows, Dp;
+};
+inline PackedRows packed_rows(const void* packed, int64_t total, int64_t r0, int64_t rows, int64_t D, int precision) {
+  const PackedLayout L = packed_layout(total, D, precision);
+  const uint8_t* b = static_cast<const uint8_t*>(packed);
+  const size_t row_bytes = size_t(L.Dp) * (precision == IEEE_PREC_FP32_SIMT ? 4 : 2);
+  PackedRows r;
+  r.hi = b + L.hi_off + size_t(r0) * row_bytes;
+  r.lo = L.has_lo ? b + L.lo_off + size_t(r0) * row_bytes : r.hi;
+  r.norm = reinterpret_cast<const float*>(b + L.norm_off) + r0;
+  r.scale = reinterpret_cast<const float*>(b + L.scale_off) + r0;
+  r.rows = rows;
+  r.Dp = L.Dp;
+  return r;
+}
+
 // ---- gallery grouping (rank.cu): open-addressing hash pid -> slot; members of a slot = the gallery items of that identity
 static constexpr long long kEmptyPid = (long long)0x8080808080808080ull;   // memset(0x80) pattern; not a usable pid
 

@@ -707,41 +707,39 @@ struct GemmLaunch {
 };
 
 template <int CG>
-static int gemm_setup(GemmLaunch& L, const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
-                      int precision, float* out, int64_t ldo, int out_box_cols, CUtensorMapSwizzle out_swizzle) {
+static int gemm_setup(GemmLaunch& L, const PackedRows& a, const PackedRows& b, int metric, int precision, float* out,
+                      int64_t ldo, int out_box_cols, CUtensorMapSwizzle out_swizzle) {
   constexpr int kBRows = BLOCK_N / CG;
-  PackedLayout lq = packed_layout(Q, D, precision), lg = packed_layout(G, D, precision);
-  const uint8_t* qb = static_cast<const uint8_t*>(q_packed);
-  const uint8_t* gb = static_cast<const uint8_t*>(g_packed);
+  const int64_t Q = a.rows, G = b.rows;
   const CUtensorMapDataType dt16 = CU_TENSOR_MAP_DATA_TYPE_UINT16;   // the copy engine only moves 16-bit words
   int rc;
-  if ((rc = make_tmap(&L.ta_hi, dt16, 2, qb + lq.hi_off, Q, lq.Dp, lq.Dp, BLOCK_M, BLOCK_K))) return rc;
-  if ((rc = make_tmap(&L.tb_hi, dt16, 2, gb + lg.hi_off, G, lg.Dp, lg.Dp, kBRows, BLOCK_K))) return rc;
+  if ((rc = make_tmap(&L.ta_hi, dt16, 2, a.hi, Q, a.Dp, a.Dp, BLOCK_M, BLOCK_K))) return rc;
+  if ((rc = make_tmap(&L.tb_hi, dt16, 2, b.hi, G, b.Dp, b.Dp, kBRows, BLOCK_K))) return rc;
   if (precision == IEEE_PREC_F16X3) {
-    if ((rc = make_tmap(&L.ta_lo, dt16, 2, qb + lq.lo_off, Q, lq.Dp, lq.Dp, BLOCK_M, BLOCK_K))) return rc;
-    if ((rc = make_tmap(&L.tb_lo, dt16, 2, gb + lg.lo_off, G, lg.Dp, lg.Dp, kBRows, BLOCK_K))) return rc;
+    if ((rc = make_tmap(&L.ta_lo, dt16, 2, a.lo, Q, a.Dp, a.Dp, BLOCK_M, BLOCK_K))) return rc;
+    if ((rc = make_tmap(&L.tb_lo, dt16, 2, b.lo, G, b.Dp, b.Dp, kBRows, BLOCK_K))) return rc;
   } else {
     L.ta_lo = L.ta_hi;
     L.tb_lo = L.tb_hi;
   }
   GemmParams& p = L.p;
   const bool euclid = metric == IEEE_METRIC_EUCLIDEAN;
-  p.rq = euclid ? reinterpret_cast<const float*>(qb + lq.norm_off) : nullptr;
-  p.rg = euclid ? reinterpret_cast<const float*>(gb + lg.norm_off) : nullptr;
-  p.sq = precision == IEEE_PREC_F16X3 ? reinterpret_cast<const float*>(qb + lq.scale_off) : nullptr;
-  p.sg = precision == IEEE_PREC_F16X3 ? reinterpret_cast<const float*>(gb + lg.scale_off) : nullptr;
+  p.rq = euclid ? a.norm : nullptr;
+  p.rg = euclid ? b.norm : nullptr;
+  p.sq = precision == IEEE_PREC_F16X3 ? a.scale : nullptr;
+  p.sg = precision == IEEE_PREC_F16X3 ? b.scale : nullptr;
   p.alpha = euclid ? -2.0f : -1.0f;
   p.base0 = metric == IEEE_METRIC_NEG_DOT ? 0.0f : 1.0f;
   p.out = out;
   p.ldo = ldo;
   p.Q = (int)Q;
   p.G = (int)G;
-  p.num_kb = (int)(lq.Dp / BLOCK_K);
+  p.num_kb = (int)(a.Dp / BLOCK_K);
   p.nseg = precision == IEEE_PREC_F16X3 ? 3 : 1;
   p.num_m_tiles = (int)((Q + BLOCK_M * CG - 1) / (BLOCK_M * CG));
   p.num_n_tiles = (int)((G + BLOCK_N - 1) / BLOCK_N);
   // raster panel: as many m tiles as keep the panel's A planes within ~40 MB of the 126 MB L2
-  const double a_tile_bytes = double(BLOCK_M * CG) * double(lq.Dp) * 2.0 * (precision == IEEE_PREC_F16X3 ? 2.0 : 1.0);
+  const double a_tile_bytes = double(BLOCK_M * CG) * double(a.Dp) * 2.0 * (precision == IEEE_PREC_F16X3 ? 2.0 : 1.0);
   int panel = (int)(40.0 * 1024 * 1024 / a_tile_bytes);
   if (g_raster_panel > 0) panel = g_raster_panel;
   p.panel_m = panel < 1 ? 1 : (panel > p.num_m_tiles ? p.num_m_tiles : panel);
@@ -778,11 +776,11 @@ static void cluster_launch_config(cudaLaunchConfig_t& cfg, cudaLaunchAttribute* 
 }
 
 template <int CG>
-static int launch_umma(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
-                       int precision, float* out, int64_t ldo, cudaStream_t stream) {
+static int launch_umma(const PackedRows& a, const PackedRows& b, int metric, int precision, float* out, int64_t ldo,
+                       cudaStream_t stream) {
   using Cfg = GemmCfg<CG>;
   GemmLaunch L;
-  int rc = gemm_setup<CG>(L, q_packed, Q, g_packed, G, D, metric, precision, out, ldo, 32, CU_TENSOR_MAP_SWIZZLE_128B);
+  int rc = gemm_setup<CG>(L, a, b, metric, precision, out, ldo, 32, CU_TENSOR_MAP_SWIZZLE_128B);
   if (rc) return rc;
   IEEE_ENSURE_DYN_SMEM(distmat_umma_kernel<CG>, Cfg::kSmemBytes);
   cudaLaunchConfig_t cfg;
@@ -800,12 +798,12 @@ constexpr float kFixTau = 0.015625f;
 size_t distmat_fixup_bytes(int64_t Q) { return align256((size_t(2 * Q + 4096) + 2) * 8); }
 
 template <int CG>
-static int launch_umma_chunked(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
-                               int precision, float* out, int64_t ldo, cudaStream_t stream, int chunk_kb, void* fix_ws,
-                               bool fix_zeroed) {
+static int launch_umma_chunked(const PackedRows& a, const PackedRows& b, int metric, int precision, float* out, int64_t ldo,
+                               cudaStream_t stream, int chunk_kb, void* fix_ws, bool fix_zeroed) {
   using Cfg = GemmCfgC<CG>;
   GemmLaunch L;
-  int rc = gemm_setup<CG>(L, q_packed, Q, g_packed, G, D, metric, precision, out, ldo, 16, CU_TENSOR_MAP_SWIZZLE_64B);
+  const int64_t Q = a.rows, G = b.rows;
+  int rc = gemm_setup<CG>(L, a, b, metric, precision, out, ldo, 16, CU_TENSOR_MAP_SWIZZLE_64B);
   if (rc) return rc;
   const bool fix = fix_ws != nullptr && metric == IEEE_METRIC_EUCLIDEAN && precision == IEEE_PREC_F16X3 &&
                    !(g_debug_flags & 32);
@@ -826,34 +824,32 @@ static int launch_umma_chunked(const void* q_packed, int64_t Q, const void* g_pa
                                      chunk_kb));
   count_launch(1, "distmat_umma_chunked_kernel");
   if (fix) {
-    PackedLayout lq = packed_layout(Q, D, precision), lg = packed_layout(G, D, precision);
-    const uint8_t* qb = static_cast<const uint8_t*>(q_packed);
-    const uint8_t* gb = static_cast<const uint8_t*>(g_packed);
     distmat_fixup_kernel<<<sm_count(), 256, 0, stream>>>(
-        reinterpret_cast<const __half*>(qb + lq.hi_off), reinterpret_cast<const __half*>(qb + lq.lo_off),
-        reinterpret_cast<const __half*>(gb + lg.hi_off), reinterpret_cast<const __half*>(gb + lg.lo_off),
-        reinterpret_cast<const float*>(qb + lq.scale_off), reinterpret_cast<const float*>(gb + lg.scale_off),
-        reinterpret_cast<const float*>(qb + lq.norm_off), reinterpret_cast<const float*>(gb + lg.norm_off), (int)lq.Dp, (int)Q,
-        (int)G, kFixTau, L.p.fix_list, L.p.fix_cap, out, ldo);
+        reinterpret_cast<const __half*>(a.hi), reinterpret_cast<const __half*>(a.lo), reinterpret_cast<const __half*>(b.hi),
+        reinterpret_cast<const __half*>(b.lo), a.scale, b.scale, a.norm, b.norm, (int)a.Dp, (int)Q, (int)G, kFixTau,
+        L.p.fix_list, L.p.fix_cap, out, ldo);
     count_launch(1, "distmat_fixup_kernel");
     IEEE_CUDA_CHECK(cudaGetLastError());
   }
   return IEEE_OK;
 }
 
-int distmat_umma(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric, int precision,
-                 float* out, int64_t ldo, cudaStream_t stream, int cta_group, void* fix_ws, bool fix_zeroed) {
+int distmat_umma_rows(const PackedRows& a, const PackedRows& b, int metric, int precision, float* out, int64_t ldo,
+                      cudaStream_t stream, int cta_group, void* fix_ws, bool fix_zeroed) {
   // chunked accumulation serves the fp32-grade mode; the 1-pass BF16 mode keeps the whole K in TMEM (throughput mode)
   if (g_accum_chunk_kb > 0 && (precision == IEEE_PREC_F16X3 || (g_debug_flags & 8))) {
     if (cta_group == 2)
-      return launch_umma_chunked<2>(q_packed, Q, g_packed, G, D, metric, precision, out, ldo, stream, g_accum_chunk_kb, fix_ws,
-                                    fix_zeroed);
-    return launch_umma_chunked<1>(q_packed, Q, g_packed, G, D, metric, precision, out, ldo, stream, g_accum_chunk_kb, fix_ws,
-                                  fix_zeroed);
+      return launch_umma_chunked<2>(a, b, metric, precision, out, ldo, stream, g_accum_chunk_kb, fix_ws, fix_zeroed);
+    return launch_umma_chunked<1>(a, b, metric, precision, out, ldo, stream, g_accum_chunk_kb, fix_ws, fix_zeroed);
   }
-  if (cta_group == 2)
-    return launch_umma<2>(q_packed, Q, g_packed, G, D, metric, precision, out, ldo, stream);
-  return launch_umma<1>(q_packed, Q, g_packed, G, D, metric, precision, out, ldo, stream);
+  if (cta_group == 2) return launch_umma<2>(a, b, metric, precision, out, ldo, stream);
+  return launch_umma<1>(a, b, metric, precision, out, ldo, stream);
+}
+
+int distmat_umma(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric, int precision,
+                 float* out, int64_t ldo, cudaStream_t stream, int cta_group, void* fix_ws, bool fix_zeroed) {
+  return distmat_umma_rows(packed_rows(q_packed, Q, 0, Q, D, precision), packed_rows(g_packed, G, 0, G, D, precision), metric,
+                           precision, out, ldo, stream, cta_group, fix_ws, fix_zeroed);
 }
 
 }  // namespace ieee

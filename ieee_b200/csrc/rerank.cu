@@ -26,6 +26,25 @@ struct RawView {            // the virtual N x N matrix [[qq, qg], [qg^T, gg]]
     if (r < Q) return c < Q ? qq[(int64_t)r * ld_qq + c] : qg[(int64_t)r * ld_qg + (c - Q)];
     return c < Q ? qg[(int64_t)c * ld_qg + (r - Q)] : gg[(int64_t)(r - Q) * ld_gg + (c - Q)];
   }
+  // the 32 x 32 tile raw[r0.., c0..] is contiguous in r (the qg^T block: r >= Q, c < Q)
+  __device__ __forceinline__ bool contiguous_in_r(int r0, int c0) const { return r0 >= Q && c0 + 31 < Q; }
+};
+
+// Columns [c0, c0 + w) of the virtual matrix (a strip, c0 and w counted in the queries or in the gallery, never both),
+// held as the two contraction outputs that make them up; `at(r, t)` is raw[r][c0 + t].
+//   top: raw rows < Q,  [Q, w]  -- qq[:, I] (A = all queries, B = q_I) or qg[:, I - Q] (A = all queries, B = g_I)
+//   bot: raw rows >= Q, [w, G] when the strip lies in the queries -- qg[I, :] (A = q_I, B = all gallery), row t =
+//        strip column t -- else [G, w] -- gg[:, I - Q] (A = all gallery, B = g_I)
+struct StripView {
+  const float *top, *bot;
+  int64_t ld_top, ld_bot;
+  int Q;
+  bool bot_by_row;
+  __device__ __forceinline__ float at(int r, int t) const {
+    if (r < Q) return top[(int64_t)r * ld_top + t];
+    return bot_by_row ? bot[(int64_t)t * ld_bot + (r - Q)] : bot[(int64_t)(r - Q) * ld_bot + t];
+  }
+  __device__ __forceinline__ bool contiguous_in_r(int r0, int) const { return bot_by_row && r0 >= Q; }
 };
 
 // ---- K1a: column maxima of raw^2 ------------------------------------------------------------------------
@@ -55,21 +74,22 @@ __global__ void __launch_bounds__(256) rr_rowmax_kernel(const float* __restrict_
   if ((threadIdx.x & 31) == 0) atomicMax(colmax_bits + r, __float_as_int(mx));
 }
 
-// ---- K1b: orig[i][j] = raw[j][i]^2 / colmax[i]; 32 x 32 tiles transposed through shared memory -----------
-__global__ void __launch_bounds__(256) rr_build_orig_kernel(RawView raw, int N, const float* __restrict__ colmax,
-                                                             float* __restrict__ orig) {
+// ---- K1b: orig[i][j] = raw[j][i]^2 / colmax[i], i < rows, j < N; 32 x 32 tiles transposed through shared memory ----
+// View = RawView (all N rows of orig) or StripView (the rows of one strip, colmax and orig offset to its first row)
+template <class View>
+__global__ void __launch_bounds__(256) rr_build_orig_kernel(View raw, int rows, int N, const float* __restrict__ colmax,
+                                                             float* __restrict__ orig, int64_t ldo) {
   __shared__ float tile[32][33];
   const int i0 = blockIdx.y * 32, j0 = blockIdx.x * 32;
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;   // 32 x 8
-  // raw[j][i] is contiguous in i except in the qg^T block (j >= Q, i < Q), which is contiguous in j
-  const bool direct = (j0 >= raw.Q) && (i0 + 31 < raw.Q);
-  if (direct) {
+  // raw[j][i] is contiguous in i except where the view says it is contiguous in j
+  if (raw.contiguous_in_r(j0, i0)) {
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
       const int i = i0 + ty + 8 * k, j = j0 + tx;
-      if (i < N && j < N) {
+      if (i < rows && j < N) {
         const float x = raw.at(j, i);
-        orig[(int64_t)i * N + j] = __fdiv_rn(__fmul_rn(x, x), colmax[i]);
+        orig[(int64_t)i * ldo + j] = __fdiv_rn(__fmul_rn(x, x), colmax[i]);
       }
     }
     return;
@@ -77,15 +97,15 @@ __global__ void __launch_bounds__(256) rr_build_orig_kernel(RawView raw, int N, 
 #pragma unroll
   for (int k = 0; k < 4; ++k) {
     const int j = j0 + ty + 8 * k, i = i0 + tx;
-    tile[ty + 8 * k][tx] = (i < N && j < N) ? raw.at(j, i) : 0.f;
+    tile[ty + 8 * k][tx] = (i < rows && j < N) ? raw.at(j, i) : 0.f;
   }
   __syncthreads();
 #pragma unroll
   for (int k = 0; k < 4; ++k) {
     const int i = i0 + ty + 8 * k, j = j0 + tx;
-    if (i < N && j < N) {
+    if (i < rows && j < N) {
       const float x = tile[tx][ty + 8 * k];
-      orig[(int64_t)i * N + j] = __fdiv_rn(__fmul_rn(x, x), colmax[i]);
+      orig[(int64_t)i * ldo + j] = __fdiv_rn(__fmul_rn(x, x), colmax[i]);
     }
   }
 }
@@ -115,6 +135,22 @@ __device__ int reciprocal_append(const int32_t* __restrict__ rank, int ldr, int 
   return n_out;
 }
 
+// weights of one row of V (rerank.py:81-82): exp(-orig[i, members]) / sum, summed in ascending member order;
+// orig_row is row i of orig (the N x N matrix, or the row as one strip holds it)
+__device__ void rr_weights(const float* __restrict__ orig_row, const int32_t* __restrict__ cols, float* __restrict__ vals,
+                           int nu, int lane) {
+  for (int t = lane; t < nu; t += 32) vals[t] = expf(-orig_row[cols[t]]);
+  __syncwarp();
+  float total = 0.f;
+  if (lane == 0)
+    for (int t = 0; t < nu; ++t) total = __fadd_rn(total, vals[t]);
+  total = __shfl_sync(0xffffffffu, total, 0);
+  for (int t = lane; t < nu; t += 32) vals[t] = __fdiv_rn(vals[t], total);
+}
+
+// kWeights: also weigh the members from orig (N x N).  Without it only the membership (columns, counts) is written,
+// from `rank` alone, and rr_weights_kernel weighs the rows strip by strip.
+template <bool kWeights>
 __global__ void __launch_bounds__(32 * kRowWarps)
 rr_krecip_kernel(const int32_t* __restrict__ rank, int ldr, const float* __restrict__ orig, int N, int k1p, int khp, int cap_v,
                  int cap_pow2, int32_t* __restrict__ v_col, float* __restrict__ v_val, int32_t* __restrict__ v_cnt) {
@@ -174,17 +210,18 @@ rr_krecip_kernel(const int32_t* __restrict__ rank, int ldr, const float* __restr
     nu += __popc(m);
   }
   __syncwarp();
-  // weights (rerank.py:81-82): exp(-orig[i, members]) / sum, summed in ascending member order
-  int32_t* cols = v_col + (int64_t)i * cap_v;
-  float* vals = v_val + (int64_t)i * cap_v;
-  for (int t = lane; t < nu; t += 32) vals[t] = expf(-orig[(int64_t)i * N + cols[t]]);
-  __syncwarp();
-  float total = 0.f;
-  if (lane == 0)
-    for (int t = 0; t < nu; ++t) total = __fadd_rn(total, vals[t]);
-  total = __shfl_sync(0xffffffffu, total, 0);
-  for (int t = lane; t < nu; t += 32) vals[t] = __fdiv_rn(vals[t], total);
+  if constexpr (kWeights) rr_weights(orig + (int64_t)i * N, v_col + (int64_t)i * cap_v, v_val + (int64_t)i * cap_v, nu, lane);
   if (lane == 0) v_cnt[i] = nu;
+}
+
+// weights of rows [row0, row0 + rows) of V from one strip of orig (row t of the strip = row row0 + t of orig)
+__global__ void __launch_bounds__(32 * kRowWarps)
+rr_weights_kernel(const float* __restrict__ orig, int64_t ldo, int row0, int rows, int cap_v, const int32_t* __restrict__ v_col,
+                  float* __restrict__ v_val, const int32_t* __restrict__ v_cnt) {
+  const int lane = threadIdx.x & 31, t = blockIdx.x * kRowWarps + (threadIdx.x >> 5);
+  if (t >= rows) return;
+  const int i = row0 + t;
+  rr_weights(orig + (int64_t)t * ldo, v_col + (int64_t)i * cap_v, v_val + (int64_t)i * cap_v, v_cnt[i], lane);
 }
 
 // ---- K4: V_qe[i] = mean_j V[rank[i][j]], j < k2; one CTA per row ------------------------------------------
@@ -313,13 +350,19 @@ __global__ void rr_col_fill_kernel(int N, int cap, const int32_t* __restrict__ c
 }
 
 // ---- K5b + K6: Jaccard accumulation for one query per CTA, then the lambda blend ----------------------------
+// Query i = row0 + blockIdx.x, output row blockIdx.x of `out`.  Dense (kBlock = false): row0 = 0, the output row
+// doubles as the accumulator (acc == out) and the original distance is read from orig.  kBlock: `out` holds the
+// query's distances to the gallery (qg rows row0..), accumulation goes to `acc`, and the original distance is
+// formed from the distance as rr_build_orig_kernel forms it (qg[i][g] = raw[Q + g][i]).
+template <bool kBlock>
 __global__ void __launch_bounds__(256)
 rr_jaccard_kernel(int Q, int G, int N, int cap, const int32_t* __restrict__ col, const float* __restrict__ val,
                   const int32_t* __restrict__ cnt, const int32_t* __restrict__ col_ptr, const int32_t* __restrict__ inv_row,
-                  const float* __restrict__ inv_val, const float* __restrict__ orig, float w_jaccard, float w_orig,
-                  float* __restrict__ out, int64_t ldo) {
-  const int i = blockIdx.x;
-  float* acc = out + (int64_t)i * ldo;     // the output row doubles as the accumulator (columns >= Q only are kept)
+                  const float* __restrict__ inv_val, const float* __restrict__ orig, const float* __restrict__ colmax, int row0,
+                  float* acc_rows, int64_t ld_acc, float w_jaccard, float w_orig, float* out, int64_t ldo) {
+  const int i = row0 + blockIdx.x;
+  float* acc = acc_rows + (int64_t)blockIdx.x * ld_acc;
+  float* dst = out + (int64_t)blockIdx.x * ldo;
   for (int g = threadIdx.x; g < G; g += blockDim.x) acc[g] = 0.f;
   __syncthreads();
   const int n = cnt[i];
@@ -337,11 +380,22 @@ rr_jaccard_kernel(int Q, int G, int N, int cap, const int32_t* __restrict__ col,
   for (int g = threadIdx.x; g < G; g += blockDim.x) {
     const float tmin = acc[g];
     const float jac = __fsub_rn(1.0f, __fdiv_rn(tmin, __fsub_rn(2.0f, tmin)));          // rerank.py:106
-    acc[g] = __fadd_rn(__fmul_rn(jac, w_jaccard), __fmul_rn(orig[(int64_t)i * N + Q + g], w_orig));   // :108
+    float o;
+    if constexpr (kBlock) {
+      const float x = dst[g];
+      o = __fdiv_rn(__fmul_rn(x, x), colmax[i]);
+    } else {
+      o = orig[(int64_t)i * N + Q + g];
+    }
+    dst[g] = __fadd_rn(__fmul_rn(jac, w_jaccard), __fmul_rn(o, w_orig));   // :108
   }
 }
 
 // ---- host ----------------------------------------------------------------------------------------------------
+int distmat_umma_rows(const PackedRows& a, const PackedRows& b, int metric, int precision, float* out, int64_t ldo,
+                      cudaStream_t stream, int cta_group, void* fix_ws, bool fix_zeroed);
+size_t distmat_fixup_bytes(int64_t Q);
+
 static inline int pow2_at_least(int x) { int p = 1; while (p < x) p <<= 1; return p; }
 static inline int half_k(int k1) {          // int(np.around(k1 / 2.)): round half to even
   const double h = k1 / 2.0;
@@ -350,12 +404,15 @@ static inline int half_k(int k1) {          // int(np.around(k1 / 2.)): round ha
   return (int)r;
 }
 
+// Workspace of both forms.  The dense form holds orig (N x N), colmax, rank and the top-k values; the streamed form
+// keeps colmax and rank in caller buffers and only the sparse state here (its strips live in a separate scratch, see
+// StripPlan), so its offsets depend on (Q, G, k1, k2) alone.
 struct RerankPlan {
   int N, k1p, khp, cap_v, cap_v_pow2, cap_e, cap_e_pow2;
   size_t off_orig, off_colmax, off_rank, off_rank_val, off_vcol, off_vval, off_vcnt, off_ecol, off_eval, off_ecnt, off_colcnt,
       off_colptr, off_cursor, off_invrow, off_invval, total;
 };
-static RerankPlan make_plan(int64_t Q, int64_t G, int k1, int k2) {
+static RerankPlan make_plan(int64_t Q, int64_t G, int k1, int k2, bool dense) {
   RerankPlan p;
   p.N = (int)(Q + G);
   p.k1p = k1 + 1;
@@ -367,10 +424,11 @@ static RerankPlan make_plan(int64_t Q, int64_t G, int k1, int k2) {
   size_t o = 0;
   auto take = [&](size_t bytes) { size_t r = o; o += align256(bytes); return r; };
   const size_t N = p.N;
-  p.off_orig = take(N * N * 4);
-  p.off_colmax = take(N * 4);
-  p.off_rank = take(N * p.k1p * 4);
-  p.off_rank_val = take(N * p.k1p * 4);
+  const size_t dn = dense ? N : 0;
+  p.off_orig = take(dn * N * 4);
+  p.off_colmax = take(dn * 4);
+  p.off_rank = take(dn * p.k1p * 4);
+  p.off_rank_val = take(dn * p.k1p * 4);
   p.off_vcol = take(N * p.cap_v * 4);
   p.off_vval = take(N * p.cap_v * 4);
   p.off_vcnt = take(N * 4);
@@ -386,9 +444,83 @@ static RerankPlan make_plan(int64_t Q, int64_t G, int k1, int k2) {
   return p;
 }
 
+// the limits both forms share; returns IEEE_OK or sets the error text
+static int check_params(const char* who, int64_t Q, int64_t G, int32_t k1, int32_t k2) {
+  IEEE_REQUIRE(Q > 0 && G > 0, "%s: bad shape Q=%lld G=%lld", who, (long long)Q, (long long)G);
+  IEEE_REQUIRE(Q + G < (int64_t(1) << 24), "%s: N = Q + G too large", who);
+  IEEE_REQUIRE(k1 >= 1 && k1 + 1 <= 512 && k2 >= 1 && k2 <= k1 + 1, "%s: need 1 <= k2 <= k1 + 1 <= 512", who);
+  IEEE_REQUIRE(k1 + 1 <= Q + G, "%s: k1 + 1 exceeds the number of samples", who);
+  const RerankPlan p = make_plan(Q, G, k1, k2, false);
+  IEEE_REQUIRE((size_t)p.cap_e_pow2 * 8 <= 160 * 1024, "%s: k2 * (k1+1) * (k1/2+2) = %d entries per row exceed the shared-memory sort",
+               who, p.cap_e);
+  return IEEE_OK;
+}
+
+// The V rows the Jaccard stage reads: V_qe (k2 > 1) or V itself.
+struct SparseRows {
+  const int32_t* col;
+  const float* val;
+  const int32_t* cnt;
+  int cap;
+};
+static SparseRows final_rows(const RerankPlan& p, uint8_t* w, int k2) {
+  if (k2 != 1)
+    return {reinterpret_cast<int32_t*>(w + p.off_ecol), reinterpret_cast<float*>(w + p.off_eval),
+            reinterpret_cast<int32_t*>(w + p.off_ecnt), p.cap_e};
+  return {reinterpret_cast<int32_t*>(w + p.off_vcol), reinterpret_cast<float*>(w + p.off_vval),
+          reinterpret_cast<int32_t*>(w + p.off_vcnt), p.cap_v};
+}
+
+// K4 + K5a: query expansion of V (built by K3) and the inverted index of the result
+static int expand_and_index(const RerankPlan& p, uint8_t* w, const int32_t* rank, int k2, cudaStream_t stream) {
+  const int N = p.N;
+  int32_t* vcol = reinterpret_cast<int32_t*>(w + p.off_vcol);
+  float* vval = reinterpret_cast<float*>(w + p.off_vval);
+  int32_t* vcnt = reinterpret_cast<int32_t*>(w + p.off_vcnt);
+  int32_t* colcnt = reinterpret_cast<int32_t*>(w + p.off_colcnt);
+  int32_t* colptr = reinterpret_cast<int32_t*>(w + p.off_colptr);
+  int32_t* cursor = reinterpret_cast<int32_t*>(w + p.off_cursor);
+  int32_t* invrow = reinterpret_cast<int32_t*>(w + p.off_invrow);
+  float* invval = reinterpret_cast<float*>(w + p.off_invval);
+  // K4
+  if (k2 != 1) {
+    const size_t smem = size_t(p.cap_e_pow2) * 8;
+    IEEE_ENSURE_DYN_SMEM(rr_expand_kernel, smem);
+    rr_expand_kernel<<<N, 256, smem, stream>>>(rank, p.k1p, N, k2, p.cap_v, vcol, vval, vcnt, p.cap_e, p.cap_e_pow2,
+                                               reinterpret_cast<int32_t*>(w + p.off_ecol), reinterpret_cast<float*>(w + p.off_eval),
+                                               reinterpret_cast<int32_t*>(w + p.off_ecnt));
+    count_launch();
+  }
+  const SparseRows f = final_rows(p, w, k2);
+  // K5a
+  IEEE_CUDA_CHECK(cudaMemsetAsync(colcnt, 0, size_t(N) * 4, stream));
+  IEEE_CUDA_CHECK(cudaMemsetAsync(cursor, 0, size_t(N) * 4, stream));
+  rr_col_count_kernel<<<N, 128, 0, stream>>>(N, f.cap, f.col, f.val, f.cnt, colcnt);
+  count_launch();
+  rr_scan_kernel<<<1, 1024, 0, stream>>>(colcnt, N, colptr);
+  count_launch();
+  rr_col_fill_kernel<<<N, 128, 0, stream>>>(N, f.cap, f.col, f.val, f.cnt, colptr, cursor, invrow, invval);
+  count_launch();
+  return IEEE_OK;
+}
+
+// K5b + K6 for query rows [row0, row0 + rows), written to out (leading dim ldo)
+template <bool kBlock>
+static void launch_jaccard(const RerankPlan& p, uint8_t* w, int64_t Q, int64_t G, int k2, double lambda_value,
+                           const float* orig, const float* colmax, int64_t row0, int64_t rows, float* acc, int64_t ld_acc,
+                           float* out, int64_t ldo, cudaStream_t stream) {
+  const SparseRows f = final_rows(p, w, k2);
+  // (1 - lambda) is formed in double and rounded to float32 once, as NumPy does with the Python float
+  rr_jaccard_kernel<kBlock><<<(unsigned)rows, 256, 0, stream>>>(
+      (int)Q, (int)G, p.N, f.cap, f.col, f.val, f.cnt, reinterpret_cast<int32_t*>(w + p.off_colptr),
+      reinterpret_cast<int32_t*>(w + p.off_invrow), reinterpret_cast<float*>(w + p.off_invval), orig, colmax, (int)row0, acc,
+      ld_acc, (float)(1.0 - lambda_value), (float)lambda_value, out, ldo);
+  count_launch();
+}
+
 size_t rerank_workspace_bytes(int64_t Q, int64_t G, int32_t k1, int32_t k2) {
   if (Q <= 0 || G <= 0 || k1 < 1 || k2 < 1) return 0;
-  return make_plan(Q, G, k1, k2).total;
+  return make_plan(Q, G, k1, k2, true).total;
 }
 
 int rerank(const float* q_g, int64_t ld_qg, const float* q_q, int64_t ld_qq, const float* g_g, int64_t ld_gg, int64_t Q,
@@ -400,29 +532,19 @@ int rerank(const float* q_g, int64_t ld_qg, const float* q_q, int64_t ld_qq, con
   IEEE_REQUIRE(k1 >= 1 && k1 + 1 <= 512 && k2 >= 1 && k2 <= k1 + 1, "rerank: need 1 <= k2 <= k1 + 1 <= 512");
   IEEE_REQUIRE(k1 + 1 <= Q + G, "rerank: k1 + 1 exceeds the number of samples");
   IEEE_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "rerank: workspace must be 256-byte aligned");
-  const RerankPlan p = make_plan(Q, G, k1, k2);
+  const RerankPlan p = make_plan(Q, G, k1, k2, true);
   if (workspace_bytes < p.total) {
     set_error("rerank: workspace too small (%zu < %zu)", workspace_bytes, p.total);
     return IEEE_ERR_WORKSPACE;
   }
-  IEEE_REQUIRE((size_t)p.cap_e_pow2 * 8 <= 160 * 1024, "rerank: k2 * (k1+1) * (k1/2+2) = %d entries per row exceed the shared-memory sort", p.cap_e);
+  int rc = check_params("rerank", Q, G, k1, k2);
+  if (rc) return rc;
   uint8_t* w = static_cast<uint8_t*>(workspace);
   const int N = p.N;
   float* orig = reinterpret_cast<float*>(w + p.off_orig);
   float* colmax = reinterpret_cast<float*>(w + p.off_colmax);
   int32_t* rank = reinterpret_cast<int32_t*>(w + p.off_rank);
   float* rank_val = reinterpret_cast<float*>(w + p.off_rank_val);
-  int32_t* vcol = reinterpret_cast<int32_t*>(w + p.off_vcol);
-  float* vval = reinterpret_cast<float*>(w + p.off_vval);
-  int32_t* vcnt = reinterpret_cast<int32_t*>(w + p.off_vcnt);
-  int32_t* ecol = reinterpret_cast<int32_t*>(w + p.off_ecol);
-  float* eval = reinterpret_cast<float*>(w + p.off_eval);
-  int32_t* ecnt = reinterpret_cast<int32_t*>(w + p.off_ecnt);
-  int32_t* colcnt = reinterpret_cast<int32_t*>(w + p.off_colcnt);
-  int32_t* colptr = reinterpret_cast<int32_t*>(w + p.off_colptr);
-  int32_t* cursor = reinterpret_cast<int32_t*>(w + p.off_cursor);
-  int32_t* invrow = reinterpret_cast<int32_t*>(w + p.off_invrow);
-  float* invval = reinterpret_cast<float*>(w + p.off_invval);
 
   // K1
   IEEE_CUDA_CHECK(cudaMemsetAsync(colmax, 0, size_t(N) * 4, stream));
@@ -441,45 +563,175 @@ int rerank(const float* q_g, int64_t ld_qg, const float* q_q, int64_t ld_qq, con
   RawView raw{q_g, q_q, g_g, ld_qg, ld_qq, ld_gg, (int)Q, (int)G};
   {
     dim3 grid((N + 31) / 32, (N + 31) / 32);
-    rr_build_orig_kernel<<<grid, 256, 0, stream>>>(raw, N, colmax, orig);
+    rr_build_orig_kernel<<<grid, 256, 0, stream>>>(raw, N, N, colmax, orig, N);
     count_launch();
   }
   // K2: first k1+1 of each row's ascending (value, index) order
-  int rc = topk(orig, N, N, N, 0, nullptr, nullptr, nullptr, nullptr, p.k1p, rank, rank_val, stream);
+  rc = topk(orig, N, N, N, 0, nullptr, nullptr, nullptr, nullptr, p.k1p, rank, rank_val, stream);
   if (rc) return rc;
   // K3
   {
     const size_t smem = size_t(kRowWarps) * (p.k1p + p.khp + p.cap_v_pow2) * 4;
-    IEEE_ENSURE_DYN_SMEM(rr_krecip_kernel, smem);
-    rr_krecip_kernel<<<(N + kRowWarps - 1) / kRowWarps, 32 * kRowWarps, smem, stream>>>(rank, p.k1p, orig, N, p.k1p, p.khp,
-                                                                                         p.cap_v, p.cap_v_pow2, vcol, vval, vcnt);
+    IEEE_ENSURE_DYN_SMEM(rr_krecip_kernel<true>, smem);
+    rr_krecip_kernel<true><<<(N + kRowWarps - 1) / kRowWarps, 32 * kRowWarps, smem, stream>>>(
+        rank, p.k1p, orig, N, p.k1p, p.khp, p.cap_v, p.cap_v_pow2, reinterpret_cast<int32_t*>(w + p.off_vcol),
+        reinterpret_cast<float*>(w + p.off_vval), reinterpret_cast<int32_t*>(w + p.off_vcnt));
     count_launch();
   }
-  // K4
-  const int32_t* fcol = vcol;
-  const float* fval = vval;
-  const int32_t* fcnt = vcnt;
-  int fcap = p.cap_v;
-  if (k2 != 1) {
-    const size_t smem = size_t(p.cap_e_pow2) * 8;
-    IEEE_ENSURE_DYN_SMEM(rr_expand_kernel, smem);
-    rr_expand_kernel<<<N, 256, smem, stream>>>(rank, p.k1p, N, k2, p.cap_v, vcol, vval, vcnt, p.cap_e, p.cap_e_pow2, ecol, eval, ecnt);
-    count_launch();
-    fcol = ecol; fval = eval; fcnt = ecnt; fcap = p.cap_e;
+  // K4 + K5a
+  if ((rc = expand_and_index(p, w, rank, k2, stream))) return rc;
+  // K5b + K6
+  launch_jaccard<false>(p, w, Q, G, k2, lambda_value, orig, nullptr, 0, Q, out, ldo, out, ldo, stream);
+  IEEE_CUDA_CHECK(cudaGetLastError());
+  return IEEE_OK;
+}
+
+// ---- streamed form: orig in column strips of the virtual matrix, never all of it -------------------------------
+// A strip is raw[:, I] for |I| <= W columns, I inside the queries or inside the gallery and starting at a multiple of
+// W (a multiple of 256) of that operand's index: every contraction output is then computed at the same position
+// inside its tile (and its 128-column fix-up span) as in the whole-matrix products, so it has the same bits.
+// Strip scratch (a buffer of its own: only the prepare call needs it): top [Q, W], bot [max(W x Gp, G x W)], orig rows
+// [W, Np], top-k values [W, k1+1], the contraction's fix-up list.
+struct StripPlan {
+  int64_t W, Gp, Np;
+  size_t off_top, off_bot, off_orig, off_val, off_fix, total;
+};
+static StripPlan make_strip_plan(int64_t Q, int64_t G, int k1, size_t strip_bytes) {
+  StripPlan s;
+  s.Gp = round_up(G, 32);
+  s.Np = round_up(Q + G, 32);
+  const int64_t per_col = 4 * (Q + s.Gp + s.Np + k1 + 1);    // scratch bytes per strip column
+  const int64_t widest = round_up(Q > G ? Q : G, 256);
+  s.W = int64_t(strip_bytes / size_t(per_col)) / 256 * 256;
+  s.W = s.W < 256 ? 256 : (s.W > widest ? widest : s.W);
+  size_t o = 0;
+  auto take = [&](size_t bytes) { size_t r = o; o += align256(bytes); return r; };
+  s.off_top = take(size_t(Q) * s.W * 4);
+  s.off_bot = take(size_t(s.W) * s.Gp * 4);
+  s.off_orig = take(size_t(s.W) * s.Np * 4);
+  s.off_val = take(size_t(s.W) * (k1 + 1) * 4);
+  s.off_fix = take(distmat_fixup_bytes(Q > G ? Q : G));
+  s.total = o + 256;
+  return s;
+}
+
+size_t rerank_stream_workspace_bytes(int64_t Q, int64_t G, int32_t k1, int32_t k2) {
+  if (check_params("rerank_stream", Q, G, k1, k2) != IEEE_OK) return 0;
+  return make_plan(Q, G, k1, k2, false).total;
+}
+
+size_t rerank_stream_scratch_bytes(int64_t Q, int64_t G, int32_t k1, size_t strip_bytes) {
+  if (check_params("rerank_stream", Q, G, k1, 1) != IEEE_OK) return 0;
+  return make_strip_plan(Q, G, k1, strip_bytes).total;
+}
+
+int rerank_stream_prepare(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
+                          int precision, int32_t k1, int32_t k2, size_t strip_bytes, float* colmax, int32_t* rank,
+                          void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes, cudaStream_t stream,
+                          int cta_group) {
+  IEEE_REQUIRE(q_packed && g_packed && colmax && rank && workspace && scratch, "rerank_stream_prepare: null pointer");
+  IEEE_REQUIRE(D > 0, "rerank_stream_prepare: bad feature width D=%lld", (long long)D);
+  int rc = check_params("rerank_stream_prepare", Q, G, k1, k2);
+  if (rc) return rc;
+  IEEE_REQUIRE(metric == IEEE_METRIC_EUCLIDEAN || metric == IEEE_METRIC_COSINE, "rerank_stream_prepare: unknown metric %d", metric);
+  IEEE_REQUIRE(precision == IEEE_PREC_F16X3 || precision == IEEE_PREC_BF16,
+               "rerank_stream_prepare: precision %d has no tensor-core contraction", precision);
+  IEEE_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0 && (reinterpret_cast<uintptr_t>(scratch) & 255) == 0,
+               "rerank_stream_prepare: workspace and scratch must be 256-byte aligned");
+  const RerankPlan p = make_plan(Q, G, k1, k2, false);
+  const StripPlan s = make_strip_plan(Q, G, k1, strip_bytes);
+  if (workspace_bytes < p.total || scratch_bytes < s.total) {
+    set_error("rerank_stream_prepare: workspace or scratch too small (%zu < %zu or %zu < %zu)", workspace_bytes, p.total,
+              scratch_bytes, s.total);
+    return IEEE_ERR_WORKSPACE;
   }
-  // K5a
-  IEEE_CUDA_CHECK(cudaMemsetAsync(colcnt, 0, size_t(N) * 4, stream));
-  IEEE_CUDA_CHECK(cudaMemsetAsync(cursor, 0, size_t(N) * 4, stream));
-  rr_col_count_kernel<<<N, 128, 0, stream>>>(N, fcap, fcol, fval, fcnt, colcnt);
-  count_launch();
-  rr_scan_kernel<<<1, 1024, 0, stream>>>(colcnt, N, colptr);
-  count_launch();
-  rr_col_fill_kernel<<<N, 128, 0, stream>>>(N, fcap, fcol, fval, fcnt, colptr, cursor, invrow, invval);
-  count_launch();
-  // K5b + K6.  (1 - lambda) is formed in double and rounded to float32 once, as NumPy does with the Python float.
-  rr_jaccard_kernel<<<(unsigned)Q, 256, 0, stream>>>((int)Q, (int)G, N, fcap, fcol, fval, fcnt, colptr, invrow, invval, orig,
-                                                     (float)(1.0 - lambda_value), (float)lambda_value, out, ldo);
-  count_launch();
+  const int N = p.N;
+  uint8_t* w = static_cast<uint8_t*>(workspace);
+  uint8_t* sc = static_cast<uint8_t*>(scratch);
+  float* top = reinterpret_cast<float*>(sc + s.off_top);
+  float* bot = reinterpret_cast<float*>(sc + s.off_bot);
+  float* orig = reinterpret_cast<float*>(sc + s.off_orig);
+  float* val = reinterpret_cast<float*>(sc + s.off_val);
+  void* fix = sc + s.off_fix;
+  int32_t* vcol = reinterpret_cast<int32_t*>(w + p.off_vcol);
+  float* vval = reinterpret_cast<float*>(w + p.off_vval);
+  int32_t* vcnt = reinterpret_cast<int32_t*>(w + p.off_vcnt);
+  int* cm_bits = reinterpret_cast<int*>(colmax);
+  const int rpb = 256;
+  auto rows_of = [&](bool gallery, int64_t r0, int64_t n) {
+    return gallery ? packed_rows(g_packed, G, r0, n, D, precision) : packed_rows(q_packed, Q, r0, n, D, precision);
+  };
+  IEEE_CUDA_CHECK(cudaMemsetAsync(colmax, 0, size_t(N) * 4, stream));
+  // pass 0: column maxima, orig rows, top-k (K1, K2); pass 1: the same orig rows again, weights of V (K3)
+  for (int pass = 0; pass < 2; ++pass) {
+    if (pass == 1) {
+      // K3, membership: from rank alone, which pass 0 has completed
+      const size_t smem = size_t(kRowWarps) * (p.k1p + p.khp + p.cap_v_pow2) * 4;
+      IEEE_ENSURE_DYN_SMEM(rr_krecip_kernel<false>, smem);
+      rr_krecip_kernel<false><<<(N + kRowWarps - 1) / kRowWarps, 32 * kRowWarps, smem, stream>>>(
+          rank, p.k1p, nullptr, N, p.k1p, p.khp, p.cap_v, p.cap_v_pow2, vcol, vval, vcnt);
+      count_launch();
+    }
+    for (int seg = 0; seg < 2; ++seg) {         // strips of the queries, then of the gallery
+      const bool gal = seg == 1;
+      const int64_t n_seg = gal ? G : Q;
+      for (int64_t c0 = 0; c0 < n_seg; c0 += s.W) {
+        const int64_t wc = (n_seg - c0) < s.W ? (n_seg - c0) : s.W;
+        const int64_t i0 = (gal ? Q : 0) + c0;  // first row of orig (column of raw) in the strip
+        // the contraction calls of the whole-matrix products, with the same operand roles
+        if ((rc = distmat_umma_rows(rows_of(false, 0, Q), rows_of(gal, c0, wc), metric, precision, top, s.W, stream, cta_group,
+                                    fix, false)))
+          return rc;
+        if (!gal) rc = distmat_umma_rows(rows_of(false, c0, wc), rows_of(true, 0, G), metric, precision, bot, s.Gp, stream,
+                                         cta_group, fix, false);
+        else rc = distmat_umma_rows(rows_of(true, 0, G), rows_of(true, c0, wc), metric, precision, bot, s.W, stream, cta_group,
+                                    fix, false);
+        if (rc) return rc;
+        const StripView view{top, bot, s.W, gal ? s.W : s.Gp, (int)Q, !gal};
+        if (pass == 0) {
+          rr_colmax_kernel<<<dim3((unsigned)((wc + 255) / 256), (unsigned)((Q + rpb - 1) / rpb)), 256, 0, stream>>>(
+              top, s.W, (int)Q, (int)wc, rpb, cm_bits + i0);
+          if (!gal) rr_rowmax_kernel<<<(unsigned)wc, 256, 0, stream>>>(bot, s.Gp, (int)wc, (int)G, cm_bits + i0);
+          else rr_colmax_kernel<<<dim3((unsigned)((wc + 255) / 256), (unsigned)((G + rpb - 1) / rpb)), 256, 0, stream>>>(
+                   bot, s.W, (int)G, (int)wc, rpb, cm_bits + i0);
+          count_launch(2);
+        }
+        rr_build_orig_kernel<<<dim3((unsigned)((N + 31) / 32), (unsigned)((wc + 31) / 32)), 256, 0, stream>>>(
+            view, (int)wc, N, colmax + i0, orig, s.Np);
+        count_launch();
+        if (pass == 0) {
+          // K2 for the strip's rows
+          if ((rc = topk(orig, s.Np, wc, N, 0, nullptr, nullptr, nullptr, nullptr, p.k1p, rank + i0 * p.k1p, val, stream)))
+            return rc;
+        } else {
+          rr_weights_kernel<<<(unsigned)((wc + kRowWarps - 1) / kRowWarps), 32 * kRowWarps, 0, stream>>>(
+              orig, s.Np, (int)i0, (int)wc, p.cap_v, vcol, vval, vcnt);
+          count_launch();
+        }
+      }
+    }
+  }
+  if ((rc = expand_and_index(p, w, rank, k2, stream))) return rc;
+  IEEE_CUDA_CHECK(cudaGetLastError());
+  return IEEE_OK;
+}
+
+int rerank_stream_block(const void* workspace, int64_t Q, int64_t G, int32_t k1, int32_t k2, const float* colmax, int64_t row0,
+                        int64_t rows, double lambda_value, float* block, int64_t ld, void* scratch, size_t scratch_bytes,
+                        cudaStream_t stream) {
+  IEEE_REQUIRE(workspace && colmax && block && scratch, "rerank_stream_block: null pointer");
+  int rc = check_params("rerank_stream_block", Q, G, k1, k2);
+  if (rc) return rc;
+  IEEE_REQUIRE(row0 >= 0 && rows >= 0 && row0 + rows <= Q && ld >= G, "rerank_stream_block: bad block rows [%lld, %lld) of %lld, ld=%lld",
+               (long long)row0, (long long)(row0 + rows), (long long)Q, (long long)ld);
+  if (scratch_bytes < size_t(rows) * size_t(G) * 4) {
+    set_error("rerank_stream_block: scratch too small (%zu < %zu)", scratch_bytes, size_t(rows) * size_t(G) * 4);
+    return IEEE_ERR_WORKSPACE;
+  }
+  if (rows == 0) return IEEE_OK;
+  const RerankPlan p = make_plan(Q, G, k1, k2, false);
+  launch_jaccard<true>(p, static_cast<uint8_t*>(const_cast<void*>(workspace)), Q, G, k2, lambda_value, nullptr, colmax, row0, rows,
+                       static_cast<float*>(scratch), G, block, ld, stream);
   IEEE_CUDA_CHECK(cudaGetLastError());
   return IEEE_OK;
 }

@@ -218,17 +218,30 @@ class RetrievalEvaluator:
 
     ``gf, g_pids, g_camids`` are THIS rank's gallery slice (the whole gallery when ``group`` is None);
     ``g_offset`` its first global row and ``g_total`` the gallery size over all ranks.
+
+    ``rerank=True`` ranks k-reciprocal re-ranked distances (rerank.py:31-113 with ``k1``, ``k2``, ``lambda_value``)
+    instead of the plain ones, with the same bits as ``re_ranking`` on the three distance matrices, but without any
+    N x N matrix (N = queries + gallery): the re-ranking state is prepared from the features in column strips
+    (ieee_rerank_stream_prepare, strips sized by ``block_bytes``) and each query block's distances are re-ranked before
+    they are ranked.  The gallery must be on this one device (no ``group``, not ``from_host``).
     """
 
     def __init__(self, gf: torch.Tensor, g_pids, g_camids, dist_metric: str = "euclidean", normalize_feature: bool = False,
                  precision: str | None = None, max_rank: int = 20, group=None, g_offset: int = 0, g_total: int | None = None,
-                 block_bytes: int = DEFAULT_BLOCK_BYTES, center: torch.Tensor | None = None, exchange: str | None = None):
+                 block_bytes: int = DEFAULT_BLOCK_BYTES, center: torch.Tensor | None = None, exchange: str | None = None,
+                 rerank: bool = False, k1: int = 20, k2: int = 6, lambda_value: float = 0.3):
         _lib.require_cuda()
         if dist_metric not in _lib.METRICS:
             raise ValueError('Unknown distance metric: {}. Please choose either "euclidean" or "cosine"'.format(dist_metric))
         self.device = gf.device if gf is not None else torch.device("cuda", torch.cuda.current_device())
         self.metric, self.normalize = dist_metric, normalize_feature
         self.precision = precision or ("bf16" if gf is not None and gf.dtype == torch.bfloat16 else "f16x3")
+        self.rerank = bool(rerank)
+        if self.rerank:
+            self._check_rerank(gf, group, k1, k2)
+        self.k1, self.k2, self.lambda_value = k1, k2, float(lambda_value)
+        self._rr = None          # re-ranking state of the last query set (_rerank_prepare)
+        self._rr_scratch = None  # the blend's accumulators, one block
         self.max_rank = max_rank
         self.group = group
         self.world = 1 if group is None else torch.distributed.get_world_size(group)
@@ -265,6 +278,73 @@ class RetrievalEvaluator:
         self._host_gallery = None
         self._label_keys = (_tensor_key(g_pids), _tensor_key(g_camids))
         self._label_refs = (g_pids, g_camids)
+
+    def _check_rerank(self, gf, group, k1, k2):
+        if group is not None:
+            raise ValueError("rerank=True needs the whole gallery on one GPU: re-ranking over a sharded gallery (group) "
+                             "is not supported")
+        if gf is None:
+            raise ValueError("rerank=True needs the gallery features on the device: from_host streams them from the host")
+        if self.precision not in ("f16x3", "bf16"):
+            raise ValueError("rerank=True computes with the tensor-core precisions f16x3 and bf16, not {}".format(self.precision))
+        if not all(isinstance(k, (int, np.integer)) and not isinstance(k, bool) for k in (k1, k2)):
+            raise ValueError("rerank=True: k1 and k2 must be integers, got k1={!r} k2={!r}".format(k1, k2))
+        # the library's size query states its limits (k1 + 1 <= 512, k2 <= k1 + 1, the expansion's sort, N < 2^24), here
+        # for the fewest queries that give k1 + 1 samples; evaluate() checks k1 + 1 <= N with the real query count
+        G = max(gf.shape[0], 1)
+        if _lib.load().ieee_rerank_stream_workspace_bytes(max(1, k1 + 1 - G), G, k1, k2) == 0:
+            raise ValueError("rerank=True: " + _lib.load().ieee_last_error().decode())
+
+    def _rerank_prepare(self, qf: torch.Tensor):
+        """Re-ranking state of this query set (ieee_rerank_stream_prepare): kept while the same, unmodified query
+        tensor is evaluated again."""
+        k1, k2 = self.k1, self.k2
+        key = (_features_key(qf), k1, k2)
+        if self._rr is not None and self._rr["key"] == key:
+            return self._rr
+        # the previous state, the distance block and the blend's accumulators are free while the strips are computed:
+        # the block budget (block_bytes) then covers the strips, and later the block and its accumulators
+        self._rr = self._block = self._rr_scratch = None
+        Q, D = qf.shape
+        G = self.G
+        if k1 + 1 > Q + G:
+            raise ValueError("rerank=True: k1 + 1 = {} exceeds the {} query and gallery samples".format(k1 + 1, Q + G))
+        lib = _lib.load()
+        ws_bytes = lib.ieee_rerank_stream_workspace_bytes(Q, G, k1, k2)
+        sc_bytes = lib.ieee_rerank_stream_scratch_bytes(Q, G, k1, self.block_bytes)
+        if ws_bytes == 0 or sc_bytes == 0:
+            raise ValueError("rerank=True: " + lib.ieee_last_error().decode())
+        qpk = self._take_early_q(qf)
+        if qpk is None:
+            qpk = PackedFeatures(qf, self.metric, self.normalize, self.precision, self.center)
+        gpk = self.chunks[0][1]
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=self.device)
+        strips = torch.empty(sc_bytes, dtype=torch.uint8, device=self.device)    # released (stream-ordered) on return
+        colmax = torch.empty(Q + G, dtype=torch.float32, device=self.device)
+        rank = torch.empty((Q + G, k1 + 1), dtype=torch.int32, device=self.device)
+        _lib.call("ieee_rerank_stream_prepare", qpk.buf.data_ptr(), Q, gpk.buf.data_ptr(), G, D, qpk.metric, qpk.precision,
+                  k1, k2, self.block_bytes, colmax.data_ptr(), rank.data_ptr(), ws.data_ptr(), ws_bytes, strips.data_ptr(),
+                  sc_bytes, _lib.stream())
+        TRACE.mark("re-ranking state prepared")
+        # qf is kept so that its address cannot be reused by another tensor while the key refers to it; k1 and k2
+        # fix the workspace's layout, so the block calls take them from here
+        self._rr = {"key": key, "qf": qf, "Q": Q, "k1": k1, "k2": k2, "packed": qpk, "ws": ws, "colmax": colmax,
+                    "rank": rank}
+        return self._rr
+
+    def _rerank_block(self, dist: torch.Tensor, row0: int) -> torch.Tensor:
+        """Queries [row0, row0 + rows) of the prepared set: distances -> re-ranked distances, in place."""
+        rr = self._rr
+        rows = dist.shape[0]
+        if rows == 0:                            # (an empty query set has no state to blend with)
+            return dist
+        if self._rr_scratch is None or self._rr_scratch.numel() < rows * self.G:
+            self._rr_scratch = torch.empty(rows * self.G, dtype=torch.float32, device=self.device)
+        _lib.call("ieee_rerank_stream_block", rr["ws"].data_ptr(), rr["Q"], self.G, rr["k1"], rr["k2"], rr["colmax"].data_ptr(),
+                  row0, rows, self.lambda_value, dist.data_ptr(), dist.stride(0), self._rr_scratch.data_ptr(),
+                  4 * self._rr_scratch.numel(), _lib.stream())
+        TRACE.mark("  re-ranking blend")
+        return dist
 
     def _prepare_gallery(self, qf_dev):
         """ieee_gallery_prepare: grouping + [centre from the query rows] + packing of a device-resident gallery -- and
@@ -321,7 +401,9 @@ class RetrievalEvaluator:
 
     # -- one query block ---------------------------------------------------------------------------------
     def _block_rows_for(self, Q: int, G: int) -> int:
-        rows = max(128, int(self.block_bytes // (4 * max(G, 1))) // 128 * 128)
+        # re-ranking: the distance block and the blend's accumulators (as large) share the budget
+        budget = self.block_bytes // 2 if self.rerank else self.block_bytes
+        rows = max(128, int(budget // (4 * max(G, 1))) // 128 * 128)
         return min(Q, rows)
 
     def _block_rows(self, Q: int) -> int:
@@ -367,6 +449,8 @@ class RetrievalEvaluator:
             if Q == 0:
                 return idx, val
             self._ensure_center(qf)
+            if self.rerank:
+                self._rerank_prepare(qf)
             self._early_q = None          # (this path packs its query blocks itself: do not keep the early copy alive)
             if self._host_gallery is not None:
                 if self._copy is None:
@@ -381,6 +465,8 @@ class RetrievalEvaluator:
             for s in range(0, Q, rows):
                 e = min(Q, s + rows)
                 dist = self._distance_block(PackedFeatures(qf[s:e], self.metric, self.normalize, self.precision, self.center))
+                if self.rerank:
+                    self._rerank_block(dist, s)
                 loc_i = idx[s:e] if self.world == 1 else torch.empty((e - s, k_eff), dtype=torch.int32, device=self.device)
                 loc_v = val[s:e] if self.world == 1 else torch.empty((e - s, k_eff), dtype=torch.float32, device=self.device)
                 _lib.call("ieee_topk", dist.data_ptr(), dist.stride(0), e - s, self.G, self.g_offset,
@@ -579,10 +665,14 @@ class RetrievalEvaluator:
     def evaluate(self, qf: torch.Tensor, q_pids, q_camids, return_distmat: bool = False, use_cap_memo: bool = True,
                  one_call: bool | None = None):
         """Returns (cmc float32 ndarray [K'], mAP float, info dict).  Queries are replicated on every rank.
-        `qf` may live in (pinned) host memory: it is copied on the copy stream ahead of the gallery chunks."""
+        `qf` may live in (pinned) host memory: it is copied on the copy stream ahead of the gallery chunks.
+        On a re-ranking evaluator every query block's distances are re-ranked before they are ranked (and returned)."""
         if one_call is None:
             one_call = os.environ.get("IEEE_B200_ONE_CALL", "1") != "0"
         qf = _as_features(qf)
+        if self.rerank:
+            qf = qf.to(self.device)
+            one_call = False             # the one-call path has no re-ranking stage: the staged block loop does
         if qf.is_cuda:
             with torch.cuda.device(self.device):
                 if qf.shape[0] > 0:
@@ -608,7 +698,10 @@ class RetrievalEvaluator:
             # queries already in HBM: pack the first block before anything else, so the GPU is busy while the host
             # prepares the rest of the step
             early_pack = None
-            if qf.is_cuda:
+            if self.rerank and Q > 0:
+                rr = self._rerank_prepare(qf)
+                early_pack = rr["packed"] if rows >= Q else None
+            if qf.is_cuda and early_pack is None:
                 early_pack = self._take_early_q(qf) if rows >= Q else None
                 if early_pack is None:
                     early_pack = PackedFeatures(qf[: min(Q, rows)], self.metric, self.normalize, self.precision, self.center)
@@ -665,7 +758,8 @@ class RetrievalEvaluator:
             self._ensure_block(rows)
 
             def contraction(s, e):
-                return self._distance_block(qf_packed(s, e))
+                dist = self._distance_block(qf_packed(s, e))
+                return self._rerank_block(dist, s) if self.rerank else dist
 
             def qf_packed(s, e):
                 if s == 0 and early_pack is not None:

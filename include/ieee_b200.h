@@ -336,6 +336,34 @@ int ieee_rerank(const float* q_g, int64_t ld_qg, const float* q_q, int64_t ld_qq
                 void* workspace, size_t workspace_bytes, ieee_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * k-reciprocal re-ranking, streamed: the same result as ieee_rerank, computed from packed features (ieee_pack_features,
+ * both operands with the same centre) without any N x N or Q x Q matrix, N = Q + G.
+ *   ieee_rerank_stream_prepare computes the virtual matrix [[qq, qg], [qg^T, gg]] in column strips (of width
+ *   strip_bytes / ~8N, a multiple of 256 columns) twice with the contraction: the first pass yields the column
+ *   maxima `colmax` (float32 [N]) and the first k1 + 1 neighbours `rank` (int32 [N, k1 + 1]) of every sample, the second
+ *   the weights of the k-reciprocal sets.  The strips live in `scratch` (ieee_rerank_stream_scratch_bytes), which is
+ *   free again when the call's work on the stream is done.  The sparse state (V, its query expansion, the inverted
+ *   index) stays in `workspace` (ieee_rerank_stream_workspace_bytes, linear in N), which must outlive the block calls.
+ *   No host synchronisation.
+ *   ieee_rerank_stream_block turns the distances of queries [row0, row0 + rows) to the gallery (float32 [rows, G],
+ *   leading dim ld, as the contraction of those packed query rows against g_packed writes them) into their re-ranked
+ *   distances, in place; scratch holds rows * G floats.  Q, G, k1, k2 and colmax are those given to the prepare call.
+ * Bit-identical to ieee_rerank on the three matrices the contraction writes for the same packed operands.  Limits as
+ * ieee_rerank: k1 + 1 <= 512 and <= N, 1 <= k2 <= k1 + 1, k2 * (k1+1) * (round(k1/2)+2) <= 16384 entries per row,
+ * N < 2^24; precision F16X3 or BF16.  The size queries need no GPU and return 0 (with ieee_last_error set) when the
+ * parameters are out of range.
+ * ---------------------------------------------------------------------------------------------- */
+size_t ieee_rerank_stream_workspace_bytes(int64_t Q, int64_t G, int32_t k1, int32_t k2);
+size_t ieee_rerank_stream_scratch_bytes(int64_t Q, int64_t G, int32_t k1, size_t strip_bytes);
+int ieee_rerank_stream_prepare(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
+                               int precision, int32_t k1, int32_t k2, size_t strip_bytes, float* colmax, int32_t* rank,
+                               void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
+                               ieee_stream_t stream);
+int ieee_rerank_stream_block(const void* workspace, int64_t Q, int64_t G, int32_t k1, int32_t k2, const float* colmax,
+                             int64_t row0, int64_t rows, double lambda_value, float* block, int64_t ld, void* scratch,
+                             size_t scratch_bytes, ieee_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
  * GNN re-ranking (alternative `rerank` mode).   Replaces torchreid/utils/GPU-Re-Ranking/gnn_reranking.py:27-59 with its
  * extensions build_adjacency_matrix_kernel.cu:10-17 and gnn_propagate_kernel.cu:8-22.
  * neg_score: float32 [N, lds] = -(X_u X_u^T) over queries followed by gallery (ieee_distmat with IEEE_METRIC_NEG_DOT),
