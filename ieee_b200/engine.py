@@ -18,6 +18,7 @@ import torch
 
 from . import _lib
 from .metrics.rank import GalleryLabels, RankStages, _as_device, copy_stream, raise_for_status
+from .peer import link_for
 from .utils.rerank import re_ranking_device
 
 DEFAULT_BLOCK_BYTES = 4 << 30   # HBM scratch for one distance block
@@ -98,26 +99,33 @@ _ONE_CALL_POOL = {}
 _RESULT_HOST = {}
 
 
-def _result_buffer(device, nbytes):
-    """Pinned host landing zone for the (cmc, summary, stats) read-back of one evaluation."""
-    key = (str(device), nbytes)
-    buf = _RESULT_HOST.get(key)
-    if buf is None:
-        buf = _RESULT_HOST[key] = torch.empty(nbytes, dtype=torch.uint8, pin_memory=True)
-    return buf
-
-
 def _one_call_buffers(key, ws_bytes, res_bytes, device):
-    """Workspace, result block and its pinned host copy of a one-call evaluation, reused per key (stream-ordered like
-    the stage pool)."""
+    """Workspace and result block of a one-call evaluation, reused per key (stream-ordered like the stage pool).  The
+    result block is zeroed once, here: the one-GPU entry point never writes its stats words."""
     buf = _ONE_CALL_POOL.get(key)
     if buf is None:
         if len(_ONE_CALL_POOL) > 8:
             _ONE_CALL_POOL.clear()
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=device)
-        res = torch.empty(res_bytes, dtype=torch.uint8, device=device)
-        buf = _ONE_CALL_POOL[key] = (ws, res, torch.empty(res_bytes, dtype=torch.uint8, pin_memory=True))
+        buf = _ONE_CALL_POOL[key] = (ws, torch.zeros(res_bytes, dtype=torch.uint8, device=device))
     return buf
+
+
+def _read_result(res: torch.Tensor):
+    """One device->host copy of a result block [stats int64[4] | summary (64 B) | cmc float32[K']] into a pooled pinned
+    buffer, then a stream synchronise.  stats = [gather overflow = needed capacity (0: all lists fitted), tie pairs,
+    longest merged list, pad].  Returns ((overflow, longest), summary, cmc); the overflow is also taken from the
+    summary, where the one-GPU one-call entry point reports it."""
+    key = (str(res.device), res.numel())
+    host = _RESULT_HOST.get(key)
+    if host is None:
+        host = _RESULT_HOST[key] = torch.empty(res.numel(), dtype=torch.uint8, pin_memory=True)
+    host.copy_(res, non_blocking=True)
+    torch.cuda.current_stream().synchronize()
+    out = host.numpy()
+    overflow, _, longest = (int(v) for v in out[:32].view(np.int64)[:3])
+    summary = _lib.EvalSummary.from_buffer_copy(out[32:96].tobytes())
+    return (overflow or summary.list_overflow, longest), summary, out[96:].view(np.float32).copy()
 
 
 def _features_key(t: torch.Tensor):
@@ -168,15 +176,24 @@ class PackedFeatures:
             raise TypeError("PackedFeatures: features must be float32 or bfloat16, got {}".format(feats.dtype))
         if feats.stride(1) != 1:
             feats = feats.contiguous()
-        self.rows, self.D = feats.shape
-        self.metric, self.precision = _lib.METRICS[metric], _lib.PRECISIONS[precision]
-        self.center = center
-        lib = _lib.load()
-        self.buf = torch.empty(max(lib.ieee_packed_bytes(self.rows, self.D, self.precision), 256), dtype=torch.uint8,
-                               device=feats.device)
+        self._allocate(*feats.shape, metric, precision, center, feats.device)
         if self.rows:
             _lib.call("ieee_pack_features", feats.data_ptr(), _lib.DTYPES[feats.dtype], feats.stride(0), self.rows, self.D,
                       self.metric, int(normalize), self.precision, _lib.ptr(center), self.buf.data_ptr(), _lib.stream())
+
+    @classmethod
+    def _empty(cls, rows: int, D: int, metric: str, precision: str, center: torch.Tensor | None, device):
+        """The buffer of `rows` packed rows, left for the caller to fill (ieee_gallery_prepare)."""
+        pk = cls.__new__(cls)
+        pk._allocate(rows, D, metric, precision, center, device)
+        return pk
+
+    def _allocate(self, rows, D, metric, precision, center, device):
+        self.rows, self.D = rows, D
+        self.metric, self.precision = _lib.METRICS[metric], _lib.PRECISIONS[precision]
+        self.center = center
+        self.buf = torch.empty(max(_lib.load().ieee_packed_bytes(rows, D, self.precision), 256), dtype=torch.uint8,
+                               device=device)
 
 
 def packed_distmat(q: PackedFeatures, g: PackedFeatures, out: torch.Tensor) -> torch.Tensor:
@@ -355,11 +372,6 @@ class RetrievalEvaluator:
         if gf.stride(1) != 1:
             gf = self._gallery_dev = gf.contiguous()
         G, D = gf.shape
-        lib = _lib.load()
-        prec = _lib.PRECISIONS[self.precision]
-        pk = PackedFeatures.__new__(PackedFeatures)
-        pk.rows, pk.D, pk.metric, pk.precision = G, D, _lib.METRICS[self.metric], prec
-        pk.buf = torch.empty(max(lib.ieee_packed_bytes(G, D, prec), 256), dtype=torch.uint8, device=self.device)
         src, ws, qpk, flags = None, None, None, _lib.PREPARE_DEFER_JOIN
         if qf_dev is not None and qf_dev.shape[0] > 0:
             src = qf_dev if qf_dev.stride(1) == 1 else qf_dev.contiguous()
@@ -369,15 +381,13 @@ class RetrievalEvaluator:
         else:
             flags |= _lib.PREPARE_KEEP_CENTER
         center = self.center if self._use_center else None
-        pk.center = center
+        pk = PackedFeatures._empty(G, D, self.metric, self.precision, center, self.device)
         if src is not None and src.shape[0] <= self._block_rows_for(src.shape[0], G):
-            qpk = PackedFeatures.__new__(PackedFeatures)
-            qpk.rows, qpk.D, qpk.metric, qpk.precision, qpk.center = src.shape[0], D, pk.metric, prec, center
-            qpk.buf = torch.empty(max(lib.ieee_packed_bytes(src.shape[0], D, prec), 256), dtype=torch.uint8, device=self.device)
+            qpk = PackedFeatures._empty(src.shape[0], D, self.metric, self.precision, center, self.device)
             self._early_q = (_features_key(qf_dev), qpk)
         cur = torch.cuda.current_stream()
         _lib.call("ieee_gallery_prepare", gf.data_ptr(), gf.stride(0), _lib.DTYPES[gf.dtype], G, D, pk.metric, int(self.normalize),
-                  prec, self.labels.pids.data_ptr(), _lib.ptr(src), src.stride(0) if src is not None else 0,
+                  pk.precision, self.labels.pids.data_ptr(), _lib.ptr(src), src.stride(0) if src is not None else 0,
                   src.shape[0] if src is not None else 0, _lib.ptr(center), pk.buf.data_ptr(),
                   self.labels.group.data_ptr(), qpk.buf.data_ptr() if qpk is not None else None, flags, _lib.ptr(ws),
                   cur.cuda_stream)
@@ -429,6 +439,37 @@ class RetrievalEvaluator:
             TRACE.mark("  chunk %d contraction" % c0)
         return out
 
+    def _query_blocks(self, qf: torch.Tensor, rows: int, pack0: PackedFeatures | None = None, q_event=None):
+        """Iterates over (s, e, distances of queries [s, e)) in blocks of `rows`: each block is packed (block 0 may come
+        packed as `pack0`), after `q_event` when the queries are still being copied, contracted against every gallery
+        chunk and, on a re-ranking evaluator, re-ranked.  Block 0 is queued before this returns, so the caller can hide
+        host work behind its contraction; every later block when the iteration reaches it, in the same scratch."""
+        Q = qf.shape[0]
+        self._ensure_block(rows)
+
+        def block(s, e, qpk):
+            if qpk is None:
+                if q_event is not None:
+                    torch.cuda.current_stream().wait_event(q_event)
+                qpk = PackedFeatures(qf[s:e], self.metric, self.normalize, self.precision, self.center)
+            dist = self._distance_block(qpk)
+            return self._rerank_block(dist, s) if self.rerank else dist
+
+        dist0 = block(0, min(Q, rows), pack0)
+
+        def blocks():
+            for s in range(0, Q, rows):
+                e = min(Q, s + rows)
+                yield s, e, dist0 if s == 0 else block(s, e, None)
+        return blocks()
+
+    def _copy_stream(self) -> torch.cuda.Stream:
+        """The copy stream, ordered after the work queued on the compute stream so far."""
+        if self._copy is None:
+            self._copy = copy_stream(self.device)
+        self._copy.wait_stream(torch.cuda.current_stream())
+        return self._copy
+
     def ranked_lists(self, qf: torch.Tensor, q_pids=None, q_camids=None, k: int = 10):
         """First ``k`` entries of every query's junk-filtered ranked list over the WHOLE (possibly sharded) gallery --
         what ``visualize_ranked_results`` walks (torchreid/utils/reidtools.py:49,109-145).
@@ -453,20 +494,11 @@ class RetrievalEvaluator:
                 self._rerank_prepare(qf)
             self._early_q = None          # (this path packs its query blocks itself: do not keep the early copy alive)
             if self._host_gallery is not None:
-                if self._copy is None:
-                    self._copy = copy_stream(self.device)
-                self._copy.wait_stream(torch.cuda.current_stream())
-                self._start_gallery_copies(self._copy)
+                self._start_gallery_copies(self._copy_stream())
             qp = _as_device(q_pids, torch.int64, self.device) if masked else None
             qc = _as_device(q_camids, torch.int64, self.device) if masked else None
-            rows = self._block_rows(Q)
-            self._ensure_block(rows)
             self.labels.wait(torch.cuda.current_stream())
-            for s in range(0, Q, rows):
-                e = min(Q, s + rows)
-                dist = self._distance_block(PackedFeatures(qf[s:e], self.metric, self.normalize, self.precision, self.center))
-                if self.rerank:
-                    self._rerank_block(dist, s)
+            for s, e, dist in self._query_blocks(qf, self._block_rows(Q)):
                 loc_i = idx[s:e] if self.world == 1 else torch.empty((e - s, k_eff), dtype=torch.int32, device=self.device)
                 loc_v = val[s:e] if self.world == 1 else torch.empty((e - s, k_eff), dtype=torch.float32, device=self.device)
                 _lib.call("ieee_topk", dist.data_ptr(), dist.stride(0), e - s, self.G, self.g_offset,
@@ -556,65 +588,25 @@ class RetrievalEvaluator:
             self.chunks.append((c0, (ev, staged)))
         self._host_gallery = None
 
-    def _evaluate_one_call(self, qf, q_pids, q_camids, return_distmat, use_cap_memo):
-        """One GPU, gallery packed in HBM, queries in HBM, one distance block: the whole evaluation is ONE foreign
-        call (ieee_retrieve_eval_prepared enqueues pack -> contraction -> gather -> count -> metrics -> reduce back to
-        back from C) and one device->host copy of (cmc, summary)."""
-        with torch.cuda.device(self.device):
-            Q, D = qf.shape
-            if qf.stride(1) != 1:
-                qf = qf.contiguous()
-            qp = _as_device(q_pids, torch.int64, self.device)
-            qc = _as_device(q_camids, torch.int64, self.device)
-            memo_key = None
-            if use_cap_memo and self._label_keys[0] is not None and _tensor_key(q_pids) is not None:
-                memo_key = (self._label_keys, _tensor_key(q_pids), self.world)
-            cap = _CAP_MEMO.get(memo_key, (0, 0))[0] if memo_key is not None else 0
-            cur = torch.cuda.current_stream()
-            self.labels.wait(cur, join=False)
-            if cap <= 0:
-                # sizing pass: the capacity query synchronises once; later calls with the same labels skip it
-                cap = self.labels.list_cap(qp)
-                if memo_key is not None:
-                    _memo_put(memo_key, (cap, 0), (self._label_refs, q_pids))
-            k_eff = min(self.max_rank, self.g_total)
-            prec = _lib.PRECISIONS[self.precision]
-            res_off = (4 * k_eff + 7) // 8 * 8                  # [cmc float32[k_eff] | pad | ieee_eval_summary]
-            ws, res, res_host = _one_call_buffers((Q, D, prec, cap, k_eff, str(self.device)),
-                                                  _lib.load().ieee_retrieve_prepared_workspace_bytes(Q, D, prec, cap),
-                                                  res_off + C.sizeof(_lib.EvalSummary), self.device)
-            pitch = (self.G + 31) // 32 * 32
-            if self._block is None or self._block.shape[0] < Q:
-                self._block = torch.empty((Q, pitch), dtype=torch.float32, device=self.device)[:, : self.G]
-            ap = torch.empty(Q, dtype=torch.float64, device=self.device)
-            first = torch.empty(Q, dtype=torch.int32, device=self.device)
-            gpk = self.chunks[0][1]
-            qpk = self._take_early_q(qf)          # packed already by ieee_gallery_prepare (first evaluation of this gallery)
-            _lib.call("ieee_retrieve_eval_prepared", qf.data_ptr(), qf.stride(0), _lib.DTYPES[qf.dtype], Q, D,
-                      _lib.METRICS[self.metric], int(self.normalize), prec, gpk.buf.data_ptr(), self.labels.group.data_ptr(),
-                      _lib.ptr(self.center), self.G, qp.data_ptr(), qc.data_ptr(), self.labels.camids.data_ptr(), self.max_rank, cap, None,
-                      self._block.data_ptr(), self._block.stride(0), res.data_ptr(), res.data_ptr() + res_off,
-                      ap.data_ptr(), first.data_ptr(), qpk.buf.data_ptr() if qpk is not None else None, ws.data_ptr(), ws.numel(),
-                      cur.cuda_stream)
-            res_host.copy_(res, non_blocking=True)
-            cur.synchronize()
-            out = res_host.numpy()
-            cmc_host = out[: 4 * k_eff].view(np.float32).copy()
-            summary = _lib.EvalSummary.from_buffer_copy(out[res_off: res_off + 64].tobytes())
-        if summary.list_overflow:
-            _memo_drop(memo_key)                 # stale hint: size the lists again (exact value, so this ends)
-            return self._evaluate_one_call(qf, q_pids, q_camids, return_distmat, use_cap_memo)
-        raise_for_status(summary, self.max_rank)
-        info = {"num_valid": summary.num_valid, "num_ties": summary.num_ties, "cap": cap, "ap": ap, "first": first,
-                "mINP": float(summary.mINP)}
-        if return_distmat:
-            info["distmat"] = self._block[:Q].clone()
-        return cmc_host, float(summary.mAP), info
+    def _memo_key(self, q_pids):
+        """Key of these labels in the capacity memo; None when a label set is not a torch tensor (no identity to key on)."""
+        if self._label_keys[0] is None or _tensor_key(q_pids) is None:
+            return None
+        return (self._label_keys, _tensor_key(q_pids), self.world)
 
-    def _evaluate_one_call_peer(self, qf, q_pids, q_camids, return_distmat, cap, width, memo_key):
-        """Sharded gallery, sizes known from an earlier evaluation with the same labels: ONE foreign call enqueues the
-        whole step (ieee_retrieve_eval_prepared_peer) -- no collective launch, no host round trip before the result."""
-        from .peer import link_for
+    def _one_resident_block(self, qf: torch.Tensor) -> bool:
+        """Queries in HBM that make one block against a gallery packed in HBM as one chunk: what a one-call evaluation
+        takes."""
+        return (qf.is_cuda and self._host_gallery is None and len(self.chunks) == 1
+                and isinstance(self.chunks[0][1], PackedFeatures) and 0 < qf.shape[0] <= self._block_rows(qf.shape[0]))
+
+    def _evaluate_one_call(self, qf, q_pids, q_camids, return_distmat, memo_key, cap, width):
+        """One resident block: the whole evaluation is ONE foreign call, which enqueues pack -> contraction -> gather ->
+        count -> metrics -> reduce back to back from C, and one device->host copy of the result block.  On one GPU that
+        is ieee_retrieve_eval_prepared (cap <= 0: size the lists here first).  A sharded gallery takes
+        ieee_retrieve_eval_prepared_peer with the sizes an earlier evaluation with the same labels memoised: no
+        collective launch, no host round trip before the result."""
+        peer = self.world > 1
         with torch.cuda.device(self.device):
             lib = _lib.load()
             Q, D = qf.shape
@@ -622,75 +614,50 @@ class RetrievalEvaluator:
                 qf = qf.contiguous()
             qp = _as_device(q_pids, torch.int64, self.device)
             qc = _as_device(q_camids, torch.int64, self.device)
-            W = min(width, self.world * cap)
             k_eff = min(self.max_rank, self.g_total)
             prec = _lib.PRECISIONS[self.precision]
-            link = link_for(self.group, self.device, lib.ieee_peer_exchange_bytes(Q, Q, cap, W, self.world))
-            ex = link.descriptor(Q, Q, Q, 0, cap, W, link.next_epoch())
-            # [stats int64[3] | pad | ieee_eval_summary | cmc float32[k_eff]]
-            ws, res, res_host = _one_call_buffers(("peer", Q, D, prec, cap, k_eff, str(self.device)),
-                                                  lib.ieee_retrieve_prepared_peer_workspace_bytes(Q, D, prec, cap),
-                                                  32 + 64 + 4 * k_eff, self.device)
+            cur = torch.cuda.current_stream()
+            if peer:
+                entry, W = "ieee_retrieve_eval_prepared_peer", min(width, self.world * cap)
+                link = link_for(self.group, self.device, lib.ieee_peer_exchange_bytes(Q, Q, cap, W, self.world))
+                ex = link.descriptor(Q, Q, Q, 0, cap, W, link.next_epoch())
+                ws_bytes = lib.ieee_retrieve_prepared_peer_workspace_bytes(Q, D, prec, cap)
+            else:
+                entry, W = "ieee_retrieve_eval_prepared", 0          # (no merged lists on one GPU)
+                if cap <= 0:
+                    # sizing pass: the capacity query synchronises once; later calls with the same labels skip it
+                    cap = self.labels.list_cap(qp)
+                    if memo_key is not None:
+                        _memo_put(memo_key, (cap, 0), (self._label_refs, q_pids))
+                ws_bytes = lib.ieee_retrieve_prepared_workspace_bytes(Q, D, prec, cap)
+            ws, res = _one_call_buffers((entry, Q, D, prec, cap, k_eff, str(self.device)), ws_bytes, 96 + 4 * k_eff, self.device)
             self._ensure_block(Q)
-            # per-query results straight into fresh arrays (every rank derives all of them itself): nothing to copy out
-            # of the exchange buffer after the result has arrived, when the GPU would be idle
+            # per-query results straight into fresh arrays (with the peer exchange every rank derives all of them
+            # itself): nothing to copy out after the result has arrived, when the GPU would be idle
             ap = torch.empty(Q, dtype=torch.float64, device=self.device)
             first = torch.empty(Q, dtype=torch.int32, device=self.device)
-            cur = torch.cuda.current_stream()
             self.labels.wait(cur, join=False)
-            gpk = self.chunks[0][1]
-            qpk = self._take_early_q(qf)
-            _lib.call("ieee_retrieve_eval_prepared_peer", qf.data_ptr(), qf.stride(0), _lib.DTYPES[qf.dtype], Q, D,
-                      _lib.METRICS[self.metric], int(self.normalize), prec, gpk.buf.data_ptr(), self.labels.group.data_ptr(),
-                      _lib.ptr(self.center), self.G, self.g_total, self.g_offset, qp.data_ptr(), qc.data_ptr(),
-                      self.labels.camids.data_ptr(), self.max_rank, self._block.data_ptr(), self._block.stride(0),
-                      res.data_ptr() + 96, res.data_ptr() + 32, res.data_ptr(), ap.data_ptr(), first.data_ptr(), C.byref(ex),
-                      qpk.buf.data_ptr() if qpk is not None else None, ws.data_ptr(), ws.numel(), cur.cuda_stream)
-            res_host.copy_(res, non_blocking=True)
-            cur.synchronize()
-            out = res_host.numpy()
-            overflow, _, longest = (int(v) for v in out[:32].view(np.int64)[:3])
-            if overflow or longest > W:
-                _memo_drop(memo_key)             # sizes no longer fit these labels: size again, collectively
-                return self.evaluate(qf, q_pids, q_camids, return_distmat, use_cap_memo=False, one_call=False)
-            summary = _lib.EvalSummary.from_buffer_copy(out[32:96].tobytes())
-            cmc_host = out[96:].view(np.float32).copy()
-        raise_for_status(summary, self.max_rank)
-        info = {"num_valid": summary.num_valid, "num_ties": summary.num_ties, "cap": cap, "ap": ap, "first": first,
-                "mINP": float(summary.mINP)}
-        if return_distmat:
-            info["distmat"] = self._block[:Q].clone()
-        return cmc_host, float(summary.mAP), info
+            qpk = self._take_early_q(qf)          # packed already by ieee_gallery_prepare (first evaluation of this gallery)
+            queries = (qf.data_ptr(), qf.stride(0), _lib.DTYPES[qf.dtype], Q, D, _lib.METRICS[self.metric], int(self.normalize),
+                       prec, self.chunks[0][1].buf.data_ptr(), self.labels.group.data_ptr(), _lib.ptr(self.center), self.G)
+            rest = (qpk.buf.data_ptr() if qpk is not None else None, ws.data_ptr(), ws.numel(), cur.cuda_stream)
+            if peer:
+                _lib.call(entry, *queries, self.g_total, self.g_offset, qp.data_ptr(), qc.data_ptr(), self.labels.camids.data_ptr(),
+                          self.max_rank, self._block.data_ptr(), self._block.stride(0), res.data_ptr() + 96, res.data_ptr() + 32,
+                          res.data_ptr(), ap.data_ptr(), first.data_ptr(), C.byref(ex), *rest)
+            else:
+                _lib.call(entry, *queries, qp.data_ptr(), qc.data_ptr(), self.labels.camids.data_ptr(), self.max_rank, cap, None,
+                          self._block.data_ptr(), self._block.stride(0), res.data_ptr() + 96, res.data_ptr() + 32,
+                          ap.data_ptr(), first.data_ptr(), *rest)
+            (overflow, longest), summary, cmc = _read_result(res)
+        if overflow or longest > W:
+            return self._retry(qf, q_pids, q_camids, return_distmat, memo_key, cap, longest, one_call=True)
+        return self._result(summary, cmc, cap, ap, first, self._block[:Q].clone() if return_distmat else None)
 
-    def evaluate(self, qf: torch.Tensor, q_pids, q_camids, return_distmat: bool = False, use_cap_memo: bool = True,
-                 one_call: bool | None = None):
-        """Returns (cmc float32 ndarray [K'], mAP float, info dict).  Queries are replicated on every rank.
-        `qf` may live in (pinned) host memory: it is copied on the copy stream ahead of the gallery chunks.
-        On a re-ranking evaluator every query block's distances are re-ranked before they are ranked (and returned)."""
-        if one_call is None:
-            one_call = os.environ.get("IEEE_B200_ONE_CALL", "1") != "0"
-        qf = _as_features(qf)
-        if self.rerank:
-            qf = qf.to(self.device)
-            one_call = False             # the one-call path has no re-ranking stage: the staged block loop does
-        if qf.is_cuda:
-            with torch.cuda.device(self.device):
-                if qf.shape[0] > 0:
-                    self._ensure_center(qf)      # one foreign call: grouping, centre, gallery pack -- the GPU is busy from here on
-                elif self._gallery_dev is not None and not self.chunks:
-                    self._use_center = False     # no query rows to take a centre from (and nothing to compare against)
-                    self._prepare_gallery(None)
-        if (one_call and self.world == 1 and qf.is_cuda and self._host_gallery is None and len(self.chunks) == 1
-                and isinstance(self.chunks[0][1], PackedFeatures) and 0 < qf.shape[0] <= self._block_rows(qf.shape[0])):
-            return self._evaluate_one_call(qf, q_pids, q_camids, return_distmat, use_cap_memo)
-        if (one_call and use_cap_memo and self.world > 1 and self.exchange == "peer" and qf.is_cuda and self._host_gallery is None
-                and len(self.chunks) == 1 and isinstance(self.chunks[0][1], PackedFeatures)
-                and 0 < qf.shape[0] <= self._block_rows(qf.shape[0]) and self._label_keys[0] is not None
-                and _tensor_key(q_pids) is not None):
-            memo_key = (self._label_keys, _tensor_key(q_pids), self.world)
-            cap, width = _CAP_MEMO.get(memo_key, (None, 0))
-            if cap is not None and width > 0:
-                return self._evaluate_one_call_peer(qf, q_pids, q_camids, return_distmat, cap, width, memo_key)
+    def _evaluate_staged(self, qf, q_pids, q_camids, return_distmat, memo_key, cap, width):
+        """The query-block loop, stage by stage: any number of blocks, host queries and a host gallery, re-ranking, and
+        both exchanges of a sharded gallery.  cap <= 0: the capacity is queried behind block 0's contraction."""
+        import torch.distributed as dist_
         with torch.cuda.device(self.device):
             TRACE.mark("evaluate: start")
             Q = qf.shape[0]
@@ -711,37 +678,33 @@ class RetrievalEvaluator:
             qc = _as_device(q_camids, torch.int64, self.device)
             ids_ready = torch.cuda.current_stream().record_event()
             q_event = None
-            pending_gallery = getattr(self, "_host_gallery", None) is not None
-            if not qf.is_cuda or pending_gallery:
-                if self._copy is None:
-                    self._copy = copy_stream(self.device)
-                self._copy.wait_stream(torch.cuda.current_stream())
+            if not qf.is_cuda or self._host_gallery is not None:
+                copy = self._copy_stream()
                 if not qf.is_cuda:                       # queries first: every contraction needs them
                     if self.world > 1:
                         # the query set is the same on every rank: each copies 1/N of it over its own PCIe link and
                         # the slices are all-gathered over NVLink instead of N full host->device copies
-                        import torch.distributed as dist_
                         rank = dist_.get_rank(self.group)
                         per = (Q + self.world - 1) // self.world
                         q_all = torch.empty((self.world * per, qf.shape[1]), dtype=qf.dtype, device=self.device)
                         mine = q_all[rank * per: (rank + 1) * per]
                         lo, hi = min(Q, rank * per), min(Q, (rank + 1) * per)
-                        with torch.cuda.stream(self._copy):
+                        with torch.cuda.stream(copy):
                             if hi > lo:
                                 mine[: hi - lo].copy_(qf[lo:hi], non_blocking=True)
                             if hi - lo < per:
                                 mine[hi - lo:].zero_()
                             dist_.all_gather_into_tensor(q_all, mine, group=self.group)
-                            q_event = self._copy.record_event()
+                            q_event = copy.record_event()
                         qf = q_all[:Q]
                     else:
                         q_dev = torch.empty(qf.shape, dtype=qf.dtype, device=self.device)
-                        with torch.cuda.stream(self._copy):
+                        with torch.cuda.stream(copy):
                             q_dev.copy_(qf, non_blocking=True)
-                            q_event = self._copy.record_event()
+                            q_event = copy.record_event()
                         qf = q_dev
-                if pending_gallery:
-                    self._start_gallery_copies(self._copy)
+                if self._host_gallery is not None:
+                    self._start_gallery_copies(copy)
                 if q_event is not None and Q > 0:
                     # host queries: the centre comes from their device copy, before any chunk is packed
                     torch.cuda.current_stream().wait_event(q_event)
@@ -750,108 +713,101 @@ class RetrievalEvaluator:
             first = torch.empty(Q, dtype=torch.int32, device=self.device)
             short = torch.empty(Q, dtype=torch.int32, device=self.device)
             inp = torch.empty(Q, dtype=torch.float64, device=self.device)
-            # one result block = one device->host copy: [stats int64[4] | summary (64 B) | cmc float32[K']];
-            # stats = [gather overflow = needed capacity (int32, 0: all lists fitted), tie pairs, longest merged list, pad]
             k_eff = min(self.max_rank, self.g_total)
-            res = torch.zeros(32 + 64 + 4 * k_eff, dtype=torch.uint8, device=self.device)
-            ties = res[:32].view(torch.int64)
-            self._ensure_block(rows)
-
-            def contraction(s, e):
-                dist = self._distance_block(qf_packed(s, e))
-                return self._rerank_block(dist, s) if self.rerank else dist
-
-            def qf_packed(s, e):
-                if s == 0 and early_pack is not None:
-                    return early_pack
-                if q_event is not None:
-                    torch.cuda.current_stream().wait_event(q_event)
-                return PackedFeatures(qf[s:e], self.metric, self.normalize, self.precision, self.center)
-
-            memo_key = None
-            if use_cap_memo and self._label_keys[0] is not None and _tensor_key(q_pids) is not None:
-                memo_key = (self._label_keys, _tensor_key(q_pids), self.world)
-            cap, width = _CAP_MEMO.get(memo_key, (None, 0)) if memo_key is not None else (None, 0)
-            if cap is not None:
-                dist = contraction(0, min(Q, rows))
-                TRACE.mark("contraction(block 0) queued (capacity memo hit)")
-            else:
+            res = torch.zeros(96 + 4 * k_eff, dtype=torch.uint8, device=self.device)    # the kernels accumulate into it
+            ties, summ, cmc = res[:32].view(torch.int64), res[32:96], res[96:].view(torch.float32)
+            blocks = self._query_blocks(qf, rows, early_pack, q_event)
+            TRACE.mark("contraction(block 0) queued")
+            if cap <= 0:
                 # The contraction of the first block is queued FIRST; the capacity is then queried on a side stream
                 # that only waits for the gallery grouping and the query ids, so its host round trip (and the
                 # host-side allocations below) hide behind the tensor-core kernel.
-                dist = contraction(0, min(Q, rows))
-                TRACE.mark("contraction(block 0) queued")
                 cap_done, cap_host = self.labels.list_cap_async(qp, ids_ready)
                 cap_done.synchronize()
                 cap = max(int(cap_host.item()), 1)
                 if self.world > 1:
                     # every rank must size its lists alike for the all-gather (after the contraction: a NCCL kernel
                     # beside the persistent GEMM would take an SM pair away from a tile cluster)
-                    import torch.distributed as dist_
                     cap_t = torch.tensor([cap], dtype=torch.int32, device=self.device)
                     dist_.all_reduce(cap_t, op=dist_.ReduceOp.MAX, group=self.group)
                     cap = int(cap_t.item())
-            full = None
+            W = min(width, self.world * cap) if width > 0 else self.world * cap     # row width of the merged counts
             peer = self.world > 1 and self.exchange == "peer" and Q > 0
-            summ, cmc = res[32:96], res[96:].view(torch.float32)
+            full = torch.empty((Q, self.G), dtype=torch.float32, device=self.device) if return_distmat else None
             if peer:
-                from .peer import link_for
                 lib = _lib.load()
-                W = min(width, self.world * cap) if width > 0 else self.world * cap
                 link = link_for(self.group, self.device, lib.ieee_peer_exchange_bytes(rows, Q, cap, W, self.world))
                 stats = torch.zeros(4, dtype=torch.int64, device=self.device)      # this rank's own statistics
-                ex = None
-                for s in range(0, Q, rows):
-                    e = min(Q, s + rows)
-                    if s > 0:
-                        dist = contraction(s, e)
-                    ex = self._rank_block_peer(dist, qp[s:e], qc[s:e], link, rows, Q, s, cap, W, stats, cmc, summ, ties, k_eff)
-                    if return_distmat:
-                        full = dist.clone() if full is None else torch.cat([full, dist], 0)
-                TRACE.mark("rank stages done")
+            for s, e, dist in blocks:
+                if peer:
+                    self._rank_block_peer(dist, qp[s:e], qc[s:e], link, rows, Q, s, cap, W, stats, cmc, summ, ties, k_eff)
+                else:
+                    self._rank_block(dist, qp[s:e], qc[s:e], cap, width, ap[s:e], first[s:e], short[s:e], ties, inp[s:e])
+                if full is not None:
+                    full[s:e].copy_(dist)
+            if not peer and self.world > 1:
+                dist_.all_reduce(ties[:2], group=self.group)          # [2] (longest merged list) is the same on every rank
+            TRACE.mark("rank stages done")
+            if peer:
                 offs = [lib.ieee_peer_result_offset(i, rows, Q, cap, W, self.world) for i in (0, 1)]
                 ap = link.view[offs[0]: offs[0] + 8 * Q].view(torch.float64)       # every rank holds all per-query results
                 first = link.view[offs[1]: offs[1] + 4 * Q].view(torch.int32)
             else:
-                for s in range(0, Q, rows):
-                    e = min(Q, s + rows)
-                    if s > 0:
-                        dist = contraction(s, e)
-                    self._rank_block(dist, qp[s:e], qc[s:e], cap, width, ap[s:e], first[s:e], short[s:e], ties, inp[s:e])
-                    if return_distmat:
-                        full = dist.clone() if full is None else torch.cat([full, dist], 0)
-                if self.world > 1:
-                    import torch.distributed as dist_
-                    dist_.all_reduce(ties[:2], group=self.group)      # [2] (longest merged list) is the same on every rank
-                TRACE.mark("rank stages done")
                 _lib.call("ieee_rank_reduce", ap.data_ptr(), first.data_ptr(), short.data_ptr(), Q, k_eff, ties.data_ptr() + 8,
                           cmc.data_ptr(), summ.data_ptr(), inp.data_ptr(), _lib.stream())
             TRACE.mark("reduce done")
-            host = _result_buffer(self.device, res.numel())                    # pinned landing zone
-            host.copy_(res, non_blocking=True)
-            torch.cuda.current_stream().synchronize()
+            (overflow, longest), summary, cmc_host = _read_result(res)
             if peer:
                 ap, first = ap.clone(), first.clone()    # the exchange buffer is overwritten by the next evaluation
-            out = host.numpy()
-            overflow, _, longest = (int(v) for v in out[:32].view(np.int64)[:3])
-            summary = _lib.EvalSummary.from_buffer_copy(out[32:96].tobytes())
-            cmc_host = out[96:].view(np.float32).copy()
-            overflow = overflow or (longest > (width if width > 0 else self.world * cap))   # rows narrower than a merged list
-            if memo_key is not None and not overflow:
-                _memo_put(memo_key, (cap, max(longest, 1)), (self._label_refs, q_pids))
-        if overflow:
-            # a list did not fit the (memoised) capacity: forget the hint and run again with the exact value
-            if not use_cap_memo:
-                raise RuntimeError("ieee_b200: per-query lists overflowed an exactly sized buffer (cap=%d, longest=%d)" % (cap, longest))
-            _memo_drop(memo_key)
-            return self.evaluate(qf, q_pids, q_camids, return_distmat, use_cap_memo=False, one_call=one_call)
+        if overflow or longest > W:
+            return self._retry(qf, q_pids, q_camids, return_distmat, memo_key, cap, longest, one_call=False)
+        if memo_key is not None:
+            _memo_put(memo_key, (cap, max(longest, 1)), (self._label_refs, q_pids))
         TRACE.report()
+        return self._result(summary, cmc_host, cap, ap, first, full)
+
+    def _retry(self, qf, q_pids, q_camids, return_distmat, memo_key, cap, longest, one_call):
+        """A list did not fit the sizes the capacity memo held: forget them and evaluate again with exact ones.  The
+        one-GPU one-call route sizes exactly itself (and memoises the new capacity); every other route runs the
+        staged loop without the memo.  Exact sizes cannot overflow, so an overflow with them is an error."""
+        if memo_key is None:
+            raise RuntimeError("ieee_b200: per-query lists overflowed an exactly sized buffer (cap=%d, longest=%d)" % (cap, longest))
+        _memo_drop(memo_key)
+        if one_call and self.world == 1:
+            return self._evaluate_one_call(qf, q_pids, q_camids, return_distmat, memo_key, 0, 0)
+        return self.evaluate(qf, q_pids, q_camids, return_distmat, use_cap_memo=False, one_call=False)
+
+    def _result(self, summary, cmc, cap, ap, first, distmat):
         raise_for_status(summary, self.max_rank)
         info = {"num_valid": summary.num_valid, "num_ties": summary.num_ties, "cap": cap, "ap": ap, "first": first,
                 "mINP": float(summary.mINP)}
-        if return_distmat:
-            info["distmat"] = full
-        return cmc_host, float(summary.mAP), info
+        if distmat is not None:
+            info["distmat"] = distmat
+        return cmc, float(summary.mAP), info
+
+    def evaluate(self, qf: torch.Tensor, q_pids, q_camids, return_distmat: bool = False, use_cap_memo: bool = True,
+                 one_call: bool = True):
+        """Returns (cmc float32 ndarray [K'], mAP float, info dict).  Queries are replicated on every rank.
+        `qf` may live in (pinned) host memory: it is copied on the copy stream ahead of the gallery chunks.
+        On a re-ranking evaluator every query block's distances are re-ranked before they are ranked (and returned).
+        one_call=False runs the staged block loop where one foreign call could do the whole evaluation (same bits)."""
+        qf = _as_features(qf)
+        if self.rerank:
+            qf = qf.to(self.device)
+            one_call = False             # the one-call path has no re-ranking stage: the staged block loop does
+        if qf.is_cuda:
+            with torch.cuda.device(self.device):
+                if qf.shape[0] > 0:
+                    self._ensure_center(qf)      # one foreign call: grouping, centre, gallery pack -- the GPU is busy from here on
+                elif self._gallery_dev is not None and not self.chunks:
+                    self._use_center = False     # no query rows to take a centre from (and nothing to compare against)
+                    self._prepare_gallery(None)
+        memo_key = self._memo_key(q_pids) if use_cap_memo else None
+        cap, width = _CAP_MEMO.get(memo_key, (0, 0))
+        # one GPU: always one call; a sharded gallery: once the memo knows the row width the peer exchange needs
+        if one_call and self._one_resident_block(qf) and (self.world == 1 or self.exchange == "peer" and width > 0):
+            return self._evaluate_one_call(qf, q_pids, q_camids, return_distmat, memo_key, cap, width)
+        return self._evaluate_staged(qf, q_pids, q_camids, return_distmat, memo_key, cap, width)
 
 
 def result_lines(cmc, mAP, ranks=(1, 5, 10, 20)):

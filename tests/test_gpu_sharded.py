@@ -259,3 +259,72 @@ def test_two_gpu_nccl_evaluation():
     s = make_retrieval_set(500, 3001, 40, 4, dim=256, sigma=2.5, seed=17, distractor_frac=0.1)
     cmc_o, map_o = R.evaluate_rank(out["d"], s.q_pids, s.g_pids, s.q_camids, s.g_camids)
     assert np.array_equal(out["cmc"], cmc_o) and abs(out["mAP"] - map_o) < 1e-9
+
+
+def _peer_one_call_worker(rank, world, port, out):
+    import torch.distributed as dist
+    from ieee_b200 import engine
+    os.environ["MASTER_ADDR"], os.environ["MASTER_PORT"] = "127.0.0.1", str(port)
+    torch.cuda.set_device(rank)
+    dev = torch.device("cuda", rank)
+    dist.init_process_group("nccl", rank=rank, world_size=world, device_id=dev)
+    s = make_retrieval_set(500, 3001, 40, 4, dim=256, sigma=2.5, seed=17, distractor_frac=0.1)
+    g0, g1 = shard_bounds(3001, world, rank)
+    # label tensors (the capacity memo is keyed on tensor identity) and one query block (default block budget)
+    qp, qc = torch.from_numpy(s.q_pids).to(dev), torch.from_numpy(s.q_camids).to(dev)
+    gp, gc = torch.from_numpy(s.g_pids[g0:g1]).to(dev), torch.from_numpy(s.g_camids[g0:g1]).to(dev)
+    qf = s.qf.to(dev)
+    ev = RetrievalEvaluator(s.gf[g0:g1].to(dev), gp, gc, group=dist.group.WORLD, g_offset=g0, g_total=3001)
+    assert ev.exchange == "peer"
+    calls, real_call = [], _lib.call
+
+    def spy(name, *args):
+        calls.append(name)
+        return real_call(name, *args)
+
+    def run(evaluator):
+        calls.clear()
+        cmc, mAP, info = evaluator.evaluate(qf, qp, qc)
+        return (cmc, mAP, info["ap"], info["first"], info["mINP"], info["num_ties"]), list(calls)
+
+    def same(a, b):
+        assert np.array_equal(a[0], b[0]) and a[1] == b[1] and torch.equal(a[2], b[2]) and torch.equal(a[3], b[3])
+        assert a[4] == b[4] and a[5] == b[5]
+
+    _lib.call = spy
+    try:
+        staged, c1 = run(ev)                                  # sizes unknown: the staged loop with the peer exchange
+        assert "ieee_rank_gather_peer" in c1 and "ieee_retrieve_eval_prepared_peer" not in c1
+        key = [k for k in engine._CAP_MEMO if k[0] == ev._label_keys][0]
+        assert engine._CAP_MEMO[key][1] > 0                   # the row width is memoised
+        hit, c2 = run(ev)                                     # memo hit: the whole step in one call
+        assert "ieee_retrieve_eval_prepared_peer" in c2 and "ieee_rank_gather_peer" not in c2
+        same(staged, hit)
+        ev_n = RetrievalEvaluator(s.gf[g0:g1].to(dev), gp, gc, group=dist.group.WORLD, g_offset=g0, g_total=3001,
+                                  exchange="nccl", center=ev.center)
+        same(hit, run(ev_n)[0])
+        engine._CAP_MEMO[key] = (2, 0)          # capacity far too small, no width: the staged route overflows, runs again
+        poisoned, c3 = run(ev)
+        assert "ieee_retrieve_eval_prepared_peer" not in c3
+        same(hit, poisoned)
+        engine._CAP_MEMO[key] = (2, 1)          # with a width: the one call overflows and the staged route runs exactly
+        fallback, c4 = run(ev)
+        assert "ieee_retrieve_eval_prepared_peer" in c4 and "ieee_rank_gather_peer" in c4
+        same(hit, fallback)
+    finally:
+        _lib.call = real_call
+    out[rank] = True
+    dist.destroy_process_group()
+
+
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
+def test_two_gpu_peer_one_call_evaluation():
+    """The memoised one-call step of a sharded gallery (ieee_retrieve_eval_prepared_peer) against the staged peer loop
+    and the NCCL exchange, bit for bit, and its overflow fall-back to the staged loop."""
+    import torch.multiprocessing as mp
+    with socket.socket() as sk:
+        sk.bind(("127.0.0.1", 0))
+        port = sk.getsockname()[1]
+    out = mp.Manager().dict()
+    mp.spawn(_peer_one_call_worker, args=(2, port, out), nprocs=2, join=True)
+    assert dict(out) == {0: True, 1: True}
