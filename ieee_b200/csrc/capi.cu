@@ -123,6 +123,18 @@ int rerank_stream_block(const void* workspace, int64_t Q, int64_t G, int32_t k1,
 size_t gnn_rerank_workspace_bytes(int64_t N, int32_t k1);
 int gnn_rerank(const float* neg_score, int64_t lds, int64_t N, int32_t k1, int32_t k2, float* A, int64_t ldA, void* workspace,
                size_t workspace_bytes, cudaStream_t stream);
+size_t gnn_stream_scratch_bytes(int64_t Q, int64_t G, int32_t k1, size_t strip_bytes);
+int gnn_stream_neighbours(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int precision, int32_t k1,
+                          size_t strip_bytes, int32_t* rank, float* S, void* scratch, size_t scratch_bytes, cudaStream_t stream,
+                          int cta_group);
+int gnn_stream_graph_bytes_sync(const int32_t* rank, int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch,
+                                size_t scratch_bytes, int64_t* sizes, cudaStream_t stream);
+int gnn_stream_graph(const int32_t* rank, const float* S, int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch,
+                     size_t scratch_bytes, void* work, size_t work_bytes, const int64_t* sizes, int64_t* a_ptr, int32_t* a_col,
+                     float* a_val, int64_t* g_ptr, int32_t* g_row, float* g_val, cudaStream_t stream);
+int gnn_stream_block(const int64_t* a_ptr, const int32_t* a_col, const float* a_val, const int64_t* g_ptr, const int32_t* g_row,
+                     const float* g_val, int64_t Q, int64_t G, int64_t row0, int64_t rows, float* block, int64_t ld,
+                     void* scratch, size_t scratch_bytes, cudaStream_t stream);
 
 static int g_cta_group = -1;   // IEEE_B200_CTA_GROUP=1|2 overrides the default (2) pairing of the tensor-core kernel
 static int cta_group_default() {
@@ -743,6 +755,44 @@ int ieee_gnn_rerank(const float* neg_score, int64_t lds, int64_t N, int32_t k1, 
   int rc = check_device();
   if (rc) return rc;
   return gnn_rerank(neg_score, lds, N, k1, k2, A, ldA, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+size_t ieee_gnn_stream_scratch_bytes(int64_t Q, int64_t G, int32_t k1, size_t strip_bytes) {
+  return gnn_stream_scratch_bytes(Q, G, k1, strip_bytes);
+}
+
+int ieee_gnn_stream_neighbours(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int precision,
+                               int32_t k1, size_t strip_bytes, int32_t* rank, float* S, void* scratch, size_t scratch_bytes,
+                               ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return gnn_stream_neighbours(q_packed, Q, g_packed, G, D, precision, k1, strip_bytes, rank, S, scratch, scratch_bytes,
+                               (cudaStream_t)stream, cta_group_default());
+}
+
+int ieee_gnn_stream_graph_bytes_sync(const int32_t* rank, int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch,
+                                     size_t scratch_bytes, int64_t* sizes, ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return gnn_stream_graph_bytes_sync(rank, Q, G, k1, k2, scratch, scratch_bytes, sizes, (cudaStream_t)stream);
+}
+
+int ieee_gnn_stream_graph(const int32_t* rank, const float* S, int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch,
+                          size_t scratch_bytes, void* work, size_t work_bytes, const int64_t* sizes, int64_t* a_ptr,
+                          int32_t* a_col, float* a_val, int64_t* g_ptr, int32_t* g_row, float* g_val, ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return gnn_stream_graph(rank, S, Q, G, k1, k2, scratch, scratch_bytes, work, work_bytes, sizes, a_ptr, a_col, a_val, g_ptr,
+                          g_row, g_val, (cudaStream_t)stream);
+}
+
+int ieee_gnn_stream_block(const int64_t* a_ptr, const int32_t* a_col, const float* a_val, const int64_t* g_ptr,
+                          const int32_t* g_row, const float* g_val, int64_t Q, int64_t G, int64_t row0, int64_t rows,
+                          float* block, int64_t ld, void* scratch, size_t scratch_bytes, ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return gnn_stream_block(a_ptr, a_col, a_val, g_ptr, g_row, g_val, Q, G, row0, rows, block, ld, scratch, scratch_bytes,
+                          (cudaStream_t)stream);
 }
 
 // ---- peer exchange (gallery sharded over the GPUs of one box) ---------------------------------------------------

@@ -855,4 +855,627 @@ int gnn_rerank(const float* neg_score, int64_t lds, int64_t N, int32_t k1, int32
   return IEEE_OK;
 }
 
+// =========================================================================================================
+// GNN re-ranking, streamed: the same A as gnn_rerank, held sparse, from packed features without any N x N matrix.
+//   neighbours  -(X_u X_u^T) in row strips (queries, then gallery; W rows each) -> top-k1 `rank`, S = val^2
+//   symbolic    every structure below is decided by `rank` alone; one CTA per row counts it in a shared-memory bitmap
+//               of N bits from A0 = rank, its transpose T0 and K2inv (the transpose of the first k2 columns of rank):
+//                 B1[r] = A0[r] u T0[r]                 A1[i] = u_{j<k2} B1[rank[i, j]]
+//                 A1^T[r] = u_{m in B1[r]} K2inv[m]     B2[r] = A1[r] u A1^T[r]     A2[i] = u_{j<k2} B2[rank[i, j]]
+//               (A1^T[r]: r in A1[c] <=> some rank[c, j < k2] lies in B1[r], B1 being structurally symmetric)
+//   numeric     B = A + A^T, propagation and normalisation row by row into CSR rows with ascending columns, then the
+//               gallery rows of A2 as CSC (rows ascending).  Structural entries whose value is 0 are kept.
+// Every value has the dense kernels' bits: the dense sums skip nothing, but an absent entry adds fma(0, s, x) = x or
+// 0 + x = x, so summing only the present entries in the same order gives the same float.
+// =========================================================================================================
+constexpr int kGnnThreads = 256;           // also the residue classes of the normalisation (gnn_normalise_kernel)
+constexpr int64_t kGnnMaxN = int64_t(1) << 20;   // the per-row bitmap: N bits of shared memory
+
+struct SpRows {                            // CSR rows (idx = columns) or CSC columns (idx = rows); val == nullptr: all 1
+  const int64_t* ptr;
+  const int32_t* idx;
+  const float* val;
+  __device__ __forceinline__ float v(int64_t p) const { return val ? val[p] : 1.0f; }
+};
+
+__device__ __forceinline__ void bm_set(uint32_t* bm, int c) { atomicOr(bm + (c >> 5), 1u << (c & 31)); }
+
+__device__ void bm_clear(uint32_t* bm, int nw) {
+  __syncthreads();
+  for (int w = threadIdx.x; w < nw; w += kGnnThreads) bm[w] = 0u;
+  __syncthreads();
+}
+
+// exclusive scan of one int per thread; wsum: 8 ints of shared memory
+__device__ int block_excl_scan(int v, int* wsum) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  int incl = v;
+  for (int o = 1; o < 32; o <<= 1) {
+    const int y = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += y;
+  }
+  if (lane == 31) wsum[w] = incl;
+  __syncthreads();
+  int off = 0;
+  for (int x = 0; x < w; ++x) off += wsum[x];
+  __syncthreads();
+  return off + incl - v;
+}
+
+// number of set bits (every thread gets it)
+__device__ int bm_count(const uint32_t* bm, int nw, int* wsum) {
+  __syncthreads();
+  int n = 0;
+  for (int w = threadIdx.x; w < nw; w += kGnnThreads) n += __popc(bm[w]);
+  for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
+  if ((threadIdx.x & 31) == 0) wsum[threadIdx.x >> 5] = n;
+  __syncthreads();
+  int t = 0;
+  for (int x = 0; x < kGnnThreads / 32; ++x) t += wsum[x];
+  __syncthreads();
+  return t;
+}
+
+// the set bits in ascending order -> out[0, count); thread t owns a contiguous run of words
+__device__ void bm_emit(const uint32_t* bm, int nw, int32_t* out, int* wsum) {
+  __syncthreads();
+  const int per = (nw + kGnnThreads - 1) / kGnnThreads, w0 = threadIdx.x * per, w1 = min(nw, w0 + per);
+  int n = 0;
+  for (int w = w0; w < w1; ++w) n += __popc(bm[w]);
+  int pos = block_excl_scan(n, wsum);
+  for (int w = w0; w < w1; ++w)
+    for (uint32_t b = bm[w]; b; b &= b - 1) out[pos++] = w * 32 + __ffs(b) - 1;
+  __syncthreads();
+}
+
+// position of column c in the ascending run idx[lo, hi) (present by construction)
+__device__ __forceinline__ int64_t find_col(const int32_t* __restrict__ idx, int64_t lo, int64_t hi, int c) {
+  while (hi - lo > 1) {
+    const int64_t mid = (lo + hi) >> 1;
+    if (idx[mid] <= c) lo = mid; else hi = mid;
+  }
+  return lo;
+}
+
+// bits of row m of a sparse operand, by worker `id` of `nt`
+// (a top-k list pads with -1 only when a row has fewer than k1 candidates, which k1 <= N rules out; skipped anyway)
+__device__ __forceinline__ void set_row(uint32_t* bm, const SpRows& a, int m, int id, int nt) {
+  for (int64_t p = a.ptr[m] + id; p < a.ptr[m + 1]; p += nt)
+    if (a.idx[p] >= 0) bm_set(bm, a.idx[p]);
+}
+// B1[m] = A0[m] u T0[m]
+__device__ __forceinline__ void set_b1(uint32_t* bm, const SpRows& a0, const SpRows& t0, int m, int id, int nt) {
+  set_row(bm, a0, m, id, nt);
+  set_row(bm, t0, m, id, nt);
+}
+// A1[m] = u_{j<k2} B1[rank[m, j]]: one warp per j
+__device__ void set_a1(uint32_t* bm, const SpRows& a0, const SpRows& t0, int k2, int m) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  for (int j = w; j < k2; j += kGnnThreads / 32) {
+    const int x = a0.idx[a0.ptr[m] + j];
+    if (x >= 0) set_b1(bm, a0, t0, x, lane, 32);
+  }
+}
+// A1^T[m] = u_{x in B1[m]} K2inv[x]: one warp per x
+__device__ void set_a1t(uint32_t* bm, const SpRows& a0, const SpRows& t0, const SpRows& k2inv, int m) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int64_t na = a0.ptr[m + 1] - a0.ptr[m], nt = t0.ptr[m + 1] - t0.ptr[m];
+  for (int64_t u = w; u < na + nt; u += kGnnThreads / 32) {
+    const int x = u < na ? a0.idx[a0.ptr[m] + u] : t0.idx[t0.ptr[m] + u - na];
+    if (x >= 0) set_row(bm, k2inv, x, lane, 32);
+  }
+}
+
+// symbolic phase: per row the nnz of B1, A1, B2, A2
+__global__ void __launch_bounds__(kGnnThreads) gnn_symbolic_kernel(SpRows a0, SpRows t0, SpRows k2inv, int N, int k2,
+                                                                    int32_t* __restrict__ cnt_b1, int32_t* __restrict__ cnt_a1,
+                                                                    int32_t* __restrict__ cnt_b2, int32_t* __restrict__ cnt_a2) {
+  extern __shared__ __align__(16) uint32_t bm[];
+  __shared__ int wsum[kGnnThreads / 32];
+  const int r = blockIdx.x, nw = (N + 31) >> 5;
+  bm_clear(bm, nw);
+  set_b1(bm, a0, t0, r, threadIdx.x, kGnnThreads);
+  int n = bm_count(bm, nw, wsum);
+  if (threadIdx.x == 0) cnt_b1[r] = n;
+  bm_clear(bm, nw);
+  set_a1(bm, a0, t0, k2, r);
+  n = bm_count(bm, nw, wsum);
+  if (threadIdx.x == 0) cnt_a1[r] = n;
+  set_a1t(bm, a0, t0, k2inv, r);
+  n = bm_count(bm, nw, wsum);
+  if (threadIdx.x == 0) cnt_b2[r] = n;
+  bm_clear(bm, nw);
+  for (int j = 0; j < k2; ++j) {
+    const int m = a0.idx[a0.ptr[r] + j];
+    if (m < 0) continue;
+    set_a1(bm, a0, t0, k2, m);
+    set_a1t(bm, a0, t0, k2inv, m);
+  }
+  n = bm_count(bm, nw, wsum);
+  if (threadIdx.x == 0) cnt_a2[r] = n;
+}
+
+// B = A + A^T row by row: ascending columns of A[r] u T[r]; values (0 + A[r][c]) + A[c][r], which is the dense
+// A[r][c] + A[c][r] (gnn_symmetrise_kernel) for every pattern of presence
+__global__ void __launch_bounds__(kGnnThreads) gnn_sum_kernel(SpRows a, SpRows t, int N, const int64_t* __restrict__ bptr,
+                                                               int32_t* __restrict__ bcol, float* __restrict__ bval) {
+  extern __shared__ __align__(16) uint32_t bm[];
+  __shared__ int wsum[kGnnThreads / 32];
+  const int r = blockIdx.x, nw = (N + 31) >> 5;
+  const int64_t b0 = bptr[r], b1 = bptr[r + 1];
+  bm_clear(bm, nw);
+  set_row(bm, a, r, threadIdx.x, kGnnThreads);
+  if (t.ptr) set_row(bm, t, r, threadIdx.x, kGnnThreads);
+  bm_emit(bm, nw, bcol + b0, wsum);
+  for (int64_t p = b0 + threadIdx.x; p < b1; p += kGnnThreads) bval[p] = 0.f;
+  __syncthreads();
+  for (int64_t p = a.ptr[r] + threadIdx.x; p < a.ptr[r + 1]; p += kGnnThreads) {
+    if (a.idx[p] < 0) continue;
+    const int64_t q = find_col(bcol, b0, b1, a.idx[p]);
+    bval[q] = __fadd_rn(bval[q], a.v(p));
+  }
+  __syncthreads();
+  if (t.ptr)
+    for (int64_t p = t.ptr[r] + threadIdx.x; p < t.ptr[r + 1]; p += kGnnThreads) {
+      const int64_t q = find_col(bcol, b0, b1, t.idx[p]);
+      bval[q] = __fadd_rn(bval[q], t.v(p));
+    }
+}
+
+// A[i] = sum_{j<k2} S[i, j] * B[rank[i, j]] in j order (gnn_propagate_kernel's FFMA chain), then A[i] /= |A[i]|_2 in
+// gnn_normalise_kernel's order: thread t sums the squares of columns c = t (mod 256) in ascending order, then the same
+// shuffle tree, warp sum and square root
+__global__ void __launch_bounds__(kGnnThreads) gnn_propagate_rows_kernel(SpRows b, const int32_t* __restrict__ rank,
+                                                                          const float* __restrict__ S, int k1, int k2, int N,
+                                                                          const int64_t* __restrict__ aptr, int32_t* __restrict__ acol,
+                                                                          float* __restrict__ aval) {
+  extern __shared__ __align__(16) uint32_t bm[];
+  __shared__ int wsum[kGnnThreads / 32];
+  __shared__ int32_t chunk_c[kGnnThreads];
+  __shared__ float chunk_v[kGnnThreads];
+  __shared__ float red[kGnnThreads / 32];
+  __shared__ float nrm_s;
+  const int i = blockIdx.x, nw = (N + 31) >> 5;
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int64_t a0 = aptr[i], a1 = aptr[i + 1];
+  const int32_t* nb = rank + (int64_t)i * k1;
+  bm_clear(bm, nw);
+  for (int j = w; j < k2; j += kGnnThreads / 32)
+    if (nb[j] >= 0) set_row(bm, b, nb[j], lane, 32);
+  bm_emit(bm, nw, acol + a0, wsum);
+  for (int64_t p = a0 + threadIdx.x; p < a1; p += kGnnThreads) aval[p] = 0.f;
+  __syncthreads();
+  for (int j = 0; j < k2; ++j) {
+    const int m = nb[j];
+    if (m < 0) continue;
+    const float s = S[(int64_t)i * k1 + j];
+    for (int64_t p = b.ptr[m] + threadIdx.x; p < b.ptr[m + 1]; p += kGnnThreads) {
+      const int64_t q = find_col(acol, a0, a1, b.idx[p]);
+      aval[q] = __fmaf_rn(b.val[p], s, aval[q]);
+    }
+    __syncthreads();
+  }
+  float s = 0.f;
+  for (int64_t base = a0; base < a1; base += kGnnThreads) {
+    const int64_t p = base + threadIdx.x;
+    chunk_c[threadIdx.x] = p < a1 ? acol[p] : -1;
+    chunk_v[threadIdx.x] = p < a1 ? aval[p] : 0.f;
+    __syncthreads();
+    const int n = a1 - base < kGnnThreads ? (int)(a1 - base) : kGnnThreads;
+    for (int u = 0; u < n; ++u)
+      if ((chunk_c[u] & (kGnnThreads - 1)) == (int)threadIdx.x) s = __fmaf_rn(chunk_v[u], chunk_v[u], s);
+    __syncthreads();
+  }
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  if (lane == 0) red[w] = s;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float t = 0.f;
+    for (int x = 0; x < kGnnThreads / 32; ++x) t += red[x];
+    nrm_s = __fsqrt_rn(t);
+  }
+  __syncthreads();
+  const float nrm = nrm_s;
+  for (int64_t p = a0 + threadIdx.x; p < a1; p += kGnnThreads) aval[p] = __fdiv_rn(aval[p], nrm);
+}
+
+// transposes: entries of rows [r0, r1) counted per column, then placed (row - r_base, value) in any order
+__global__ void gnn_col_count_kernel(SpRows a, int r0, int r1, int32_t* __restrict__ cnt) {
+  const int r = r0 + blockIdx.x * (blockDim.x / 32) + (threadIdx.x >> 5);
+  if (r >= r1) return;
+  for (int64_t p = a.ptr[r] + (threadIdx.x & 31); p < a.ptr[r + 1]; p += 32) atomicAdd(cnt + a.idx[p], 1);
+}
+__global__ void gnn_col_fill_kernel(SpRows a, int r0, int r1, int r_base, const int64_t* __restrict__ tptr,
+                                    int32_t* __restrict__ cursor, int32_t* __restrict__ tidx, float* __restrict__ tval) {
+  const int r = r0 + blockIdx.x * (blockDim.x / 32) + (threadIdx.x >> 5);
+  if (r >= r1) return;
+  for (int64_t p = a.ptr[r] + (threadIdx.x & 31); p < a.ptr[r + 1]; p += 32) {
+    const int c = a.idx[p];
+    const int64_t q = tptr[c] + atomicAdd(cursor + c, 1);
+    tidx[q] = r - r_base;
+    if (tval) tval[q] = a.v(p);
+  }
+}
+// K2inv and the transpose of A0 straight from rank (columns j < kk of every row)
+__global__ void gnn_rank_count_kernel(const int32_t* __restrict__ rank, int64_t N, int k1, int kk, int32_t* __restrict__ cnt) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= N * kk) return;
+  const int64_t i = e / kk;
+  const int32_t c = rank[i * k1 + (e - i * kk)];
+  if (c >= 0) atomicAdd(cnt + c, 1);
+}
+__global__ void gnn_rank_fill_kernel(const int32_t* __restrict__ rank, int64_t N, int k1, int kk, const int64_t* __restrict__ tptr,
+                                     int32_t* __restrict__ cursor, int32_t* __restrict__ tidx) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= N * kk) return;
+  const int64_t i = e / kk;
+  const int32_t c = rank[i * k1 + (e - i * kk)];
+  if (c >= 0) tidx[tptr[c] + atomicAdd(cursor + c, 1)] = (int32_t)i;
+}
+// exclusive scan int32[n] -> int64[n + 1]; single CTA
+__global__ void __launch_bounds__(1024) gnn_scan64_kernel(const int32_t* __restrict__ in, int64_t n, int64_t* __restrict__ out) {
+  __shared__ long long wsum[32];
+  __shared__ long long carry;
+  if (threadIdx.x == 0) carry = 0;
+  __syncthreads();
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  for (int64_t base = 0; base < n; base += 1024) {
+    const int64_t i = base + threadIdx.x;
+    const long long v = i < n ? in[i] : 0;
+    long long incl = v;
+    for (int o = 1; o < 32; o <<= 1) {
+      const long long y = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += y;
+    }
+    if (lane == 31) wsum[w] = incl;
+    __syncthreads();
+    long long off = carry;
+    for (int x = 0; x < w; ++x) off += wsum[x];
+    if (i < n) out[i] = off + incl - v;
+    __syncthreads();
+    if (threadIdx.x == 1023) carry = off + incl;
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) out[n] = carry;
+}
+__global__ void gnn_iota_kernel(int64_t* __restrict__ ptr, int64_t n, int step) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i <= n) ptr[i] = i * step;
+}
+// the gallery CSC: each column's rows ascending (a bitmap of G bits), values looked up in the CSR rows
+__global__ void __launch_bounds__(kGnnThreads) gnn_col_sort_kernel(const int64_t* __restrict__ gptr, int32_t* __restrict__ grow,
+                                                                    float* __restrict__ gval, SpRows a, int Q, int G) {
+  extern __shared__ __align__(16) uint32_t bm[];
+  __shared__ int wsum[kGnnThreads / 32];
+  const int c = blockIdx.x, nw = (G + 31) >> 5;
+  const int64_t p0 = gptr[c], p1 = gptr[c + 1];
+  if (p0 == p1) return;
+  bm_clear(bm, nw);
+  for (int64_t p = p0 + threadIdx.x; p < p1; p += kGnnThreads) bm_set(bm, grow[p]);
+  bm_emit(bm, nw, grow + p0, wsum);
+  for (int64_t p = p0 + threadIdx.x; p < p1; p += kGnnThreads) {
+    const int r = Q + grow[p];
+    gval[p] = a.val[find_col(a.idx, a.ptr[r], a.ptr[r + 1], c)];
+  }
+}
+// -(A2[q] . A2[Q + g]) for queries [row0, row0 + rows): scattered through the gallery CSC, columns of A2[q] ascending,
+// into a float64 accumulator row (a product of two floats is exact in float64), rounded to float32 once
+__global__ void __launch_bounds__(kGnnThreads) gnn_block_kernel(SpRows a, SpRows gcsc, int G, int row0, double* __restrict__ acc_rows,
+                                                                 float* __restrict__ block, int64_t ld) {
+  const int q = row0 + blockIdx.x;
+  double* acc = acc_rows + (int64_t)blockIdx.x * G;
+  float* out = block + (int64_t)blockIdx.x * ld;
+  for (int g = threadIdx.x; g < G; g += kGnnThreads) acc[g] = 0.0;
+  __syncthreads();
+  for (int64_t p = a.ptr[q]; p < a.ptr[q + 1]; ++p) {
+    const int c = a.idx[p];
+    const double x = a.val[p];
+    for (int64_t e = gcsc.ptr[c] + threadIdx.x; e < gcsc.ptr[c + 1]; e += kGnnThreads) {
+      const int g = gcsc.idx[e];
+      acc[g] = __fma_rn(x, (double)gcsc.val[e], acc[g]);      // rows are distinct inside a column
+    }
+    __syncthreads();
+  }
+  for (int g = threadIdx.x; g < G; g += kGnnThreads) out[g] = -__double2float_rn(acc[g]);
+}
+
+static int gnn_stream_check(const char* who, int64_t Q, int64_t G, int32_t k1, int32_t k2) {
+  IEEE_REQUIRE(Q > 0 && G > 0, "%s: bad shape Q=%lld G=%lld", who, (long long)Q, (long long)G);
+  IEEE_REQUIRE(Q + G <= kGnnMaxN, "%s: N = Q + G = %lld exceeds %lld", who, (long long)(Q + G), (long long)kGnnMaxN);
+  IEEE_REQUIRE(k2 >= 1 && k2 <= k1 && k1 <= 1024, "%s: need 1 <= k2 <= k1 <= 1024, got k1=%d k2=%d", who, k1, k2);
+  IEEE_REQUIRE(k1 <= Q + G, "%s: k1 = %d exceeds the %lld query and gallery samples", who, k1, (long long)(Q + G));
+  return IEEE_OK;
+}
+
+// Scratch of the neighbour and graph calls (one buffer, used by one phase after the other): the strips [W, ld] with
+// their top-k values, or the index both graph calls share (A0's row offsets, T0, K2inv, per-row counts and offsets).
+struct GnnScratch {
+  int64_t N, W, ld;
+  size_t off_strip, off_val, strips;
+  size_t off_a0p, off_t0p, off_t0i, off_k2p, off_k2i, off_cnt, off_cursor, off_cntr[4], off_ptr[4], off_tot, index;
+  size_t total;
+};
+static GnnScratch gnn_scratch_plan(int64_t Q, int64_t G, int k1, size_t strip_bytes) {
+  GnnScratch s;
+  s.N = Q + G;
+  s.ld = round_up(s.N, 32);
+  const int64_t per_row = 4 * (s.ld + k1);
+  const int64_t widest = round_up(Q > G ? Q : G, 256);
+  s.W = int64_t(strip_bytes / size_t(per_row)) / 256 * 256;
+  s.W = s.W < 256 ? 256 : (s.W > widest ? widest : s.W);
+  size_t o = 0;
+  auto take = [&](size_t bytes) { size_t r = o; o += align256(bytes); return r; };
+  s.off_strip = take(size_t(s.W) * s.ld * 4);
+  s.off_val = take(size_t(s.W) * k1 * 4);
+  s.strips = o;
+  o = 0;
+  const size_t N = s.N, p8 = (N + 1) * 8;
+  s.off_a0p = take(p8);
+  s.off_t0p = take(p8);
+  s.off_t0i = take(N * k1 * 4);
+  s.off_k2p = take(p8);
+  s.off_k2i = take(N * k1 * 4);
+  s.off_cnt = take(N * 4);
+  s.off_cursor = take(N * 4);
+  for (int x = 0; x < 4; ++x) s.off_cntr[x] = take(N * 4);
+  for (int x = 0; x < 4; ++x) s.off_ptr[x] = take(p8);
+  s.off_tot = take(64);
+  s.index = o;
+  s.total = (s.strips > s.index ? s.strips : s.index) + 256;
+  return s;
+}
+
+size_t gnn_stream_scratch_bytes(int64_t Q, int64_t G, int32_t k1, size_t strip_bytes) {
+  if (gnn_stream_check("gnn_stream", Q, G, k1, 1) != IEEE_OK) return 0;
+  return gnn_scratch_plan(Q, G, k1, strip_bytes).total;
+}
+
+int gnn_stream_neighbours(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int precision, int32_t k1,
+                          size_t strip_bytes, int32_t* rank, float* S, void* scratch, size_t scratch_bytes, cudaStream_t stream,
+                          int cta_group) {
+  IEEE_REQUIRE(q_packed && g_packed && rank && S && scratch, "gnn_stream_neighbours: null pointer");
+  IEEE_REQUIRE(D > 0, "gnn_stream_neighbours: bad feature width D=%lld", (long long)D);
+  int rc = gnn_stream_check("gnn_stream_neighbours", Q, G, k1, 1);
+  if (rc) return rc;
+  IEEE_REQUIRE(precision == IEEE_PREC_F16X3 || precision == IEEE_PREC_BF16,
+               "gnn_stream_neighbours: precision %d has no tensor-core contraction", precision);
+  IEEE_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 255) == 0, "gnn_stream_neighbours: scratch must be 256-byte aligned");
+  const GnnScratch s = gnn_scratch_plan(Q, G, k1, strip_bytes);
+  if (scratch_bytes < s.total) {
+    set_error("gnn_stream_neighbours: scratch too small (%zu < %zu)", scratch_bytes, s.total);
+    return IEEE_ERR_WORKSPACE;
+  }
+  uint8_t* sc = static_cast<uint8_t*>(scratch);
+  float* strip = reinterpret_cast<float*>(sc + s.off_strip);
+  float* val = reinterpret_cast<float*>(sc + s.off_val);
+  const int64_t N = Q + G;
+  auto rows_of = [&](bool gallery, int64_t r0, int64_t n) {
+    return gallery ? packed_rows(g_packed, G, r0, n, D, precision) : packed_rows(q_packed, Q, r0, n, D, precision);
+  };
+  // NEG_DOT has no centre and no near-duplicate fix-up, so an output's bits do not depend on where it sits in its
+  // tile: the strips give the bits of the whole -(X_u X_u^T) product
+  for (int seg = 0; seg < 2; ++seg) {
+    const bool gal = seg == 1;
+    const int64_t n_seg = gal ? G : Q;
+    for (int64_t r0 = 0; r0 < n_seg; r0 += s.W) {
+      const int64_t wr = (n_seg - r0) < s.W ? (n_seg - r0) : s.W;
+      const int64_t i0 = (gal ? Q : 0) + r0;
+      if ((rc = distmat_umma_rows(rows_of(gal, r0, wr), rows_of(false, 0, Q), IEEE_METRIC_NEG_DOT, precision, strip, s.ld, stream,
+                                  cta_group, nullptr, false)))
+        return rc;
+      if ((rc = distmat_umma_rows(rows_of(gal, r0, wr), rows_of(true, 0, G), IEEE_METRIC_NEG_DOT, precision, strip + Q, s.ld,
+                                  stream, cta_group, nullptr, false)))
+        return rc;
+      if ((rc = topk(strip, s.ld, wr, N, 0, nullptr, nullptr, nullptr, nullptr, k1, rank + i0 * k1, val, stream))) return rc;
+      const int64_t nk = wr * k1;
+      gnn_square_kernel<<<(unsigned)((nk + 255) / 256), 256, 0, stream>>>(val, S + i0 * k1, nk);
+      count_launch();
+    }
+  }
+  IEEE_CUDA_CHECK(cudaGetLastError());
+  return IEEE_OK;
+}
+
+// The index of the graph calls, and the offsets of the numeric phase's work buffer (B1, A1, A1^T, B2).
+struct GnnIndex {
+  int64_t *a0p, *t0p, *k2p, *ptr[4], *tot;     // ptr: B1, A1, B2, A2
+  int32_t *t0i, *k2i, *cnt, *cursor, *cntr[4];
+};
+static GnnIndex gnn_index(const GnnScratch& s, void* scratch) {
+  uint8_t* b = static_cast<uint8_t*>(scratch);
+  GnnIndex x;
+  x.a0p = reinterpret_cast<int64_t*>(b + s.off_a0p);
+  x.t0p = reinterpret_cast<int64_t*>(b + s.off_t0p);
+  x.k2p = reinterpret_cast<int64_t*>(b + s.off_k2p);
+  x.t0i = reinterpret_cast<int32_t*>(b + s.off_t0i);
+  x.k2i = reinterpret_cast<int32_t*>(b + s.off_k2i);
+  x.cnt = reinterpret_cast<int32_t*>(b + s.off_cnt);
+  x.cursor = reinterpret_cast<int32_t*>(b + s.off_cursor);
+  for (int i = 0; i < 4; ++i) {
+    x.cntr[i] = reinterpret_cast<int32_t*>(b + s.off_cntr[i]);
+    x.ptr[i] = reinterpret_cast<int64_t*>(b + s.off_ptr[i]);
+  }
+  x.tot = reinterpret_cast<int64_t*>(b + s.off_tot);
+  return x;
+}
+struct GnnWork {
+  size_t off_b1c, off_b1v, off_a1c, off_a1v, off_tp, off_ti, off_tv, off_b2c, off_b2v, total;
+};
+static GnnWork gnn_work_plan(int64_t N, int k2, int64_t nb1, int64_t na1, int64_t nb2) {
+  GnnWork w{};
+  size_t o = 0;
+  auto take = [&](size_t bytes) { size_t r = o; o += align256(bytes); return r; };
+  if (k2 != 1) {
+    w.off_b1c = take(size_t(nb1) * 4);
+    w.off_b1v = take(size_t(nb1) * 4);
+    w.off_a1c = take(size_t(na1) * 4);
+    w.off_a1v = take(size_t(na1) * 4);
+    w.off_tp = take(size_t(N + 1) * 8);
+    w.off_ti = take(size_t(na1) * 4);
+    w.off_tv = take(size_t(na1) * 4);
+    w.off_b2c = take(size_t(nb2) * 4);
+    w.off_b2v = take(size_t(nb2) * 4);
+  }
+  w.total = o + 256;
+  return w;
+}
+
+static size_t gnn_bitmap_smem(int64_t n) { return size_t((n + 31) / 32) * 4; }
+
+// counts per column of rank[:, :kk] -> offsets, then the rows of every column (any order)
+static int gnn_rank_transpose(const int32_t* rank, int64_t N, int k1, int kk, const GnnIndex& x, int64_t* tptr, int32_t* tidx,
+                              cudaStream_t stream) {
+  const int64_t nk = N * kk;
+  IEEE_CUDA_CHECK(cudaMemsetAsync(x.cnt, 0, size_t(N) * 4, stream));
+  IEEE_CUDA_CHECK(cudaMemsetAsync(x.cursor, 0, size_t(N) * 4, stream));
+  gnn_rank_count_kernel<<<(unsigned)((nk + 255) / 256), 256, 0, stream>>>(rank, N, k1, kk, x.cnt);
+  gnn_scan64_kernel<<<1, 1024, 0, stream>>>(x.cnt, N, tptr);
+  gnn_rank_fill_kernel<<<(unsigned)((nk + 255) / 256), 256, 0, stream>>>(rank, N, k1, kk, tptr, x.cursor, tidx);
+  count_launch(3);
+  return IEEE_OK;
+}
+// rows [r0, r1) of `a` -> CSC (row indices relative to r_base) with values
+static int gnn_sparse_transpose(const SpRows& a, int64_t N, int r0, int r1, int r_base, const GnnIndex& x, int64_t* tptr,
+                                int32_t* tidx, float* tval, cudaStream_t stream) {
+  IEEE_CUDA_CHECK(cudaMemsetAsync(x.cnt, 0, size_t(N) * 4, stream));
+  IEEE_CUDA_CHECK(cudaMemsetAsync(x.cursor, 0, size_t(N) * 4, stream));
+  const unsigned blocks = (unsigned)((r1 - r0 + 7) / 8);
+  if (blocks) gnn_col_count_kernel<<<blocks, 256, 0, stream>>>(a, r0, r1, x.cnt);
+  gnn_scan64_kernel<<<1, 1024, 0, stream>>>(x.cnt, N, tptr);
+  if (blocks) gnn_col_fill_kernel<<<blocks, 256, 0, stream>>>(a, r0, r1, r_base, tptr, x.cursor, tidx, tval);
+  count_launch(3);
+  return IEEE_OK;
+}
+
+int gnn_stream_graph_bytes_sync(const int32_t* rank, int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch,
+                                size_t scratch_bytes, int64_t* sizes, cudaStream_t stream) {
+  IEEE_REQUIRE(rank && scratch && sizes, "gnn_stream_graph_bytes_sync: null pointer");
+  int rc = gnn_stream_check("gnn_stream_graph_bytes_sync", Q, G, k1, k2);
+  if (rc) return rc;
+  IEEE_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 255) == 0, "gnn_stream_graph_bytes_sync: scratch must be 256-byte aligned");
+  const GnnScratch s = gnn_scratch_plan(Q, G, k1, 0);
+  if (scratch_bytes < s.index) {
+    set_error("gnn_stream_graph_bytes_sync: scratch too small (%zu < %zu)", scratch_bytes, s.index);
+    return IEEE_ERR_WORKSPACE;
+  }
+  const int64_t N = Q + G;
+  const GnnIndex x = gnn_index(s, scratch);
+  int64_t tot[4] = {N * k1, N * k1, N * k1, N * k1};     // nnz of B1, A1, B2, A2 (k2 == 1: A2 = A0)
+  int64_t nnz_gal = G * k1;
+  if (k2 != 1) {
+    gnn_iota_kernel<<<(unsigned)((N + 256) / 256), 256, 0, stream>>>(x.a0p, N, k1);
+    count_launch();
+    if ((rc = gnn_rank_transpose(rank, N, k1, k1, x, x.t0p, x.t0i, stream))) return rc;
+    if ((rc = gnn_rank_transpose(rank, N, k1, k2, x, x.k2p, x.k2i, stream))) return rc;
+    const SpRows a0{x.a0p, rank, nullptr}, t0{x.t0p, x.t0i, nullptr}, k2inv{x.k2p, x.k2i, nullptr};
+    const size_t smem = gnn_bitmap_smem(N);
+    IEEE_ENSURE_DYN_SMEM(gnn_symbolic_kernel, smem);
+    gnn_symbolic_kernel<<<(unsigned)N, kGnnThreads, smem, stream>>>(a0, t0, k2inv, (int)N, k2, x.cntr[0], x.cntr[1], x.cntr[2],
+                                                                     x.cntr[3]);
+    count_launch();
+    for (int i = 0; i < 4; ++i) {
+      gnn_scan64_kernel<<<1, 1024, 0, stream>>>(x.cntr[i], N, x.ptr[i]);
+      count_launch();
+    }
+    int64_t host[5];
+    for (int i = 0; i < 4; ++i) IEEE_CUDA_CHECK(cudaMemcpyAsync(host + i, x.ptr[i] + N, 8, cudaMemcpyDeviceToHost, stream));
+    IEEE_CUDA_CHECK(cudaMemcpyAsync(host + 4, x.ptr[3] + Q, 8, cudaMemcpyDeviceToHost, stream));
+    IEEE_CUDA_CHECK(cudaStreamSynchronize(stream));
+    for (int i = 0; i < 4; ++i) tot[i] = host[i];
+    nnz_gal = host[3] - host[4];
+  }
+  IEEE_REQUIRE(tot[3] < (int64_t(1) << 40), "gnn_stream_graph_bytes_sync: nnz overflow");
+  sizes[0] = tot[3];
+  sizes[1] = nnz_gal;
+  sizes[2] = (int64_t)gnn_work_plan(N, k2, tot[0], tot[1], tot[2]).total;
+  sizes[3] = tot[0];
+  sizes[4] = tot[1];
+  sizes[5] = tot[2];
+  return IEEE_OK;
+}
+
+int gnn_stream_graph(const int32_t* rank, const float* S, int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch,
+                     size_t scratch_bytes, void* work, size_t work_bytes, const int64_t* sizes, int64_t* a_ptr, int32_t* a_col,
+                     float* a_val, int64_t* g_ptr, int32_t* g_row, float* g_val, cudaStream_t stream) {
+  IEEE_REQUIRE(rank && S && scratch && work && sizes && a_ptr && a_col && a_val && g_ptr && g_row && g_val,
+               "gnn_stream_graph: null pointer");
+  int rc = gnn_stream_check("gnn_stream_graph", Q, G, k1, k2);
+  if (rc) return rc;
+  IEEE_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 255) == 0 && (reinterpret_cast<uintptr_t>(work) & 255) == 0,
+               "gnn_stream_graph: scratch and work must be 256-byte aligned");
+  const int64_t N = Q + G;
+  const GnnScratch s = gnn_scratch_plan(Q, G, k1, 0);
+  const GnnWork wp = gnn_work_plan(N, k2, sizes[3], sizes[4], sizes[5]);
+  if (scratch_bytes < s.index || work_bytes < wp.total) {
+    set_error("gnn_stream_graph: scratch or work too small (%zu < %zu or %zu < %zu)", scratch_bytes, s.index, work_bytes, wp.total);
+    return IEEE_ERR_WORKSPACE;
+  }
+  const GnnIndex x = gnn_index(s, scratch);
+  const size_t smem = gnn_bitmap_smem(N);
+  uint8_t* w = static_cast<uint8_t*>(work);
+  if (k2 == 1) {
+    // A2 = A0: the neighbour lists with ascending columns, all values 1
+    gnn_iota_kernel<<<(unsigned)((N + 256) / 256), 256, 0, stream>>>(a_ptr, N, k1);
+    count_launch();
+    IEEE_ENSURE_DYN_SMEM(gnn_sum_kernel, smem);
+    gnn_sum_kernel<<<(unsigned)N, kGnnThreads, smem, stream>>>(SpRows{a_ptr, rank, nullptr}, SpRows{nullptr, nullptr, nullptr},
+                                                               (int)N, a_ptr, a_col, a_val);
+    count_launch();
+  } else {
+    int32_t* b1c = reinterpret_cast<int32_t*>(w + wp.off_b1c);
+    float* b1v = reinterpret_cast<float*>(w + wp.off_b1v);
+    int32_t* a1c = reinterpret_cast<int32_t*>(w + wp.off_a1c);
+    float* a1v = reinterpret_cast<float*>(w + wp.off_a1v);
+    int64_t* tp = reinterpret_cast<int64_t*>(w + wp.off_tp);
+    int32_t* ti = reinterpret_cast<int32_t*>(w + wp.off_ti);
+    float* tv = reinterpret_cast<float*>(w + wp.off_tv);
+    int32_t* b2c = reinterpret_cast<int32_t*>(w + wp.off_b2c);
+    float* b2v = reinterpret_cast<float*>(w + wp.off_b2v);
+    IEEE_ENSURE_DYN_SMEM(gnn_sum_kernel, smem);
+    IEEE_ENSURE_DYN_SMEM(gnn_propagate_rows_kernel, smem);
+    // B1 = A0 + A0^T, A1 = P(B1)
+    gnn_sum_kernel<<<(unsigned)N, kGnnThreads, smem, stream>>>(SpRows{x.a0p, rank, nullptr}, SpRows{x.t0p, x.t0i, nullptr}, (int)N,
+                                                               x.ptr[0], b1c, b1v);
+    gnn_propagate_rows_kernel<<<(unsigned)N, kGnnThreads, smem, stream>>>(SpRows{x.ptr[0], b1c, b1v}, rank, S, k1, k2, (int)N,
+                                                                          x.ptr[1], a1c, a1v);
+    count_launch(2);
+    // B2 = A1 + A1^T, A2 = P(B2)
+    const SpRows a1{x.ptr[1], a1c, a1v};
+    if ((rc = gnn_sparse_transpose(a1, N, 0, (int)N, 0, x, tp, ti, tv, stream))) return rc;
+    gnn_sum_kernel<<<(unsigned)N, kGnnThreads, smem, stream>>>(a1, SpRows{tp, ti, tv}, (int)N, x.ptr[2], b2c, b2v);
+    IEEE_CUDA_CHECK(cudaMemcpyAsync(a_ptr, x.ptr[3], size_t(N + 1) * 8, cudaMemcpyDeviceToDevice, stream));
+    gnn_propagate_rows_kernel<<<(unsigned)N, kGnnThreads, smem, stream>>>(SpRows{x.ptr[2], b2c, b2v}, rank, S, k1, k2, (int)N,
+                                                                          a_ptr, a_col, a_val);
+    count_launch(2);
+  }
+  // the gallery rows of A2 as CSC, rows ascending
+  const SpRows a2{a_ptr, a_col, a_val};
+  if ((rc = gnn_sparse_transpose(a2, N, (int)Q, (int)N, (int)Q, x, g_ptr, g_row, nullptr, stream))) return rc;
+  const size_t gsmem = gnn_bitmap_smem(G);
+  IEEE_ENSURE_DYN_SMEM(gnn_col_sort_kernel, gsmem);
+  gnn_col_sort_kernel<<<(unsigned)N, kGnnThreads, gsmem, stream>>>(g_ptr, g_row, g_val, a2, (int)Q, (int)G);
+  count_launch();
+  IEEE_CUDA_CHECK(cudaGetLastError());
+  return IEEE_OK;
+}
+
+int gnn_stream_block(const int64_t* a_ptr, const int32_t* a_col, const float* a_val, const int64_t* g_ptr, const int32_t* g_row,
+                     const float* g_val, int64_t Q, int64_t G, int64_t row0, int64_t rows, float* block, int64_t ld,
+                     void* scratch, size_t scratch_bytes, cudaStream_t stream) {
+  IEEE_REQUIRE(a_ptr && a_col && a_val && g_ptr && g_row && g_val && block && scratch, "gnn_stream_block: null pointer");
+  IEEE_REQUIRE(Q > 0 && G > 0 && Q + G <= kGnnMaxN, "gnn_stream_block: bad shape Q=%lld G=%lld", (long long)Q, (long long)G);
+  IEEE_REQUIRE(row0 >= 0 && rows >= 0 && row0 + rows <= Q && ld >= G, "gnn_stream_block: bad block rows [%lld, %lld) of %lld, ld=%lld",
+               (long long)row0, (long long)(row0 + rows), (long long)Q, (long long)ld);
+  if (scratch_bytes < size_t(rows) * size_t(G) * 8) {
+    set_error("gnn_stream_block: scratch too small (%zu < %zu)", scratch_bytes, size_t(rows) * size_t(G) * 8);
+    return IEEE_ERR_WORKSPACE;
+  }
+  if (rows == 0) return IEEE_OK;
+  gnn_block_kernel<<<(unsigned)rows, kGnnThreads, 0, stream>>>(SpRows{a_ptr, a_col, a_val}, SpRows{g_ptr, g_row, g_val}, (int)G,
+                                                                (int)row0, static_cast<double*>(scratch), block, ld);
+  count_launch();
+  IEEE_CUDA_CHECK(cudaGetLastError());
+  return IEEE_OK;
+}
+
 }  // namespace ieee

@@ -190,7 +190,8 @@ class PackedFeatures:
 
     def _allocate(self, rows, D, metric, precision, center, device):
         self.rows, self.D = rows, D
-        self.metric, self.precision = _lib.METRICS[metric], _lib.PRECISIONS[precision]
+        self.metric = _lib.METRICS[metric] if metric in _lib.METRICS else _lib.INTERNAL_METRICS[metric]
+        self.precision = _lib.PRECISIONS[precision]
         self.center = center
         self.buf = torch.empty(max(_lib.load().ieee_packed_bytes(rows, D, self.precision), 256), dtype=torch.uint8,
                                device=device)
@@ -236,24 +237,40 @@ class RetrievalEvaluator:
     ``gf, g_pids, g_camids`` are THIS rank's gallery slice (the whole gallery when ``group`` is None);
     ``g_offset`` its first global row and ``g_total`` the gallery size over all ranks.
 
-    ``rerank=True`` ranks k-reciprocal re-ranked distances (rerank.py:31-113 with ``k1``, ``k2``, ``lambda_value``)
-    instead of the plain ones, with the same bits as ``re_ranking`` on the three distance matrices, but without any
-    N x N matrix (N = queries + gallery): the re-ranking state is prepared from the features in column strips
-    (ieee_rerank_stream_prepare, strips sized by ``block_bytes``) and each query block's distances are re-ranked before
-    they are ranked.  The gallery must be on this one device (no ``group``, not ``from_host``).
+    ``rerank=True`` ranks k-reciprocal re-ranked distances (rerank.py:31-113 with ``k1``, ``k2``, ``lambda_value``;
+    k1, k2 default to 20, 6) instead of the plain ones, with the same bits as ``re_ranking`` on the three distance
+    matrices, but without any N x N matrix (N = queries + gallery): the re-ranking state is prepared from the features
+    in column strips (ieee_rerank_stream_prepare, strips sized by ``block_bytes``) and each query block's distances are
+    re-ranked before they are ranked.  The gallery must be on this one device (no ``group``, not ``from_host``).
+
+    ``rerank="gnn"`` ranks the GNN re-ranked similarity (gnn_reranking.py:27-59; k1, k2 default to 26, 7, the reference
+    driver's values), negated so that it ranks as a distance: what ``gnn_reranking_distmat`` computes on the
+    evaluator's features.  The score is X X^T of the features after ``normalize_feature``, packed with the negative dot
+    product and no centre; ``dist_metric`` and ``lambda_value`` are not used.  The adjacency is held sparse
+    (ieee_gnn_stream_*: neighbours from row strips sized by ``block_bytes``, then A as CSR rows and an inverted index of
+    its gallery rows), and a query block's distances come from it instead of a contraction.  Same limits on the
+    gallery as ``rerank=True``; 1 <= k2 <= k1 <= min(N, 1024).
     """
 
     def __init__(self, gf: torch.Tensor, g_pids, g_camids, dist_metric: str = "euclidean", normalize_feature: bool = False,
                  precision: str | None = None, max_rank: int = 20, group=None, g_offset: int = 0, g_total: int | None = None,
                  block_bytes: int = DEFAULT_BLOCK_BYTES, center: torch.Tensor | None = None, exchange: str | None = None,
-                 rerank: bool = False, k1: int = 20, k2: int = 6, lambda_value: float = 0.3):
+                 rerank: bool | str = False, k1: int | None = None, k2: int | None = None, lambda_value: float = 0.3):
         _lib.require_cuda()
         if dist_metric not in _lib.METRICS:
             raise ValueError('Unknown distance metric: {}. Please choose either "euclidean" or "cosine"'.format(dist_metric))
+        if isinstance(rerank, str) and rerank != "gnn":
+            raise ValueError('rerank must be False, True or "gnn", got {!r}'.format(rerank))
         self.device = gf.device if gf is not None else torch.device("cuda", torch.cuda.current_device())
-        self.metric, self.normalize = dist_metric, normalize_feature
+        self.gnn = rerank == "gnn"
+        # GNN re-ranking scores with the negative dot product whatever the distance metric (gnn_reranking.py:31)
+        self.metric, self.normalize = ("neg_dot" if self.gnn else dist_metric), normalize_feature
         self.precision = precision or ("bf16" if gf is not None and gf.dtype == torch.bfloat16 else "f16x3")
         self.rerank = bool(rerank)
+        if k1 is None:
+            k1 = 26 if self.gnn else 20
+        if k2 is None:
+            k2 = 7 if self.gnn else 6
         if self.rerank:
             self._check_rerank(gf, group, k1, k2)
         self.k1, self.k2, self.lambda_value = k1, k2, float(lambda_value)
@@ -274,7 +291,7 @@ class RetrievalEvaluator:
         # queries are replicated on every rank of a sharded gallery, so all shards -- and a single-GPU evaluation of
         # the same queries -- derive the same vector without exchanging anything.  The gallery is therefore packed
         # on the first evaluate(), or here when the caller hands a centre in.
-        self._use_center = centering_applies(dist_metric, self.precision)
+        self._use_center = not self.gnn and centering_applies(dist_metric, self.precision)
         self.center = center
         self._gallery_dev = gf
         # the gallery as packed row chunks [(first row, PackedFeatures)]: one chunk when the features are already
@@ -297,15 +314,25 @@ class RetrievalEvaluator:
         self._label_refs = (g_pids, g_camids)
 
     def _check_rerank(self, gf, group, k1, k2):
+        mode = 'rerank="gnn"' if self.gnn else "rerank=True"
         if group is not None:
-            raise ValueError("rerank=True needs the whole gallery on one GPU: re-ranking over a sharded gallery (group) "
-                             "is not supported")
+            raise ValueError("{} needs the whole gallery on one GPU: re-ranking over a sharded gallery (group) "
+                             "is not supported".format(mode))
         if gf is None:
-            raise ValueError("rerank=True needs the gallery features on the device: from_host streams them from the host")
+            raise ValueError("{} needs the gallery features on the device: from_host streams them from the host".format(mode))
         if self.precision not in ("f16x3", "bf16"):
-            raise ValueError("rerank=True computes with the tensor-core precisions f16x3 and bf16, not {}".format(self.precision))
+            raise ValueError("{} computes with the tensor-core precisions f16x3 and bf16, not {}".format(mode, self.precision))
         if not all(isinstance(k, (int, np.integer)) and not isinstance(k, bool) for k in (k1, k2)):
-            raise ValueError("rerank=True: k1 and k2 must be integers, got k1={!r} k2={!r}".format(k1, k2))
+            raise ValueError("{}: k1 and k2 must be integers, got k1={!r} k2={!r}".format(mode, k1, k2))
+        if self.gnn:
+            if not 1 <= k2 <= k1 <= 1024:
+                raise ValueError('rerank="gnn" needs 1 <= k2 <= k1 <= min(N, 1024), got k1={} k2={}'.format(k1, k2))
+            # the library's size query states the other limits (N <= 2^20), here for the fewest queries that give k1
+            # samples; the first evaluate() checks k1 <= N with the real query count
+            G = max(gf.shape[0], 1)
+            if _lib.load().ieee_gnn_stream_scratch_bytes(max(1, k1 - G), G, k1, 0) == 0:
+                raise ValueError('rerank="gnn": ' + _lib.load().ieee_last_error().decode())
+            return
         # the library's size query states its limits (k1 + 1 <= 512, k2 <= k1 + 1, the expansion's sort, N < 2^24), here
         # for the fewest queries that give k1 + 1 samples; evaluate() checks k1 + 1 <= N with the real query count
         G = max(gf.shape[0], 1)
@@ -313,8 +340,8 @@ class RetrievalEvaluator:
             raise ValueError("rerank=True: " + _lib.load().ieee_last_error().decode())
 
     def _rerank_prepare(self, qf: torch.Tensor):
-        """Re-ranking state of this query set (ieee_rerank_stream_prepare): kept while the same, unmodified query
-        tensor is evaluated again."""
+        """Re-ranking state of this query set (ieee_rerank_stream_prepare, or the ieee_gnn_stream_* calls): kept while
+        the same, unmodified query tensor is evaluated again with the same k1 and k2."""
         k1, k2 = self.k1, self.k2
         key = (_features_key(qf), k1, k2)
         if self._rr is not None and self._rr["key"] == key:
@@ -322,6 +349,9 @@ class RetrievalEvaluator:
         # the previous state, the distance block and the blend's accumulators are free while the strips are computed:
         # the block budget (block_bytes) then covers the strips, and later the block and its accumulators
         self._rr = self._block = self._rr_scratch = None
+        if self.gnn:
+            self._rr = self._gnn_prepare(qf, key)
+            return self._rr
         Q, D = qf.shape
         G = self.G
         if k1 + 1 > Q + G:
@@ -348,6 +378,64 @@ class RetrievalEvaluator:
         self._rr = {"key": key, "qf": qf, "Q": Q, "k1": k1, "k2": k2, "packed": qpk, "ws": ws, "colmax": colmax,
                     "rank": rank}
         return self._rr
+
+    def _gnn_prepare(self, qf: torch.Tensor, key):
+        """GNN state of this query set: neighbours from row strips, the symbolic phase (one host round trip sizes every
+        structure), then the numeric phase: A as CSR rows and the CSC of its gallery rows."""
+        k1, k2 = self.k1, self.k2
+        Q, D = qf.shape
+        G = self.G
+        N = Q + G
+        if k1 > N:
+            raise ValueError('rerank="gnn": k1 = {} exceeds the {} query and gallery samples'.format(k1, N))
+        lib = _lib.load()
+        sc_bytes = lib.ieee_gnn_stream_scratch_bytes(Q, G, k1, self.block_bytes)
+        if sc_bytes == 0:
+            raise ValueError('rerank="gnn": ' + lib.ieee_last_error().decode())
+        qpk = self._take_early_q(qf)
+        if qpk is None:
+            qpk = PackedFeatures(qf, self.metric, self.normalize, self.precision, None)
+        gpk = self.chunks[0][1]
+        dev = self.device
+        scratch = torch.empty(sc_bytes, dtype=torch.uint8, device=dev)     # strips, then the graph calls' index
+        rank = torch.empty((N, k1), dtype=torch.int32, device=dev)
+        S = torch.empty((N, k1), dtype=torch.float32, device=dev)
+        _lib.call("ieee_gnn_stream_neighbours", qpk.buf.data_ptr(), Q, gpk.buf.data_ptr(), G, D, qpk.precision, k1,
+                  self.block_bytes, rank.data_ptr(), S.data_ptr(), scratch.data_ptr(), sc_bytes, _lib.stream())
+        TRACE.mark("GNN neighbours")
+        sizes = (C.c_int64 * 6)()
+        _lib.call("ieee_gnn_stream_graph_bytes_sync", rank.data_ptr(), Q, G, k1, k2, scratch.data_ptr(), sc_bytes, sizes,
+                  _lib.stream())
+        TRACE.mark("GNN symbolic phase")
+        nnz, nnz_g, work_bytes = sizes[0], sizes[1], sizes[2]
+        work = torch.empty(work_bytes, dtype=torch.uint8, device=dev)    # released (stream-ordered) on return
+        a_ptr = torch.empty(N + 1, dtype=torch.int64, device=dev)
+        a_col = torch.empty(nnz, dtype=torch.int32, device=dev)
+        a_val = torch.empty(nnz, dtype=torch.float32, device=dev)
+        g_ptr = torch.empty(N + 1, dtype=torch.int64, device=dev)
+        g_row = torch.empty(nnz_g, dtype=torch.int32, device=dev)
+        g_val = torch.empty(nnz_g, dtype=torch.float32, device=dev)
+        _lib.call("ieee_gnn_stream_graph", rank.data_ptr(), S.data_ptr(), Q, G, k1, k2, scratch.data_ptr(), sc_bytes,
+                  work.data_ptr(), work_bytes, sizes, a_ptr.data_ptr(), a_col.data_ptr(), a_val.data_ptr(), g_ptr.data_ptr(),
+                  g_row.data_ptr(), g_val.data_ptr(), _lib.stream())
+        TRACE.mark("GNN numeric phase")
+        return {"key": key, "qf": qf, "Q": Q, "k1": k1, "k2": k2, "rank": rank, "S": S, "a_ptr": a_ptr, "a_col": a_col,
+                "a_val": a_val, "g_ptr": g_ptr, "g_row": g_row, "g_val": g_val, "scratch_bytes": sc_bytes,
+                "work_bytes": work_bytes}
+
+    def _gnn_block(self, s: int, e: int) -> torch.Tensor:
+        """-(A[q] . A[Q + g]) of queries [s, e) into the scratch block (accumulated in float64): no contraction."""
+        dist = self._block[: e - s]
+        if e > s:
+            rr = self._rr
+            if self._rr_scratch is None or self._rr_scratch.numel() < (e - s) * self.G:
+                self._rr_scratch = torch.empty((e - s) * self.G, dtype=torch.float64, device=self.device)
+            _lib.call("ieee_gnn_stream_block", rr["a_ptr"].data_ptr(), rr["a_col"].data_ptr(), rr["a_val"].data_ptr(),
+                      rr["g_ptr"].data_ptr(), rr["g_row"].data_ptr(), rr["g_val"].data_ptr(), rr["Q"], self.G, s, e - s,
+                      dist.data_ptr(), dist.stride(0), self._rr_scratch.data_ptr(), 8 * self._rr_scratch.numel(),
+                      _lib.stream())
+            TRACE.mark("  GNN similarity")
+        return dist
 
     def _rerank_block(self, dist: torch.Tensor, row0: int) -> torch.Tensor:
         """Queries [row0, row0 + rows) of the prepared set: distances -> re-ranked distances, in place."""
@@ -411,8 +499,9 @@ class RetrievalEvaluator:
 
     # -- one query block ---------------------------------------------------------------------------------
     def _block_rows_for(self, Q: int, G: int) -> int:
-        # re-ranking: the distance block and the blend's accumulators (as large) share the budget
-        budget = self.block_bytes // 2 if self.rerank else self.block_bytes
+        # re-ranking: the distance block and its accumulators share the budget (k-reciprocal: float32, as large as the
+        # block; GNN: float64, twice as large)
+        budget = self.block_bytes // (3 if self.gnn else 2) if self.rerank else self.block_bytes
         rows = max(128, int(budget // (4 * max(G, 1))) // 128 * 128)
         return min(Q, rows)
 
@@ -448,6 +537,8 @@ class RetrievalEvaluator:
         self._ensure_block(rows)
 
         def block(s, e, qpk):
+            if self.gnn:
+                return self._gnn_block(s, e)
             if qpk is None:
                 if q_event is not None:
                     torch.cuda.current_stream().wait_event(q_event)
@@ -667,8 +758,8 @@ class RetrievalEvaluator:
             early_pack = None
             if self.rerank and Q > 0:
                 rr = self._rerank_prepare(qf)
-                early_pack = rr["packed"] if rows >= Q else None
-            if qf.is_cuda and early_pack is None:
+                early_pack = rr.get("packed") if rows >= Q else None
+            if qf.is_cuda and early_pack is None and not self.gnn:
                 early_pack = self._take_early_q(qf) if rows >= Q else None
                 if early_pack is None:
                     early_pack = PackedFeatures(qf[: min(Q, rows)], self.metric, self.normalize, self.precision, self.center)

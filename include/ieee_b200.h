@@ -376,6 +376,40 @@ int ieee_gnn_rerank(const float* neg_score, int64_t lds, int64_t N, int32_t k1, 
                     void* workspace, size_t workspace_bytes, ieee_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * GNN re-ranking, streamed: the A of ieee_gnn_rerank held sparse, computed from packed features (ieee_pack_features with
+ * IEEE_METRIC_NEG_DOT, no centre) without any N x N matrix, N = Q + G.  Memory grows linearly in N and in the number
+ * of adjacency entries.
+ *   ieee_gnn_stream_neighbours computes -(X_u X_u^T) in row strips (queries, then gallery; strip_bytes / ~4N rows, a
+ *   multiple of 256) with the contraction, and from each strip the first k1 neighbours `rank` (int32 [N, k1], ties by
+ *   index) and S = score^2 (float32 [N, k1]).  No host synchronisation.
+ *   ieee_gnn_stream_graph_bytes_sync (symbolic phase) derives every adjacency structure from `rank` alone and waits for
+ *   its sizes: sizes (host int64[6]) = {nnz of A, nnz of A's gallery rows, work bytes of ieee_gnn_stream_graph, and
+ *   three sizes that call reads back}.  It keeps an index in `scratch` for the next call.
+ *   ieee_gnn_stream_graph (numeric phase) writes A as CSR (a_ptr int64 [N + 1], a_col int32 ascending, a_val float32)
+ *   and A's gallery rows as CSC (g_ptr int64 [N + 1] over the N columns, g_row int32 gallery indices ascending, g_val
+ *   float32).  Structural entries whose value is 0 are kept.  `work` is free again when its work on the stream is done.
+ *   ieee_gnn_stream_block writes -(A[q] . A[Q + g]) for queries [row0, row0 + rows) into block (float32 [rows, G],
+ *   leading dim ld), summed in float64 (scratch: rows * G doubles) in ascending column order and rounded once: the bits
+ *   do not depend on the block size.
+ * rank, S and A have the bits ieee_gnn_rerank gives on the -(X_u X_u^T) the contraction writes for the same packed rows;
+ * only the final product differs from the dense path's tensor-core contraction (k2 == 1: A holds 0 and 1 and the products
+ * are the same integers).  Limits: 1 <= k2 <= k1 <= min(N, 1024), N <= 2^20; precision F16X3 or BF16.
+ * ieee_gnn_stream_scratch_bytes needs no GPU and returns 0 (with ieee_last_error set) when the parameters are out of range.
+ * ---------------------------------------------------------------------------------------------- */
+size_t ieee_gnn_stream_scratch_bytes(int64_t Q, int64_t G, int32_t k1, size_t strip_bytes);
+int ieee_gnn_stream_neighbours(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int precision,
+                               int32_t k1, size_t strip_bytes, int32_t* rank, float* S, void* scratch, size_t scratch_bytes,
+                               ieee_stream_t stream);
+int ieee_gnn_stream_graph_bytes_sync(const int32_t* rank, int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch,
+                                     size_t scratch_bytes, int64_t* sizes, ieee_stream_t stream);
+int ieee_gnn_stream_graph(const int32_t* rank, const float* S, int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch,
+                          size_t scratch_bytes, void* work, size_t work_bytes, const int64_t* sizes, int64_t* a_ptr,
+                          int32_t* a_col, float* a_val, int64_t* g_ptr, int32_t* g_row, float* g_val, ieee_stream_t stream);
+int ieee_gnn_stream_block(const int64_t* a_ptr, const int32_t* a_col, const float* a_val, const int64_t* g_ptr,
+                          const int32_t* g_row, const float* g_val, int64_t Q, int64_t G, int64_t row0, int64_t rows,
+                          float* block, int64_t ld, void* scratch, size_t scratch_bytes, ieee_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Peer exchange: the two exchange steps of a gallery sharded over the GPUs of one box (relevant lists to every rank,
  * partial counts to every rank) as STORES into NVLink peer memory from inside the rank kernels, with flag words for
  * the hand-over -- no collective launches between the kernels of a step.
