@@ -82,6 +82,12 @@ SIGNATURES = {
     "ieee_rerank_stream_scratch_bytes": (sz, [i64, i64, i32, sz]),
     "ieee_rerank_stream_prepare": (C.c_int, [vp, i64, vp, i64, i64, C.c_int, C.c_int, i32, i32, sz, vp, vp, vp, sz, vp, sz, vp]),
     "ieee_rerank_stream_block": (C.c_int, [vp, i64, i64, i32, i32, vp, i64, i64, C.c_double, vp, i64, vp, sz, vp]),
+    "ieee_rerank_stream_window_workspace_bytes": (sz, [i64, i64, i32, i32, i64]),
+    "ieee_rerank_stream_v_layout": (C.c_int, [i64, i64, i32, i32, C.POINTER(i64), C.POINTER(sz), C.POINTER(sz), C.POINTER(sz)]),
+    "ieee_rerank_stream_pass": (C.c_int, [i32, vp, i64, vp, i64, i64, C.c_int, C.c_int, i32, i32, sz, i64, i64, i64, i64, vp, vp,
+                                          vp, sz, vp, sz, vp]),
+    "ieee_rerank_stream_finish": (C.c_int, [vp, sz, i64, i64, i32, i32, i64, i64, vp, vp]),
+    "ieee_rerank_stream_block_window": (C.c_int, [vp, i64, i64, i32, i32, i64, vp, i64, i64, C.c_double, vp, i64, vp, sz, vp]),
     "ieee_gnn_stream_scratch_bytes": (sz, [i64, i64, i32, sz]),
     "ieee_gnn_stream_neighbours": (C.c_int, [vp, i64, vp, i64, i64, C.c_int, i32, sz, vp, vp, vp, sz, vp]),
     "ieee_gnn_stream_graph_bytes_sync": (C.c_int, [vp, i64, i64, i32, i32, vp, sz, C.POINTER(i64), vp]),

@@ -119,6 +119,18 @@ int rerank_stream_prepare(const void* q_packed, int64_t Q, const void* g_packed,
 int rerank_stream_block(const void* workspace, int64_t Q, int64_t G, int32_t k1, int32_t k2, const float* colmax, int64_t row0,
                         int64_t rows, double lambda_value, float* block, int64_t ld, void* scratch, size_t scratch_bytes,
                         cudaStream_t stream);
+size_t rerank_stream_window_workspace_bytes(int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t Gs);
+int rerank_stream_v_layout(int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t* cap, size_t* off_col, size_t* off_val,
+                           size_t* off_cnt);
+int rerank_stream_pass(int pass, const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
+                       int precision, int32_t k1, int32_t k2, size_t strip_bytes, int64_t q0, int64_t q1, int64_t g0, int64_t g1,
+                       float* colmax, int32_t* rank, void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
+                       cudaStream_t stream, int cta_group);
+int rerank_stream_finish(void* workspace, size_t workspace_bytes, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t g0,
+                         int64_t Gs, const int32_t* rank, cudaStream_t stream);
+int rerank_stream_block_window(const void* workspace, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t Gs,
+                               const float* colmax, int64_t row0, int64_t rows, double lambda_value, float* block, int64_t ld,
+                               void* scratch, size_t scratch_bytes, cudaStream_t stream);
 
 size_t gnn_rerank_workspace_bytes(int64_t N, int32_t k1);
 int gnn_rerank(const float* neg_score, int64_t lds, int64_t N, int32_t k1, int32_t k2, float* A, int64_t ldA, void* workspace,
@@ -746,6 +758,41 @@ int ieee_rerank_stream_block(const void* workspace, int64_t Q, int64_t G, int32_
   if (rc) return rc;
   return rerank_stream_block(workspace, Q, G, k1, k2, colmax, row0, rows, lambda_value, block, ld, scratch, scratch_bytes,
                              (cudaStream_t)stream);
+}
+
+size_t ieee_rerank_stream_window_workspace_bytes(int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t Gs) {
+  return rerank_stream_window_workspace_bytes(Q, G, k1, k2, Gs);
+}
+
+int ieee_rerank_stream_v_layout(int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t* cap, size_t* off_col, size_t* off_val,
+                                size_t* off_cnt) {
+  return rerank_stream_v_layout(Q, G, k1, k2, cap, off_col, off_val, off_cnt);
+}
+
+int ieee_rerank_stream_pass(int32_t pass, const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
+                            int precision, int32_t k1, int32_t k2, size_t strip_bytes, int64_t q0, int64_t q1, int64_t g0,
+                            int64_t g1, float* colmax, int32_t* rank, void* workspace, size_t workspace_bytes, void* scratch,
+                            size_t scratch_bytes, ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return rerank_stream_pass(pass, q_packed, Q, g_packed, G, D, metric, precision, k1, k2, strip_bytes, q0, q1, g0, g1, colmax,
+                            rank, workspace, workspace_bytes, scratch, scratch_bytes, (cudaStream_t)stream, cta_group_default());
+}
+
+int ieee_rerank_stream_finish(void* workspace, size_t workspace_bytes, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t g0,
+                              int64_t Gs, const int32_t* rank, ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return rerank_stream_finish(workspace, workspace_bytes, Q, G, k1, k2, g0, Gs, rank, (cudaStream_t)stream);
+}
+
+int ieee_rerank_stream_block_window(const void* workspace, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t Gs,
+                                    const float* colmax, int64_t row0, int64_t rows, double lambda_value, float* block,
+                                    int64_t ld, void* scratch, size_t scratch_bytes, ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return rerank_stream_block_window(workspace, Q, G, k1, k2, Gs, colmax, row0, rows, lambda_value, block, ld, scratch,
+                                    scratch_bytes, (cudaStream_t)stream);
 }
 
 size_t ieee_gnn_rerank_workspace_bytes(int64_t N, int32_t k1) { return gnn_rerank_workspace_bytes(N, k1); }

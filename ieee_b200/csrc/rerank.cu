@@ -224,7 +224,11 @@ rr_weights_kernel(const float* __restrict__ orig, int64_t ldo, int row0, int row
   rr_weights(orig + (int64_t)t * ldo, v_col + (int64_t)i * cap_v, v_val + (int64_t)i * cap_v, v_cnt[i], lane);
 }
 
-// ---- K4: V_qe[i] = mean_j V[rank[i][j]], j < k2; one CTA per row ------------------------------------------
+// Rows of a gallery window: the Q query rows, then the gallery rows [Q + g0, Q + g0 + Gs).  Window row m is sample
+// m < Q ? m : m + g0; with g0 = 0 and Gs = G the window is every sample.
+__device__ __forceinline__ int window_sample(int m, int Q, int g0) { return m < Q ? m : m + g0; }
+
+// ---- K4: V_qe[m] = mean_j V[rank[i][j]], j < k2, i the sample of window row m; one CTA per window row ------------
 __device__ __forceinline__ void block_sort_u64(uint64_t* s, int n) {
   for (int k = 2; k <= n; k <<= 1) {
     for (int j = k >> 1; j > 0; j >>= 1) {
@@ -242,17 +246,18 @@ __device__ __forceinline__ void block_sort_u64(uint64_t* s, int n) {
 }
 
 __global__ void __launch_bounds__(256)
-rr_expand_kernel(const int32_t* __restrict__ rank, int ldr, int N, int k2, int cap_v, const int32_t* __restrict__ v_col,
+rr_expand_kernel(const int32_t* __restrict__ rank, int ldr, int Q, int g0, int k2, int cap_v, const int32_t* __restrict__ v_col,
                  const float* __restrict__ v_val, const int32_t* __restrict__ v_cnt, int cap_e, int cap_e_pow2,
                  int32_t* __restrict__ e_col, float* __restrict__ e_val, int32_t* __restrict__ e_cnt) {
   extern __shared__ __align__(16) uint8_t ex_raw[];
   uint64_t* keys = reinterpret_cast<uint64_t*>(ex_raw);                  // (col * k2 + j) << 32 | float bits
   __shared__ int n_items, n_out;
-  const int i = blockIdx.x;
+  const int i = blockIdx.x;                                              // output row (window row)
+  const int sample = window_sample(i, Q, g0);
   if (threadIdx.x == 0) { n_items = 0; n_out = 0; }
   __syncthreads();
   for (int j = 0; j < k2; ++j) {
-    const int r = rank[(int64_t)i * ldr + j];
+    const int r = rank[(int64_t)sample * ldr + j];
     if (r < 0) continue;
     const int n = v_cnt[r];
     __shared__ int base;
@@ -304,9 +309,11 @@ rr_expand_kernel(const int32_t* __restrict__ rank, int ldr, int N, int k2, int c
 }
 
 // ---- K5a: inverted index (CSC of the row-sparse matrix), zero values excluded (rerank.py:93: V[:, i] != 0) ----
-__global__ void rr_col_count_kernel(int N, int cap, const int32_t* __restrict__ col, const float* __restrict__ val,
+// One CTA per window row r; its entries are read from row window_sample(r, Q, shift) of the row-sparse matrix (shift =
+// g0 when that matrix is V, indexed by sample; 0 when it is V_qe, already indexed by window row) and listed as row r.
+__global__ void rr_col_count_kernel(int Q, int shift, int cap, const int32_t* __restrict__ col, const float* __restrict__ val,
                                     const int32_t* __restrict__ cnt, int32_t* __restrict__ col_count) {
-  const int r = blockIdx.x;
+  const int r = window_sample(blockIdx.x, Q, shift);
   const int n = cnt[r];
   for (int t = threadIdx.x; t < n; t += blockDim.x)
     if (val[(int64_t)r * cap + t] != 0.f) atomicAdd(col_count + col[(int64_t)r * cap + t], 1);
@@ -334,17 +341,17 @@ __global__ void __launch_bounds__(1024) rr_scan_kernel(const int32_t* __restrict
   }
   if (threadIdx.x == 0) out[N] = carry;
 }
-__global__ void rr_col_fill_kernel(int N, int cap, const int32_t* __restrict__ col, const float* __restrict__ val,
+__global__ void rr_col_fill_kernel(int Q, int shift, int cap, const int32_t* __restrict__ col, const float* __restrict__ val,
                                    const int32_t* __restrict__ cnt, const int32_t* __restrict__ col_ptr,
                                    int32_t* __restrict__ cursor, int32_t* __restrict__ inv_row, float* __restrict__ inv_val) {
-  const int r = blockIdx.x;
+  const int r = window_sample(blockIdx.x, Q, shift);
   const int n = cnt[r];
   for (int t = threadIdx.x; t < n; t += blockDim.x) {
     const float v = val[(int64_t)r * cap + t];
     if (v == 0.f) continue;
     const int c = col[(int64_t)r * cap + t];
     const int pos = col_ptr[c] + atomicAdd(cursor + c, 1);
-    inv_row[pos] = r;
+    inv_row[pos] = blockIdx.x;
     inv_val[pos] = v;
   }
 }
@@ -354,16 +361,20 @@ __global__ void rr_col_fill_kernel(int N, int cap, const int32_t* __restrict__ c
 // doubles as the accumulator (acc == out) and the original distance is read from orig.  kBlock: `out` holds the
 // query's distances to the gallery (qg rows row0..), accumulation goes to `acc`, and the original distance is
 // formed from the distance as rr_build_orig_kernel forms it (qg[i][g] = raw[Q + g][i]).
+// The inverted index holds the rows of one gallery window (Q query rows, then Gs gallery rows, see window_sample): row
+// r >= Q of the index is column r - Q of the window, so acc and out are Gs wide.  Each acc[g] gets at most one add per
+// column of row i (rows are distinct inside a column), in the ascending column order, so a window has the bits of the
+// same columns of the whole gallery whatever order the index was filled in.
 template <bool kBlock>
 __global__ void __launch_bounds__(256)
-rr_jaccard_kernel(int Q, int G, int N, int cap, const int32_t* __restrict__ col, const float* __restrict__ val,
+rr_jaccard_kernel(int Q, int Gs, int N, int cap, const int32_t* __restrict__ col, const float* __restrict__ val,
                   const int32_t* __restrict__ cnt, const int32_t* __restrict__ col_ptr, const int32_t* __restrict__ inv_row,
                   const float* __restrict__ inv_val, const float* __restrict__ orig, const float* __restrict__ colmax, int row0,
                   float* acc_rows, int64_t ld_acc, float w_jaccard, float w_orig, float* out, int64_t ldo) {
   const int i = row0 + blockIdx.x;
   float* acc = acc_rows + (int64_t)blockIdx.x * ld_acc;
   float* dst = out + (int64_t)blockIdx.x * ldo;
-  for (int g = threadIdx.x; g < G; g += blockDim.x) acc[g] = 0.f;
+  for (int g = threadIdx.x; g < Gs; g += blockDim.x) acc[g] = 0.f;
   __syncthreads();
   const int n = cnt[i];
   for (int t = 0; t < n; ++t) {            // ascending column order (rerank.py:99-105)
@@ -377,7 +388,7 @@ rr_jaccard_kernel(int Q, int G, int N, int cap, const int32_t* __restrict__ col,
     }
     __syncthreads();
   }
-  for (int g = threadIdx.x; g < G; g += blockDim.x) {
+  for (int g = threadIdx.x; g < Gs; g += blockDim.x) {
     const float tmin = acc[g];
     const float jac = __fsub_rn(1.0f, __fdiv_rn(tmin, __fsub_rn(2.0f, tmin)));          // rerank.py:106
     float o;
@@ -406,15 +417,18 @@ static inline int half_k(int k1) {          // int(np.around(k1 / 2.)): round ha
 
 // Workspace of both forms.  The dense form holds orig (N x N), colmax, rank and the top-k values; the streamed form
 // keeps colmax and rank in caller buffers and only the sparse state here (its strips live in a separate scratch, see
-// StripPlan), so its offsets depend on (Q, G, k1, k2) alone.
+// StripPlan), so its offsets depend on (Q, G, k1, k2, Gs) alone.  V holds all N rows; its query expansion and the
+// inverted index hold the M = Q + Gs rows of a gallery window (window_sample): the whole gallery when Gs = G.  V comes
+// first, so its offsets do not depend on the window.
 struct RerankPlan {
-  int N, k1p, khp, cap_v, cap_v_pow2, cap_e, cap_e_pow2;
-  size_t off_orig, off_colmax, off_rank, off_rank_val, off_vcol, off_vval, off_vcnt, off_ecol, off_eval, off_ecnt, off_colcnt,
-      off_colptr, off_cursor, off_invrow, off_invval, total;
+  int N, M, k1p, khp, cap_v, cap_v_pow2, cap_e, cap_e_pow2;
+  size_t off_orig, off_colmax, off_rank, off_rank_val, off_vcol, off_vval, off_vcnt, v_end, off_ecol, off_eval, off_ecnt,
+      off_colcnt, off_colptr, off_cursor, off_invrow, off_invval, total;
 };
-static RerankPlan make_plan(int64_t Q, int64_t G, int k1, int k2, bool dense) {
+static RerankPlan make_plan(int64_t Q, int64_t G, int k1, int k2, bool dense, int64_t Gs) {
   RerankPlan p;
   p.N = (int)(Q + G);
+  p.M = (int)(Q + Gs);
   p.k1p = k1 + 1;
   p.khp = half_k(k1) + 1;
   p.cap_v = p.k1p * (p.khp + 1);
@@ -423,7 +437,7 @@ static RerankPlan make_plan(int64_t Q, int64_t G, int k1, int k2, bool dense) {
   p.cap_e_pow2 = pow2_at_least(p.cap_e);
   size_t o = 0;
   auto take = [&](size_t bytes) { size_t r = o; o += align256(bytes); return r; };
-  const size_t N = p.N;
+  const size_t N = p.N, M = p.M;
   const size_t dn = dense ? N : 0;
   p.off_orig = take(dn * N * 4);
   p.off_colmax = take(dn * 4);
@@ -432,14 +446,15 @@ static RerankPlan make_plan(int64_t Q, int64_t G, int k1, int k2, bool dense) {
   p.off_vcol = take(N * p.cap_v * 4);
   p.off_vval = take(N * p.cap_v * 4);
   p.off_vcnt = take(N * 4);
-  p.off_ecol = take(k2 > 1 ? N * p.cap_e * 4 : 0);
-  p.off_eval = take(k2 > 1 ? N * p.cap_e * 4 : 0);
-  p.off_ecnt = take(k2 > 1 ? N * 4 : 0);
-  p.off_colcnt = take(N * 4);
+  p.v_end = o;
+  p.off_ecol = take(k2 > 1 ? M * p.cap_e * 4 : 0);
+  p.off_eval = take(k2 > 1 ? M * p.cap_e * 4 : 0);
+  p.off_ecnt = take(k2 > 1 ? M * 4 : 0);
+  p.off_colcnt = take(N * 4);                 // the index's columns are samples: all N of them
   p.off_colptr = take((N + 1) * 4);
   p.off_cursor = take(N * 4);
-  p.off_invrow = take(N * p.cap_e * 4);
-  p.off_invval = take(N * p.cap_e * 4);
+  p.off_invrow = take(M * p.cap_e * 4);
+  p.off_invval = take(M * p.cap_e * 4);
   p.total = o + 256;
   return p;
 }
@@ -450,7 +465,7 @@ static int check_params(const char* who, int64_t Q, int64_t G, int32_t k1, int32
   IEEE_REQUIRE(Q + G < (int64_t(1) << 24), "%s: N = Q + G too large", who);
   IEEE_REQUIRE(k1 >= 1 && k1 + 1 <= 512 && k2 >= 1 && k2 <= k1 + 1, "%s: need 1 <= k2 <= k1 + 1 <= 512", who);
   IEEE_REQUIRE(k1 + 1 <= Q + G, "%s: k1 + 1 exceeds the number of samples", who);
-  const RerankPlan p = make_plan(Q, G, k1, k2, false);
+  const RerankPlan p = make_plan(Q, G, k1, k2, false, G);
   IEEE_REQUIRE((size_t)p.cap_e_pow2 * 8 <= 160 * 1024, "%s: k2 * (k1+1) * (k1/2+2) = %d entries per row exceed the shared-memory sort",
                who, p.cap_e);
   return IEEE_OK;
@@ -471,9 +486,11 @@ static SparseRows final_rows(const RerankPlan& p, uint8_t* w, int k2) {
           reinterpret_cast<int32_t*>(w + p.off_vcnt), p.cap_v};
 }
 
-// K4 + K5a: query expansion of V (built by K3) and the inverted index of the result
-static int expand_and_index(const RerankPlan& p, uint8_t* w, const int32_t* rank, int k2, cudaStream_t stream) {
-  const int N = p.N;
+// K4 + K5a over the rows of the gallery window that starts at gallery row g0: query expansion of V (built by K3) and
+// the inverted index of the result
+static int expand_and_index(const RerankPlan& p, uint8_t* w, const int32_t* rank, int k2, int64_t Q, int64_t g0,
+                            cudaStream_t stream) {
+  const int N = p.N, M = p.M;
   int32_t* vcol = reinterpret_cast<int32_t*>(w + p.off_vcol);
   float* vval = reinterpret_cast<float*>(w + p.off_vval);
   int32_t* vcnt = reinterpret_cast<int32_t*>(w + p.off_vcnt);
@@ -486,33 +503,34 @@ static int expand_and_index(const RerankPlan& p, uint8_t* w, const int32_t* rank
   if (k2 != 1) {
     const size_t smem = size_t(p.cap_e_pow2) * 8;
     IEEE_ENSURE_DYN_SMEM(rr_expand_kernel, smem);
-    rr_expand_kernel<<<N, 256, smem, stream>>>(rank, p.k1p, N, k2, p.cap_v, vcol, vval, vcnt, p.cap_e, p.cap_e_pow2,
-                                               reinterpret_cast<int32_t*>(w + p.off_ecol), reinterpret_cast<float*>(w + p.off_eval),
-                                               reinterpret_cast<int32_t*>(w + p.off_ecnt));
+    rr_expand_kernel<<<M, 256, smem, stream>>>(rank, p.k1p, (int)Q, (int)g0, k2, p.cap_v, vcol, vval, vcnt, p.cap_e,
+                                               p.cap_e_pow2, reinterpret_cast<int32_t*>(w + p.off_ecol),
+                                               reinterpret_cast<float*>(w + p.off_eval), reinterpret_cast<int32_t*>(w + p.off_ecnt));
     count_launch();
   }
   const SparseRows f = final_rows(p, w, k2);
+  const int shift = k2 != 1 ? 0 : (int)g0;     // V_qe rows are window rows already, V rows are samples
   // K5a
   IEEE_CUDA_CHECK(cudaMemsetAsync(colcnt, 0, size_t(N) * 4, stream));
   IEEE_CUDA_CHECK(cudaMemsetAsync(cursor, 0, size_t(N) * 4, stream));
-  rr_col_count_kernel<<<N, 128, 0, stream>>>(N, f.cap, f.col, f.val, f.cnt, colcnt);
+  rr_col_count_kernel<<<M, 128, 0, stream>>>((int)Q, shift, f.cap, f.col, f.val, f.cnt, colcnt);
   count_launch();
   rr_scan_kernel<<<1, 1024, 0, stream>>>(colcnt, N, colptr);
   count_launch();
-  rr_col_fill_kernel<<<N, 128, 0, stream>>>(N, f.cap, f.col, f.val, f.cnt, colptr, cursor, invrow, invval);
+  rr_col_fill_kernel<<<M, 128, 0, stream>>>((int)Q, shift, f.cap, f.col, f.val, f.cnt, colptr, cursor, invrow, invval);
   count_launch();
   return IEEE_OK;
 }
 
-// K5b + K6 for query rows [row0, row0 + rows), written to out (leading dim ldo)
+// K5b + K6 for query rows [row0, row0 + rows) against the window's p.M - Q gallery rows, written to out (leading dim ldo)
 template <bool kBlock>
-static void launch_jaccard(const RerankPlan& p, uint8_t* w, int64_t Q, int64_t G, int k2, double lambda_value,
-                           const float* orig, const float* colmax, int64_t row0, int64_t rows, float* acc, int64_t ld_acc,
-                           float* out, int64_t ldo, cudaStream_t stream) {
+static void launch_jaccard(const RerankPlan& p, uint8_t* w, int64_t Q, int k2, double lambda_value, const float* orig,
+                           const float* colmax, int64_t row0, int64_t rows, float* acc, int64_t ld_acc, float* out, int64_t ldo,
+                           cudaStream_t stream) {
   const SparseRows f = final_rows(p, w, k2);
   // (1 - lambda) is formed in double and rounded to float32 once, as NumPy does with the Python float
   rr_jaccard_kernel<kBlock><<<(unsigned)rows, 256, 0, stream>>>(
-      (int)Q, (int)G, p.N, f.cap, f.col, f.val, f.cnt, reinterpret_cast<int32_t*>(w + p.off_colptr),
+      (int)Q, p.M - (int)Q, p.N, f.cap, f.col, f.val, f.cnt, reinterpret_cast<int32_t*>(w + p.off_colptr),
       reinterpret_cast<int32_t*>(w + p.off_invrow), reinterpret_cast<float*>(w + p.off_invval), orig, colmax, (int)row0, acc,
       ld_acc, (float)(1.0 - lambda_value), (float)lambda_value, out, ldo);
   count_launch();
@@ -520,7 +538,7 @@ static void launch_jaccard(const RerankPlan& p, uint8_t* w, int64_t Q, int64_t G
 
 size_t rerank_workspace_bytes(int64_t Q, int64_t G, int32_t k1, int32_t k2) {
   if (Q <= 0 || G <= 0 || k1 < 1 || k2 < 1) return 0;
-  return make_plan(Q, G, k1, k2, true).total;
+  return make_plan(Q, G, k1, k2, true, G).total;
 }
 
 int rerank(const float* q_g, int64_t ld_qg, const float* q_q, int64_t ld_qq, const float* g_g, int64_t ld_gg, int64_t Q,
@@ -532,7 +550,7 @@ int rerank(const float* q_g, int64_t ld_qg, const float* q_q, int64_t ld_qq, con
   IEEE_REQUIRE(k1 >= 1 && k1 + 1 <= 512 && k2 >= 1 && k2 <= k1 + 1, "rerank: need 1 <= k2 <= k1 + 1 <= 512");
   IEEE_REQUIRE(k1 + 1 <= Q + G, "rerank: k1 + 1 exceeds the number of samples");
   IEEE_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "rerank: workspace must be 256-byte aligned");
-  const RerankPlan p = make_plan(Q, G, k1, k2, true);
+  const RerankPlan p = make_plan(Q, G, k1, k2, true, G);
   if (workspace_bytes < p.total) {
     set_error("rerank: workspace too small (%zu < %zu)", workspace_bytes, p.total);
     return IEEE_ERR_WORKSPACE;
@@ -579,17 +597,18 @@ int rerank(const float* q_g, int64_t ld_qg, const float* q_q, int64_t ld_qq, con
     count_launch();
   }
   // K4 + K5a
-  if ((rc = expand_and_index(p, w, rank, k2, stream))) return rc;
+  if ((rc = expand_and_index(p, w, rank, k2, Q, 0, stream))) return rc;
   // K5b + K6
-  launch_jaccard<false>(p, w, Q, G, k2, lambda_value, orig, nullptr, 0, Q, out, ldo, out, ldo, stream);
+  launch_jaccard<false>(p, w, Q, k2, lambda_value, orig, nullptr, 0, Q, out, ldo, out, ldo, stream);
   IEEE_CUDA_CHECK(cudaGetLastError());
   return IEEE_OK;
 }
 
 // ---- streamed form: orig in column strips of the virtual matrix, never all of it -------------------------------
 // A strip is raw[:, I] for |I| <= W columns, I inside the queries or inside the gallery and starting at a multiple of
-// W (a multiple of 256) of that operand's index: every contraction output is then computed at the same position
-// inside its tile (and its 128-column fix-up span) as in the whole-matrix products, so it has the same bits.
+// 256 of that operand's index: every contraction output is then computed at the same position inside its tile (and
+// its 128-column fix-up span) as in the whole-matrix products, so it has the same bits whatever W (a multiple of 256)
+// is and wherever the strips of a sample range start.
 // Strip scratch (a buffer of its own: only the prepare call needs it): top [Q, W], bot [max(W x Gp, G x W)], orig rows
 // [W, Np], top-k values [W, k1+1], the contraction's fix-up list.
 struct StripPlan {
@@ -615,9 +634,17 @@ static StripPlan make_strip_plan(int64_t Q, int64_t G, int k1, size_t strip_byte
   return s;
 }
 
-size_t rerank_stream_workspace_bytes(int64_t Q, int64_t G, int32_t k1, int32_t k2) {
+size_t rerank_stream_window_workspace_bytes(int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t Gs) {
   if (check_params("rerank_stream", Q, G, k1, k2) != IEEE_OK) return 0;
-  return make_plan(Q, G, k1, k2, false).total;
+  if (Gs < 0 || Gs > G) {
+    set_error("rerank_stream: gallery window of %lld rows outside the gallery of %lld", (long long)Gs, (long long)G);
+    return 0;
+  }
+  return make_plan(Q, G, k1, k2, false, Gs).total;
+}
+
+size_t rerank_stream_workspace_bytes(int64_t Q, int64_t G, int32_t k1, int32_t k2) {
+  return rerank_stream_window_workspace_bytes(Q, G, k1, k2, G);
 }
 
 size_t rerank_stream_scratch_bytes(int64_t Q, int64_t G, int32_t k1, size_t strip_bytes) {
@@ -625,23 +652,48 @@ size_t rerank_stream_scratch_bytes(int64_t Q, int64_t G, int32_t k1, size_t stri
   return make_strip_plan(Q, G, k1, strip_bytes).total;
 }
 
-int rerank_stream_prepare(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
-                          int precision, int32_t k1, int32_t k2, size_t strip_bytes, float* colmax, int32_t* rank,
-                          void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes, cudaStream_t stream,
-                          int cta_group) {
-  IEEE_REQUIRE(q_packed && g_packed && colmax && rank && workspace && scratch, "rerank_stream_prepare: null pointer");
-  IEEE_REQUIRE(D > 0, "rerank_stream_prepare: bad feature width D=%lld", (long long)D);
-  int rc = check_params("rerank_stream_prepare", Q, G, k1, k2);
+int rerank_stream_v_layout(int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t* cap, size_t* off_col, size_t* off_val,
+                           size_t* off_cnt) {
+  IEEE_REQUIRE(cap && off_col && off_val && off_cnt, "rerank_stream_v_layout: null pointer");
+  int rc = check_params("rerank_stream_v_layout", Q, G, k1, k2);
   if (rc) return rc;
-  IEEE_REQUIRE(metric == IEEE_METRIC_EUCLIDEAN || metric == IEEE_METRIC_COSINE, "rerank_stream_prepare: unknown metric %d", metric);
+  const RerankPlan p = make_plan(Q, G, k1, k2, false, G);
+  *cap = p.cap_v;
+  *off_col = p.off_vcol;
+  *off_val = p.off_vval;
+  *off_cnt = p.off_vcnt;
+  return IEEE_OK;
+}
+
+// One pass over the strips of the owned samples [q0, q1) and [Q + g0, Q + g1) (each range starting at a multiple of 256
+// of its segment and ending at one or at the segment's end).  Pass 0 (K1, K2): colmax and rank of the owned samples.
+// Pass 1 (K3): V's membership (columns, counts) of all N rows from `rank`, which must be complete, and the weights of
+// the owned rows from their strips, which need their colmax.
+int rerank_stream_pass(int pass, const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
+                       int precision, int32_t k1, int32_t k2, size_t strip_bytes, int64_t q0, int64_t q1, int64_t g0, int64_t g1,
+                       float* colmax, int32_t* rank, void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
+                       cudaStream_t stream, int cta_group) {
+  IEEE_REQUIRE(pass == 0 || pass == 1, "rerank_stream_pass: pass must be 0 or 1, got %d", pass);
+  IEEE_REQUIRE(q_packed && g_packed && colmax && rank && scratch && (pass == 0 || workspace), "rerank_stream_pass: null pointer");
+  IEEE_REQUIRE(D > 0, "rerank_stream_pass: bad feature width D=%lld", (long long)D);
+  int rc = check_params("rerank_stream_pass", Q, G, k1, k2);
+  if (rc) return rc;
+  IEEE_REQUIRE(metric == IEEE_METRIC_EUCLIDEAN || metric == IEEE_METRIC_COSINE, "rerank_stream_pass: unknown metric %d", metric);
   IEEE_REQUIRE(precision == IEEE_PREC_F16X3 || precision == IEEE_PREC_BF16,
-               "rerank_stream_prepare: precision %d has no tensor-core contraction", precision);
+               "rerank_stream_pass: precision %d has no tensor-core contraction", precision);
   IEEE_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0 && (reinterpret_cast<uintptr_t>(scratch) & 255) == 0,
-               "rerank_stream_prepare: workspace and scratch must be 256-byte aligned");
-  const RerankPlan p = make_plan(Q, G, k1, k2, false);
+               "rerank_stream_pass: workspace and scratch must be 256-byte aligned");
+  auto range_ok = [](int64_t a, int64_t b, int64_t n) {
+    return a == b ? 0 <= a && a <= n : 0 <= a && a < b && b <= n && a % 256 == 0 && (b == n || b % 256 == 0);
+  };
+  IEEE_REQUIRE(range_ok(q0, q1, Q) && range_ok(g0, g1, G),
+               "rerank_stream_pass: owned samples [%lld, %lld) of %lld queries and [%lld, %lld) of %lld gallery rows must start "
+               "at a multiple of 256 and end at one or at the end, or be empty", (long long)q0, (long long)q1, (long long)Q, (long long)g0,
+               (long long)g1, (long long)G);
+  const RerankPlan p = make_plan(Q, G, k1, k2, false, 0);
   const StripPlan s = make_strip_plan(Q, G, k1, strip_bytes);
-  if (workspace_bytes < p.total || scratch_bytes < s.total) {
-    set_error("rerank_stream_prepare: workspace or scratch too small (%zu < %zu or %zu < %zu)", workspace_bytes, p.total,
+  if ((pass == 1 && workspace_bytes < p.v_end) || scratch_bytes < s.total) {
+    set_error("rerank_stream_pass: workspace or scratch too small (%zu < %zu or %zu < %zu)", workspace_bytes, p.v_end,
               scratch_bytes, s.total);
     return IEEE_ERR_WORKSPACE;
   }
@@ -661,57 +713,115 @@ int rerank_stream_prepare(const void* q_packed, int64_t Q, const void* g_packed,
   auto rows_of = [&](bool gallery, int64_t r0, int64_t n) {
     return gallery ? packed_rows(g_packed, G, r0, n, D, precision) : packed_rows(q_packed, Q, r0, n, D, precision);
   };
-  IEEE_CUDA_CHECK(cudaMemsetAsync(colmax, 0, size_t(N) * 4, stream));
-  // pass 0: column maxima, orig rows, top-k (K1, K2); pass 1: the same orig rows again, weights of V (K3)
-  for (int pass = 0; pass < 2; ++pass) {
-    if (pass == 1) {
-      // K3, membership: from rank alone, which pass 0 has completed
-      const size_t smem = size_t(kRowWarps) * (p.k1p + p.khp + p.cap_v_pow2) * 4;
-      IEEE_ENSURE_DYN_SMEM(rr_krecip_kernel<false>, smem);
-      rr_krecip_kernel<false><<<(N + kRowWarps - 1) / kRowWarps, 32 * kRowWarps, smem, stream>>>(
-          rank, p.k1p, nullptr, N, p.k1p, p.khp, p.cap_v, p.cap_v_pow2, vcol, vval, vcnt);
+  if (pass == 0) {
+    if (q1 > q0) IEEE_CUDA_CHECK(cudaMemsetAsync(colmax + q0, 0, size_t(q1 - q0) * 4, stream));
+    if (g1 > g0) IEEE_CUDA_CHECK(cudaMemsetAsync(colmax + Q + g0, 0, size_t(g1 - g0) * 4, stream));
+  } else {
+    // K3, membership: from rank alone
+    const size_t smem = size_t(kRowWarps) * (p.k1p + p.khp + p.cap_v_pow2) * 4;
+    IEEE_ENSURE_DYN_SMEM(rr_krecip_kernel<false>, smem);
+    rr_krecip_kernel<false><<<(N + kRowWarps - 1) / kRowWarps, 32 * kRowWarps, smem, stream>>>(
+        rank, p.k1p, nullptr, N, p.k1p, p.khp, p.cap_v, p.cap_v_pow2, vcol, vval, vcnt);
+    count_launch();
+  }
+  for (int seg = 0; seg < 2; ++seg) {         // strips of the queries, then of the gallery
+    const bool gal = seg == 1;
+    const int64_t a = gal ? g0 : q0, b = gal ? g1 : q1;
+    for (int64_t c0 = a; c0 < b; c0 += s.W) {
+      const int64_t wc = (b - c0) < s.W ? (b - c0) : s.W;
+      const int64_t i0 = (gal ? Q : 0) + c0;  // first row of orig (column of raw) in the strip
+      // the contraction calls of the whole-matrix products, with the same operand roles
+      if ((rc = distmat_umma_rows(rows_of(false, 0, Q), rows_of(gal, c0, wc), metric, precision, top, s.W, stream, cta_group,
+                                  fix, false)))
+        return rc;
+      if (!gal) rc = distmat_umma_rows(rows_of(false, c0, wc), rows_of(true, 0, G), metric, precision, bot, s.Gp, stream,
+                                       cta_group, fix, false);
+      else rc = distmat_umma_rows(rows_of(true, 0, G), rows_of(true, c0, wc), metric, precision, bot, s.W, stream, cta_group,
+                                  fix, false);
+      if (rc) return rc;
+      const StripView view{top, bot, s.W, gal ? s.W : s.Gp, (int)Q, !gal};
+      if (pass == 0) {
+        rr_colmax_kernel<<<dim3((unsigned)((wc + 255) / 256), (unsigned)((Q + rpb - 1) / rpb)), 256, 0, stream>>>(
+            top, s.W, (int)Q, (int)wc, rpb, cm_bits + i0);
+        if (!gal) rr_rowmax_kernel<<<(unsigned)wc, 256, 0, stream>>>(bot, s.Gp, (int)wc, (int)G, cm_bits + i0);
+        else rr_colmax_kernel<<<dim3((unsigned)((wc + 255) / 256), (unsigned)((G + rpb - 1) / rpb)), 256, 0, stream>>>(
+                 bot, s.W, (int)G, (int)wc, rpb, cm_bits + i0);
+        count_launch(2);
+      }
+      rr_build_orig_kernel<<<dim3((unsigned)((N + 31) / 32), (unsigned)((wc + 31) / 32)), 256, 0, stream>>>(
+          view, (int)wc, N, colmax + i0, orig, s.Np);
       count_launch();
-    }
-    for (int seg = 0; seg < 2; ++seg) {         // strips of the queries, then of the gallery
-      const bool gal = seg == 1;
-      const int64_t n_seg = gal ? G : Q;
-      for (int64_t c0 = 0; c0 < n_seg; c0 += s.W) {
-        const int64_t wc = (n_seg - c0) < s.W ? (n_seg - c0) : s.W;
-        const int64_t i0 = (gal ? Q : 0) + c0;  // first row of orig (column of raw) in the strip
-        // the contraction calls of the whole-matrix products, with the same operand roles
-        if ((rc = distmat_umma_rows(rows_of(false, 0, Q), rows_of(gal, c0, wc), metric, precision, top, s.W, stream, cta_group,
-                                    fix, false)))
+      if (pass == 0) {
+        // K2 for the strip's rows
+        if ((rc = topk(orig, s.Np, wc, N, 0, nullptr, nullptr, nullptr, nullptr, p.k1p, rank + i0 * p.k1p, val, stream)))
           return rc;
-        if (!gal) rc = distmat_umma_rows(rows_of(false, c0, wc), rows_of(true, 0, G), metric, precision, bot, s.Gp, stream,
-                                         cta_group, fix, false);
-        else rc = distmat_umma_rows(rows_of(true, 0, G), rows_of(true, c0, wc), metric, precision, bot, s.W, stream, cta_group,
-                                    fix, false);
-        if (rc) return rc;
-        const StripView view{top, bot, s.W, gal ? s.W : s.Gp, (int)Q, !gal};
-        if (pass == 0) {
-          rr_colmax_kernel<<<dim3((unsigned)((wc + 255) / 256), (unsigned)((Q + rpb - 1) / rpb)), 256, 0, stream>>>(
-              top, s.W, (int)Q, (int)wc, rpb, cm_bits + i0);
-          if (!gal) rr_rowmax_kernel<<<(unsigned)wc, 256, 0, stream>>>(bot, s.Gp, (int)wc, (int)G, cm_bits + i0);
-          else rr_colmax_kernel<<<dim3((unsigned)((wc + 255) / 256), (unsigned)((G + rpb - 1) / rpb)), 256, 0, stream>>>(
-                   bot, s.W, (int)G, (int)wc, rpb, cm_bits + i0);
-          count_launch(2);
-        }
-        rr_build_orig_kernel<<<dim3((unsigned)((N + 31) / 32), (unsigned)((wc + 31) / 32)), 256, 0, stream>>>(
-            view, (int)wc, N, colmax + i0, orig, s.Np);
+      } else {
+        rr_weights_kernel<<<(unsigned)((wc + kRowWarps - 1) / kRowWarps), 32 * kRowWarps, 0, stream>>>(
+            orig, s.Np, (int)i0, (int)wc, p.cap_v, vcol, vval, vcnt);
         count_launch();
-        if (pass == 0) {
-          // K2 for the strip's rows
-          if ((rc = topk(orig, s.Np, wc, N, 0, nullptr, nullptr, nullptr, nullptr, p.k1p, rank + i0 * p.k1p, val, stream)))
-            return rc;
-        } else {
-          rr_weights_kernel<<<(unsigned)((wc + kRowWarps - 1) / kRowWarps), 32 * kRowWarps, 0, stream>>>(
-              orig, s.Np, (int)i0, (int)wc, p.cap_v, vcol, vval, vcnt);
-          count_launch();
-        }
       }
     }
   }
-  if ((rc = expand_and_index(p, w, rank, k2, stream))) return rc;
+  IEEE_CUDA_CHECK(cudaGetLastError());
+  return IEEE_OK;
+}
+
+// K4 + K5a over the gallery window [g0, g0 + Gs): needs rank and V of every sample
+int rerank_stream_finish(void* workspace, size_t workspace_bytes, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t g0,
+                         int64_t Gs, const int32_t* rank, cudaStream_t stream) {
+  IEEE_REQUIRE(workspace && rank, "rerank_stream_finish: null pointer");
+  int rc = check_params("rerank_stream_finish", Q, G, k1, k2);
+  if (rc) return rc;
+  IEEE_REQUIRE(g0 >= 0 && Gs >= 0 && g0 + Gs <= G, "rerank_stream_finish: gallery window [%lld, %lld) outside [0, %lld)",
+               (long long)g0, (long long)(g0 + Gs), (long long)G);
+  IEEE_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "rerank_stream_finish: workspace must be 256-byte aligned");
+  const RerankPlan p = make_plan(Q, G, k1, k2, false, Gs);
+  if (workspace_bytes < p.total) {
+    set_error("rerank_stream_finish: workspace too small (%zu < %zu)", workspace_bytes, p.total);
+    return IEEE_ERR_WORKSPACE;
+  }
+  if ((rc = expand_and_index(p, static_cast<uint8_t*>(workspace), rank, k2, Q, g0, stream))) return rc;
+  IEEE_CUDA_CHECK(cudaGetLastError());
+  return IEEE_OK;
+}
+
+int rerank_stream_prepare(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int metric,
+                          int precision, int32_t k1, int32_t k2, size_t strip_bytes, float* colmax, int32_t* rank,
+                          void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes, cudaStream_t stream,
+                          int cta_group) {
+  int rc = check_params("rerank_stream_prepare", Q, G, k1, k2);
+  if (rc) return rc;
+  const size_t need = make_plan(Q, G, k1, k2, false, G).total;
+  if (workspace_bytes < need) {                 // before any work is queued
+    set_error("rerank_stream_prepare: workspace too small (%zu < %zu)", workspace_bytes, need);
+    return IEEE_ERR_WORKSPACE;
+  }
+  for (int pass = 0; pass < 2; ++pass)
+    if ((rc = rerank_stream_pass(pass, q_packed, Q, g_packed, G, D, metric, precision, k1, k2, strip_bytes, 0, Q, 0, G, colmax,
+                                 rank, workspace, workspace_bytes, scratch, scratch_bytes, stream, cta_group)))
+      return rc;
+  return rerank_stream_finish(workspace, workspace_bytes, Q, G, k1, k2, 0, G, rank, stream);
+}
+
+// K5b + K6 of queries [row0, row0 + rows) against the gallery window the finish call indexed (Gs columns)
+int rerank_stream_block_window(const void* workspace, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t Gs,
+                               const float* colmax, int64_t row0, int64_t rows, double lambda_value, float* block, int64_t ld,
+                               void* scratch, size_t scratch_bytes, cudaStream_t stream) {
+  IEEE_REQUIRE(workspace && colmax && block && scratch, "rerank_stream_block: null pointer");
+  int rc = check_params("rerank_stream_block", Q, G, k1, k2);
+  if (rc) return rc;
+  IEEE_REQUIRE(Gs >= 0 && Gs <= G, "rerank_stream_block: gallery window of %lld rows outside the gallery of %lld",
+               (long long)Gs, (long long)G);
+  IEEE_REQUIRE(row0 >= 0 && rows >= 0 && row0 + rows <= Q && ld >= Gs, "rerank_stream_block: bad block rows [%lld, %lld) of %lld, ld=%lld",
+               (long long)row0, (long long)(row0 + rows), (long long)Q, (long long)ld);
+  if (scratch_bytes < size_t(rows) * size_t(Gs) * 4) {
+    set_error("rerank_stream_block: scratch too small (%zu < %zu)", scratch_bytes, size_t(rows) * size_t(Gs) * 4);
+    return IEEE_ERR_WORKSPACE;
+  }
+  if (rows == 0 || Gs == 0) return IEEE_OK;
+  const RerankPlan p = make_plan(Q, G, k1, k2, false, Gs);
+  launch_jaccard<true>(p, static_cast<uint8_t*>(const_cast<void*>(workspace)), Q, k2, lambda_value, nullptr, colmax, row0, rows,
+                       static_cast<float*>(scratch), Gs, block, ld, stream);
   IEEE_CUDA_CHECK(cudaGetLastError());
   return IEEE_OK;
 }
@@ -719,21 +829,8 @@ int rerank_stream_prepare(const void* q_packed, int64_t Q, const void* g_packed,
 int rerank_stream_block(const void* workspace, int64_t Q, int64_t G, int32_t k1, int32_t k2, const float* colmax, int64_t row0,
                         int64_t rows, double lambda_value, float* block, int64_t ld, void* scratch, size_t scratch_bytes,
                         cudaStream_t stream) {
-  IEEE_REQUIRE(workspace && colmax && block && scratch, "rerank_stream_block: null pointer");
-  int rc = check_params("rerank_stream_block", Q, G, k1, k2);
-  if (rc) return rc;
-  IEEE_REQUIRE(row0 >= 0 && rows >= 0 && row0 + rows <= Q && ld >= G, "rerank_stream_block: bad block rows [%lld, %lld) of %lld, ld=%lld",
-               (long long)row0, (long long)(row0 + rows), (long long)Q, (long long)ld);
-  if (scratch_bytes < size_t(rows) * size_t(G) * 4) {
-    set_error("rerank_stream_block: scratch too small (%zu < %zu)", scratch_bytes, size_t(rows) * size_t(G) * 4);
-    return IEEE_ERR_WORKSPACE;
-  }
-  if (rows == 0) return IEEE_OK;
-  const RerankPlan p = make_plan(Q, G, k1, k2, false);
-  launch_jaccard<true>(p, static_cast<uint8_t*>(const_cast<void*>(workspace)), Q, G, k2, lambda_value, nullptr, colmax, row0, rows,
-                       static_cast<float*>(scratch), G, block, ld, stream);
-  IEEE_CUDA_CHECK(cudaGetLastError());
-  return IEEE_OK;
+  return rerank_stream_block_window(workspace, Q, G, k1, k2, G, colmax, row0, rows, lambda_value, block, ld, scratch,
+                                    scratch_bytes, stream);
 }
 
 // =========================================================================================================

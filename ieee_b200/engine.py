@@ -144,6 +144,16 @@ def shard_bounds(num_rows: int, world: int, rank: int) -> tuple[int, int]:
     return start, start + base + (1 if rank < rem else 0)
 
 
+def rerank_owned(Q: int, G: int, world: int, rank: int) -> tuple[int, int, int, int]:
+    """Samples whose strips ``rank`` computes when ``world`` ranks prepare k-reciprocal re-ranking together: queries
+    [q0, q1) and gallery rows [g0, g1).  Each segment is cut into 256-sample strips, dealt out as shard_bounds deals
+    rows: every range starts at a multiple of 256 of its segment, and ranks differ by at most one strip per segment."""
+    def split(n):
+        a, b = shard_bounds((n + 255) // 256, world, rank)
+        return min(n, 256 * a), min(n, 256 * b)
+    return split(Q) + split(G)
+
+
 def centering_applies(metric: str, precision: str) -> bool:
     """Euclidean operands are packed relative to a common centre (ieee_pack_features); cosine is not translation
     invariant and the 1-pass bf16 mode multiplies bf16 inputs exactly as they are."""
@@ -241,7 +251,18 @@ class RetrievalEvaluator:
     k1, k2 default to 20, 6) instead of the plain ones, with the same bits as ``re_ranking`` on the three distance
     matrices, but without any N x N matrix (N = queries + gallery): the re-ranking state is prepared from the features
     in column strips (ieee_rerank_stream_prepare, strips sized by ``block_bytes``) and each query block's distances are
-    re-ranked before they are ranked.  The gallery must be on this one device (no ``group``, not ``from_host``).
+    re-ranked before they are ranked.  The gallery must be in HBM (not ``from_host``).
+
+    With ``group`` (a torch.distributed process group; NCCL for device tensors) and ``rerank=True`` the re-ranking is
+    over the whole sharded gallery, with the bits of one GPU holding it all: every rank returns what a one-GPU
+    ``rerank=True`` evaluator returns (ieee_rerank_stream_pass / _finish / _block_window).  The slices must tile
+    [0, g_total) in rank order (checked once, collectively; ValueError on every rank otherwise).  During the prepare
+    call every rank holds the whole gallery packed (about 4 bytes per feature, gathered from the slices and freed when
+    the prepare returns) and computes the strips of its share of the samples (rerank_owned); the small state (colmax,
+    neighbour lists, the k-reciprocal sets) is all-gathered.  What stays is sized by this rank's slice of Gs rows:
+    about 8 (k1+1)(round(k1/2)+2) bytes per sample of the whole set plus k2 times that per query and per slice row
+    (2 KB * N + 24 KB * (Q + Gs) at k1 = 20, k2 = 6), plus ``block_bytes``.  The plain sharded path's condition for
+    the bits of one GPU applies to the query blocks' own distances (this rank's contraction against its slice).
 
     ``rerank="gnn"`` ranks the GNN re-ranked similarity (gnn_reranking.py:27-59; k1, k2 default to 26, 7, the reference
     driver's values), negated so that it ranks as a distance: what ``gnn_reranking_distmat`` computes on the
@@ -249,7 +270,7 @@ class RetrievalEvaluator:
     product and no centre; ``dist_metric`` and ``lambda_value`` are not used.  The adjacency is held sparse
     (ieee_gnn_stream_*: neighbours from row strips sized by ``block_bytes``, then A as CSR rows and an inverted index of
     its gallery rows), and a query block's distances come from it instead of a contraction.  Same limits on the
-    gallery as ``rerank=True``; 1 <= k2 <= k1 <= min(N, 1024).
+    gallery as ``rerank=True``, and no ``group``; 1 <= k2 <= k1 <= min(N, 1024).
     """
 
     def __init__(self, gf: torch.Tensor, g_pids, g_camids, dist_metric: str = "euclidean", normalize_feature: bool = False,
@@ -272,7 +293,7 @@ class RetrievalEvaluator:
         if k2 is None:
             k2 = 7 if self.gnn else 6
         if self.rerank:
-            self._check_rerank(gf, group, k1, k2)
+            self._check_rerank(gf, group, k1, k2, g_total)
         self.k1, self.k2, self.lambda_value = k1, k2, float(lambda_value)
         self._rr = None          # re-ranking state of the last query set (_rerank_prepare)
         self._rr_scratch = None  # the blend's accumulators, one block
@@ -312,12 +333,32 @@ class RetrievalEvaluator:
         self._host_gallery = None
         self._label_keys = (_tensor_key(g_pids), _tensor_key(g_camids))
         self._label_refs = (g_pids, g_camids)
+        self._slices = self._gallery_slices() if self.rerank and group is not None else None
 
-    def _check_rerank(self, gf, group, k1, k2):
+    def _gallery_slices(self):
+        """[(g_offset, rows)] of every rank, all-gathered once.  Every rank gets the same list and so reaches the same
+        verdict: slices that do not tile [0, g_total) in rank order raise ValueError on every rank."""
+        import torch.distributed as dist_
+        with torch.cuda.device(self.device):
+            mine = torch.tensor([self.g_offset, self.G, self.g_total], dtype=torch.int64, device=self.device)
+            every = torch.empty((self.world, 3), dtype=torch.int64, device=self.device)
+            dist_.all_gather_into_tensor(every, mine, group=self.group)
+            every = every.cpu().tolist()
+        total = every[0][2]
+        starts = [sum(e[1] for e in every[:r]) for r in range(self.world)]
+        if any(e[0] != s or e[2] != total for e, s in zip(every, starts)) or starts[-1] + every[-1][1] != total:
+            raise ValueError("rerank=True over a sharded gallery: the slices (g_offset, rows, g_total) of the ranks {} do "
+                             "not tile [0, g_total) in rank order".format([tuple(e) for e in every]))
+        return [(off, rows) for off, rows, _ in every]
+
+    def _check_rerank(self, gf, group, k1, k2, g_total):
         mode = 'rerank="gnn"' if self.gnn else "rerank=True"
-        if group is not None:
+        if group is not None and self.gnn:
             raise ValueError("{} needs the whole gallery on one GPU: re-ranking over a sharded gallery (group) "
                              "is not supported".format(mode))
+        if group is not None and not (torch.distributed.is_available() and isinstance(group, torch.distributed.ProcessGroup)):
+            raise ValueError("rerank=True over a sharded gallery needs a torch.distributed process group as group, "
+                             "got {!r}".format(type(group).__name__))
         if gf is None:
             raise ValueError("{} needs the gallery features on the device: from_host streams them from the host".format(mode))
         if self.precision not in ("f16x3", "bf16"):
@@ -335,7 +376,7 @@ class RetrievalEvaluator:
             return
         # the library's size query states its limits (k1 + 1 <= 512, k2 <= k1 + 1, the expansion's sort, N < 2^24), here
         # for the fewest queries that give k1 + 1 samples; evaluate() checks k1 + 1 <= N with the real query count
-        G = max(gf.shape[0], 1)
+        G = max(gf.shape[0] if g_total is None else g_total, 1)
         if _lib.load().ieee_rerank_stream_workspace_bytes(max(1, k1 + 1 - G), G, k1, k2) == 0:
             raise ValueError("rerank=True: " + _lib.load().ieee_last_error().decode())
 
@@ -353,31 +394,89 @@ class RetrievalEvaluator:
             self._rr = self._gnn_prepare(qf, key)
             return self._rr
         Q, D = qf.shape
-        G = self.G
+        G = self.g_total
         if k1 + 1 > Q + G:
             raise ValueError("rerank=True: k1 + 1 = {} exceeds the {} query and gallery samples".format(k1 + 1, Q + G))
         lib = _lib.load()
-        ws_bytes = lib.ieee_rerank_stream_workspace_bytes(Q, G, k1, k2)
+        ws_bytes = lib.ieee_rerank_stream_window_workspace_bytes(Q, G, k1, k2, self.G)
         sc_bytes = lib.ieee_rerank_stream_scratch_bytes(Q, G, k1, self.block_bytes)
         if ws_bytes == 0 or sc_bytes == 0:
             raise ValueError("rerank=True: " + lib.ieee_last_error().decode())
         qpk = self._take_early_q(qf)
         if qpk is None:
             qpk = PackedFeatures(qf, self.metric, self.normalize, self.precision, self.center)
-        gpk = self.chunks[0][1]
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=self.device)
         strips = torch.empty(sc_bytes, dtype=torch.uint8, device=self.device)    # released (stream-ordered) on return
         colmax = torch.empty(Q + G, dtype=torch.float32, device=self.device)
         rank = torch.empty((Q + G, k1 + 1), dtype=torch.int32, device=self.device)
-        _lib.call("ieee_rerank_stream_prepare", qpk.buf.data_ptr(), Q, gpk.buf.data_ptr(), G, D, qpk.metric, qpk.precision,
-                  k1, k2, self.block_bytes, colmax.data_ptr(), rank.data_ptr(), ws.data_ptr(), ws_bytes, strips.data_ptr(),
-                  sc_bytes, _lib.stream())
+        if self.group is None:
+            _lib.call("ieee_rerank_stream_prepare", qpk.buf.data_ptr(), Q, self.chunks[0][1].buf.data_ptr(), G, D, qpk.metric,
+                      qpk.precision, k1, k2, self.block_bytes, colmax.data_ptr(), rank.data_ptr(), ws.data_ptr(), ws_bytes,
+                      strips.data_ptr(), sc_bytes, _lib.stream())
+        else:
+            self._rerank_prepare_sharded(qpk, colmax, rank, ws, strips)
         TRACE.mark("re-ranking state prepared")
         # qf is kept so that its address cannot be reused by another tensor while the key refers to it; k1 and k2
         # fix the workspace's layout, so the block calls take them from here
         self._rr = {"key": key, "qf": qf, "Q": Q, "k1": k1, "k2": k2, "packed": qpk, "ws": ws, "colmax": colmax,
                     "rank": rank}
         return self._rr
+
+    def _rerank_prepare_sharded(self, qpk: PackedFeatures, colmax, rank, ws, strips):
+        """The prepare call's phases with the ranks' exchanges between them: pass 0 and pass 1 over this rank's share of
+        the strips (rerank_owned), each followed by an all-gather of the owned rows (colmax and rank, then V's values),
+        and the finish over this rank's gallery slice.  The strips need every gallery row: the slices are all-gathered
+        and packed whole for the two passes and freed on return."""
+        import torch.distributed as dist_
+        Q, G, k1, k2 = qpk.rows, self.g_total, self.k1, self.k2
+        gpk = self._whole_gallery()
+        TRACE.mark("re-ranking: whole gallery gathered and packed")
+        owned = [rerank_owned(Q, G, self.world, r) for r in range(self.world)]
+        q0, q1, g0, g1 = owned[dist_.get_rank(self.group)]
+        cap, off_col, off_val, off_cnt = C.c_int64(), C.c_size_t(), C.c_size_t(), C.c_size_t()
+        _lib.call("ieee_rerank_stream_v_layout", Q, G, k1, k2, C.byref(cap), C.byref(off_col), C.byref(off_val), C.byref(off_cnt))
+        v_val = ws[off_val.value: off_val.value + 4 * (Q + G) * cap.value].view(torch.float32).view(Q + G, cap.value)
+        for step, shared in ((0, (colmax, rank)), (1, (v_val,))):
+            _lib.call("ieee_rerank_stream_pass", step, qpk.buf.data_ptr(), Q, gpk.buf.data_ptr(), G, qpk.D, qpk.metric,
+                      qpk.precision, k1, k2, self.block_bytes, q0, q1, g0, g1, colmax.data_ptr(), rank.data_ptr(), ws.data_ptr(),
+                      ws.numel(), strips.data_ptr(), strips.numel(), _lib.stream())
+            TRACE.mark("re-ranking: pass %d" % step)
+            for t in shared:
+                self._all_gather_owned(t, owned, Q)
+            TRACE.mark("re-ranking: exchange after pass %d" % step)
+        del gpk
+        _lib.call("ieee_rerank_stream_finish", ws.data_ptr(), ws.numel(), Q, G, k1, k2, self.g_offset, self.G, rank.data_ptr(),
+                  _lib.stream())
+
+    def _whole_gallery(self) -> PackedFeatures:
+        """Every rank's gallery slice, all-gathered (padded to the largest) and packed as one tensor with this evaluator's
+        centre: packing is per row, so these are the bytes one GPU packs from the whole gallery."""
+        import torch.distributed as dist_
+        gf = self._gallery_dev
+        rows = max(n for _, n in self._slices)
+        send = torch.zeros((rows, gf.shape[1]), dtype=gf.dtype, device=self.device)
+        send[: gf.shape[0]] = gf
+        recv = torch.empty((self.world, rows, gf.shape[1]), dtype=gf.dtype, device=self.device)
+        dist_.all_gather_into_tensor(recv, send, group=self.group)
+        del send
+        whole = torch.cat([recv[r, :n] for r, (_, n) in enumerate(self._slices)])
+        del recv
+        return PackedFeatures(whole, self.metric, self.normalize, self.precision, self.center)
+
+    def _all_gather_owned(self, t: torch.Tensor, owned, Q: int):
+        """Rows [q0, q1) and [Q + g0, Q + g1) of t ([Q + G, ...]), computed by each rank (owned = rerank_owned of every
+        rank), from that rank into t on every rank: one all-gather, padded to the largest share."""
+        import torch.distributed as dist_
+        dev = self.device
+        idx = [torch.cat([torch.arange(q0, q1), torch.arange(Q + g0, Q + g1)]).to(dev) for q0, q1, g0, g1 in owned]
+        rows = max(len(i) for i in idx)
+        mine = idx[dist_.get_rank(self.group)]
+        send = torch.zeros((rows,) + t.shape[1:], dtype=t.dtype, device=dev)
+        send[: len(mine)] = t[mine]
+        recv = torch.empty((self.world * rows,) + t.shape[1:], dtype=t.dtype, device=dev)
+        dist_.all_gather_into_tensor(recv, send, group=self.group)
+        at = torch.cat([r * rows + torch.arange(len(i), device=dev) for r, i in enumerate(idx)])
+        t[torch.cat(idx)] = recv[at]
 
     def _gnn_prepare(self, qf: torch.Tensor, key):
         """GNN state of this query set: neighbours from row strips, the symbolic phase (one host round trip sizes every
@@ -438,16 +537,17 @@ class RetrievalEvaluator:
         return dist
 
     def _rerank_block(self, dist: torch.Tensor, row0: int) -> torch.Tensor:
-        """Queries [row0, row0 + rows) of the prepared set: distances -> re-ranked distances, in place."""
+        """Queries [row0, row0 + rows) of the prepared set: distances to this rank's gallery rows -> re-ranked distances,
+        in place."""
         rr = self._rr
         rows = dist.shape[0]
         if rows == 0:                            # (an empty query set has no state to blend with)
             return dist
         if self._rr_scratch is None or self._rr_scratch.numel() < rows * self.G:
             self._rr_scratch = torch.empty(rows * self.G, dtype=torch.float32, device=self.device)
-        _lib.call("ieee_rerank_stream_block", rr["ws"].data_ptr(), rr["Q"], self.G, rr["k1"], rr["k2"], rr["colmax"].data_ptr(),
-                  row0, rows, self.lambda_value, dist.data_ptr(), dist.stride(0), self._rr_scratch.data_ptr(),
-                  4 * self._rr_scratch.numel(), _lib.stream())
+        _lib.call("ieee_rerank_stream_block_window", rr["ws"].data_ptr(), rr["Q"], self.g_total, rr["k1"], rr["k2"], self.G,
+                  rr["colmax"].data_ptr(), row0, rows, self.lambda_value, dist.data_ptr(), dist.stride(0),
+                  self._rr_scratch.data_ptr(), 4 * self._rr_scratch.numel(), _lib.stream())
         TRACE.mark("  re-ranking blend")
         return dist
 

@@ -363,6 +363,46 @@ int ieee_rerank_stream_block(const void* workspace, int64_t Q, int64_t G, int32_
                              int64_t row0, int64_t rows, double lambda_value, float* block, int64_t ld, void* scratch,
                              size_t scratch_bytes, ieee_stream_t stream);
 
+/* k-reciprocal re-ranking, streamed, in phases: the prepare call split so that S processes, each holding a gallery slice
+ * [g0, g0 + Gs) (the slices tiling [0, G) in order) and the replicated queries, share its strips and end with the state
+ * of their own slice.  ieee_rerank_stream_prepare is pass 0, pass 1 and finish over every sample with the window
+ * (0, G); ieee_rerank_stream_block is ieee_rerank_stream_block_window with Gs = G.  Same limits as above.
+ *   ieee_rerank_stream_pass needs the whole gallery packed (g_packed, G rows, as for the prepare call) and computes the
+ *   strips of the owned samples only: queries [q0, q1) and gallery rows [g0, g1), each range starting at a multiple of
+ *   256 of its segment and ending at one or at the segment's end (an empty range is allowed).  The bits do not depend on
+ *   the ranges or on strip_bytes.
+ *     pass 0 writes colmax and rank of the owned samples (colmax[i], rank[i, :] for i in [q0, q1) and [Q + g0, Q + g1)).
+ *       workspace may be null.  Exchange: every process needs colmax [N] and rank [N, k1 + 1] of all samples before
+ *       pass 1 (an all-gather of the owned rows).
+ *     pass 1 writes V's columns and counts of all N rows (from rank alone, the same on every process) and V's values of
+ *       the owned rows.  workspace: ieee_rerank_stream_window_workspace_bytes of this process's window (V comes first).
+ *       Exchange: every process needs V's values of all rows before finish; ieee_rerank_stream_v_layout says where they
+ *       are (an all-gather of the owned rows of a [N, cap] float32 array).
+ *   ieee_rerank_stream_finish builds the query expansion and the inverted index of the gallery window [g0, g0 + Gs) from
+ *   rank and V of every sample; the workspace then serves block calls for that window only.
+ *   ieee_rerank_stream_block_window re-ranks the distances of queries [row0, row0 + rows) to the window's Gs gallery rows
+ *   (float32 [rows, Gs], leading dim ld), in place: the same bits as columns [g0, g0 + Gs) of ieee_rerank_stream_block on
+ *   the whole gallery's distances.  scratch holds rows * Gs floats.
+ *   ieee_rerank_stream_window_workspace_bytes: V of N rows plus expansion and index of Q + Gs rows, about
+ *   8 c N + 16 k2 c (Q + Gs) bytes with c = (k1+1)(round(k1/2)+2) (k2 = 1: 8 c N + 8 c (Q + Gs)); for Gs = G it is
+ *   ieee_rerank_stream_workspace_bytes.  Returns 0 with ieee_last_error set when out of range.
+ *   ieee_rerank_stream_v_layout: V in the workspace is three arrays of N rows, cap entries each: columns (int32 [N, cap])
+ *   at byte offset off_col, values (float32 [N, cap]) at off_val, counts (int32 [N]) at off_cnt; row i holds cnt[i] valid
+ *   entries.  The same for every window.  Needs no GPU.
+ * ---------------------------------------------------------------------------------------------- */
+size_t ieee_rerank_stream_window_workspace_bytes(int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t Gs);
+int ieee_rerank_stream_v_layout(int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t* cap, size_t* off_col, size_t* off_val,
+                                size_t* off_cnt);
+int ieee_rerank_stream_pass(int32_t pass, const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D,
+                            int metric, int precision, int32_t k1, int32_t k2, size_t strip_bytes, int64_t q0, int64_t q1,
+                            int64_t g0, int64_t g1, float* colmax, int32_t* rank, void* workspace, size_t workspace_bytes,
+                            void* scratch, size_t scratch_bytes, ieee_stream_t stream);
+int ieee_rerank_stream_finish(void* workspace, size_t workspace_bytes, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t g0,
+                              int64_t Gs, const int32_t* rank, ieee_stream_t stream);
+int ieee_rerank_stream_block_window(const void* workspace, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t Gs,
+                                    const float* colmax, int64_t row0, int64_t rows, double lambda_value, float* block,
+                                    int64_t ld, void* scratch, size_t scratch_bytes, ieee_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------
  * GNN re-ranking (alternative `rerank` mode).   Replaces torchreid/utils/GPU-Re-Ranking/gnn_reranking.py:27-59 with its
  * extensions build_adjacency_matrix_kernel.cu:10-17 and gnn_propagate_kernel.cu:8-22.
