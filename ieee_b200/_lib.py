@@ -93,6 +93,13 @@ SIGNATURES = {
     "ieee_gnn_stream_graph_bytes_sync": (C.c_int, [vp, i64, i64, i32, i32, vp, sz, C.POINTER(i64), vp]),
     "ieee_gnn_stream_graph": (C.c_int, [vp, vp, i64, i64, i32, i32, vp, sz, vp, sz, C.POINTER(i64), vp, vp, vp, vp, vp, vp, vp]),
     "ieee_gnn_stream_block": (C.c_int, [vp, vp, vp, vp, vp, vp, i64, i64, i64, i64, vp, i64, vp, sz, vp]),
+    "ieee_gnn_stream_neighbours_rows": (C.c_int, [vp, i64, vp, i64, i64, C.c_int, i32, sz, i64, i64, i64, i64, vp, vp, vp, sz, vp]),
+    "ieee_gnn_stream_layout": (C.c_int, [i64, i64, i32, i32, C.POINTER(i64), C.POINTER(sz)]),
+    "ieee_gnn_stream_symbolic": (C.c_int, [vp, i64, i64, i32, i32, i64, i64, i64, i64, vp, sz, vp]),
+    "ieee_gnn_stream_sizes_sync": (C.c_int, [i64, i64, i32, i32, vp, sz, C.POINTER(i64), vp]),
+    "ieee_gnn_stream_numeric": (C.c_int, [i32, vp, vp, i64, i64, i32, i32, i64, i64, i64, i64, vp, sz, vp, sz, C.POINTER(i64), vp, vp,
+                                          vp, vp]),
+    "ieee_gnn_stream_csc": (C.c_int, [i64, i64, i32, i64, i64, i64, i64, vp, sz, vp, vp, vp, vp, vp, vp, vp]),
 }
 
 MAX_PEERS = 16

@@ -144,6 +144,20 @@ int gnn_stream_graph_bytes_sync(const int32_t* rank, int64_t Q, int64_t G, int32
 int gnn_stream_graph(const int32_t* rank, const float* S, int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch,
                      size_t scratch_bytes, void* work, size_t work_bytes, const int64_t* sizes, int64_t* a_ptr, int32_t* a_col,
                      float* a_val, int64_t* g_ptr, int32_t* g_row, float* g_val, cudaStream_t stream);
+int gnn_stream_neighbours_rows(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int precision,
+                               int32_t k1, size_t strip_bytes, int64_t q0, int64_t q1, int64_t g0, int64_t g1, int32_t* rank,
+                               float* S, void* scratch, size_t scratch_bytes, cudaStream_t stream, int cta_group);
+int gnn_stream_layout(int64_t Q, int64_t G, int32_t k1, int32_t k2, const int64_t* sizes, size_t* off);
+int gnn_stream_symbolic(const int32_t* rank, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t q0, int64_t q1, int64_t g0,
+                        int64_t g1, void* scratch, size_t scratch_bytes, cudaStream_t stream);
+int gnn_stream_sizes_sync(int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch, size_t scratch_bytes, int64_t* sizes,
+                          cudaStream_t stream);
+int gnn_stream_numeric(int step, const int32_t* rank, const float* S, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t q0,
+                       int64_t q1, int64_t g0, int64_t g1, void* scratch, size_t scratch_bytes, void* work, size_t work_bytes,
+                       const int64_t* sizes, int64_t* a_ptr, int32_t* a_col, float* a_val, cudaStream_t stream);
+int gnn_stream_csc(int64_t Q, int64_t G, int32_t k1, int64_t q0, int64_t q1, int64_t g0, int64_t g1, void* scratch,
+                   size_t scratch_bytes, const int64_t* a_ptr, const int32_t* a_col, const float* a_val, int64_t* g_ptr,
+                   int32_t* g_row, float* g_val, cudaStream_t stream);
 int gnn_stream_block(const int64_t* a_ptr, const int32_t* a_col, const float* a_val, const int64_t* g_ptr, const int32_t* g_row,
                      const float* g_val, int64_t Q, int64_t G, int64_t row0, int64_t rows, float* block, int64_t ld,
                      void* scratch, size_t scratch_bytes, cudaStream_t stream);
@@ -840,6 +854,52 @@ int ieee_gnn_stream_block(const int64_t* a_ptr, const int32_t* a_col, const floa
   if (rc) return rc;
   return gnn_stream_block(a_ptr, a_col, a_val, g_ptr, g_row, g_val, Q, G, row0, rows, block, ld, scratch, scratch_bytes,
                           (cudaStream_t)stream);
+}
+
+int ieee_gnn_stream_neighbours_rows(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int precision,
+                                    int32_t k1, size_t strip_bytes, int64_t q0, int64_t q1, int64_t g0, int64_t g1, int32_t* rank,
+                                    float* S, void* scratch, size_t scratch_bytes, ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return gnn_stream_neighbours_rows(q_packed, Q, g_packed, G, D, precision, k1, strip_bytes, q0, q1, g0, g1, rank, S, scratch,
+                                    scratch_bytes, (cudaStream_t)stream, cta_group_default());
+}
+
+int ieee_gnn_stream_layout(int64_t Q, int64_t G, int32_t k1, int32_t k2, const int64_t* sizes, size_t* off) {
+  return gnn_stream_layout(Q, G, k1, k2, sizes, off);
+}
+
+int ieee_gnn_stream_symbolic(const int32_t* rank, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t q0, int64_t q1, int64_t g0,
+                             int64_t g1, void* scratch, size_t scratch_bytes, ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return gnn_stream_symbolic(rank, Q, G, k1, k2, q0, q1, g0, g1, scratch, scratch_bytes, (cudaStream_t)stream);
+}
+
+int ieee_gnn_stream_sizes_sync(int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch, size_t scratch_bytes, int64_t* sizes,
+                               ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return gnn_stream_sizes_sync(Q, G, k1, k2, scratch, scratch_bytes, sizes, (cudaStream_t)stream);
+}
+
+int ieee_gnn_stream_numeric(int32_t step, const int32_t* rank, const float* S, int64_t Q, int64_t G, int32_t k1, int32_t k2,
+                            int64_t q0, int64_t q1, int64_t g0, int64_t g1, void* scratch, size_t scratch_bytes, void* work,
+                            size_t work_bytes, const int64_t* sizes, int64_t* a_ptr, int32_t* a_col, float* a_val,
+                            ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return gnn_stream_numeric(step, rank, S, Q, G, k1, k2, q0, q1, g0, g1, scratch, scratch_bytes, work, work_bytes, sizes, a_ptr,
+                            a_col, a_val, (cudaStream_t)stream);
+}
+
+int ieee_gnn_stream_csc(int64_t Q, int64_t G, int32_t k1, int64_t q0, int64_t q1, int64_t g0, int64_t g1, void* scratch,
+                        size_t scratch_bytes, const int64_t* a_ptr, const int32_t* a_col, const float* a_val, int64_t* g_ptr,
+                        int32_t* g_row, float* g_val, ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return gnn_stream_csc(Q, G, k1, q0, q1, g0, g1, scratch, scratch_bytes, a_ptr, a_col, a_val, g_ptr, g_row, g_val,
+                        (cudaStream_t)stream);
 }
 
 // ---- peer exchange (gallery sharded over the GPUs of one box) ---------------------------------------------------

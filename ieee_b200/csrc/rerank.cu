@@ -975,6 +975,15 @@ struct SpRows {                            // CSR rows (idx = columns) or CSC co
   __device__ __forceinline__ float v(int64_t p) const { return val ? val[p] : 1.0f; }
 };
 
+// The rows (or columns) a call covers: [a0, a0 + na), then [b0, b0 + nb) -- a process's queries, then its gallery rows,
+// as indices among all N samples.  Block i of a launch over count() rows takes row(i); the whole range is {0, Q, Q, G}.
+struct GnnRows {
+  int a0, na, b0, nb;
+  __host__ __device__ int count() const { return na + nb; }
+  __device__ __forceinline__ int row(int i) const { return i < na ? a0 + i : b0 + i - na; }
+  __device__ __forceinline__ bool owns(int c) const { return (c >= a0 && c < a0 + na) || (c >= b0 && c < b0 + nb); }
+};
+
 __device__ __forceinline__ void bm_set(uint32_t* bm, int c) { atomicOr(bm + (c >> 5), 1u << (c & 31)); }
 
 __device__ void bm_clear(uint32_t* bm, int nw) {
@@ -1065,11 +1074,12 @@ __device__ void set_a1t(uint32_t* bm, const SpRows& a0, const SpRows& t0, const 
 
 // symbolic phase: per row the nnz of B1, A1, B2, A2
 __global__ void __launch_bounds__(kGnnThreads) gnn_symbolic_kernel(SpRows a0, SpRows t0, SpRows k2inv, int N, int k2,
-                                                                    int32_t* __restrict__ cnt_b1, int32_t* __restrict__ cnt_a1,
-                                                                    int32_t* __restrict__ cnt_b2, int32_t* __restrict__ cnt_a2) {
+                                                                    GnnRows own, int32_t* __restrict__ cnt_b1,
+                                                                    int32_t* __restrict__ cnt_a1, int32_t* __restrict__ cnt_b2,
+                                                                    int32_t* __restrict__ cnt_a2) {
   extern __shared__ __align__(16) uint32_t bm[];
   __shared__ int wsum[kGnnThreads / 32];
-  const int r = blockIdx.x, nw = (N + 31) >> 5;
+  const int r = own.row(blockIdx.x), nw = (N + 31) >> 5;
   bm_clear(bm, nw);
   set_b1(bm, a0, t0, r, threadIdx.x, kGnnThreads);
   int n = bm_count(bm, nw, wsum);
@@ -1094,11 +1104,12 @@ __global__ void __launch_bounds__(kGnnThreads) gnn_symbolic_kernel(SpRows a0, Sp
 
 // B = A + A^T row by row: ascending columns of A[r] u T[r]; values (0 + A[r][c]) + A[c][r], which is the dense
 // A[r][c] + A[c][r] (gnn_symmetrise_kernel) for every pattern of presence
-__global__ void __launch_bounds__(kGnnThreads) gnn_sum_kernel(SpRows a, SpRows t, int N, const int64_t* __restrict__ bptr,
-                                                               int32_t* __restrict__ bcol, float* __restrict__ bval) {
+__global__ void __launch_bounds__(kGnnThreads) gnn_sum_kernel(SpRows a, SpRows t, int N, GnnRows own,
+                                                               const int64_t* __restrict__ bptr, int32_t* __restrict__ bcol,
+                                                               float* __restrict__ bval) {
   extern __shared__ __align__(16) uint32_t bm[];
   __shared__ int wsum[kGnnThreads / 32];
-  const int r = blockIdx.x, nw = (N + 31) >> 5;
+  const int r = own.row(blockIdx.x), nw = (N + 31) >> 5;
   const int64_t b0 = bptr[r], b1 = bptr[r + 1];
   bm_clear(bm, nw);
   set_row(bm, a, r, threadIdx.x, kGnnThreads);
@@ -1124,15 +1135,15 @@ __global__ void __launch_bounds__(kGnnThreads) gnn_sum_kernel(SpRows a, SpRows t
 // shuffle tree, warp sum and square root
 __global__ void __launch_bounds__(kGnnThreads) gnn_propagate_rows_kernel(SpRows b, const int32_t* __restrict__ rank,
                                                                           const float* __restrict__ S, int k1, int k2, int N,
-                                                                          const int64_t* __restrict__ aptr, int32_t* __restrict__ acol,
-                                                                          float* __restrict__ aval) {
+                                                                          GnnRows own, const int64_t* __restrict__ aptr,
+                                                                          int32_t* __restrict__ acol, float* __restrict__ aval) {
   extern __shared__ __align__(16) uint32_t bm[];
   __shared__ int wsum[kGnnThreads / 32];
   __shared__ int32_t chunk_c[kGnnThreads];
   __shared__ float chunk_v[kGnnThreads];
   __shared__ float red[kGnnThreads / 32];
   __shared__ float nrm_s;
-  const int i = blockIdx.x, nw = (N + 31) >> 5;
+  const int i = own.row(blockIdx.x), nw = (N + 31) >> 5;
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int64_t a0 = aptr[i], a1 = aptr[i + 1];
   const int32_t* nb = rank + (int64_t)i * k1;
@@ -1239,14 +1250,22 @@ __global__ void gnn_iota_kernel(int64_t* __restrict__ ptr, int64_t n, int step) 
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i <= n) ptr[i] = i * step;
 }
-// the gallery CSC: each column's rows ascending (a bitmap of G bits), values looked up in the CSR rows
+// the gallery CSC: each owned column's rows ascending (a bitmap of G bits), values looked up in the CSR rows; every
+// other column's entries are set to 0, so that summing the processes' CSCs as integers assembles the whole one
 __global__ void __launch_bounds__(kGnnThreads) gnn_col_sort_kernel(const int64_t* __restrict__ gptr, int32_t* __restrict__ grow,
-                                                                    float* __restrict__ gval, SpRows a, int Q, int G) {
+                                                                    float* __restrict__ gval, SpRows a, int Q, int G, GnnRows own) {
   extern __shared__ __align__(16) uint32_t bm[];
   __shared__ int wsum[kGnnThreads / 32];
   const int c = blockIdx.x, nw = (G + 31) >> 5;
   const int64_t p0 = gptr[c], p1 = gptr[c + 1];
   if (p0 == p1) return;
+  if (!own.owns(c)) {
+    for (int64_t p = p0 + threadIdx.x; p < p1; p += kGnnThreads) {
+      grow[p] = 0;
+      gval[p] = 0.f;
+    }
+    return;
+  }
   bm_clear(bm, nw);
   for (int64_t p = p0 + threadIdx.x; p < p1; p += kGnnThreads) bm_set(bm, grow[p]);
   bm_emit(bm, nw, grow + p0, wsum);
@@ -1327,13 +1346,29 @@ size_t gnn_stream_scratch_bytes(int64_t Q, int64_t G, int32_t k1, size_t strip_b
   return gnn_scratch_plan(Q, G, k1, strip_bytes).total;
 }
 
-int gnn_stream_neighbours(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int precision, int32_t k1,
-                          size_t strip_bytes, int32_t* rank, float* S, void* scratch, size_t scratch_bytes, cudaStream_t stream,
-                          int cta_group) {
+// The owned rows [q0, q1) and [g0, g1) of the phase calls: each empty, or starting at a multiple of 256 of its segment and
+// ending at one or at the segment's end.
+static int gnn_owned(const char* who, int64_t Q, int64_t G, int64_t q0, int64_t q1, int64_t g0, int64_t g1, GnnRows* own) {
+  auto range_ok = [](int64_t a, int64_t b, int64_t n) {
+    return a == b ? 0 <= a && a <= n : 0 <= a && a < b && b <= n && a % 256 == 0 && (b == n || b % 256 == 0);
+  };
+  IEEE_REQUIRE(range_ok(q0, q1, Q) && range_ok(g0, g1, G),
+               "%s: owned rows [%lld, %lld) of %lld queries and [%lld, %lld) of %lld gallery rows must start at a multiple "
+               "of 256 and end at one or at the end, or be empty", who, (long long)q0, (long long)q1, (long long)Q, (long long)g0,
+               (long long)g1, (long long)G);
+  *own = GnnRows{(int)q0, (int)(q1 - q0), (int)(Q + g0), (int)(g1 - g0)};
+  return IEEE_OK;
+}
+
+int gnn_stream_neighbours_rows(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int precision,
+                               int32_t k1, size_t strip_bytes, int64_t q0, int64_t q1, int64_t g0, int64_t g1, int32_t* rank,
+                               float* S, void* scratch, size_t scratch_bytes, cudaStream_t stream, int cta_group) {
   IEEE_REQUIRE(q_packed && g_packed && rank && S && scratch, "gnn_stream_neighbours: null pointer");
   IEEE_REQUIRE(D > 0, "gnn_stream_neighbours: bad feature width D=%lld", (long long)D);
   int rc = gnn_stream_check("gnn_stream_neighbours", Q, G, k1, 1);
   if (rc) return rc;
+  GnnRows own;
+  if ((rc = gnn_owned("gnn_stream_neighbours", Q, G, q0, q1, g0, g1, &own))) return rc;
   IEEE_REQUIRE(precision == IEEE_PREC_F16X3 || precision == IEEE_PREC_BF16,
                "gnn_stream_neighbours: precision %d has no tensor-core contraction", precision);
   IEEE_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 255) == 0, "gnn_stream_neighbours: scratch must be 256-byte aligned");
@@ -1353,9 +1388,9 @@ int gnn_stream_neighbours(const void* q_packed, int64_t Q, const void* g_packed,
   // tile: the strips give the bits of the whole -(X_u X_u^T) product
   for (int seg = 0; seg < 2; ++seg) {
     const bool gal = seg == 1;
-    const int64_t n_seg = gal ? G : Q;
-    for (int64_t r0 = 0; r0 < n_seg; r0 += s.W) {
-      const int64_t wr = (n_seg - r0) < s.W ? (n_seg - r0) : s.W;
+    const int64_t a = gal ? g0 : q0, b = gal ? g1 : q1;
+    for (int64_t r0 = a; r0 < b; r0 += s.W) {
+      const int64_t wr = (b - r0) < s.W ? (b - r0) : s.W;
       const int64_t i0 = (gal ? Q : 0) + r0;
       if ((rc = distmat_umma_rows(rows_of(gal, r0, wr), rows_of(false, 0, Q), IEEE_METRIC_NEG_DOT, precision, strip, s.ld, stream,
                                   cta_group, nullptr, false)))
@@ -1371,6 +1406,13 @@ int gnn_stream_neighbours(const void* q_packed, int64_t Q, const void* g_packed,
   }
   IEEE_CUDA_CHECK(cudaGetLastError());
   return IEEE_OK;
+}
+
+int gnn_stream_neighbours(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int precision, int32_t k1,
+                          size_t strip_bytes, int32_t* rank, float* S, void* scratch, size_t scratch_bytes, cudaStream_t stream,
+                          int cta_group) {
+  return gnn_stream_neighbours_rows(q_packed, Q, g_packed, G, D, precision, k1, strip_bytes, 0, Q, 0, G, rank, S, scratch,
+                                    scratch_bytes, stream, cta_group);
 }
 
 // The index of the graph calls, and the offsets of the numeric phase's work buffer (B1, A1, A1^T, B2).
@@ -1444,15 +1486,62 @@ static int gnn_sparse_transpose(const SpRows& a, int64_t N, int r0, int r1, int 
   return IEEE_OK;
 }
 
-int gnn_stream_graph_bytes_sync(const int32_t* rank, int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch,
-                                size_t scratch_bytes, int64_t* sizes, cudaStream_t stream) {
-  IEEE_REQUIRE(rank && scratch && sizes, "gnn_stream_graph_bytes_sync: null pointer");
-  int rc = gnn_stream_check("gnn_stream_graph_bytes_sync", Q, G, k1, k2);
+int gnn_stream_layout(int64_t Q, int64_t G, int32_t k1, int32_t k2, const int64_t* sizes, size_t* off) {
+  IEEE_REQUIRE(off, "gnn_stream_layout: null pointer");
+  int rc = gnn_stream_check("gnn_stream_layout", Q, G, k1, k2);
   if (rc) return rc;
-  IEEE_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 255) == 0, "gnn_stream_graph_bytes_sync: scratch must be 256-byte aligned");
+  const GnnScratch s = gnn_scratch_plan(Q, G, k1, 0);
+  for (int i = 0; i < 4; ++i) off[i] = s.off_cntr[i];
+  if (sizes) {
+    const GnnWork w = gnn_work_plan(Q + G, k2, sizes[3], sizes[4], sizes[5]);
+    const size_t o[6] = {w.off_b1c, w.off_b1v, w.off_a1c, w.off_a1v, w.off_b2c, w.off_b2v};
+    for (int i = 0; i < 6; ++i) off[4 + i] = o[i];
+  }
+  return IEEE_OK;
+}
+
+// index of the graph calls (A0's row offsets, T0, K2inv; every process builds all of it), then the nnz of B1, A1, B2 and
+// A2 of the owned rows; k2 == 1 has nothing to count (A2 = A0)
+int gnn_stream_symbolic(const int32_t* rank, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t q0, int64_t q1, int64_t g0,
+                        int64_t g1, void* scratch, size_t scratch_bytes, cudaStream_t stream) {
+  IEEE_REQUIRE(rank && scratch, "gnn_stream_symbolic: null pointer");
+  int rc = gnn_stream_check("gnn_stream_symbolic", Q, G, k1, k2);
+  if (rc) return rc;
+  GnnRows own;
+  if ((rc = gnn_owned("gnn_stream_symbolic", Q, G, q0, q1, g0, g1, &own))) return rc;
+  IEEE_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 255) == 0, "gnn_stream_symbolic: scratch must be 256-byte aligned");
   const GnnScratch s = gnn_scratch_plan(Q, G, k1, 0);
   if (scratch_bytes < s.index) {
-    set_error("gnn_stream_graph_bytes_sync: scratch too small (%zu < %zu)", scratch_bytes, s.index);
+    set_error("gnn_stream_symbolic: scratch too small (%zu < %zu)", scratch_bytes, s.index);
+    return IEEE_ERR_WORKSPACE;
+  }
+  if (k2 == 1) return IEEE_OK;
+  const int64_t N = Q + G;
+  const GnnIndex x = gnn_index(s, scratch);
+  gnn_iota_kernel<<<(unsigned)((N + 256) / 256), 256, 0, stream>>>(x.a0p, N, k1);
+  count_launch();
+  if ((rc = gnn_rank_transpose(rank, N, k1, k1, x, x.t0p, x.t0i, stream))) return rc;
+  if ((rc = gnn_rank_transpose(rank, N, k1, k2, x, x.k2p, x.k2i, stream))) return rc;
+  const SpRows a0{x.a0p, rank, nullptr}, t0{x.t0p, x.t0i, nullptr}, k2inv{x.k2p, x.k2i, nullptr};
+  const size_t smem = gnn_bitmap_smem(N);
+  IEEE_ENSURE_DYN_SMEM(gnn_symbolic_kernel, smem);
+  if (own.count())
+    gnn_symbolic_kernel<<<(unsigned)own.count(), kGnnThreads, smem, stream>>>(a0, t0, k2inv, (int)N, k2, own, x.cntr[0], x.cntr[1],
+                                                                              x.cntr[2], x.cntr[3]);
+  if (own.count()) count_launch();
+  IEEE_CUDA_CHECK(cudaGetLastError());
+  return IEEE_OK;
+}
+
+// row offsets of B1, A1, B2, A2 from the counts of all N rows, and the one wait for their totals
+int gnn_stream_sizes_sync(int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch, size_t scratch_bytes, int64_t* sizes,
+                          cudaStream_t stream) {
+  IEEE_REQUIRE(scratch && sizes, "gnn_stream_sizes_sync: null pointer");
+  int rc = gnn_stream_check("gnn_stream_sizes_sync", Q, G, k1, k2);
+  if (rc) return rc;
+  const GnnScratch s = gnn_scratch_plan(Q, G, k1, 0);
+  if (scratch_bytes < s.index) {
+    set_error("gnn_stream_sizes_sync: scratch too small (%zu < %zu)", scratch_bytes, s.index);
     return IEEE_ERR_WORKSPACE;
   }
   const int64_t N = Q + G;
@@ -1460,16 +1549,6 @@ int gnn_stream_graph_bytes_sync(const int32_t* rank, int64_t Q, int64_t G, int32
   int64_t tot[4] = {N * k1, N * k1, N * k1, N * k1};     // nnz of B1, A1, B2, A2 (k2 == 1: A2 = A0)
   int64_t nnz_gal = G * k1;
   if (k2 != 1) {
-    gnn_iota_kernel<<<(unsigned)((N + 256) / 256), 256, 0, stream>>>(x.a0p, N, k1);
-    count_launch();
-    if ((rc = gnn_rank_transpose(rank, N, k1, k1, x, x.t0p, x.t0i, stream))) return rc;
-    if ((rc = gnn_rank_transpose(rank, N, k1, k2, x, x.k2p, x.k2i, stream))) return rc;
-    const SpRows a0{x.a0p, rank, nullptr}, t0{x.t0p, x.t0i, nullptr}, k2inv{x.k2p, x.k2i, nullptr};
-    const size_t smem = gnn_bitmap_smem(N);
-    IEEE_ENSURE_DYN_SMEM(gnn_symbolic_kernel, smem);
-    gnn_symbolic_kernel<<<(unsigned)N, kGnnThreads, smem, stream>>>(a0, t0, k2inv, (int)N, k2, x.cntr[0], x.cntr[1], x.cntr[2],
-                                                                     x.cntr[3]);
-    count_launch();
     for (int i = 0; i < 4; ++i) {
       gnn_scan64_kernel<<<1, 1024, 0, stream>>>(x.cntr[i], N, x.ptr[i]);
       count_launch();
@@ -1481,13 +1560,128 @@ int gnn_stream_graph_bytes_sync(const int32_t* rank, int64_t Q, int64_t G, int32
     for (int i = 0; i < 4; ++i) tot[i] = host[i];
     nnz_gal = host[3] - host[4];
   }
-  IEEE_REQUIRE(tot[3] < (int64_t(1) << 40), "gnn_stream_graph_bytes_sync: nnz overflow");
+  IEEE_REQUIRE(tot[3] < (int64_t(1) << 40), "gnn_stream_sizes_sync: nnz overflow");
   sizes[0] = tot[3];
   sizes[1] = nnz_gal;
   sizes[2] = (int64_t)gnn_work_plan(N, k2, tot[0], tot[1], tot[2]).total;
   sizes[3] = tot[0];
   sizes[4] = tot[1];
   sizes[5] = tot[2];
+  return IEEE_OK;
+}
+
+int gnn_stream_graph_bytes_sync(const int32_t* rank, int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch,
+                                size_t scratch_bytes, int64_t* sizes, cudaStream_t stream) {
+  IEEE_REQUIRE(sizes, "gnn_stream_graph_bytes_sync: null pointer");
+  int rc = gnn_stream_symbolic(rank, Q, G, k1, k2, 0, Q, 0, G, scratch, scratch_bytes, stream);
+  if (rc) return rc;
+  return gnn_stream_sizes_sync(Q, G, k1, k2, scratch, scratch_bytes, sizes, stream);
+}
+
+// One step of the numeric phase over the owned rows: 0 B1 = A0 + A0^T, 1 A1 = P(B1), 2 A1^T (all rows, from the whole
+// A1) and B2 = A1 + A1^T, 3 A2 = P(B2) (k2 == 1: A2 = A0) into a_ptr (all rows) and a_col / a_val.  When the owned rows
+// are not all N rows, the entries of every other row are set to 0 (see gnn_col_sort_kernel).
+int gnn_stream_numeric(int step, const int32_t* rank, const float* S, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t q0,
+                       int64_t q1, int64_t g0, int64_t g1, void* scratch, size_t scratch_bytes, void* work, size_t work_bytes,
+                       const int64_t* sizes, int64_t* a_ptr, int32_t* a_col, float* a_val, cudaStream_t stream) {
+  IEEE_REQUIRE(step >= 0 && step <= 3, "gnn_stream_numeric: step must be 0 to 3, got %d", step);
+  IEEE_REQUIRE(rank && S && scratch && work && sizes && (step < 3 || (a_ptr && a_col && a_val)), "gnn_stream_numeric: null pointer");
+  int rc = gnn_stream_check("gnn_stream_numeric", Q, G, k1, k2);
+  if (rc) return rc;
+  IEEE_REQUIRE(k2 != 1 || step == 3, "gnn_stream_numeric: with k2 = 1 there is only step 3 (A2 = A0), got step %d", step);
+  GnnRows own;
+  if ((rc = gnn_owned("gnn_stream_numeric", Q, G, q0, q1, g0, g1, &own))) return rc;
+  IEEE_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 255) == 0 && (reinterpret_cast<uintptr_t>(work) & 255) == 0,
+               "gnn_stream_numeric: scratch and work must be 256-byte aligned");
+  const int64_t N = Q + G;
+  const GnnScratch s = gnn_scratch_plan(Q, G, k1, 0);
+  const GnnWork wp = gnn_work_plan(N, k2, sizes[3], sizes[4], sizes[5]);
+  if (scratch_bytes < s.index || work_bytes < wp.total) {
+    set_error("gnn_stream_numeric: scratch or work too small (%zu < %zu or %zu < %zu)", scratch_bytes, s.index, work_bytes,
+              wp.total);
+    return IEEE_ERR_WORKSPACE;
+  }
+  const bool part = own.count() != N;
+  const unsigned rows = (unsigned)own.count();
+  const GnnIndex x = gnn_index(s, scratch);
+  const size_t smem = gnn_bitmap_smem(N);
+  uint8_t* w = static_cast<uint8_t*>(work);
+  int32_t* b1c = reinterpret_cast<int32_t*>(w + wp.off_b1c);
+  float* b1v = reinterpret_cast<float*>(w + wp.off_b1v);
+  int32_t* a1c = reinterpret_cast<int32_t*>(w + wp.off_a1c);
+  float* a1v = reinterpret_cast<float*>(w + wp.off_a1v);
+  int32_t* b2c = reinterpret_cast<int32_t*>(w + wp.off_b2c);
+  float* b2v = reinterpret_cast<float*>(w + wp.off_b2v);
+  auto clear = [&](void* col, void* val, int64_t nnz) -> int {
+    if (part && nnz) {
+      IEEE_CUDA_CHECK(cudaMemsetAsync(col, 0, size_t(nnz) * 4, stream));
+      IEEE_CUDA_CHECK(cudaMemsetAsync(val, 0, size_t(nnz) * 4, stream));
+    }
+    return IEEE_OK;
+  };
+  IEEE_ENSURE_DYN_SMEM(gnn_sum_kernel, smem);
+  IEEE_ENSURE_DYN_SMEM(gnn_propagate_rows_kernel, smem);
+  if (step == 0) {            // B1 = A0 + A0^T
+    if ((rc = clear(b1c, b1v, sizes[3]))) return rc;
+    if (rows)
+      gnn_sum_kernel<<<rows, kGnnThreads, smem, stream>>>(SpRows{x.a0p, rank, nullptr}, SpRows{x.t0p, x.t0i, nullptr}, (int)N, own,
+                                                          x.ptr[0], b1c, b1v);
+  } else if (step == 1) {     // A1 = P(B1)
+    if ((rc = clear(a1c, a1v, sizes[4]))) return rc;
+    if (rows)
+      gnn_propagate_rows_kernel<<<rows, kGnnThreads, smem, stream>>>(SpRows{x.ptr[0], b1c, b1v}, rank, S, k1, k2, (int)N, own,
+                                                                     x.ptr[1], a1c, a1v);
+  } else if (step == 2) {     // B2 = A1 + A1^T
+    int64_t* tp = reinterpret_cast<int64_t*>(w + wp.off_tp);
+    int32_t* ti = reinterpret_cast<int32_t*>(w + wp.off_ti);
+    float* tv = reinterpret_cast<float*>(w + wp.off_tv);
+    const SpRows a1{x.ptr[1], a1c, a1v};
+    if ((rc = gnn_sparse_transpose(a1, N, 0, (int)N, 0, x, tp, ti, tv, stream))) return rc;
+    if ((rc = clear(b2c, b2v, sizes[5]))) return rc;
+    if (rows) gnn_sum_kernel<<<rows, kGnnThreads, smem, stream>>>(a1, SpRows{tp, ti, tv}, (int)N, own, x.ptr[2], b2c, b2v);
+  } else if (k2 == 1) {       // A2 = A0: the neighbour lists with ascending columns, all values 1
+    gnn_iota_kernel<<<(unsigned)((N + 256) / 256), 256, 0, stream>>>(a_ptr, N, k1);
+    count_launch();
+    if ((rc = clear(a_col, a_val, sizes[0]))) return rc;
+    if (rows)
+      gnn_sum_kernel<<<rows, kGnnThreads, smem, stream>>>(SpRows{a_ptr, rank, nullptr}, SpRows{nullptr, nullptr, nullptr}, (int)N,
+                                                          own, a_ptr, a_col, a_val);
+  } else {                    // A2 = P(B2)
+    IEEE_CUDA_CHECK(cudaMemcpyAsync(a_ptr, x.ptr[3], size_t(N + 1) * 8, cudaMemcpyDeviceToDevice, stream));
+    if ((rc = clear(a_col, a_val, sizes[0]))) return rc;
+    if (rows)
+      gnn_propagate_rows_kernel<<<rows, kGnnThreads, smem, stream>>>(SpRows{x.ptr[2], b2c, b2v}, rank, S, k1, k2, (int)N, own,
+                                                                     a_ptr, a_col, a_val);
+  }
+  count_launch();
+  IEEE_CUDA_CHECK(cudaGetLastError());
+  return IEEE_OK;
+}
+
+// the gallery rows of A2 (all of them) as CSC, rows ascending in the owned columns (the owned rows' indices)
+int gnn_stream_csc(int64_t Q, int64_t G, int32_t k1, int64_t q0, int64_t q1, int64_t g0, int64_t g1, void* scratch,
+                   size_t scratch_bytes, const int64_t* a_ptr, const int32_t* a_col, const float* a_val, int64_t* g_ptr,
+                   int32_t* g_row, float* g_val, cudaStream_t stream) {
+  IEEE_REQUIRE(scratch && a_ptr && a_col && a_val && g_ptr && g_row && g_val, "gnn_stream_csc: null pointer");
+  int rc = gnn_stream_check("gnn_stream_csc", Q, G, k1, 1);
+  if (rc) return rc;
+  GnnRows own;
+  if ((rc = gnn_owned("gnn_stream_csc", Q, G, q0, q1, g0, g1, &own))) return rc;
+  IEEE_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 255) == 0, "gnn_stream_csc: scratch must be 256-byte aligned");
+  const GnnScratch s = gnn_scratch_plan(Q, G, k1, 0);
+  if (scratch_bytes < s.index) {
+    set_error("gnn_stream_csc: scratch too small (%zu < %zu)", scratch_bytes, s.index);
+    return IEEE_ERR_WORKSPACE;
+  }
+  const int64_t N = Q + G;
+  const GnnIndex x = gnn_index(s, scratch);
+  const SpRows a2{a_ptr, a_col, a_val};
+  if ((rc = gnn_sparse_transpose(a2, N, (int)Q, (int)N, (int)Q, x, g_ptr, g_row, nullptr, stream))) return rc;
+  const size_t gsmem = gnn_bitmap_smem(G);
+  IEEE_ENSURE_DYN_SMEM(gnn_col_sort_kernel, gsmem);
+  gnn_col_sort_kernel<<<(unsigned)N, kGnnThreads, gsmem, stream>>>(g_ptr, g_row, g_val, a2, (int)Q, (int)G, own);
+  count_launch();
+  IEEE_CUDA_CHECK(cudaGetLastError());
   return IEEE_OK;
 }
 
@@ -1498,62 +1692,11 @@ int gnn_stream_graph(const int32_t* rank, const float* S, int64_t Q, int64_t G, 
                "gnn_stream_graph: null pointer");
   int rc = gnn_stream_check("gnn_stream_graph", Q, G, k1, k2);
   if (rc) return rc;
-  IEEE_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 255) == 0 && (reinterpret_cast<uintptr_t>(work) & 255) == 0,
-               "gnn_stream_graph: scratch and work must be 256-byte aligned");
-  const int64_t N = Q + G;
-  const GnnScratch s = gnn_scratch_plan(Q, G, k1, 0);
-  const GnnWork wp = gnn_work_plan(N, k2, sizes[3], sizes[4], sizes[5]);
-  if (scratch_bytes < s.index || work_bytes < wp.total) {
-    set_error("gnn_stream_graph: scratch or work too small (%zu < %zu or %zu < %zu)", scratch_bytes, s.index, work_bytes, wp.total);
-    return IEEE_ERR_WORKSPACE;
-  }
-  const GnnIndex x = gnn_index(s, scratch);
-  const size_t smem = gnn_bitmap_smem(N);
-  uint8_t* w = static_cast<uint8_t*>(work);
-  if (k2 == 1) {
-    // A2 = A0: the neighbour lists with ascending columns, all values 1
-    gnn_iota_kernel<<<(unsigned)((N + 256) / 256), 256, 0, stream>>>(a_ptr, N, k1);
-    count_launch();
-    IEEE_ENSURE_DYN_SMEM(gnn_sum_kernel, smem);
-    gnn_sum_kernel<<<(unsigned)N, kGnnThreads, smem, stream>>>(SpRows{a_ptr, rank, nullptr}, SpRows{nullptr, nullptr, nullptr},
-                                                               (int)N, a_ptr, a_col, a_val);
-    count_launch();
-  } else {
-    int32_t* b1c = reinterpret_cast<int32_t*>(w + wp.off_b1c);
-    float* b1v = reinterpret_cast<float*>(w + wp.off_b1v);
-    int32_t* a1c = reinterpret_cast<int32_t*>(w + wp.off_a1c);
-    float* a1v = reinterpret_cast<float*>(w + wp.off_a1v);
-    int64_t* tp = reinterpret_cast<int64_t*>(w + wp.off_tp);
-    int32_t* ti = reinterpret_cast<int32_t*>(w + wp.off_ti);
-    float* tv = reinterpret_cast<float*>(w + wp.off_tv);
-    int32_t* b2c = reinterpret_cast<int32_t*>(w + wp.off_b2c);
-    float* b2v = reinterpret_cast<float*>(w + wp.off_b2v);
-    IEEE_ENSURE_DYN_SMEM(gnn_sum_kernel, smem);
-    IEEE_ENSURE_DYN_SMEM(gnn_propagate_rows_kernel, smem);
-    // B1 = A0 + A0^T, A1 = P(B1)
-    gnn_sum_kernel<<<(unsigned)N, kGnnThreads, smem, stream>>>(SpRows{x.a0p, rank, nullptr}, SpRows{x.t0p, x.t0i, nullptr}, (int)N,
-                                                               x.ptr[0], b1c, b1v);
-    gnn_propagate_rows_kernel<<<(unsigned)N, kGnnThreads, smem, stream>>>(SpRows{x.ptr[0], b1c, b1v}, rank, S, k1, k2, (int)N,
-                                                                          x.ptr[1], a1c, a1v);
-    count_launch(2);
-    // B2 = A1 + A1^T, A2 = P(B2)
-    const SpRows a1{x.ptr[1], a1c, a1v};
-    if ((rc = gnn_sparse_transpose(a1, N, 0, (int)N, 0, x, tp, ti, tv, stream))) return rc;
-    gnn_sum_kernel<<<(unsigned)N, kGnnThreads, smem, stream>>>(a1, SpRows{tp, ti, tv}, (int)N, x.ptr[2], b2c, b2v);
-    IEEE_CUDA_CHECK(cudaMemcpyAsync(a_ptr, x.ptr[3], size_t(N + 1) * 8, cudaMemcpyDeviceToDevice, stream));
-    gnn_propagate_rows_kernel<<<(unsigned)N, kGnnThreads, smem, stream>>>(SpRows{x.ptr[2], b2c, b2v}, rank, S, k1, k2, (int)N,
-                                                                          a_ptr, a_col, a_val);
-    count_launch(2);
-  }
-  // the gallery rows of A2 as CSC, rows ascending
-  const SpRows a2{a_ptr, a_col, a_val};
-  if ((rc = gnn_sparse_transpose(a2, N, (int)Q, (int)N, (int)Q, x, g_ptr, g_row, nullptr, stream))) return rc;
-  const size_t gsmem = gnn_bitmap_smem(G);
-  IEEE_ENSURE_DYN_SMEM(gnn_col_sort_kernel, gsmem);
-  gnn_col_sort_kernel<<<(unsigned)N, kGnnThreads, gsmem, stream>>>(g_ptr, g_row, g_val, a2, (int)Q, (int)G);
-  count_launch();
-  IEEE_CUDA_CHECK(cudaGetLastError());
-  return IEEE_OK;
+  for (int step = k2 == 1 ? 3 : 0; step < 4; ++step)
+    if ((rc = gnn_stream_numeric(step, rank, S, Q, G, k1, k2, 0, Q, 0, G, scratch, scratch_bytes, work, work_bytes, sizes, a_ptr,
+                                 a_col, a_val, stream)))
+      return rc;
+  return gnn_stream_csc(Q, G, k1, 0, Q, 0, G, scratch, scratch_bytes, a_ptr, a_col, a_val, g_ptr, g_row, g_val, stream);
 }
 
 int gnn_stream_block(const int64_t* a_ptr, const int32_t* a_col, const float* a_val, const int64_t* g_ptr, const int32_t* g_row,

@@ -271,12 +271,28 @@ class RetrievalEvaluator:
     (ieee_gnn_stream_*: neighbours from row strips sized by ``block_bytes``, then A as CSR rows and an inverted index of
     its gallery rows), and a query block's distances come from it instead of a contraction.  Same limits on the
     gallery as ``rerank=True``, and no ``group``; 1 <= k2 <= k1 <= min(N, 1024).
+
+    With ``query_group`` (a torch.distributed process group, NCCL) and ``rerank="gnn"``, the ranks of the group share
+    the GNN re-ranking: every rank holds the whole gallery (``gf``, ``g_pids``, ``g_camids``) and is handed the whole
+    query set, and every rank returns what an evaluator without ``query_group`` returns, bit for bit (cmc, mAP, ap,
+    first, mINP and ``ranked_lists`` of all queries).  Each rank owns the queries and gallery rows rerank_owned(Q, G,
+    world, rank) gives: it computes those rows of every stage whose work grows as N^2 (neighbour lists, the symbolic
+    counts, the rows of the adjacency's structures, the sort of the same columns of the CSC) and evaluates its own
+    queries; the stages linear in the adjacency's entries run on every rank (ieee_gnn_stream_neighbours_rows /
+    _symbolic / _sizes_sync / _numeric / _csc).  The per-query results are all-gathered and reduced on every rank.
+    ``return_distmat=True`` returns this rank's own query rows only: rows [q0, q1) of the queries, (q0, q1) =
+    rerank_owned(Q, G, world, rank)[:2] (possibly none).  This buys time, not memory: while the state is built every rank
+    holds B1, A1, B2 and the CSC whole, as one GPU does.  The ranks must agree on G, D, dtype, precision,
+    normalize_feature, k1 and k2 (checked once at construction) and on the number of queries (checked by every
+    evaluate); ValueError on every rank otherwise.  ``query_group`` cannot be combined with ``group``, and plain and
+    k-reciprocal evaluation take ``group`` instead.
     """
 
     def __init__(self, gf: torch.Tensor, g_pids, g_camids, dist_metric: str = "euclidean", normalize_feature: bool = False,
                  precision: str | None = None, max_rank: int = 20, group=None, g_offset: int = 0, g_total: int | None = None,
                  block_bytes: int = DEFAULT_BLOCK_BYTES, center: torch.Tensor | None = None, exchange: str | None = None,
-                 rerank: bool | str = False, k1: int | None = None, k2: int | None = None, lambda_value: float = 0.3):
+                 rerank: bool | str = False, k1: int | None = None, k2: int | None = None, lambda_value: float = 0.3,
+                 query_group=None):
         _lib.require_cuda()
         if dist_metric not in _lib.METRICS:
             raise ValueError('Unknown distance metric: {}. Please choose either "euclidean" or "cosine"'.format(dist_metric))
@@ -288,6 +304,8 @@ class RetrievalEvaluator:
         self.metric, self.normalize = ("neg_dot" if self.gnn else dist_metric), normalize_feature
         self.precision = precision or ("bf16" if gf is not None and gf.dtype == torch.bfloat16 else "f16x3")
         self.rerank = bool(rerank)
+        if query_group is not None:
+            self._check_query_group(query_group, group)
         if k1 is None:
             k1 = 26 if self.gnn else 20
         if k2 is None:
@@ -334,6 +352,54 @@ class RetrievalEvaluator:
         self._label_keys = (_tensor_key(g_pids), _tensor_key(g_camids))
         self._label_refs = (g_pids, g_camids)
         self._slices = self._gallery_slices() if self.rerank and group is not None else None
+        self.query_group = query_group
+        if query_group is not None:
+            self._q_world = torch.distributed.get_world_size(query_group)
+            self._q_rank = torch.distributed.get_rank(query_group)
+            self._check_ranks_agree(gf)
+
+    def _check_query_group(self, query_group, group):
+        if not (torch.distributed.is_available() and isinstance(query_group, torch.distributed.ProcessGroup)):
+            raise ValueError("query_group must be a torch.distributed process group, got {!r}".format(type(query_group).__name__))
+        if group is not None:
+            raise ValueError("query_group (every rank holds the whole gallery) cannot be combined with group (a sharded "
+                             "gallery)")
+        if not self.gnn:
+            raise ValueError('query_group shares GNN re-ranking (rerank="gnn") only: plain and k-reciprocal evaluation run '
+                             "on several GPUs over a sharded gallery with group=")
+
+    def _check_ranks_agree(self, gf):
+        """One all-gather at construction: every rank of query_group must hold the same gallery shape and settings (not
+        block_bytes: the bits depend on neither strip width nor block size).  ValueError on every rank otherwise."""
+        import torch.distributed as dist_
+        mine = [self.G, gf.shape[1], _lib.DTYPES[gf.dtype], _lib.PRECISIONS[self.precision], int(self.normalize), self.k1, self.k2]
+        with torch.cuda.device(self.device):
+            every = torch.empty((self._q_world, len(mine)), dtype=torch.int64, device=self.device)
+            dist_.all_gather_into_tensor(every, torch.tensor(mine, dtype=torch.int64, device=self.device), group=self.query_group)
+            every = every.cpu().tolist()
+        if any(e != every[0] for e in every):
+            raise ValueError("query_group: the ranks disagree on (G, D, dtype, precision, normalize_feature, k1, k2): "
+                             "{}".format([tuple(e) for e in every]))
+
+    def _agree_on_queries(self, qf: torch.Tensor):
+        """One all-gather per evaluation of a query_group: the ranks must hold the same number of queries (ValueError on
+        every rank otherwise), and when any rank has no GNN state for these queries, every rank prepares it anew, so that
+        all of them take part in the same exchanges."""
+        import torch.distributed as dist_
+        key = (_features_key(qf), self.k1, self.k2)
+        fresh = int(self._rr is None or self._rr["key"] != key)
+        every = torch.empty((self._q_world, 2), dtype=torch.int64, device=self.device)
+        dist_.all_gather_into_tensor(every, torch.tensor([qf.shape[0], fresh], dtype=torch.int64, device=self.device),
+                                     group=self.query_group)
+        every = every.cpu().tolist()
+        if any(q != every[0][0] for q, _ in every):
+            raise ValueError("query_group: the ranks hold different numbers of queries: {}".format([q for q, _ in every]))
+        if any(f for _, f in every):
+            self._rr = None
+
+    def _query_range(self, Q: int) -> tuple[int, int]:
+        """Queries [q0, q1) this rank evaluates: its own (rerank_owned) with a query_group, else all of them."""
+        return rerank_owned(Q, self.G, self._q_world, self._q_rank)[:2] if self.query_group is not None else (0, Q)
 
     def _gallery_slices(self):
         """[(g_offset, rows)] of every rank, all-gathered once.  Every rank gets the same list and so reaches the same
@@ -463,18 +529,20 @@ class RetrievalEvaluator:
         del recv
         return PackedFeatures(whole, self.metric, self.normalize, self.precision, self.center)
 
-    def _all_gather_owned(self, t: torch.Tensor, owned, Q: int):
+    def _all_gather_owned(self, t: torch.Tensor, owned, Q: int, group=None):
         """Rows [q0, q1) and [Q + g0, Q + g1) of t ([Q + G, ...]), computed by each rank (owned = rerank_owned of every
-        rank), from that rank into t on every rank: one all-gather, padded to the largest share."""
+        rank), from that rank into t on every rank of `group` (default: the gallery's): one all-gather, padded to the
+        largest share."""
         import torch.distributed as dist_
+        group = self.group if group is None else group
         dev = self.device
         idx = [torch.cat([torch.arange(q0, q1), torch.arange(Q + g0, Q + g1)]).to(dev) for q0, q1, g0, g1 in owned]
         rows = max(len(i) for i in idx)
-        mine = idx[dist_.get_rank(self.group)]
+        mine = idx[dist_.get_rank(group)]
         send = torch.zeros((rows,) + t.shape[1:], dtype=t.dtype, device=dev)
         send[: len(mine)] = t[mine]
-        recv = torch.empty((self.world * rows,) + t.shape[1:], dtype=t.dtype, device=dev)
-        dist_.all_gather_into_tensor(recv, send, group=self.group)
+        recv = torch.empty((len(owned) * rows,) + t.shape[1:], dtype=t.dtype, device=dev)
+        dist_.all_gather_into_tensor(recv, send, group=group)
         at = torch.cat([r * rows + torch.arange(len(i), device=dev) for r, i in enumerate(idx)])
         t[torch.cat(idx)] = recv[at]
 
@@ -499,6 +567,9 @@ class RetrievalEvaluator:
         scratch = torch.empty(sc_bytes, dtype=torch.uint8, device=dev)     # strips, then the graph calls' index
         rank = torch.empty((N, k1), dtype=torch.int32, device=dev)
         S = torch.empty((N, k1), dtype=torch.float32, device=dev)
+        if self.query_group is not None:
+            state = self._gnn_prepare_shared(qpk, gpk, rank, S, scratch)
+            return dict(state, key=key, qf=qf, Q=Q, k1=k1, k2=k2, rank=rank, S=S, scratch_bytes=sc_bytes)
         _lib.call("ieee_gnn_stream_neighbours", qpk.buf.data_ptr(), Q, gpk.buf.data_ptr(), G, D, qpk.precision, k1,
                   self.block_bytes, rank.data_ptr(), S.data_ptr(), scratch.data_ptr(), sc_bytes, _lib.stream())
         TRACE.mark("GNN neighbours")
@@ -520,6 +591,74 @@ class RetrievalEvaluator:
         TRACE.mark("GNN numeric phase")
         return {"key": key, "qf": qf, "Q": Q, "k1": k1, "k2": k2, "rank": rank, "S": S, "a_ptr": a_ptr, "a_col": a_col,
                 "a_val": a_val, "g_ptr": g_ptr, "g_row": g_row, "g_val": g_val, "scratch_bytes": sc_bytes,
+                "work_bytes": work_bytes}
+
+    def _gnn_prepare_shared(self, qpk: PackedFeatures, gpk: PackedFeatures, rank, S, scratch):
+        """_gnn_prepare's calls in phases, shared by the ranks of query_group (all holding the whole gallery and query set):
+        each rank computes the rows it owns (rerank_owned) of every stage whose work grows as N^2, and replicates the
+        stages linear in the adjacency's entries.  Neighbour lists and counts are all-gathered; the CSR structures and
+        the CSC, where every rank holds zeros but in its own rows, are summed as int32 (an exact move of each entry's bits).
+        Every rank ends with the one-GPU rank, S, a_ptr, A's gallery rows and CSC, and its own query rows of A."""
+        import torch.distributed as dist_
+        qg = self.query_group
+        Q, G, k1, k2 = qpk.rows, self.G, self.k1, self.k2
+        N, dev, stream = Q + G, self.device, _lib.stream()
+        owned = [rerank_owned(Q, G, self._q_world, r) for r in range(self._q_world)]
+        own = owned[self._q_rank]
+        sc = (scratch.data_ptr(), scratch.numel())
+
+        def summed(t):
+            dist_.all_reduce(t.view(torch.int32), group=qg)
+
+        _lib.call("ieee_gnn_stream_neighbours_rows", qpk.buf.data_ptr(), Q, gpk.buf.data_ptr(), G, qpk.D, qpk.precision, k1,
+                  self.block_bytes, *own, rank.data_ptr(), S.data_ptr(), *sc, stream)
+        TRACE.mark("GNN neighbours")
+        for t in (rank, S):
+            self._all_gather_owned(t, owned, Q, qg)
+        TRACE.mark("GNN exchange: rank, S")
+        _lib.call("ieee_gnn_stream_symbolic", rank.data_ptr(), Q, G, k1, k2, *own, *sc, stream)
+        TRACE.mark("GNN symbolic phase")
+        off = (C.c_size_t * 10)()
+        _lib.call("ieee_gnn_stream_layout", Q, G, k1, k2, None, off)
+        if k2 != 1:
+            for i in range(4):
+                self._all_gather_owned(scratch[off[i]: off[i] + 4 * N].view(torch.int32), owned, Q, qg)
+        TRACE.mark("GNN exchange: counts")
+        sizes = (C.c_int64 * 6)()
+        _lib.call("ieee_gnn_stream_sizes_sync", Q, G, k1, k2, *sc, sizes, stream)
+        TRACE.mark("GNN sizes")
+        nnz, nnz_g, work_bytes = sizes[0], sizes[1], sizes[2]
+        work = torch.empty(work_bytes, dtype=torch.uint8, device=dev)    # released (stream-ordered) on return
+        a_ptr = torch.empty(N + 1, dtype=torch.int64, device=dev)
+        a_col = torch.empty(nnz, dtype=torch.int32, device=dev)
+        a_val = torch.empty(nnz, dtype=torch.float32, device=dev)
+        g_ptr = torch.empty(N + 1, dtype=torch.int64, device=dev)
+        g_row = torch.empty(nnz_g, dtype=torch.int32, device=dev)
+        g_val = torch.empty(nnz_g, dtype=torch.float32, device=dev)
+        a = (a_ptr.data_ptr(), a_col.data_ptr(), a_val.data_ptr())
+
+        def numeric(step):
+            _lib.call("ieee_gnn_stream_numeric", step, rank.data_ptr(), S.data_ptr(), Q, G, k1, k2, *own, *sc, work.data_ptr(),
+                      work_bytes, sizes, *a, stream)
+            TRACE.mark("GNN numeric step %d" % step)
+
+        if k2 != 1:
+            _lib.call("ieee_gnn_stream_layout", Q, G, k1, k2, sizes, off)
+            for step, n in enumerate((sizes[3], sizes[4], sizes[5])):        # B1, A1, B2: columns and values
+                numeric(step)
+                for o in (off[4 + 2 * step], off[5 + 2 * step]):
+                    summed(work[o: o + 4 * n])
+                TRACE.mark("GNN exchange after step %d" % step)
+        numeric(3)
+        summed(a_col[nnz - nnz_g:])                     # A2's gallery rows: its query rows stay with their owners
+        summed(a_val[nnz - nnz_g:])
+        TRACE.mark("GNN exchange: gallery rows of A")
+        _lib.call("ieee_gnn_stream_csc", Q, G, k1, *own, *sc, *a, g_ptr.data_ptr(), g_row.data_ptr(), g_val.data_ptr(), stream)
+        TRACE.mark("GNN CSC")
+        summed(g_row)
+        summed(g_val)
+        TRACE.mark("GNN exchange: CSC")
+        return {"a_ptr": a_ptr, "a_col": a_col, "a_val": a_val, "g_ptr": g_ptr, "g_row": g_row, "g_val": g_val,
                 "work_bytes": work_bytes}
 
     def _gnn_block(self, s: int, e: int) -> torch.Tensor:
@@ -632,8 +771,9 @@ class RetrievalEvaluator:
         """Iterates over (s, e, distances of queries [s, e)) in blocks of `rows`: each block is packed (block 0 may come
         packed as `pack0`), after `q_event` when the queries are still being copied, contracted against every gallery
         chunk and, on a re-ranking evaluator, re-ranked.  Block 0 is queued before this returns, so the caller can hide
-        host work behind its contraction; every later block when the iteration reaches it, in the same scratch."""
-        Q = qf.shape[0]
+        host work behind its contraction; every later block when the iteration reaches it, in the same scratch.  With a
+        query_group only this rank's queries (_query_range) are iterated."""
+        q0, Q = self._query_range(qf.shape[0])
         self._ensure_block(rows)
 
         def block(s, e, qpk):
@@ -646,12 +786,12 @@ class RetrievalEvaluator:
             dist = self._distance_block(qpk)
             return self._rerank_block(dist, s) if self.rerank else dist
 
-        dist0 = block(0, min(Q, rows), pack0)
+        dist0 = block(q0, min(Q, q0 + rows), pack0)
 
         def blocks():
-            for s in range(0, Q, rows):
+            for s in range(q0, Q, rows):
                 e = min(Q, s + rows)
-                yield s, e, dist0 if s == 0 else block(s, e, None)
+                yield s, e, dist0 if s == q0 else block(s, e, None)
         return blocks()
 
     def _copy_stream(self) -> torch.cuda.Stream:
@@ -675,6 +815,8 @@ class RetrievalEvaluator:
         with torch.cuda.device(self.device):
             qf = qf.to(self.device, non_blocking=True)
             Q = qf.shape[0]
+            if self.query_group is not None:
+                self._agree_on_queries(qf)
             k_eff = max(1, min(int(k), self.g_total))
             idx = torch.empty((Q, k_eff), dtype=torch.int32, device=self.device)
             val = torch.empty((Q, k_eff), dtype=torch.float32, device=self.device)
@@ -704,7 +846,14 @@ class RetrievalEvaluator:
                     dist_.all_gather_into_tensor(all_v, loc_v, group=self.group)
                     _lib.call("ieee_topk_merge", all_i.data_ptr(), all_v.data_ptr(), self.world, e - s, k_eff,
                               idx[s:e].data_ptr(), val[s:e].data_ptr(), _lib.stream())
+            if self.query_group is not None:
+                for t in (idx, val):
+                    self._all_gather_owned(t, self._owned_queries(Q), Q, self.query_group)
         return idx, val
+
+    def _owned_queries(self, Q: int):
+        """The query rows every rank of query_group evaluates, in _all_gather_owned's form."""
+        return [rerank_owned(Q, self.G, self._q_world, r)[:2] + (0, 0) for r in range(self._q_world)]
 
     def _rank_block_peer(self, dist, qp, qc, link, Qb_max, Qtot, q_base, cap, W, stats, cmc, summ, stats_out, k_eff):
         """gather -> count -> metrics of one query block with the exchanges as stores into peer memory; the metrics
@@ -924,7 +1073,8 @@ class RetrievalEvaluator:
                     cap = int(cap_t.item())
             W = min(width, self.world * cap) if width > 0 else self.world * cap     # row width of the merged counts
             peer = self.world > 1 and self.exchange == "peer" and Q > 0
-            full = torch.empty((Q, self.G), dtype=torch.float32, device=self.device) if return_distmat else None
+            q0, q1 = self._query_range(Q)
+            full = torch.empty((q1 - q0, self.G), dtype=torch.float32, device=self.device) if return_distmat else None
             if peer:
                 lib = _lib.load()
                 link = link_for(self.group, self.device, lib.ieee_peer_exchange_bytes(rows, Q, cap, W, self.world))
@@ -935,9 +1085,16 @@ class RetrievalEvaluator:
                 else:
                     self._rank_block(dist, qp[s:e], qc[s:e], cap, width, ap[s:e], first[s:e], short[s:e], ties, inp[s:e])
                 if full is not None:
-                    full[s:e].copy_(dist)
+                    full[s - q0:e - q0].copy_(dist)
             if not peer and self.world > 1:
                 dist_.all_reduce(ties[:2], group=self.group)          # [2] (longest merged list) is the same on every rank
+            if self.query_group is not None:
+                # every rank's per-query results in query order, and the statistics of all queries: the reduction below
+                # then runs on the same inputs on every rank, and a list overflow is decided by all of them together
+                for t in (ap, first, short, inp):
+                    self._all_gather_owned(t, self._owned_queries(Q), Q, self.query_group)
+                dist_.all_reduce(ties[:2], group=self.query_group)
+                dist_.all_reduce(ties[2:3], op=dist_.ReduceOp.MAX, group=self.query_group)
             TRACE.mark("rank stages done")
             if peer:
                 offs = [lib.ieee_peer_result_offset(i, rows, Q, cap, W, self.world) for i in (0, 1)]
@@ -986,6 +1143,9 @@ class RetrievalEvaluator:
         if self.rerank:
             qf = qf.to(self.device)
             one_call = False             # the one-call path has no re-ranking stage: the staged block loop does
+        if self.query_group is not None:
+            with torch.cuda.device(self.device):
+                self._agree_on_queries(qf)
         if qf.is_cuda:
             with torch.cuda.device(self.device):
                 if qf.shape[0] > 0:

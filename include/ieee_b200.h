@@ -449,6 +449,55 @@ int ieee_gnn_stream_block(const int64_t* a_ptr, const int32_t* a_col, const floa
                           const int32_t* g_row, const float* g_val, int64_t Q, int64_t G, int64_t row0, int64_t rows,
                           float* block, int64_t ld, void* scratch, size_t scratch_bytes, ieee_stream_t stream);
 
+/* GNN re-ranking, streamed, in phases: the calls above split so that S processes, each holding the whole gallery and the
+ * whole query set, share the work that grows as N^2 and end with the same state.  Every row-parallel kernel computes a
+ * row from `rank`, S and the structures before it only, so which process computes a row does not change its bits.
+ * ieee_gnn_stream_neighbours is ieee_gnn_stream_neighbours_rows over all rows; ieee_gnn_stream_graph_bytes_sync is
+ * ieee_gnn_stream_symbolic over all rows followed by ieee_gnn_stream_sizes_sync; ieee_gnn_stream_graph is the numeric
+ * steps (k2 == 1: step 3 only) followed by ieee_gnn_stream_csc, over all rows.  Same limits as above.
+ * The owned rows of a process are queries [q0, q1) and gallery rows [g0, g1) (rows Q + g0 to Q + g1 of the N samples),
+ * each range starting at a multiple of 256 of its segment and ending at one or at the segment's end, or empty; the CSC
+ * columns with the same indices are its owned columns.  Other ranges give IEEE_ERR_INVALID.
+ *   ieee_gnn_stream_neighbours_rows writes rank and S of the owned rows.  Exchange: every process needs rank and S of all
+ *   N rows before the next call (an all-gather of the owned rows).
+ *   ieee_gnn_stream_symbolic builds the index in scratch (every process, all rows: linear in N k1) and counts the nnz of
+ *   B1, A1, B2 and A2 of the owned rows into four int32 [N] arrays of scratch (k2 == 1: nothing to count).  No host
+ *   synchronisation.  Exchange: every process needs the four counts of all rows (an all-gather of the owned rows; offsets
+ *   from ieee_gnn_stream_layout).
+ *   ieee_gnn_stream_sizes_sync scans the counts into row offsets and waits for the totals: sizes as
+ *   ieee_gnn_stream_graph_bytes_sync gives them, the same on every process.  The one host round trip.
+ *   ieee_gnn_stream_numeric, step 0: B1, 1: A1, 2: B2 (after the transpose of the whole A1, computed by every process),
+ *   3: A2 into a_ptr (all rows), a_col and a_val.  B1, A1 and B2 are CSR arrays in `work` (offsets from
+ *   ieee_gnn_stream_layout).  Each step writes the owned rows' entries and, unless every row is owned, sets every other
+ *   row's entries to 0.  Exchange: every process needs all of B1 before step 1, all of A1 before step 2, all of B2 before
+ *   step 3, and A2's gallery rows (entries [sizes[0] - sizes[1], sizes[0])) before ieee_gnn_stream_csc.  Because every
+ *   entry is 0 on all processes but the one that owns its row, an all-reduce that sums these arrays as int32 moves each
+ *   entry's bits exactly.  With k2 == 1 only step 3 exists (A2 = A0).
+ *   ieee_gnn_stream_csc builds the CSC of A2's gallery rows (g_ptr of all columns, every process), sorts the owned
+ *   columns and, unless every column is owned, sets every other column's entries to 0.  Exchange: g_row and g_val as
+ *   above.  Then every process holds the a_ptr, A2's gallery rows and the CSC one process builds, and ieee_gnn_stream_block
+ *   serves any of its owned query rows.
+ *   ieee_gnn_stream_layout needs no GPU: off[0..3] = byte offsets in scratch of the counts of B1, A1, B2, A2; with sizes
+ *   (those of ieee_gnn_stream_sizes_sync), off[4..9] = byte offsets in work of B1's columns and values, A1's columns and
+ *   values, B2's columns and values (k2 != 1).
+ * Memory: every process holds B1, A1, B2 and the CSC whole while the state is built, as one process does.
+ * ---------------------------------------------------------------------------------------------- */
+int ieee_gnn_stream_neighbours_rows(const void* q_packed, int64_t Q, const void* g_packed, int64_t G, int64_t D, int precision,
+                                    int32_t k1, size_t strip_bytes, int64_t q0, int64_t q1, int64_t g0, int64_t g1, int32_t* rank,
+                                    float* S, void* scratch, size_t scratch_bytes, ieee_stream_t stream);
+int ieee_gnn_stream_layout(int64_t Q, int64_t G, int32_t k1, int32_t k2, const int64_t* sizes, size_t* off);
+int ieee_gnn_stream_symbolic(const int32_t* rank, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t q0, int64_t q1, int64_t g0,
+                             int64_t g1, void* scratch, size_t scratch_bytes, ieee_stream_t stream);
+int ieee_gnn_stream_sizes_sync(int64_t Q, int64_t G, int32_t k1, int32_t k2, void* scratch, size_t scratch_bytes, int64_t* sizes,
+                               ieee_stream_t stream);
+int ieee_gnn_stream_numeric(int32_t step, const int32_t* rank, const float* S, int64_t Q, int64_t G, int32_t k1, int32_t k2,
+                            int64_t q0, int64_t q1, int64_t g0, int64_t g1, void* scratch, size_t scratch_bytes, void* work,
+                            size_t work_bytes, const int64_t* sizes, int64_t* a_ptr, int32_t* a_col, float* a_val,
+                            ieee_stream_t stream);
+int ieee_gnn_stream_csc(int64_t Q, int64_t G, int32_t k1, int64_t q0, int64_t q1, int64_t g0, int64_t g1, void* scratch,
+                        size_t scratch_bytes, const int64_t* a_ptr, const int32_t* a_col, const float* a_val, int64_t* g_ptr,
+                        int32_t* g_row, float* g_val, ieee_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Peer exchange: the two exchange steps of a gallery sharded over the GPUs of one box (relevant lists to every rank,
  * partial counts to every rank) as STORES into NVLink peer memory from inside the rank kernels, with flag words for
