@@ -44,6 +44,7 @@ SIGNATURES = {
     "ieee_set_accum_chunk": (C.c_int, [C.c_int]),
     "ieee_packed_bytes": (sz, [i64, i64, C.c_int]),
     "ieee_pack_features": (C.c_int, [vp, C.c_int, i64, i64, i64, C.c_int, C.c_int, C.c_int, vp, vp, vp]),
+    "ieee_packed_copy_rows": (C.c_int, [vp, i64, i64, vp, i64, i64, i64, i64, C.c_int, vp]),
     "ieee_distmat_fixup_bytes": (sz, [i64]),
     "ieee_distmat_packed": (C.c_int, [vp, i64, vp, i64, i64, C.c_int, C.c_int, vp, i64, vp, vp]),
     "ieee_distmat_workspace_bytes": (sz, [i64, i64, i64, C.c_int]),
@@ -88,6 +89,13 @@ SIGNATURES = {
                                           vp, sz, vp, sz, vp]),
     "ieee_rerank_stream_finish": (C.c_int, [vp, sz, i64, i64, i32, i32, i64, i64, vp, vp]),
     "ieee_rerank_stream_block_window": (C.c_int, [vp, i64, i64, i32, i32, i64, vp, i64, i64, C.c_double, vp, i64, vp, sz, vp]),
+    "ieee_rerank_stream_part_width": (i64, [i64, i64, i32, i64, i64, i64, i64, sz]),
+    "ieee_rerank_stream_part_scratch_bytes": (sz, [i64, i64, i32, i64, i64, i64, i64, i64]),
+    "ieee_rerank_stream_part_contract": (C.c_int, [i32, vp, i64, vp, vp, i64, i64, C.c_int, C.c_int, i32, i64, i64, i64, i64, i64,
+                                                   i64, i64, vp, vp, sz, vp]),
+    "ieee_rerank_stream_part_topk": (C.c_int, [i64, i64, i32, i64, i64, i64, i64, i64, i64, i64, vp, vp, vp, vp, sz, vp]),
+    "ieee_rerank_stream_part_members": (C.c_int, [i64, i64, i32, i32, i64, i64, i64, i64, i64, i64, i64, vp, vp, sz, vp, sz, vp]),
+    "ieee_rerank_stream_part_weights": (C.c_int, [vp, sz, i64, i64, i32, i32, i64, i64, vp]),
     "ieee_gnn_stream_scratch_bytes": (sz, [i64, i64, i32, sz]),
     "ieee_gnn_stream_neighbours": (C.c_int, [vp, i64, vp, i64, i64, C.c_int, i32, sz, vp, vp, vp, sz, vp]),
     "ieee_gnn_stream_graph_bytes_sync": (C.c_int, [vp, i64, i64, i32, i32, vp, sz, C.POINTER(i64), vp]),

@@ -131,6 +131,22 @@ int rerank_stream_finish(void* workspace, size_t workspace_bytes, int64_t Q, int
 int rerank_stream_block_window(const void* workspace, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t Gs,
                                const float* colmax, int64_t row0, int64_t rows, double lambda_value, float* block, int64_t ld,
                                void* scratch, size_t scratch_bytes, cudaStream_t stream);
+int64_t rerank_stream_part_width(int64_t Q, int64_t G, int32_t k1, int64_t qa, int64_t qb, int64_t ga, int64_t gb,
+                                 size_t strip_bytes);
+size_t rerank_stream_part_scratch_bytes(int64_t Q, int64_t G, int32_t k1, int64_t qa, int64_t qb, int64_t ga, int64_t gb,
+                                        int64_t W);
+int rerank_stream_part_contract(int pass, const void* q_packed, int64_t Q, const void* g_part, const void* g_strip, int64_t G,
+                                int64_t D, int metric, int precision, int32_t k1, int64_t qa, int64_t qb, int64_t ga, int64_t gb,
+                                int64_t W, int64_t i0, int64_t wc, float* colmax, void* scratch, size_t scratch_bytes,
+                                cudaStream_t stream, int cta_group);
+int rerank_stream_part_topk(int64_t Q, int64_t G, int32_t k1, int64_t qa, int64_t qb, int64_t ga, int64_t gb, int64_t W,
+                            int64_t i0, int64_t wc, const float* colmax, int32_t* idx, float* val, void* scratch,
+                            size_t scratch_bytes, cudaStream_t stream);
+int rerank_stream_part_members(int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t qa, int64_t qb, int64_t ga, int64_t gb,
+                               int64_t W, int64_t i0, int64_t wc, const float* colmax, void* workspace, size_t workspace_bytes,
+                               const void* scratch, size_t scratch_bytes, cudaStream_t stream);
+int rerank_stream_part_weights(void* workspace, size_t workspace_bytes, int64_t Q, int64_t G, int32_t k1, int32_t k2,
+                               int64_t row0, int64_t rows, cudaStream_t stream);
 
 size_t gnn_rerank_workspace_bytes(int64_t N, int32_t k1);
 int gnn_rerank(const float* neg_score, int64_t lds, int64_t N, int32_t k1, int32_t k2, float* A, int64_t ldA, void* workspace,
@@ -306,6 +322,26 @@ int ieee_set_cta_group(int cg) {
 size_t ieee_packed_bytes(int64_t rows, int64_t D, int precision) {
   if (rows < 0 || D <= 0) return 0;
   return packed_layout(rows, D, precision).total;
+}
+
+int ieee_packed_copy_rows(const void* src, int64_t src_rows, int64_t src_r0, void* dst, int64_t dst_rows, int64_t dst_r0,
+                          int64_t n, int64_t D, int precision, ieee_stream_t stream) {
+  IEEE_REQUIRE(src && dst, "packed_copy_rows: null pointer");
+  IEEE_REQUIRE(D > 0 && precision >= 0 && precision <= IEEE_PREC_FP32_SIMT, "packed_copy_rows: bad D=%lld or precision %d",
+               (long long)D, precision);
+  IEEE_REQUIRE(n >= 0 && src_r0 >= 0 && src_r0 + n <= src_rows && dst_r0 >= 0 && dst_r0 + n <= dst_rows,
+               "packed_copy_rows: rows [%lld, %lld) of %lld to [%lld, %lld) of %lld", (long long)src_r0, (long long)(src_r0 + n),
+               (long long)src_rows, (long long)dst_r0, (long long)(dst_r0 + n), (long long)dst_rows);
+  if (n == 0) return IEEE_OK;
+  const PackedRows a = packed_rows(src, src_rows, src_r0, n, D, precision), b = packed_rows(dst, dst_rows, dst_r0, n, D, precision);
+  const size_t plane = size_t(n) * size_t(a.Dp) * (precision == IEEE_PREC_FP32_SIMT ? 4 : 2);
+  cudaStream_t st = (cudaStream_t)stream;
+  IEEE_CUDA_CHECK(cudaMemcpyAsync(const_cast<uint8_t*>(b.hi), a.hi, plane, cudaMemcpyDeviceToDevice, st));
+  if (precision == IEEE_PREC_F16X3)
+    IEEE_CUDA_CHECK(cudaMemcpyAsync(const_cast<uint8_t*>(b.lo), a.lo, plane, cudaMemcpyDeviceToDevice, st));
+  IEEE_CUDA_CHECK(cudaMemcpyAsync(const_cast<float*>(b.norm), a.norm, size_t(n) * 4, cudaMemcpyDeviceToDevice, st));
+  IEEE_CUDA_CHECK(cudaMemcpyAsync(const_cast<float*>(b.scale), a.scale, size_t(n) * 4, cudaMemcpyDeviceToDevice, st));
+  return IEEE_OK;
 }
 
 int ieee_pack_features(const void* x, int dtype, int64_t ld, int64_t rows, int64_t D, int metric, int normalize,
@@ -807,6 +843,51 @@ int ieee_rerank_stream_block_window(const void* workspace, int64_t Q, int64_t G,
   if (rc) return rc;
   return rerank_stream_block_window(workspace, Q, G, k1, k2, Gs, colmax, row0, rows, lambda_value, block, ld, scratch,
                                     scratch_bytes, (cudaStream_t)stream);
+}
+
+int64_t ieee_rerank_stream_part_width(int64_t Q, int64_t G, int32_t k1, int64_t qa, int64_t qb, int64_t ga, int64_t gb,
+                                      size_t strip_bytes) {
+  return rerank_stream_part_width(Q, G, k1, qa, qb, ga, gb, strip_bytes);
+}
+
+size_t ieee_rerank_stream_part_scratch_bytes(int64_t Q, int64_t G, int32_t k1, int64_t qa, int64_t qb, int64_t ga, int64_t gb,
+                                             int64_t width) {
+  return rerank_stream_part_scratch_bytes(Q, G, k1, qa, qb, ga, gb, width);
+}
+
+int ieee_rerank_stream_part_contract(int32_t pass, const void* q_packed, int64_t Q, const void* g_part, const void* g_strip,
+                                     int64_t G, int64_t D, int metric, int precision, int32_t k1, int64_t qa, int64_t qb,
+                                     int64_t ga, int64_t gb, int64_t width, int64_t i0, int64_t wc, float* colmax, void* scratch,
+                                     size_t scratch_bytes, ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return rerank_stream_part_contract(pass, q_packed, Q, g_part, g_strip, G, D, metric, precision, k1, qa, qb, ga, gb, width, i0,
+                                     wc, colmax, scratch, scratch_bytes, (cudaStream_t)stream, cta_group_default());
+}
+
+int ieee_rerank_stream_part_topk(int64_t Q, int64_t G, int32_t k1, int64_t qa, int64_t qb, int64_t ga, int64_t gb, int64_t width,
+                                 int64_t i0, int64_t wc, const float* colmax, int32_t* idx, float* val, void* scratch,
+                                 size_t scratch_bytes, ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return rerank_stream_part_topk(Q, G, k1, qa, qb, ga, gb, width, i0, wc, colmax, idx, val, scratch, scratch_bytes,
+                                 (cudaStream_t)stream);
+}
+
+int ieee_rerank_stream_part_members(int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t qa, int64_t qb, int64_t ga, int64_t gb,
+                                    int64_t width, int64_t i0, int64_t wc, const float* colmax, void* workspace,
+                                    size_t workspace_bytes, const void* scratch, size_t scratch_bytes, ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return rerank_stream_part_members(Q, G, k1, k2, qa, qb, ga, gb, width, i0, wc, colmax, workspace, workspace_bytes, scratch,
+                                    scratch_bytes, (cudaStream_t)stream);
+}
+
+int ieee_rerank_stream_part_weights(void* workspace, size_t workspace_bytes, int64_t Q, int64_t G, int32_t k1, int32_t k2,
+                                    int64_t row0, int64_t rows, ieee_stream_t stream) {
+  int rc = check_device();
+  if (rc) return rc;
+  return rerank_stream_part_weights(workspace, workspace_bytes, Q, G, k1, k2, row0, rows, (cudaStream_t)stream);
 }
 
 size_t ieee_gnn_rerank_workspace_bytes(int64_t N, int32_t k1) { return gnn_rerank_workspace_bytes(N, k1); }

@@ -136,10 +136,10 @@ __device__ int reciprocal_append(const int32_t* __restrict__ rank, int ldr, int 
 }
 
 // weights of one row of V (rerank.py:81-82): exp(-orig[i, members]) / sum, summed in ascending member order;
-// orig_row is row i of orig (the N x N matrix, or the row as one strip holds it)
-__device__ void rr_weights(const float* __restrict__ orig_row, const int32_t* __restrict__ cols, float* __restrict__ vals,
-                           int nu, int lane) {
-  for (int t = lane; t < nu; t += 32) vals[t] = expf(-orig_row[cols[t]]);
+// orig_row is row i of orig (the N x N matrix, or the row as one strip holds it), or, with cols == nullptr, the members'
+// values orig[i, members] themselves in member order (then it may be vals: each entry is read before it is written)
+__device__ void rr_weights(const float* orig_row, const int32_t* __restrict__ cols, float* vals, int nu, int lane) {
+  for (int t = lane; t < nu; t += 32) vals[t] = expf(-(cols ? orig_row[cols[t]] : orig_row[t]));
   __syncwarp();
   float total = 0.f;
   if (lane == 0)
@@ -214,14 +214,40 @@ rr_krecip_kernel(const int32_t* __restrict__ rank, int ldr, const float* __restr
   if (lane == 0) v_cnt[i] = nu;
 }
 
-// weights of rows [row0, row0 + rows) of V from one strip of orig (row t of the strip = row row0 + t of orig)
+// weights of rows [row0, row0 + rows) of V from one strip of orig (row t of the strip = row row0 + t of orig), or, with
+// orig == nullptr, from the members' values already in v_val (rr_part_members_kernel), in place
 __global__ void __launch_bounds__(32 * kRowWarps)
 rr_weights_kernel(const float* __restrict__ orig, int64_t ldo, int row0, int rows, int cap_v, const int32_t* __restrict__ v_col,
-                  float* __restrict__ v_val, const int32_t* __restrict__ v_cnt) {
+                  float* v_val, const int32_t* __restrict__ v_cnt) {
   const int lane = threadIdx.x & 31, t = blockIdx.x * kRowWarps + (threadIdx.x >> 5);
   if (t >= rows) return;
   const int i = row0 + t;
-  rr_weights(orig + (int64_t)t * ldo, v_col + (int64_t)i * cap_v, v_val + (int64_t)i * cap_v, v_cnt[i], lane);
+  float* vals = v_val + (int64_t)i * cap_v;
+  if (orig) rr_weights(orig + (int64_t)t * ldo, v_col + (int64_t)i * cap_v, vals, v_cnt[i], lane);
+  else rr_weights(vals, nullptr, vals, v_cnt[i], lane);
+}
+
+// orig[i, c] of the members c of V's rows i = row0 + t, t < rows, from one strip's part (a StripView whose rows are this
+// part's columns: queries [qa, qa + qn), then gallery rows [ga, ga + gn)), formed as rr_build_orig_kernel forms them;
+// members outside the part, and the row's entries past its count, get 0.  One warp per row.
+__global__ void __launch_bounds__(32 * kRowWarps)
+rr_part_members_kernel(StripView part, int Q, int qa, int qn, int ga, int gn, int row0, int rows, const float* __restrict__ colmax,
+                       int cap_v, const int32_t* __restrict__ v_col, float* __restrict__ v_val, const int32_t* __restrict__ v_cnt) {
+  const int lane = threadIdx.x & 31, t = blockIdx.x * kRowWarps + (threadIdx.x >> 5);
+  if (t >= rows) return;
+  const int i = row0 + t, n = v_cnt[i];
+  for (int u = lane; u < cap_v; u += 32) {
+    float v = 0.f;
+    if (u < n) {
+      const int c = v_col[(int64_t)i * cap_v + u];
+      const int r = c < Q ? (c >= qa && c < qa + qn ? c - qa : -1) : (c - Q >= ga && c - Q < ga + gn ? qn + (c - Q - ga) : -1);
+      if (r >= 0) {
+        const float x = part.at(r, t);
+        v = __fdiv_rn(__fmul_rn(x, x), colmax[i]);
+      }
+    }
+    v_val[(int64_t)i * cap_v + u] = v;
+  }
 }
 
 // Rows of a gallery window: the Q query rows, then the gallery rows [Q + g0, Q + g0 + Gs).  Window row m is sample
@@ -674,7 +700,9 @@ int rerank_stream_pass(int pass, const void* q_packed, int64_t Q, const void* g_
                        float* colmax, int32_t* rank, void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
                        cudaStream_t stream, int cta_group) {
   IEEE_REQUIRE(pass == 0 || pass == 1, "rerank_stream_pass: pass must be 0 or 1, got %d", pass);
-  IEEE_REQUIRE(q_packed && g_packed && colmax && rank && scratch && (pass == 0 || workspace), "rerank_stream_pass: null pointer");
+  const bool strips = q1 > q0 || g1 > g0;     // without owned samples no strip is computed: g_packed and scratch go unread
+  IEEE_REQUIRE(q_packed && (g_packed || !strips) && colmax && rank && (scratch || !strips) && (pass == 0 || workspace),
+               "rerank_stream_pass: null pointer");
   IEEE_REQUIRE(D > 0, "rerank_stream_pass: bad feature width D=%lld", (long long)D);
   int rc = check_params("rerank_stream_pass", Q, G, k1, k2);
   if (rc) return rc;
@@ -692,7 +720,7 @@ int rerank_stream_pass(int pass, const void* q_packed, int64_t Q, const void* g_
                (long long)g1, (long long)G);
   const RerankPlan p = make_plan(Q, G, k1, k2, false, 0);
   const StripPlan s = make_strip_plan(Q, G, k1, strip_bytes);
-  if ((pass == 1 && workspace_bytes < p.v_end) || scratch_bytes < s.total) {
+  if ((pass == 1 && workspace_bytes < p.v_end) || (strips && scratch_bytes < s.total)) {
     set_error("rerank_stream_pass: workspace or scratch too small (%zu < %zu or %zu < %zu)", workspace_bytes, p.v_end,
               scratch_bytes, s.total);
     return IEEE_ERR_WORKSPACE;
@@ -831,6 +859,233 @@ int rerank_stream_block(const void* workspace, int64_t Q, int64_t G, int32_t k1,
                         cudaStream_t stream) {
   return rerank_stream_block_window(workspace, Q, G, k1, k2, G, colmax, row0, rows, lambda_value, block, ld, scratch,
                                     scratch_bytes, stream);
+}
+
+// ---- strips computed jointly: each process contracts its part of every strip row --------------------------------
+// Every process walks the same strips; for each it holds the part of raw[:, I] in its query rows [qa, qb) (A-operand rows
+// of the contraction: their position does not change an output's bits) and its gallery range [ga, gb) (ga a multiple of
+// 256, so the gallery columns of a query strip sit at their one-GPU positions in tiles and fix-up spans).  The part is a
+// StripView with qn = qb - qa in place of Q: part row r is raw row qa + r (r < qn) or Q + ga + (r - qn).
+// Part scratch: top [qn, W], bot [max(W x gnp, gn x W)], orig part [W, Pp], the contraction's fix-up list.
+struct PartPlan {
+  int64_t W, qn, gn, gnp, Pp;
+  size_t off_top, off_bot, off_orig, off_fix, total;
+};
+static PartPlan make_part_plan(int64_t qn, int64_t gn, int64_t W) {
+  PartPlan s;
+  s.W = W;
+  s.qn = qn;
+  s.gn = gn;
+  s.gnp = round_up(gn, 32);
+  s.Pp = round_up(qn + gn, 32);
+  size_t o = 0;
+  auto take = [&](size_t bytes) { size_t r = o; o += align256(bytes); return r; };
+  s.off_top = take(size_t(qn) * W * 4);
+  s.off_bot = take(size_t(W) * s.gnp * 4);
+  s.off_orig = take(size_t(W) * s.Pp * 4);
+  const int64_t a_rows = qn > gn ? (qn > W ? qn : W) : (gn > W ? gn : W);
+  s.off_fix = take(distmat_fixup_bytes(a_rows));
+  s.total = o + 256;
+  return s;
+}
+
+static int check_parts(const char* who, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t qa, int64_t qb, int64_t ga,
+                       int64_t gb, int64_t W) {
+  int rc = check_params(who, Q, G, k1, k2);
+  if (rc) return rc;
+  IEEE_REQUIRE(0 <= qa && qa <= qb && qb <= Q, "%s: query part [%lld, %lld) outside [0, %lld)", who, (long long)qa,
+               (long long)qb, (long long)Q);
+  IEEE_REQUIRE(ga == gb ? 0 <= ga && ga <= G : 0 <= ga && ga < gb && gb <= G && ga % 256 == 0,
+               "%s: gallery part [%lld, %lld) of %lld rows must start at a multiple of 256 or be empty", who, (long long)ga,
+               (long long)gb, (long long)G);
+  IEEE_REQUIRE(W > 0 && W % 256 == 0, "%s: strip width %lld is not a positive multiple of 256", who, (long long)W);
+  return IEEE_OK;
+}
+
+// the strip of samples [i0, i0 + wc): inside the queries or inside the gallery, starting at a multiple of 256 of its segment
+static int check_strip(const char* who, int64_t Q, int64_t G, int64_t W, int64_t i0, int64_t wc) {
+  const bool gal = i0 >= Q;
+  const int64_t c0 = gal ? i0 - Q : i0, n = gal ? G : Q;
+  IEEE_REQUIRE(i0 >= 0 && wc > 0 && wc <= W && c0 % 256 == 0 && c0 + wc <= n,
+               "%s: strip [%lld, %lld) must lie in the queries or in the gallery, start at a multiple of 256 of that segment "
+               "and be at most %lld wide", who, (long long)i0, (long long)(i0 + wc), (long long)W);
+  return IEEE_OK;
+}
+
+int64_t rerank_stream_part_width(int64_t Q, int64_t G, int32_t k1, int64_t qa, int64_t qb, int64_t ga, int64_t gb,
+                                 size_t strip_bytes) {
+  if (check_parts("rerank_stream_part_width", Q, G, k1, 1, qa, qb, ga, gb, 256) != IEEE_OK) return 0;
+  const int64_t qn = qb - qa, gn = gb - ga;
+  const int64_t per_col = 4 * (qn + round_up(gn, 32) + round_up(qn + gn, 32));    // scratch bytes per strip column
+  const int64_t widest = round_up(Q > G ? Q : G, 256);
+  int64_t W = per_col > 0 ? int64_t(strip_bytes / size_t(per_col)) / 256 * 256 : widest;
+  return W < 256 ? 256 : (W > widest ? widest : W);
+}
+
+size_t rerank_stream_part_scratch_bytes(int64_t Q, int64_t G, int32_t k1, int64_t qa, int64_t qb, int64_t ga, int64_t gb,
+                                        int64_t W) {
+  if (check_parts("rerank_stream_part_scratch_bytes", Q, G, k1, 1, qa, qb, ga, gb, W) != IEEE_OK) return 0;
+  return make_part_plan(qb - qa, gb - ga, W).total;
+}
+
+// the common arguments of the part calls; fills the plan and the strip's view of the scratch
+static int part_setup(const char* who, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t qa, int64_t qb, int64_t ga,
+                      int64_t gb, int64_t W, int64_t i0, int64_t wc, const void* scratch, size_t scratch_bytes, PartPlan& s,
+                      StripView& view) {
+  int rc = check_parts(who, Q, G, k1, k2, qa, qb, ga, gb, W);
+  if (rc) return rc;
+  if ((rc = check_strip(who, Q, G, W, i0, wc))) return rc;
+  IEEE_REQUIRE(scratch && (reinterpret_cast<uintptr_t>(scratch) & 255) == 0, "%s: scratch must be non-null and 256-byte aligned",
+               who);
+  s = make_part_plan(qb - qa, gb - ga, W);
+  if (scratch_bytes < s.total) {
+    set_error("%s: scratch too small (%zu < %zu)", who, scratch_bytes, s.total);
+    return IEEE_ERR_WORKSPACE;
+  }
+  const uint8_t* sc = static_cast<const uint8_t*>(scratch);
+  const bool gal = i0 >= Q;
+  view = StripView{reinterpret_cast<const float*>(sc + s.off_top), reinterpret_cast<const float*>(sc + s.off_bot), W,
+                   gal ? W : s.gnp, (int)s.qn, !gal};
+  return IEEE_OK;
+}
+
+// Contractions of one strip's part, with the same operand roles as rerank_stream_pass: top = q[qa, qb) x strip, bot =
+// q_I x g[ga, gb) (a query strip) or g[ga, gb) x g_I (a gallery strip).  g_part holds the packed gallery rows [ga, gb)
+// (gb - ga rows; unread when empty), g_strip a gallery strip's wc packed rows (unread for a query strip).  Pass 0 also
+// writes the part's maxima of raw^2 over each strip column to colmax[i0, i0 + wc) (as int bits, after clearing them).
+int rerank_stream_part_contract(int pass, const void* q_packed, int64_t Q, const void* g_part, const void* g_strip, int64_t G,
+                                int64_t D, int metric, int precision, int32_t k1, int64_t qa, int64_t qb, int64_t ga, int64_t gb,
+                                int64_t W, int64_t i0, int64_t wc, float* colmax, void* scratch, size_t scratch_bytes,
+                                cudaStream_t stream, int cta_group) {
+  const char* who = "rerank_stream_part_contract";
+  IEEE_REQUIRE(pass == 0 || pass == 1, "%s: pass must be 0 or 1, got %d", who, pass);
+  IEEE_REQUIRE(D > 0, "%s: bad feature width D=%lld", who, (long long)D);
+  IEEE_REQUIRE(metric == IEEE_METRIC_EUCLIDEAN || metric == IEEE_METRIC_COSINE, "%s: unknown metric %d", who, metric);
+  IEEE_REQUIRE(precision == IEEE_PREC_F16X3 || precision == IEEE_PREC_BF16, "%s: precision %d has no tensor-core contraction",
+               who, precision);
+  PartPlan s;
+  StripView view;
+  int rc = part_setup(who, Q, G, k1, 1, qa, qb, ga, gb, W, i0, wc, scratch, scratch_bytes, s, view);
+  if (rc) return rc;
+  const bool gal = i0 >= Q;
+  IEEE_REQUIRE(q_packed && colmax && (g_part || gb == ga) && (g_strip || !gal), "%s: null pointer", who);
+  uint8_t* sc = static_cast<uint8_t*>(scratch);
+  float* top = reinterpret_cast<float*>(sc + s.off_top);
+  float* bot = reinterpret_cast<float*>(sc + s.off_bot);
+  void* fix = sc + s.off_fix;
+  const int64_t qn = s.qn, gn = s.gn;
+  const PackedRows strip = gal ? packed_rows(g_strip, wc, 0, wc, D, precision) : packed_rows(q_packed, Q, i0, wc, D, precision);
+  const PackedRows part_g = packed_rows(g_part, gn, 0, gn, D, precision);
+  if (qn > 0 && (rc = distmat_umma_rows(packed_rows(q_packed, Q, qa, qn, D, precision), strip, metric, precision, top, W, stream,
+                                        cta_group, fix, false)))
+    return rc;
+  if (gn > 0 && (rc = gal ? distmat_umma_rows(part_g, strip, metric, precision, bot, W, stream, cta_group, fix, false)
+                          : distmat_umma_rows(strip, part_g, metric, precision, bot, s.gnp, stream, cta_group, fix, false)))
+    return rc;
+  if (pass == 0) {
+    int* cm_bits = reinterpret_cast<int*>(colmax) + i0;
+    const int rpb = 256;
+    IEEE_CUDA_CHECK(cudaMemsetAsync(cm_bits, 0, size_t(wc) * 4, stream));
+    if (qn > 0) {
+      rr_colmax_kernel<<<dim3((unsigned)((wc + 255) / 256), (unsigned)((qn + rpb - 1) / rpb)), 256, 0, stream>>>(
+          top, W, (int)qn, (int)wc, rpb, cm_bits);
+      count_launch();
+    }
+    if (gn > 0) {
+      if (!gal) rr_rowmax_kernel<<<(unsigned)wc, 256, 0, stream>>>(bot, s.gnp, (int)wc, (int)gn, cm_bits);
+      else rr_colmax_kernel<<<dim3((unsigned)((wc + 255) / 256), (unsigned)((gn + rpb - 1) / rpb)), 256, 0, stream>>>(
+               bot, W, (int)gn, (int)wc, rpb, cm_bits);
+      count_launch();
+    }
+  }
+  IEEE_CUDA_CHECK(cudaGetLastError());
+  return IEEE_OK;
+}
+
+// orig of the strip's rows over the part's columns (colmax complete), then the first k1 + 1 of each row's ascending
+// (value, index) order in each of the part's two column ranges: list 0 over the queries [qa, qb), list 1 over the gallery
+// rows [ga, gb), with global sample indices.  idx, val: [2][wc][k1 + 1]; an empty range's list is all -1.
+int rerank_stream_part_topk(int64_t Q, int64_t G, int32_t k1, int64_t qa, int64_t qb, int64_t ga, int64_t gb, int64_t W,
+                            int64_t i0, int64_t wc, const float* colmax, int32_t* idx, float* val, void* scratch,
+                            size_t scratch_bytes, cudaStream_t stream) {
+  const char* who = "rerank_stream_part_topk";
+  PartPlan s;
+  StripView view;
+  int rc = part_setup(who, Q, G, k1, 1, qa, qb, ga, gb, W, i0, wc, scratch, scratch_bytes, s, view);
+  if (rc) return rc;
+  IEEE_REQUIRE(colmax && idx && val, "%s: null pointer", who);
+  float* orig = reinterpret_cast<float*>(static_cast<uint8_t*>(scratch) + s.off_orig);
+  const int64_t qn = s.qn, gn = s.gn, P = qn + gn, k1p = k1 + 1;
+  if (P > 0) {
+    rr_build_orig_kernel<<<dim3((unsigned)((P + 31) / 32), (unsigned)((wc + 31) / 32)), 256, 0, stream>>>(
+        view, (int)wc, (int)P, colmax + i0, orig, s.Pp);
+    count_launch();
+  }
+  for (int l = 0; l < 2; ++l) {
+    const int64_t n = l == 0 ? qn : gn;
+    int32_t* li = idx + l * wc * k1p;
+    float* lv = val + l * wc * k1p;
+    if (n == 0) {
+      IEEE_CUDA_CHECK(cudaMemsetAsync(li, 0xFF, size_t(wc * k1p) * 4, stream));
+      continue;
+    }
+    if ((rc = topk(orig + (l == 0 ? 0 : qn), s.Pp, wc, n, l == 0 ? qa : Q + ga, nullptr, nullptr, nullptr, nullptr, (int32_t)k1p,
+                   li, lv, stream)))
+      return rc;
+  }
+  IEEE_CUDA_CHECK(cudaGetLastError());
+  return IEEE_OK;
+}
+
+// V's values of the strip's rows as far as the part holds them: row i = i0 + t of the V value array gets orig[i, c] at
+// its members c inside the part and 0 everywhere else (membership from rerank_stream_pass(1, ...), colmax complete).
+// Summed over the processes (int32 bits: every entry has one non-zero contributor) these are the members' values.
+int rerank_stream_part_members(int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t qa, int64_t qb, int64_t ga, int64_t gb,
+                               int64_t W, int64_t i0, int64_t wc, const float* colmax, void* workspace, size_t workspace_bytes,
+                               const void* scratch, size_t scratch_bytes, cudaStream_t stream) {
+  const char* who = "rerank_stream_part_members";
+  PartPlan s;
+  StripView view;
+  int rc = part_setup(who, Q, G, k1, k2, qa, qb, ga, gb, W, i0, wc, scratch, scratch_bytes, s, view);
+  if (rc) return rc;
+  IEEE_REQUIRE(colmax && workspace && (reinterpret_cast<uintptr_t>(workspace) & 255) == 0,
+               "%s: null pointer or workspace not 256-byte aligned", who);
+  const RerankPlan p = make_plan(Q, G, k1, k2, false, 0);
+  if (workspace_bytes < p.v_end) {
+    set_error("%s: workspace too small (%zu < %zu)", who, workspace_bytes, p.v_end);
+    return IEEE_ERR_WORKSPACE;
+  }
+  uint8_t* w = static_cast<uint8_t*>(workspace);
+  rr_part_members_kernel<<<(unsigned)((wc + kRowWarps - 1) / kRowWarps), 32 * kRowWarps, 0, stream>>>(
+      view, (int)Q, (int)qa, (int)s.qn, (int)ga, (int)s.gn, (int)i0, (int)wc, colmax, p.cap_v,
+      reinterpret_cast<int32_t*>(w + p.off_vcol), reinterpret_cast<float*>(w + p.off_vval), reinterpret_cast<int32_t*>(w + p.off_vcnt));
+  count_launch();
+  IEEE_CUDA_CHECK(cudaGetLastError());
+  return IEEE_OK;
+}
+
+// V's weights of rows [row0, row0 + rows) from their members' values (the summed rerank_stream_part_members), in place
+int rerank_stream_part_weights(void* workspace, size_t workspace_bytes, int64_t Q, int64_t G, int32_t k1, int32_t k2,
+                               int64_t row0, int64_t rows, cudaStream_t stream) {
+  const char* who = "rerank_stream_part_weights";
+  int rc = check_params(who, Q, G, k1, k2);
+  if (rc) return rc;
+  IEEE_REQUIRE(workspace && (reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "%s: workspace null or not 256-byte aligned", who);
+  IEEE_REQUIRE(row0 >= 0 && rows >= 0 && row0 + rows <= Q + G, "%s: rows [%lld, %lld) outside [0, %lld)", who, (long long)row0,
+               (long long)(row0 + rows), (long long)(Q + G));
+  const RerankPlan p = make_plan(Q, G, k1, k2, false, 0);
+  if (workspace_bytes < p.v_end) {
+    set_error("%s: workspace too small (%zu < %zu)", who, workspace_bytes, p.v_end);
+    return IEEE_ERR_WORKSPACE;
+  }
+  if (rows == 0) return IEEE_OK;
+  uint8_t* w = static_cast<uint8_t*>(workspace);
+  rr_weights_kernel<<<(unsigned)((rows + kRowWarps - 1) / kRowWarps), 32 * kRowWarps, 0, stream>>>(
+      nullptr, 0, (int)row0, (int)rows, p.cap_v, reinterpret_cast<int32_t*>(w + p.off_vcol), reinterpret_cast<float*>(w + p.off_vval),
+      reinterpret_cast<int32_t*>(w + p.off_vcnt));
+  count_launch();
+  IEEE_CUDA_CHECK(cudaGetLastError());
+  return IEEE_OK;
 }
 
 // =========================================================================================================

@@ -154,6 +154,16 @@ def rerank_owned(Q: int, G: int, world: int, rank: int) -> tuple[int, int, int, 
     return split(Q) + split(G)
 
 
+def rerank_ranges(offsets: list[int], G: int) -> list[tuple[int, int]]:
+    """Gallery rows [a, b) whose columns each rank computes in the strips when ranks holding slices that start at
+    ``offsets`` (rank order, tiling [0, G)) prepare k-reciprocal re-ranking together: a is the rank's slice start rounded
+    up to a multiple of 256 (0 for the first rank), b the next rank's a (G for the last).  The ranges tile [0, G) in rank
+    order and start at multiples of 256, where the contraction puts a column as it does for the whole gallery; a range
+    is empty when its slice holds no such start, and reaches up to 255 rows into the slices after its own."""
+    a = [0] + [min(G, (o + 255) // 256 * 256) for o in offsets[1:]]
+    return [(a[r], a[r + 1] if r + 1 < len(a) else G) for r in range(len(a))]
+
+
 def centering_applies(metric: str, precision: str) -> bool:
     """Euclidean operands are packed relative to a common centre (ieee_pack_features); cosine is not translation
     invariant and the 1-pass bf16 mode multiplies bf16 inputs exactly as they are."""
@@ -256,10 +266,12 @@ class RetrievalEvaluator:
     With ``group`` (a torch.distributed process group; NCCL for device tensors) and ``rerank=True`` the re-ranking is
     over the whole sharded gallery, with the bits of one GPU holding it all: every rank returns what a one-GPU
     ``rerank=True`` evaluator returns (ieee_rerank_stream_pass / _finish / _block_window).  The slices must tile
-    [0, g_total) in rank order (checked once, collectively; ValueError on every rank otherwise).  During the prepare
-    call every rank holds the whole gallery packed (about 4 bytes per feature, gathered from the slices and freed when
-    the prepare returns) and computes the strips of its share of the samples (rerank_owned); the small state (colmax,
-    neighbour lists, the k-reciprocal sets) is all-gathered.  What stays is sized by this rank's slice of Gs rows:
+    [0, g_total) in rank order (checked once, collectively; ValueError on every rank otherwise).  No rank holds the
+    whole gallery: the ranks compute every strip of the prepare call together, each the columns of its share of the
+    queries (rerank_owned) and of its gallery range (rerank_ranges: its slice, 256-aligned, so up to 255 rows of the
+    next slices are sent to it once).  A gallery strip's rows are exchanged for that strip alone, and the strips' small
+    results (column maxima, neighbour lists, the k-reciprocal weights' inputs) are reduced across the ranks; the ranks
+    share one strip width, the narrowest their ``block_bytes`` allow.  What stays is sized by this rank's slice of Gs rows:
     about 8 (k1+1)(round(k1/2)+2) bytes per sample of the whole set plus k2 times that per query and per slice row
     (2 KB * N + 24 KB * (Q + Gs) at k1 = 20, k2 = 6), plus ``block_bytes``.  The plain sharded path's condition for
     the bits of one GPU applies to the query blocks' own distances (this rank's contraction against its slice).
@@ -402,20 +414,21 @@ class RetrievalEvaluator:
         return rerank_owned(Q, self.G, self._q_world, self._q_rank)[:2] if self.query_group is not None else (0, Q)
 
     def _gallery_slices(self):
-        """[(g_offset, rows)] of every rank, all-gathered once.  Every rank gets the same list and so reaches the same
-        verdict: slices that do not tile [0, g_total) in rank order raise ValueError on every rank."""
+        """[(g_offset, rows, block_bytes)] of every rank, all-gathered once.  Every rank gets the same list and so reaches
+        the same verdict: slices that do not tile [0, g_total) in rank order raise ValueError on every rank.  From the
+        block_bytes of all ranks every rank derives the same strip width."""
         import torch.distributed as dist_
         with torch.cuda.device(self.device):
-            mine = torch.tensor([self.g_offset, self.G, self.g_total], dtype=torch.int64, device=self.device)
-            every = torch.empty((self.world, 3), dtype=torch.int64, device=self.device)
-            dist_.all_gather_into_tensor(every, mine, group=self.group)
+            mine = torch.tensor([self.g_offset, self.G, self.g_total, self.block_bytes], dtype=torch.int64, device=self.device)
+            every = torch.empty((self.world, 4), dtype=torch.int64, device=self.device)
+            dist_.all_gather_into_tensor(every.view(-1), mine, group=self.group)
             every = every.cpu().tolist()
         total = every[0][2]
         starts = [sum(e[1] for e in every[:r]) for r in range(self.world)]
         if any(e[0] != s or e[2] != total for e, s in zip(every, starts)) or starts[-1] + every[-1][1] != total:
             raise ValueError("rerank=True over a sharded gallery: the slices (g_offset, rows, g_total) of the ranks {} do "
-                             "not tile [0, g_total) in rank order".format([tuple(e) for e in every]))
-        return [(off, rows) for off, rows, _ in every]
+                             "not tile [0, g_total) in rank order".format([tuple(e[:3]) for e in every]))
+        return [(off, rows, bb) for off, rows, _, bb in every]
 
     def _check_rerank(self, gf, group, k1, k2, g_total):
         mode = 'rerank="gnn"' if self.gnn else "rerank=True"
@@ -465,14 +478,16 @@ class RetrievalEvaluator:
             raise ValueError("rerank=True: k1 + 1 = {} exceeds the {} query and gallery samples".format(k1 + 1, Q + G))
         lib = _lib.load()
         ws_bytes = lib.ieee_rerank_stream_window_workspace_bytes(Q, G, k1, k2, self.G)
-        sc_bytes = lib.ieee_rerank_stream_scratch_bytes(Q, G, k1, self.block_bytes)
+        # (a sharded prepare sizes its own scratch for its part of the strips)
+        sc_bytes = lib.ieee_rerank_stream_scratch_bytes(Q, G, k1, self.block_bytes) if self.group is None else 1
         if ws_bytes == 0 or sc_bytes == 0:
             raise ValueError("rerank=True: " + lib.ieee_last_error().decode())
         qpk = self._take_early_q(qf)
         if qpk is None:
             qpk = PackedFeatures(qf, self.metric, self.normalize, self.precision, self.center)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=self.device)
-        strips = torch.empty(sc_bytes, dtype=torch.uint8, device=self.device)    # released (stream-ordered) on return
+        if self.group is None:
+            strips = torch.empty(sc_bytes, dtype=torch.uint8, device=self.device)    # released (stream-ordered) on return
         colmax = torch.empty(Q + G, dtype=torch.float32, device=self.device)
         rank = torch.empty((Q + G, k1 + 1), dtype=torch.int32, device=self.device)
         if self.group is None:
@@ -480,7 +495,7 @@ class RetrievalEvaluator:
                       qpk.precision, k1, k2, self.block_bytes, colmax.data_ptr(), rank.data_ptr(), ws.data_ptr(), ws_bytes,
                       strips.data_ptr(), sc_bytes, _lib.stream())
         else:
-            self._rerank_prepare_sharded(qpk, colmax, rank, ws, strips)
+            self._rerank_prepare_sharded(qpk, colmax, rank, ws)
         TRACE.mark("re-ranking state prepared")
         # qf is kept so that its address cannot be reused by another tensor while the key refers to it; k1 and k2
         # fix the workspace's layout, so the block calls take them from here
@@ -488,46 +503,113 @@ class RetrievalEvaluator:
                     "rank": rank}
         return self._rr
 
-    def _rerank_prepare_sharded(self, qpk: PackedFeatures, colmax, rank, ws, strips):
-        """The prepare call's phases with the ranks' exchanges between them: pass 0 and pass 1 over this rank's share of
-        the strips (rerank_owned), each followed by an all-gather of the owned rows (colmax and rank, then V's values),
-        and the finish over this rank's gallery slice.  The strips need every gallery row: the slices are all-gathered
-        and packed whole for the two passes and freed on return."""
+    def _rerank_prepare_sharded(self, qpk: PackedFeatures, colmax, rank, ws):
+        """The prepare call's passes with every strip computed by all ranks together, each the part of every strip row in
+        its columns: its share of the queries (rerank_owned) and its gallery range (rerank_ranges), packed once.  Per strip
+        of pass 0 the part's column maxima are all-reduced (MAX), and the part's two top-(k1+1) lists all-gathered and
+        merged into `rank`; pass 1 writes V's membership of all rows from `rank`, then per strip the members' values in the
+        part, summed across the ranks (int32: one non-zero contributor each) and weighed.  A gallery strip's rows are
+        summed from the slices that hold them (zeros elsewhere) and packed by every rank.  The finish covers this rank's
+        slice."""
         import torch.distributed as dist_
-        Q, G, k1, k2 = qpk.rows, self.g_total, self.k1, self.k2
-        gpk = self._whole_gallery()
-        TRACE.mark("re-ranking: whole gallery gathered and packed")
-        owned = [rerank_owned(Q, G, self.world, r) for r in range(self.world)]
-        q0, q1, g0, g1 = owned[dist_.get_rank(self.group)]
+        Q, G, k1, k2, D = qpk.rows, self.g_total, self.k1, self.k2, qpk.D
+        lib, dev, stream, k1p = _lib.load(), self.device, _lib.stream(), k1 + 1
+        me, world = dist_.get_rank(self.group), self.world
+        ranges = rerank_ranges([off for off, _, _ in self._slices], G)
+        parts = [rerank_owned(Q, G, world, r)[:2] + ranges[r] for r in range(world)]
+        W = min(lib.ieee_rerank_stream_part_width(Q, G, k1, *part, bb) for part, (_, _, bb) in zip(parts, self._slices))
+        part = parts[me]
+        sc_bytes = lib.ieee_rerank_stream_part_scratch_bytes(Q, G, k1, *part, W) if W else 0
+        if sc_bytes == 0:
+            raise ValueError("rerank=True: " + lib.ieee_last_error().decode())
+        scratch = torch.empty(sc_bytes, dtype=torch.uint8, device=dev)         # released (stream-ordered) on return
+        gpart = self._gallery_range(ranges)
+        TRACE.mark("re-ranking: gallery range packed")
         cap, off_col, off_val, off_cnt = C.c_int64(), C.c_size_t(), C.c_size_t(), C.c_size_t()
         _lib.call("ieee_rerank_stream_v_layout", Q, G, k1, k2, C.byref(cap), C.byref(off_col), C.byref(off_val), C.byref(off_cnt))
-        v_val = ws[off_val.value: off_val.value + 4 * (Q + G) * cap.value].view(torch.float32).view(Q + G, cap.value)
-        for step, shared in ((0, (colmax, rank)), (1, (v_val,))):
-            _lib.call("ieee_rerank_stream_pass", step, qpk.buf.data_ptr(), Q, gpk.buf.data_ptr(), G, qpk.D, qpk.metric,
-                      qpk.precision, k1, k2, self.block_bytes, q0, q1, g0, g1, colmax.data_ptr(), rank.data_ptr(), ws.data_ptr(),
-                      ws.numel(), strips.data_ptr(), strips.numel(), _lib.stream())
-            TRACE.mark("re-ranking: pass %d" % step)
-            for t in shared:
-                self._all_gather_owned(t, owned, Q)
-            TRACE.mark("re-ranking: exchange after pass %d" % step)
-        del gpk
-        _lib.call("ieee_rerank_stream_finish", ws.data_ptr(), ws.numel(), Q, G, k1, k2, self.g_offset, self.G, rank.data_ptr(),
-                  _lib.stream())
+        v_val = ws[off_val.value: off_val.value + 4 * (Q + G) * cap.value].view(torch.int32).view(Q + G, cap.value)
+        gf, off = self._gallery_dev, self.g_offset
+        raw = torch.empty((W, D), dtype=gf.dtype, device=dev)                   # a gallery strip's rows
+        lists = torch.empty((2, 2 * W * k1p), dtype=torch.int32, device=dev)    # this rank's lists: indices, value bits
+        every = torch.empty((2, world * 2 * W * k1p), dtype=torch.int32, device=dev)
+        merged_val = torch.empty(W * k1p, dtype=torch.float32, device=dev)
+        common = (Q, G, k1) + part + (W,)
 
-    def _whole_gallery(self) -> PackedFeatures:
-        """Every rank's gallery slice, all-gathered (padded to the largest) and packed as one tensor with this evaluator's
-        centre: packing is per row, so these are the bytes one GPU packs from the whole gallery."""
+        def strips():
+            for i0, n in ((0, Q), (Q, G)):
+                for c0 in range(0, n, W):
+                    yield i0 + c0, min(W, n - c0)
+
+        def contract(step, i0, wc):
+            g_strip = None
+            if i0 >= Q:                          # this rank's rows of the strip, zeros elsewhere, summed across the ranks
+                c0 = i0 - Q
+                lo, hi = max(c0, off), min(c0 + wc, off + self.G)
+                raw[:wc].zero_()
+                if lo < hi:
+                    raw[lo - c0: hi - c0] = gf[lo - off: hi - off]
+                words = (wc * D * raw.element_size() + 3) // 4
+                dist_.all_reduce(raw.view(-1).view(torch.uint8)[: 4 * words].view(torch.int32), group=self.group)
+                g_strip = PackedFeatures(raw[:wc], self.metric, self.normalize, self.precision, self.center)
+            _lib.call("ieee_rerank_stream_part_contract", step, qpk.buf.data_ptr(), Q, _lib.ptr(gpart and gpart.buf),
+                      _lib.ptr(g_strip and g_strip.buf), G, D, qpk.metric, qpk.precision, k1, *part, W, i0, wc,
+                      colmax.data_ptr(), scratch.data_ptr(), sc_bytes, stream)
+
+        for i0, wc in strips():                  # pass 0: colmax and rank
+            contract(0, i0, wc)
+            dist_.all_reduce(colmax[i0: i0 + wc].view(torch.int32), op=dist_.ReduceOp.MAX, group=self.group)
+            n = 2 * wc * k1p
+            mine, got = lists[:, :n], every[:, : world * n]
+            _lib.call("ieee_rerank_stream_part_topk", *common, i0, wc, colmax.data_ptr(), mine[0].data_ptr(), mine[1].data_ptr(),
+                      scratch.data_ptr(), sc_bytes, stream)
+            for t in range(2):
+                dist_.all_gather_into_tensor(got[t], mine[t].contiguous(), group=self.group)
+            _lib.call("ieee_topk_merge", got[0].data_ptr(), got[1].data_ptr(), 2 * world, wc, k1p, rank[i0].data_ptr(),
+                      merged_val.data_ptr(), stream)
+        TRACE.mark("re-ranking: pass 0")
+        # V's membership of every row from rank alone: no owned strips, so no gallery operand and no strip scratch
+        _lib.call("ieee_rerank_stream_pass", 1, qpk.buf.data_ptr(), Q, None, G, D, qpk.metric, qpk.precision, k1, k2,
+                  self.block_bytes, 0, 0, 0, 0, colmax.data_ptr(), rank.data_ptr(), ws.data_ptr(), ws.numel(), None, 0, stream)
+        for i0, wc in strips():                  # pass 1: V's values
+            contract(1, i0, wc)
+            _lib.call("ieee_rerank_stream_part_members", *common[:3], k2, *common[3:], i0, wc, colmax.data_ptr(), ws.data_ptr(),
+                      ws.numel(), scratch.data_ptr(), sc_bytes, stream)
+            dist_.all_reduce(v_val[i0: i0 + wc], group=self.group)
+            _lib.call("ieee_rerank_stream_part_weights", ws.data_ptr(), ws.numel(), Q, G, k1, k2, i0, wc, stream)
+        TRACE.mark("re-ranking: pass 1")
+        _lib.call("ieee_rerank_stream_finish", ws.data_ptr(), ws.numel(), Q, G, k1, k2, self.g_offset, self.G, rank.data_ptr(),
+                  stream)
+
+    def _gallery_range(self, ranges) -> PackedFeatures | None:
+        """This rank's gallery range (rerank_ranges) packed with the evaluator's centre, or None when it is empty: the
+        range's rows of the packed slice, then the rows up to the range's end, taken from the heads of the next slices
+        (the rows before each one's own range, fewer than 256), all-gathered and packed here.  Packing is per row, so
+        these are the bytes one GPU packs for these rows."""
         import torch.distributed as dist_
-        gf = self._gallery_dev
-        rows = max(n for _, n in self._slices)
-        send = torch.zeros((rows, gf.shape[1]), dtype=gf.dtype, device=self.device)
-        send[: gf.shape[0]] = gf
-        recv = torch.empty((self.world, rows, gf.shape[1]), dtype=gf.dtype, device=self.device)
-        dist_.all_gather_into_tensor(recv, send, group=self.group)
-        del send
-        whole = torch.cat([recv[r, :n] for r, (_, n) in enumerate(self._slices)])
-        del recv
-        return PackedFeatures(whole, self.metric, self.normalize, self.precision, self.center)
+        gf, me, off, n = self._gallery_dev, dist_.get_rank(self.group), self.g_offset, self.G
+        heads = [min(rows, a - o) for (o, rows, _), (a, _) in zip(self._slices, ranges)]
+        h = max(heads)
+        if h > 0:                                # the same verdict on every rank: all of them take part
+            send = torch.zeros((h, gf.shape[1]), dtype=gf.dtype, device=self.device)
+            send[: heads[me]] = gf[: heads[me]]
+            recv = torch.empty((self.world, h, gf.shape[1]), dtype=gf.dtype, device=self.device)
+            dist_.all_gather_into_tensor(recv.view(-1, gf.shape[1]), send, group=self.group)
+        a, b = ranges[me]
+        if a == b:
+            return None
+        slice_pk = self.chunks[0][1]
+        if (a, b) == (off, off + n):
+            return slice_pk
+        pk = PackedFeatures._empty(b - a, slice_pk.D, self.metric, self.precision, self.center, self.device)
+        _lib.call("ieee_packed_copy_rows", slice_pk.buf.data_ptr(), n, a - off, pk.buf.data_ptr(), b - a, 0, off + n - a,
+                  pk.D, pk.precision, _lib.stream())
+        if b > off + n:
+            tail = torch.cat([recv[s, : heads[s]] for s in range(me + 1, self.world) if self._slices[s][0] < b])
+            assert tail.shape[0] == b - (off + n)
+            tpk = PackedFeatures(tail, self.metric, self.normalize, self.precision, self.center)
+            _lib.call("ieee_packed_copy_rows", tpk.buf.data_ptr(), tail.shape[0], 0, pk.buf.data_ptr(), b - a, off + n - a,
+                      tail.shape[0], pk.D, pk.precision, _lib.stream())
+        return pk
 
     def _all_gather_owned(self, t: torch.Tensor, owned, Q: int, group=None):
         """Rows [q0, q1) and [Q + g0, Q + g1) of t ([Q + G, ...]), computed by each rank (owned = rerank_owned of every

@@ -122,6 +122,10 @@ size_t ieee_packed_bytes(int64_t rows, int64_t D, int precision);
  * same centre. */
 int ieee_pack_features(const void* x, int dtype, int64_t ld, int64_t rows, int64_t D, int metric, int normalize,
                        int precision, const float* center, void* packed, ieee_stream_t stream);
+/* Copy packed rows [src_r0, src_r0 + n) of an operand of src_rows rows to rows [dst_r0, dst_r0 + n) of one of dst_rows
+ * rows (both packed for D and `precision`): the bytes packing those rows into dst would write. */
+int ieee_packed_copy_rows(const void* src, int64_t src_rows, int64_t src_r0, void* dst, int64_t dst_rows, int64_t dst_r0,
+                          int64_t n, int64_t D, int precision, ieee_stream_t stream);
 /* Centre for ieee_pack_features: column mean over up to max_rows (0: 64) evenly strided rows of x, scaled to unit
  * length when `normalize` is set (the rows will be).  Deterministic (fixed summation order).  center: float32[D];
  * workspace: ieee_feature_center_workspace_bytes(D). */
@@ -370,7 +374,7 @@ int ieee_rerank_stream_block(const void* workspace, int64_t Q, int64_t G, int32_
  *   ieee_rerank_stream_pass needs the whole gallery packed (g_packed, G rows, as for the prepare call) and computes the
  *   strips of the owned samples only: queries [q0, q1) and gallery rows [g0, g1), each range starting at a multiple of
  *   256 of its segment and ending at one or at the segment's end (an empty range is allowed).  The bits do not depend on
- *   the ranges or on strip_bytes.
+ *   the ranges or on strip_bytes.  With both ranges empty no strip is computed, and g_packed and scratch may be null.
  *     pass 0 writes colmax and rank of the owned samples (colmax[i], rank[i, :] for i in [q0, q1) and [Q + g0, Q + g1)).
  *       workspace may be null.  Exchange: every process needs colmax [N] and rank [N, k1 + 1] of all samples before
  *       pass 1 (an all-gather of the owned rows).
@@ -402,6 +406,48 @@ int ieee_rerank_stream_finish(void* workspace, size_t workspace_bytes, int64_t Q
 int ieee_rerank_stream_block_window(const void* workspace, int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t Gs,
                                     const float* colmax, int64_t row0, int64_t rows, double lambda_value, float* block,
                                     int64_t ld, void* scratch, size_t scratch_bytes, ieee_stream_t stream);
+
+/* k-reciprocal re-ranking, streamed, with strips computed jointly: passes 0 and 1 of the phased form for S processes
+ * of which none holds the whole gallery.  Every process walks the same strips [i0, i0 + wc) of all N samples (inside the
+ * queries or inside the gallery, starting at a multiple of 256 of that segment, wc <= width, width a multiple of 256 that
+ * all processes share) and computes its PART of each strip row: the columns of its queries [qa, qb) (any split of
+ * [0, Q)) and of its gallery range [ga, gb) (ga a multiple of 256; the ranges tile [0, G)).  The bits equal
+ * ieee_rerank_stream_pass's for any parts and width.  The part scratch (ieee_rerank_stream_part_scratch_bytes) must hold
+ * its contents from a contract call to the calls of the same strip that follow it.
+ *   ieee_rerank_stream_part_contract: the strip's contractions over the part.  q_packed: all Q queries; g_part: the
+ *     packed gallery rows [ga, gb) (gb - ga rows; unread when empty); g_strip: a gallery strip's wc rows packed on their
+ *     own (unread for a query strip).  All packed with the same centre.  Pass 0 also writes the part's maxima of raw^2
+ *     over the strip's columns to colmax[i0, i0 + wc).  Exchange: an all-reduce MAX of those wc words as int32 (the
+ *     values are >= 0, so the bits order as the floats do).
+ *   ieee_rerank_stream_part_topk (pass 0, colmax of the strip complete): the first k1 + 1 of each strip row's ascending
+ *     (value, index) order in each of the part's column ranges, with global sample indices: idx, val [2][wc][k1 + 1],
+ *     list 0 over the queries, list 1 over the gallery range; an empty range's list is all -1.  Exchange: all-gather the
+ *     lists, then ieee_topk_merge of the 2 S lists (shards = 2 S) into rank[i0, i0 + wc) gives the one-GPU rows.
+ *   ieee_rerank_stream_part_members (pass 1, after ieee_rerank_stream_pass(1, ...) with empty owned ranges has written
+ *     V's membership of all rows, and with colmax complete): V's values of rows [i0, i0 + wc) where the member falls in
+ *     the part, 0 elsewhere.  Exchange: an all-reduce SUM of those rows of the value array (ieee_rerank_stream_v_layout)
+ *     as int32: each entry has one non-zero contributor, so the sum is its exact bits.
+ *   ieee_rerank_stream_part_weights: the weights of V's rows [row0, row0 + rows) from those values, in place.
+ *   ieee_rerank_stream_part_width: the widest strip width (a multiple of 256, at least 256) whose part scratch fits in
+ *     strip_bytes; ieee_rerank_stream_part_scratch_bytes: the part scratch for a width.  Both need no GPU and return 0
+ *     (with ieee_last_error set) when the parameters are out of range.
+ * ---------------------------------------------------------------------------------------------- */
+int64_t ieee_rerank_stream_part_width(int64_t Q, int64_t G, int32_t k1, int64_t qa, int64_t qb, int64_t ga, int64_t gb,
+                                      size_t strip_bytes);
+size_t ieee_rerank_stream_part_scratch_bytes(int64_t Q, int64_t G, int32_t k1, int64_t qa, int64_t qb, int64_t ga, int64_t gb,
+                                             int64_t width);
+int ieee_rerank_stream_part_contract(int32_t pass, const void* q_packed, int64_t Q, const void* g_part, const void* g_strip,
+                                     int64_t G, int64_t D, int metric, int precision, int32_t k1, int64_t qa, int64_t qb,
+                                     int64_t ga, int64_t gb, int64_t width, int64_t i0, int64_t wc, float* colmax, void* scratch,
+                                     size_t scratch_bytes, ieee_stream_t stream);
+int ieee_rerank_stream_part_topk(int64_t Q, int64_t G, int32_t k1, int64_t qa, int64_t qb, int64_t ga, int64_t gb, int64_t width,
+                                 int64_t i0, int64_t wc, const float* colmax, int32_t* idx, float* val, void* scratch,
+                                 size_t scratch_bytes, ieee_stream_t stream);
+int ieee_rerank_stream_part_members(int64_t Q, int64_t G, int32_t k1, int32_t k2, int64_t qa, int64_t qb, int64_t ga, int64_t gb,
+                                    int64_t width, int64_t i0, int64_t wc, const float* colmax, void* workspace,
+                                    size_t workspace_bytes, const void* scratch, size_t scratch_bytes, ieee_stream_t stream);
+int ieee_rerank_stream_part_weights(void* workspace, size_t workspace_bytes, int64_t Q, int64_t G, int32_t k1, int32_t k2,
+                                    int64_t row0, int64_t rows, ieee_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
  * GNN re-ranking (alternative `rerank` mode).   Replaces torchreid/utils/GPU-Re-Ranking/gnn_reranking.py:27-59 with its

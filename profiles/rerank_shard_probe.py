@@ -4,8 +4,9 @@ over NCCL, the gallery split with shard_bounds.
 
 Per rank, from the evaluator's CUDA-event marks (IEEE_B200_TRACE; an interval is charged to the mark that ends it) of
 one evaluate() after a warm-up evaluate() of another query tensor:
-  prepare  gather + pack (the whole gallery, and the query pack before it), pass 0, its exchange (colmax and rank),
-           pass 1, its exchange (V's values), finish (query expansion and inverted index of the rank's slice)
+  prepare  range (the rank's gallery range packed, and the query pack before it), pass 0 (colmax and rank, with the
+           per-strip exchanges: strip rows, colmax, neighbour lists), pass 1 (V, with the per-strip exchanges: strip
+           rows, V's values), finish (query expansion and inverted index of the rank's slice)
   blocks   per query block: contraction against the slice, re-ranking blend, rank stages (gather, exchanges, counts)
 and the peak of torch.cuda.max_memory_allocated over that evaluate().  Every rank compares its cmc, mAP, ap and first
 with a one-GPU rerank=True evaluator on the whole gallery, run first in the rank-0 process of world size 1 and saved.
@@ -27,9 +28,8 @@ os.environ["IEEE_B200_TRACE"] = "1"
 from ieee_b200 import engine                                                 # noqa: E402
 from ieee_b200.engine import RetrievalEvaluator, shard_bounds                # noqa: E402
 
-PREPARE = [("gather+pack", "re-ranking: whole gallery"), ("pass 0", "re-ranking: pass 0"),
-           ("exchange 0", "re-ranking: exchange after pass 0"), ("pass 1", "re-ranking: pass 1"),
-           ("exchange 1", "re-ranking: exchange after pass 1"), ("finish", "re-ranking state prepared")]
+PREPARE = [("range", "re-ranking: gallery range"), ("pass 0", "re-ranking: pass 0"), ("pass 1", "re-ranking: pass 1"),
+           ("finish", "re-ranking state prepared")]
 
 
 def make_set(Q, G, D=2304, ids=3000, sigma=3.0, seed=0):
