@@ -132,6 +132,9 @@ SIGNATURES.update({
     "ieee_retrieve_prepared_peer_workspace_bytes": (sz, [i64, i64, C.c_int, i32]),
     "ieee_retrieve_eval_prepared_peer": (C.c_int, [vp, i64, C.c_int, i64, i64, C.c_int, C.c_int, C.c_int, vp, vp, vp, i64, i64, i64,
                                                    vp, vp, vp, i32, vp, i64, vp, vp, vp, vp, vp, _PEER, vp, vp, sz, vp]),
+    "ieee_retrieve_eval_prepared_peer_dev_epoch": (C.c_int, [vp, i64, C.c_int, i64, i64, C.c_int, C.c_int, C.c_int, vp, vp, vp, i64,
+                                                             i64, i64, vp, vp, vp, i32, vp, i64, vp, vp, vp, vp, vp, _PEER, vp, vp,
+                                                             vp, sz, vp]),
 })
 
 _lib = None

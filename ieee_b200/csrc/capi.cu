@@ -41,6 +41,9 @@ static void tl_mark(const char* name) {
 static void tl_enter(cudaStream_t stream, const char* what) {
   tl_on = (g_debug_flags & 128) != 0;
   if (!tl_on) return;
+  // a captured step gets no marks: they would be events of the capture, which the timeline cannot read back
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(stream, &cs) != cudaSuccess || cs != cudaStreamCaptureStatusNone) { tl_on = false; return; }
   tl_stream = stream;
   tl_mark(what);
 }
@@ -241,7 +244,12 @@ static int side_lane_join(cudaStream_t stream) {
     std::lock_guard<std::mutex> lock(g_side_mutex);
     join = g_side[dev].join;
   }
-  if (join != nullptr) IEEE_CUDA_CHECK(cudaStreamWaitEvent(stream, join, 0));
+  if (join == nullptr) return IEEE_OK;
+  // under stream capture the event was recorded outside the capture: the graph gets an external wait node, so every
+  // replay waits for whatever the side lane was last given, as an eager call does
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  IEEE_CUDA_CHECK(cudaStreamIsCapturing(stream, &cs));
+  IEEE_CUDA_CHECK(cudaStreamWaitEvent(stream, join, cs == cudaStreamCaptureStatusActive ? cudaEventWaitExternal : 0));
   return IEEE_OK;
 }
 }  // namespace ieee
@@ -699,6 +707,10 @@ int ieee_retrieve_eval_prepared(const void* qf, int64_t ldq, int dtype, int64_t 
       return rc;
   }
   if (cap <= 0) {
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    IEEE_CUDA_CHECK(cudaStreamIsCapturing(stream, &cs));
+    IEEE_REQUIRE(cs == cudaStreamCaptureStatusNone,
+                 "retrieve: cap <= 0 sizes the lists with a host round trip, which a stream capture cannot hold: pass cap > 0");
     int32_t need = 0;
     if ((rc = ieee_rank_list_cap_sync(group, G, q_pids, Q, scratch, &need, stream_))) return rc;
     cap = need < 1 ? 1 : need;
@@ -1037,18 +1049,19 @@ int ieee_peer_free(void* ptr) {
   return IEEE_OK;
 }
 
-static int peer_view(const ieee_peer_exchange* ex, PeerView* v) {
+static int peer_view(const ieee_peer_exchange* ex, PeerView* v, unsigned long long* epoch_dev = nullptr) {
   IEEE_REQUIRE(ex != nullptr, "peer exchange: null descriptor");
   IEEE_REQUIRE(ex->shards >= 1 && ex->shards <= kMaxPeers && ex->my_shard >= 0 && ex->my_shard < ex->shards,
                "peer exchange: bad shard %d of %d", ex->my_shard, ex->shards);
   IEEE_REQUIRE(ex->Qb > 0 && ex->Qb <= ex->Qb_max && ex->q_base >= 0 && ex->q_base + ex->Qb <= ex->Qtot && ex->cap >= 1 &&
-                   ex->W >= 1 && ex->epoch > 0,
+                   ex->W >= 1 && (ex->epoch > 0 || epoch_dev != nullptr),
                "peer exchange: bad block (Qb=%lld q_base=%lld Qtot=%lld cap=%d W=%d)", (long long)ex->Qb,
                (long long)ex->q_base, (long long)ex->Qtot, ex->cap, ex->W);
   *v = no_peers();
   v->shards = ex->shards;
   v->my = ex->my_shard;
   v->epoch = ex->epoch;
+  v->epoch_dev = epoch_dev;
   for (int s = 0; s < ex->shards; ++s) {
     IEEE_REQUIRE(ex->base[s] != nullptr, "peer exchange: buffer of shard %d is not mapped", s);
     v->base[s] = static_cast<uint8_t*>(ex->base[s]);
@@ -1099,13 +1112,13 @@ size_t ieee_retrieve_prepared_peer_workspace_bytes(int64_t Q, int64_t D, int pre
          2 * align256(size_t(Q) * 4) + 256 + 256;
 }
 
-int ieee_retrieve_eval_prepared_peer(const void* qf, int64_t ldq, int dtype, int64_t Q, int64_t D, int metric, int normalize,
+static int retrieve_eval_prepared_peer(const void* qf, int64_t ldq, int dtype, int64_t Q, int64_t D, int metric, int normalize,
                                      int precision, const void* g_packed, const void* group, const float* center, int64_t G,
                                      int64_t G_total, int64_t g_offset, const int64_t* q_pids, const int64_t* q_camids,
                                      const int64_t* g_camids, int32_t max_rank, float* distmat, int64_t ld, float* cmc,
                                      ieee_eval_summary* summary, int64_t* stats_out, double* per_query_ap,
-                                     int32_t* per_query_first, const ieee_peer_exchange* ex, const void* q_packed_ready,
-                                     void* workspace, size_t workspace_bytes, ieee_stream_t stream_) {
+                                     int32_t* per_query_first, const ieee_peer_exchange* ex, unsigned long long* epoch_dev,
+                                     const void* q_packed_ready, void* workspace, size_t workspace_bytes, ieee_stream_t stream_) {
   int rc = check_device();
   if (rc) return rc;
   cudaStream_t stream = (cudaStream_t)stream_;
@@ -1140,14 +1153,46 @@ int ieee_retrieve_eval_prepared_peer(const void* qf, int64_t ldq, int dtype, int
   }
   if ((rc = distmat_packed(q_packed, Q, g_packed, G, D, metric, precision, distmat, ld, fix, stream_, true))) return rc;
   if ((rc = side_lane_join(stream))) return rc;      // a grouping ieee_gallery_prepare left on the side lane
-  if ((rc = ieee_rank_gather_peer(distmat, ld, G, q_pids, q_camids, g_camids, group, g_offset, n_rel, junk, n_junk, stats, ex,
-                                  stream_)))
-    return rc;
-  if ((rc = ieee_rank_count_peer(distmat, ld, G, g_offset, n_rel, junk, n_junk, stats, ex, stream_))) return rc;
   PeerView v;
-  if ((rc = peer_view(ex, &v))) return rc;
+  if ((rc = peer_view(ex, &v, epoch_dev))) return rc;
+  if ((rc = rank_gather(distmat, ld, v.Qb, G, q_pids, q_camids, g_camids, group, g_offset, v.cap, nullptr, n_rel, junk, n_junk,
+                        reinterpret_cast<int32_t*>(stats), stream, &v)))
+    return rc;
+  const uint64_t* rel_all = reinterpret_cast<const uint64_t*>(v.base[v.my] + v.off_rel);
+  if ((rc = rank_count(distmat, ld, v.Qb, G, g_offset, v.shards, v.cap, v.W, rel_all, n_rel, junk, n_junk, nullptr, stats + 1,
+                       stream, &v)))
+    return rc;
   return rank_metrics_peer(&v, G_total, max_rank, stats, cmc, summary, reinterpret_cast<long long*>(stats_out), ex->Qtot, stream,
                            per_query_ap, per_query_first);
+}
+
+int ieee_retrieve_eval_prepared_peer(const void* qf, int64_t ldq, int dtype, int64_t Q, int64_t D, int metric, int normalize,
+                                     int precision, const void* g_packed, const void* group, const float* center, int64_t G,
+                                     int64_t G_total, int64_t g_offset, const int64_t* q_pids, const int64_t* q_camids,
+                                     const int64_t* g_camids, int32_t max_rank, float* distmat, int64_t ld, float* cmc,
+                                     ieee_eval_summary* summary, int64_t* stats_out, double* per_query_ap,
+                                     int32_t* per_query_first, const ieee_peer_exchange* ex, const void* q_packed_ready,
+                                     void* workspace, size_t workspace_bytes, ieee_stream_t stream_) {
+  return retrieve_eval_prepared_peer(qf, ldq, dtype, Q, D, metric, normalize, precision, g_packed, group, center, G, G_total,
+                                     g_offset, q_pids, q_camids, g_camids, max_rank, distmat, ld, cmc, summary, stats_out,
+                                     per_query_ap, per_query_first, ex, nullptr, q_packed_ready, workspace, workspace_bytes,
+                                     stream_);
+}
+
+int ieee_retrieve_eval_prepared_peer_dev_epoch(const void* qf, int64_t ldq, int dtype, int64_t Q, int64_t D, int metric,
+                                               int normalize, int precision, const void* g_packed, const void* group,
+                                               const float* center, int64_t G, int64_t G_total, int64_t g_offset,
+                                               const int64_t* q_pids, const int64_t* q_camids, const int64_t* g_camids,
+                                               int32_t max_rank, float* distmat, int64_t ld, float* cmc, ieee_eval_summary* summary,
+                                               int64_t* stats_out, double* per_query_ap, int32_t* per_query_first,
+                                               const ieee_peer_exchange* ex, uint64_t* epoch, const void* q_packed_ready,
+                                               void* workspace, size_t workspace_bytes, ieee_stream_t stream_) {
+  IEEE_REQUIRE(epoch != nullptr, "retrieve (peer, device epoch): null epoch word");
+  IEEE_REQUIRE((reinterpret_cast<uintptr_t>(epoch) & 7) == 0, "retrieve (peer, device epoch): the epoch word must be 8-byte aligned");
+  return retrieve_eval_prepared_peer(qf, ldq, dtype, Q, D, metric, normalize, precision, g_packed, group, center, G, G_total,
+                                     g_offset, q_pids, q_camids, g_camids, max_rank, distmat, ld, cmc, summary, stats_out,
+                                     per_query_ap, per_query_first, ex, reinterpret_cast<unsigned long long*>(epoch),
+                                     q_packed_ready, workspace, workspace_bytes, stream_);
 }
 
 size_t ieee_peer_result_offset(int which, int64_t Qb_max, int64_t Qtot, int32_t cap, int32_t W, int32_t shards) {

@@ -166,6 +166,9 @@ constexpr size_t kPeerTicketOffset = 448;   // a word of the header no flag uses
 struct PeerView {
   int shards, my;                  // shards == 0: no peer exchange (single GPU / NCCL path)
   unsigned long long epoch;        // one per query block, increasing
+  // device-resident epoch (replayable steps): when set, every kernel of the step reads the epoch from this word instead
+  // of `epoch`, and the metrics kernel's last CTA advances it once its reduction is over
+  unsigned long long* epoch_dev;
   uint8_t* base[kMaxPeers];        // every rank's buffer as mapped into this process; base[my] is this rank's own
   unsigned long long off_rel;      // uint64 [shards][Qb][cap + 1]   relevant lists (+ length), slot s written by shard s
   unsigned long long off_cnt;      // int32  [shards][Qb][W + 2]     partial counts, slot s written by shard s
@@ -210,6 +213,8 @@ __device__ __forceinline__ void st_release_sys(unsigned long long* p, unsigned l
 __device__ __forceinline__ void peer_signal_and_wait(const PeerView& pv, int phase, const unsigned long long* stats_src = nullptr) {
   if (threadIdx.x < 32) {
     const int lane = threadIdx.x;
+    // (a device epoch is written only by the step's last CTA, after every read of it: all CTAs read the same value)
+    const unsigned long long epoch = pv.epoch_dev ? *reinterpret_cast<volatile const unsigned long long*>(pv.epoch_dev) : pv.epoch;
     unsigned long long* hdr = reinterpret_cast<unsigned long long*>(pv.base[pv.my] + 384);
     unsigned long long* sent = hdr + phase;          // epoch this rank has signalled
     unsigned long long* seen = hdr + 4 + phase;      // epoch for which all peers' flags were already observed here
@@ -217,9 +222,9 @@ __device__ __forceinline__ void peer_signal_and_wait(const PeerView& pv, int pha
     unsigned long long have = 0;
     if (lane == 0) have = *reinterpret_cast<volatile unsigned long long*>(seen);
     have = __shfl_sync(0xffffffffu, have, 0);
-    if (have < pv.epoch) {
+    if (have < epoch) {
       bool first = false;
-      if (lane == 0) first = atomicMax(sent, pv.epoch) < pv.epoch;
+      if (lane == 0) first = atomicMax(sent, epoch) < epoch;
       first = __shfl_sync(0xffffffffu, first, 0);
       if (first) {
         if (stats_src != nullptr && lane < pv.shards) {
@@ -229,21 +234,21 @@ __device__ __forceinline__ void peer_signal_and_wait(const PeerView& pv, int pha
         __threadfence_system();
         __syncwarp();
         if (lane < pv.shards)
-          st_release_sys(reinterpret_cast<unsigned long long*>(pv.base[lane] + 128 * phase) + pv.my, pv.epoch);
+          st_release_sys(reinterpret_cast<unsigned long long*>(pv.base[lane] + 128 * phase) + pv.my, epoch);
       }
       // lane s polls the flag of shard s: the S loads are in flight together
       const unsigned long long* mine = reinterpret_cast<const unsigned long long*>(pv.base[pv.my] + 128 * phase);
       const long long t0 = clock64();
       bool ok = lane >= pv.shards;
       while (!__all_sync(0xffffffffu, ok)) {
-        if (!ok) ok = ld_acquire_sys(mine + lane) >= pv.epoch;
+        if (!ok) ok = ld_acquire_sys(mine + lane) >= epoch;
         if (clock64() - t0 > 8000000000ll) {
-          if (!ok) printf("ieee_b200: rank %d waited in vain for shard %d (phase %d, epoch %llu)\n", pv.my, lane, phase, pv.epoch);
+          if (!ok) printf("ieee_b200: rank %d waited in vain for shard %d (phase %d, epoch %llu)\n", pv.my, lane, phase, epoch);
           __trap();
         }
       }
       __threadfence();
-      if (lane == 0) atomicMax(seen, pv.epoch);
+      if (lane == 0) atomicMax(seen, epoch);
     } else {
       __threadfence();     // order this CTA's reads of the exchanged data after its read of `seen`
     }

@@ -1219,6 +1219,9 @@ __global__ void __launch_bounds__(1024) rank_metrics_kernel(const int32_t* __res
   if (!reduce_now) return;
   if (!last_cta_done(ticket)) return;
   reduce_body(rs_raw, ap, first, is_short, Qred, max_rank, ties, cmc, summary, inp, overflow, pv, stats_out);
+  // every CTA of this step's count and metrics kernels has read the device epoch by now (each took its ticket after
+  // its wait): the next replay of the step uses the next value
+  if (pv.epoch_dev != nullptr && threadIdx.x == 0) *pv.epoch_dev += 1;
 }
 
 // Peer exchange, last stage of a query block (see rank_metrics_kernel).  cmc / summary / stats_out are written when
@@ -1233,6 +1236,7 @@ int rank_metrics_peer(const PeerView* peers, int64_t G_total, int32_t max_rank, 
   const PeerView& v = *peers;
   const int last = (v.q_base + v.Qb == Qtot) ? 1 : 0;
   IEEE_REQUIRE(!last || (cmc && summary), "rank_metrics_peer: the last block needs the result buffers");
+  IEEE_REQUIRE(last || v.epoch_dev == nullptr, "rank_metrics_peer: a device epoch advances on the last block only");
   uint8_t* mine = v.base[v.my];
   const size_t smem = 2 * 1024 * 8 + size_t(max_rank + 1) * 4;
   IEEE_ENSURE_DYN_SMEM(rank_metrics_kernel, smem);

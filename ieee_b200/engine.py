@@ -18,7 +18,7 @@ import torch
 
 from . import _lib
 from .metrics.rank import GalleryLabels, RankStages, _as_device, copy_stream, raise_for_status
-from .peer import link_for
+from .peer import PeerLink, link_for
 from .utils.rerank import re_ranking_device
 
 DEFAULT_BLOCK_BYTES = 4 << 30   # HBM scratch for one distance block
@@ -122,7 +122,11 @@ def _read_result(res: torch.Tensor):
         host = _RESULT_HOST[key] = torch.empty(res.numel(), dtype=torch.uint8, pin_memory=True)
     host.copy_(res, non_blocking=True)
     torch.cuda.current_stream().synchronize()
-    out = host.numpy()
+    return _parse_result(host.numpy())
+
+
+def _parse_result(out: np.ndarray):
+    """((overflow, longest), summary, cmc) from the host copy of a result block (see _read_result); cmc is a copy."""
     overflow, _, longest = (int(v) for v in out[:32].view(np.int64)[:3])
     summary = _lib.EvalSummary.from_buffer_copy(out[32:96].tobytes())
     return (overflow or summary.list_overflow, longest), summary, out[96:].view(np.float32).copy()
@@ -831,10 +835,13 @@ class RetrievalEvaluator:
 
     def _ensure_block(self, rows: int):
         if self._block is None or self._block.shape[0] < rows:
-            # row pitch padded to 128 bytes: the contraction's TMA-store epilogue and the rank kernels'
-            # 16-byte loads both want aligned rows (G itself is arbitrary, e.g. 15913)
-            pitch = (self.G + 31) // 32 * 32
-            self._block = torch.empty((rows, pitch), dtype=torch.float32, device=self.device)[:, : self.G]
+            self._block = self._new_block(rows)
+
+    def _new_block(self, rows: int) -> torch.Tensor:
+        # row pitch padded to 128 bytes: the contraction's TMA-store epilogue and the rank kernels'
+        # 16-byte loads both want aligned rows (G itself is arbitrary, e.g. 15913)
+        pitch = (self.G + 31) // 32 * 32
+        return torch.empty((rows, pitch), dtype=torch.float32, device=self.device)[:, : self.G]
 
     def _distance_block(self, qpk: PackedFeatures) -> torch.Tensor:
         """Distances of one packed query block against this rank's gallery rows, into the scratch block."""
@@ -1060,21 +1067,34 @@ class RetrievalEvaluator:
             first = torch.empty(Q, dtype=torch.int32, device=self.device)
             self.labels.wait(cur, join=False)
             qpk = self._take_early_q(qf)          # packed already by ieee_gallery_prepare (first evaluation of this gallery)
-            queries = (qf.data_ptr(), qf.stride(0), _lib.DTYPES[qf.dtype], Q, D, _lib.METRICS[self.metric], int(self.normalize),
-                       prec, self.chunks[0][1].buf.data_ptr(), self.labels.group.data_ptr(), _lib.ptr(self.center), self.G)
-            rest = (qpk.buf.data_ptr() if qpk is not None else None, ws.data_ptr(), ws.numel(), cur.cuda_stream)
-            if peer:
-                _lib.call(entry, *queries, self.g_total, self.g_offset, qp.data_ptr(), qc.data_ptr(), self.labels.camids.data_ptr(),
-                          self.max_rank, self._block.data_ptr(), self._block.stride(0), res.data_ptr() + 96, res.data_ptr() + 32,
-                          res.data_ptr(), ap.data_ptr(), first.data_ptr(), C.byref(ex), *rest)
-            else:
-                _lib.call(entry, *queries, qp.data_ptr(), qc.data_ptr(), self.labels.camids.data_ptr(), self.max_rank, cap, None,
-                          self._block.data_ptr(), self._block.stride(0), res.data_ptr() + 96, res.data_ptr() + 32,
-                          ap.data_ptr(), first.data_ptr(), *rest)
+            self._one_call_launch(qf, qp, qc, cap, self._block, ws, res, ap, first, qpk, ex if peer else None)
             (overflow, longest), summary, cmc = _read_result(res)
         if overflow or longest > W:
             return self._retry(qf, q_pids, q_camids, return_distmat, memo_key, cap, longest, one_call=True)
         return self._result(summary, cmc, cap, ap, first, self._block[:Q].clone() if return_distmat else None)
+
+    def _one_call_launch(self, qf, qp, qc, cap, block, ws, res, ap, first, qpk=None, ex=None, epoch=None):
+        """Enqueue one resident block's evaluation on the current stream: ieee_retrieve_eval_prepared (cap > 0 here, or
+        <= 0 to size the lists first), or with an exchange descriptor `ex` ieee_retrieve_eval_prepared_peer, whose epoch
+        comes from `ex` or, with `epoch` (int64 [1] on the device), from that word (..._dev_epoch).  Results go into
+        `res` (the result block), `ap`, `first` and the distance block `block`."""
+        Q, D = qf.shape
+        queries = (qf.data_ptr(), qf.stride(0), _lib.DTYPES[qf.dtype], Q, D, _lib.METRICS[self.metric], int(self.normalize),
+                   _lib.PRECISIONS[self.precision], self.chunks[0][1].buf.data_ptr(), self.labels.group.data_ptr(),
+                   _lib.ptr(self.center), self.G)
+        rest = (qpk.buf.data_ptr() if qpk is not None else None, ws.data_ptr(), ws.numel(), _lib.stream())
+        outs = (block.data_ptr(), block.stride(0), res.data_ptr() + 96, res.data_ptr() + 32)
+        if ex is None:
+            _lib.call("ieee_retrieve_eval_prepared", *queries, qp.data_ptr(), qc.data_ptr(), self.labels.camids.data_ptr(),
+                      self.max_rank, cap, None, *outs, ap.data_ptr(), first.data_ptr(), *rest)
+        elif epoch is None:
+            _lib.call("ieee_retrieve_eval_prepared_peer", *queries, self.g_total, self.g_offset, qp.data_ptr(), qc.data_ptr(),
+                      self.labels.camids.data_ptr(), self.max_rank, *outs, res.data_ptr(), ap.data_ptr(), first.data_ptr(),
+                      C.byref(ex), *rest)
+        else:
+            _lib.call("ieee_retrieve_eval_prepared_peer_dev_epoch", *queries, self.g_total, self.g_offset, qp.data_ptr(),
+                      qc.data_ptr(), self.labels.camids.data_ptr(), self.max_rank, *outs, res.data_ptr(), ap.data_ptr(),
+                      first.data_ptr(), C.byref(ex), epoch.data_ptr(), *rest)
 
     def _evaluate_staged(self, qf, q_pids, q_camids, return_distmat, memo_key, cap, width):
         """The query-block loop, stage by stage: any number of blocks, host queries and a host gallery, re-ranking, and
@@ -1241,6 +1261,138 @@ class RetrievalEvaluator:
         if one_call and self._one_resident_block(qf) and (self.world == 1 or self.exchange == "peer" and width > 0):
             return self._evaluate_one_call(qf, q_pids, q_camids, return_distmat, memo_key, cap, width)
         return self._evaluate_staged(qf, q_pids, q_camids, return_distmat, memo_key, cap, width)
+
+    def capture(self, qf: torch.Tensor, q_pids, q_camids, return_distmat: bool = False) -> "CapturedEvaluation":
+        """The evaluation of one query block captured as a CUDA graph, for callers who evaluate the same shapes over and
+        over: a replay costs one graph launch and one wait, with no evaluator bookkeeping, allocation or foreign call.
+        Runs one ordinary evaluate() first (it fixes the centre, packs the gallery and sizes the lists), then captures
+        the one-call step on a side stream with a private memory pool.  See CapturedEvaluation.
+
+        Plain evaluation of a device-resident gallery only; ValueError for re-ranking, from_host, query_group, more
+        queries than one block holds, a sharded gallery whose exchange is not "peer", and the library's debug timeline
+        (ieee_set_debug_flags bit 7)."""
+        qf = _as_features(qf)
+        reason = self._capture_unsupported(qf.shape[0])
+        if reason is not None:
+            raise ValueError("capture: " + reason)
+        return CapturedEvaluation(self, qf, q_pids, q_camids, return_distmat)
+
+    def _capture_unsupported(self, Q: int) -> str | None:
+        if self.query_group is not None:
+            return "query_group shares GNN re-ranking across ranks; its exchanges are collectives a graph does not hold"
+        if self.rerank:
+            return "re-ranking ({}) runs the staged block loop, which is not captured".format(
+                'rerank="gnn"' if self.gnn else "rerank=True")
+        if self._gallery_dev is None:
+            return "the gallery is streamed from the host (from_host); a captured step needs it in HBM"
+        if self.world > 1 and self.exchange != "peer":
+            return 'a sharded gallery is captured with exchange="peer" only, not {!r}'.format(self.exchange)
+        if Q == 0 or self._block_rows(Q) < Q:
+            return "{} queries do not make one query block ({} rows fit block_bytes={})".format(
+                Q, self._block_rows_for(1 << 40, self.G), self.block_bytes)
+        lib = _lib.load()
+        flags = lib.ieee_set_debug_flags(0)
+        lib.ieee_set_debug_flags(flags)
+        if flags & 128:
+            return "the library's debug timeline (ieee_set_debug_flags bit 7) records events a graph cannot hold"
+        return None
+
+
+class CapturedEvaluation:
+    """One query block's evaluation captured as a CUDA graph (RetrievalEvaluator.capture).
+
+    ``qf``, ``q_pids`` and ``q_camids`` are the graph's static inputs on the evaluator's device (the features in the
+    dtype evaluate() computes from, the labels as int64), initialised from capture()'s arguments: copy the next query
+    set into them (same shapes), then ``replay()``.  It returns what ``evaluate()`` of the evaluator returns for their
+    current contents, bit for bit: (cmc, mAP, info) with ``ap``, ``first``, ``mINP``, ``num_valid``, ``num_ties``,
+    ``cap`` and, when captured with ``return_distmat=True``, ``distmat``.  The tensors in ``info`` are the graph's own
+    outputs: the next replay overwrites them.  ``launch()`` only enqueues the graph on the current stream and
+    ``result()`` waits for that launch and parses it.
+
+    The handle owns everything its step writes (workspace, distance block, per-query arrays, result block and its pinned
+    host copy) and, on a sharded gallery, an exchange buffer of its own whose epoch lives in a device word the step
+    advances itself: eager evaluations keep their own buffers and epochs.  Every rank must replay as often as the
+    others, as every rank calls evaluate() alike.  When a replay's lists outgrow the captured capacity (or, sharded, the
+    merged lists the row width), the result block says so; the handle then evaluates once eagerly to size the lists
+    exactly, captures again and replays.  A sharded handle's exchange buffer stays allocated, as the pooled ones do."""
+
+    def __init__(self, ev: RetrievalEvaluator, qf: torch.Tensor, q_pids, q_camids, return_distmat: bool):
+        self._ev, self._return_distmat = ev, return_distmat
+        dev = ev.device
+        _, _, info = ev.evaluate(qf, q_pids, q_camids)
+        with torch.cuda.device(dev):
+            self.qf = torch.empty(qf.shape, dtype=qf.dtype, device=dev).copy_(qf)
+            self.q_pids = _as_device(q_pids, torch.int64, dev).clone()
+            self.q_camids = _as_device(q_camids, torch.int64, dev).clone()
+            self._done = torch.cuda.Event()
+        self._capture(info["cap"], ev._memo_key(q_pids))
+
+    def _capture(self, cap: int, memo_key):
+        ev, lib, dev = self._ev, _lib.load(), self._ev.device
+        Q, D = self.qf.shape
+        prec = _lib.PRECISIONS[ev.precision]
+        k_eff = min(ev.max_rank, ev.g_total)
+        with torch.cuda.device(dev):
+            ex = self.epoch = None
+            W = 0                                 # (no merged lists on one GPU)
+            if ev.world > 1:
+                # the merged lists' width the memo learnt with these labels, else the widest they can be; the ranks agree
+                # on both sizes (they fix the exchange buffer's layout)
+                width = _CAP_MEMO.get(memo_key, (0, 0))[1] if memo_key is not None else 0
+                sizes = torch.tensor([cap, min(width, ev.world * cap) if width > 0 else ev.world * cap], device=dev)
+                torch.distributed.all_reduce(sizes, op=torch.distributed.ReduceOp.MAX, group=ev.group)
+                cap, W = (int(v) for v in sizes.tolist())
+                self._link = PeerLink(ev.group, dev, lib.ieee_peer_exchange_bytes(Q, Q, cap, W, ev.world))
+                ex = self._link.descriptor(Q, Q, Q, 0, cap, W, 0)
+                self.epoch = torch.ones(1, dtype=torch.int64, device=dev)
+                ws_bytes = lib.ieee_retrieve_prepared_peer_workspace_bytes(Q, D, prec, cap)
+            else:
+                ws_bytes = lib.ieee_retrieve_prepared_workspace_bytes(Q, D, prec, cap)
+            self._ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            # zeroed once: the one-GPU step never writes the statistics words
+            self._res = torch.zeros(96 + 4 * k_eff, dtype=torch.uint8, device=dev)
+            self._host = torch.empty(self._res.numel(), dtype=torch.uint8, pin_memory=True)
+            self._block = ev._new_block(Q)
+            self.ap = torch.empty(Q, dtype=torch.float64, device=dev)
+            self.first = torch.empty(Q, dtype=torch.int32, device=dev)
+            graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(graph):         # a side stream and a private memory pool
+                # the step packs the queries itself: nothing was packed ahead for the static input
+                ev._one_call_launch(self.qf, self.q_pids, self.q_camids, cap, self._block, self._ws, self._res, self.ap,
+                                    self.first, None, ex, self.epoch)
+                self._host.copy_(self._res, non_blocking=True)
+        self._graph, self._ex, self.cap, self.W = graph, ex, cap, W
+
+    def launch(self):
+        """Enqueue one replay on the current stream and return at once."""
+        self._graph.replay()                     # (on the current stream of the device it was captured on)
+        self._done.record(torch.cuda.current_stream(self._ev.device))
+
+    def result(self):
+        """Wait for the last launch() and return its (cmc, mAP, info)."""
+        return self._finish(retry=True)
+
+    def replay(self):
+        """launch() + result()."""
+        self.launch()
+        return self._finish(retry=True)
+
+    def _finish(self, retry: bool):
+        self._done.synchronize()
+        (overflow, longest), summary, cmc = _parse_result(self._host.numpy())
+        if overflow or longest > self.W:
+            if not retry:
+                raise RuntimeError("ieee_b200: per-query lists overflowed an exactly sized buffer (cap=%d, longest=%d)"
+                                   % (self.cap, longest))
+            # exact sizes from one eager evaluation of the same contents (collective on a sharded gallery: every rank
+            # sees the same statistics, so all of them get here), then a graph with those sizes
+            ev = self._ev
+            _, _, info = ev.evaluate(self.qf, self.q_pids, self.q_camids)
+            self._capture(info["cap"], ev._memo_key(self.q_pids))
+            self.launch()
+            return self._finish(retry=False)
+        return self._ev._result(summary, cmc, self.cap, self.ap, self.first,
+                                self._block if self._return_distmat else None)
 
 
 def result_lines(cmc, mAP, ranks=(1, 5, 10, 20)):

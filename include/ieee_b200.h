@@ -293,7 +293,10 @@ int ieee_eval_market1501_f64(const double* distmat, int64_t ld, int64_t Q, int64
  * cap > 0  : list-capacity HINT (e.g. the value a previous call reported); fully asynchronous.  If a query needs
  *            more, summary->list_overflow holds the needed capacity and the other results are meaningless.
  * cap <= 0 : the capacity is queried first (one stream synchronisation, ieee_rank_list_cap_sync) and written to
- *            *cap_host_out when that is not NULL.
+ *            *cap_host_out when that is not NULL.  IEEE_ERR_INVALID while `stream` is being captured.
+ * With cap > 0, ieee_retrieve_eval_prepared (and ieee_retrieve_eval_prepared_peer_dev_epoch below) may be captured into
+ * a CUDA graph and replayed: they neither
+ * synchronise nor allocate, the side-lane join becomes an external event wait, and the debug timeline records no marks.
  * distmat  : float32 [Q, ld] scratch for the distance block, ld >= G (ld % 32 == 0 keeps the TMA-store epilogue);
  *            holds the distance matrix on return (compute_distance_matrix's result, distance.py:6).
  * cmc: float[max_rank] device; summary: device; per_query_ap (double[Q]) / per_query_first (int32[Q]) may be NULL.
@@ -611,6 +614,20 @@ int ieee_retrieve_eval_prepared_peer(const void* qf, int64_t ldq, int dtype, int
                                      int32_t* per_query_first /* int32[Q], may be NULL */, const ieee_peer_exchange* ex,
                                      const void* q_packed /* as in ieee_retrieve_eval_prepared */, void* workspace,
                                      size_t workspace_bytes, ieee_stream_t stream);
+/* The same step with the epoch in a device word instead of ex->epoch (ignored), so that the step can be captured into a
+ * CUDA graph and replayed: every kernel of the step reads *epoch, and the metrics kernel's last CTA adds one to it after
+ * its reduction, when no kernel of the step reads it any more.  *epoch starts at 1 or above, and the word serves one
+ * exchange buffer set whose epochs come from no other source: never mix this call and host epochs on the same buffers.
+ * Every rank must replay its step as many times as the others.  The call itself never synchronises or allocates. */
+int ieee_retrieve_eval_prepared_peer_dev_epoch(const void* qf, int64_t ldq, int dtype, int64_t Q, int64_t D, int metric,
+                                               int normalize, int precision, const void* g_packed, const void* group,
+                                               const float* center, int64_t G, int64_t G_total, int64_t g_offset,
+                                               const int64_t* q_pids, const int64_t* q_camids, const int64_t* g_camids,
+                                               int32_t max_rank, float* distmat, int64_t ld, float* cmc, ieee_eval_summary* summary,
+                                               int64_t* stats_out, double* per_query_ap, int32_t* per_query_first,
+                                               const ieee_peer_exchange* ex, uint64_t* epoch /* device, 8-byte aligned */,
+                                               const void* q_packed, void* workspace, size_t workspace_bytes,
+                                               ieee_stream_t stream);
 /* Byte offset of a per-query result array inside an exchange buffer: which = 0 AP (double[Qtot]), 1 first hit
  * (int32[Qtot]), 2 mINP term (double[Qtot]), 3 short-list flag (int32[Qtot]). */
 size_t ieee_peer_result_offset(int which, int64_t Qb_max, int64_t Qtot, int32_t cap, int32_t W, int32_t shards);
